@@ -23,6 +23,9 @@ One JSON line on stdout (rank 0).  value = tiles/s with inputs resident in HBM; 
 from pinned HOST buffers (H2D of every input + D2H of the metric records inside the timed region).  After the timed
 regions the GPU arm re-runs the `--cpu-tiles` tiles that the cpu_baseline leg processes and compares its per-tile records
 with the oracle's bit for bit; a mismatch is reported in `check` and makes the exit code 3.
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB): the
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -64,7 +67,8 @@ class Workload:
         return {k: t[k] for k in self.keys}
 
     def gpu_step(self, ops, src):
-        """-> dict of per-tile record tensors: aji [B,2], pq [B,4], counts [B,5,C] (+ caji [B,C,2], cpq [B,C,4])"""
+        """-> dict of per-tile record tensors: aji [B,2], pq [B,4], counts [B,5,C] (+ caji [B,C,2], cpq [B,C,4]), and the
+        maps they were computed from: sem [B,H,W] uint8, inst [B,H,W] int32"""
         raise NotImplementedError
 
     def cpu_tile(self, t, literal=True):
@@ -120,7 +124,7 @@ class DistMonuseg(Workload):
         inst = ops.postproc_dist(src["dist_logit"])
         aji, pq = ops.pair_metrics_bin(inst, src["gt_inst"])
         counts, _ = ops.sem_counts(cls, src["gt_sem"], self.C)
-        return dict(aji=aji, pq=pq, counts=counts)
+        return dict(aji=aji, pq=pq, counts=counts, sem=cls, inst=inst)
 
     def cpu_tile(self, t, literal=True):
         from oracle import postprocess as opp
@@ -151,9 +155,9 @@ class UnetCpm17(Workload):
         counts, _ = ops.sem_counts(sem, src["gt_sem"], self.C)
         if self.multi:
             r = ops.pair_metrics_multiclass(inst, sem, src["gt_inst"], src["gt_sem"], self.C)
-            return dict(aji=r["bin_aji"], pq=r["bin_pq"], counts=counts, caji=r["aji"], cpq=r["pq"])
+            return dict(aji=r["bin_aji"], pq=r["bin_pq"], counts=counts, caji=r["aji"], cpq=r["pq"], sem=sem, inst=inst)
         aji, pq = ops.pair_metrics_bin(inst, src["gt_inst"])
-        return dict(aji=aji, pq=pq, counts=counts)
+        return dict(aji=aji, pq=pq, counts=counts, sem=sem, inst=inst)
 
     def cpu_tile(self, t, literal=True):
         from oracle import postprocess as opp
@@ -186,7 +190,7 @@ class HoverConsep(Workload):
         inst = ops.postproc_hover(src["fore_map"], src["hv_map"])
         aji, pq = ops.pair_metrics_bin(inst, src["gt_inst"])
         counts, _ = ops.sem_counts(cls, src["gt_sem"], self.C)
-        return dict(aji=aji, pq=pq, counts=counts)
+        return dict(aji=aji, pq=pq, counts=counts, sem=cls, inst=inst)
 
     def cpu_tile(self, t, literal=True):
         from oracle import postprocess as opp
@@ -209,7 +213,7 @@ class CdnetConsep(Workload):
         sem, inst = ops.postproc_unet(r["cls"], 2, 3, 2)
         aji, pq = ops.pair_metrics_bin(inst, src["gt_inst"])
         counts, _ = ops.sem_counts(sem, src["gt_sem"], self.C)
-        return dict(aji=aji, pq=pq, counts=counts)
+        return dict(aji=aji, pq=pq, counts=counts, sem=sem, inst=inst)
 
     def cpu_tile(self, t, literal=True):
         from oracle import postprocess as opp
@@ -248,6 +252,27 @@ def stack_batch(tiles, batch, dihedral=True):
         for key in keys:
             out[key].append(var(key, t[key], k))
     return {k: np.stack(v) for k, v in out.items()}
+
+
+DUMP_BYTES = 64 * 10 ** 6          # --dump-outputs writes at most this much
+
+
+def outputs_to_dump(rec, seed=0):
+    """One step's outputs (``Workload.gpu_step``) as host arrays for --dump-outputs: every per-tile record in full
+    (float64), and the sem / inst maps of a fixed, seeded sample of the batch's tiles (float32, exact below 2**24) with
+    their batch indices in ``sample_tiles``, at most DUMP_BYTES in all."""
+    import torch
+    out = {k: v.double().cpu().numpy() for k, v in rec.items() if k not in ("sem", "inst")}
+    B, H, W = rec["inst"].shape
+    if int(rec["inst"].max()) >= 1 << 24:
+        raise ValueError("instance ids of 2**24 and above are not exact in float32")
+    room = DUMP_BYTES - sum(v.nbytes for v in out.values()) - 8 * B
+    idx = np.sort(np.random.default_rng(seed).choice(B, min(B, room // (2 * 4 * H * W)), replace=False))
+    sel = torch.from_numpy(idx).to(rec["inst"].device)
+    out["sample_tiles"] = idx.astype(np.float64)
+    for k in ("sem", "inst"):
+        out[k] = rec[k].index_select(0, sel).float().cpu().numpy()
+    return out
 
 
 # Algorithmic bytes per pixel and LAUNCH of every kernel's own inputs + outputs, touched once (DESIGN.md §4); a step's
@@ -445,9 +470,11 @@ def run_b200(a):
     pinned_np = {k: v.numpy() for k, v in pinned.items()}
     ctx = _lib.get_ctx(local)
     acc = torch.zeros(R, dtype=torch.float64, device=dev)
+    last = {}                                              # outputs of the latest plain step (--dump-outputs)
 
     def step(src):
-        acc.add_(wl.flat(wl.gpu_step(ops, src)).sum(0))
+        last["rec"] = wl.gpu_step(ops, src)
+        acc.add_(wl.flat(last["rec"]).sum(0))
         return acc
 
     def barrier():
@@ -496,10 +523,12 @@ def run_b200(a):
         VL = max(1, a.value_lanes)
         vstreams = [torch.cuda.Stream(dev) for _ in range(VL)]
         vacc = [torch.zeros(R, dtype=torch.float64, device=dev) for _ in range(VL)]
+        vout = [None] * VL                                 # each graph's outputs: rewritten in place by every replay
         graphs = []
 
         def lane_step(k):
-            vacc[k].add_(wl.flat(wl.gpu_step(ops, devt)).sum(0))
+            vout[k] = wl.gpu_step(ops, devt)
+            vacc[k].add_(wl.flat(vout[k]).sum(0))
 
         torch.cuda.synchronize()
         for k in range(VL):
@@ -556,6 +585,9 @@ def run_b200(a):
         launches = launches_per_step * a.steps             # replayed launches are not seen by the library's counter
     value = world * B * a.steps / (ms / 1e3)
     acc_value = acc.clone()
+    dump = None
+    if a.dump_outputs and rank == 0:
+        dump = outputs_to_dump(last["rec"] if a.no_graph else vout[(turn[0] - 1) % VL])
 
     # e2e: same calls, inputs are pinned host buffers (the library stages them), result record read back.
     # The batch is fed in chunks that alternate between lanes (own stream + own workspace), so the PCIe transfer of one
@@ -719,6 +751,10 @@ def run_b200(a):
         "gpu_launches": launches, "clocks": clocks, "roofline": roof, "cpu_baseline": cpu,
         "check": dict(check or {}, aji_of_timed_batch=(inter / union) if union else None),
     }
+    if dump is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -762,7 +798,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="time plain launches instead of a CUDA-graph replay of the step")
     ap.add_argument("--value-lanes", type=int, default=3, help="resident-input steps alternate between this many streams")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy: "
+                    "the per-tile records, and the sem / inst maps of a seeded sample of the batch's tiles")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     rc = run_reference(a) if a.impl == "reference" else run_b200(a)
     sys.exit(rc or 0)
 

@@ -1,5 +1,6 @@
 """CPU suite: the oracle against the golden vectors produced by the reference's own code
 (tests/golden/make_golden.py) and against independent scipy implementations."""
+import hashlib
 import os
 
 import numpy as np
@@ -387,9 +388,30 @@ def test_oracle_ddm_enhancement_both_variants():
             assert np.array_equal(got, m["e%d_%s" % (j, key)][0]), (j, key)
 
 
+def _reg_inputs(m, name, j):
+    """The head outputs make_golden_r2.py's recorder network fed DIST.inference ("d") / HoverNet.inference ("h"), drawn
+    again from its seed in its order (per TTA variant: ``calls`` patches, the whole image or split windows; per patch:
+    the heads).  The stored digest pins them to what the reference was run on.  -> [head][variant] int8 quarter units"""
+    H, W, window, overlap, T = [int(v) for v in m["%s%d_meta" % (name, j)]]
+    rots = [int(r) for r in m["%s%d_rots" % (name, j)]]
+    chans = (2, 1) if name == "d" else (3, 2, 2)
+    rng = np.random.default_rng(9840 + 10 * j + len(chans))
+    out = [[] for _ in chans]
+    for t in range(T):
+        ph, pw = (window, window) if window else ((W, H) if (rots[t] // 90) % 2 else (H, W))
+        calls = [[rng.integers(-12, 13, (1, c, ph, pw)).astype(np.int8) for c in chans]
+                 for _ in range(int(m["%s%d_calls" % (name, j)]))]
+        for h in range(len(chans)):
+            w = np.stack([c[h] for c in calls])                                 # [M, 1, C, h, w]
+            out[h].append(np.ascontiguousarray(np.moveaxis(w, 1, 0)) if window else w[0])
+    digest = hashlib.sha256(b"".join(v.tobytes() for head in out for v in head)).hexdigest()
+    assert digest == str(m["%s%d_sha256" % (name, j)]), "%s%d: the seeded draw no longer gives the golden inputs" % (name, j)
+    return out
+
+
 def _reg_case(m, name, j, h):
     H, W, window, overlap, T = [int(v) for v in m["%s%d_meta" % (name, j)]]
-    variants = [m["%s%d_h%d_v%d" % (name, j, h, t)].astype(np.float32) / 4.0 for t in range(T)]
+    variants = [v.astype(np.float32) / 4.0 for v in _reg_inputs(m, name, j)[h]]
     return H, W, window, overlap, variants, [int(r) for r in m["%s%d_rots" % (name, j)]], [str(f) for f in m["%s%d_flips" % (name, j)]]
 
 
