@@ -1,6 +1,7 @@
 """GPU parity tests: every operator of the C-ABI CUDA library against the CPU oracle (and scipy where the
 reference calls scipy directly) on seeded inputs.  Integer outputs must be bit-exact."""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -13,6 +14,9 @@ from tiseg_b200 import ops, synth  # noqa: E402
 from oracle import metrics as om  # noqa: E402
 from oracle import postprocess as opp  # noqa: E402
 from oracle import skimage_port as sk  # noqa: E402
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import topology as T  # noqa: E402
 
 G = os.path.join(os.path.dirname(__file__), "golden")
 SHAPES = [(1, 1), (1, 40), (37, 1), (5, 33), (64, 64), (50, 97), (130, 257)]
@@ -53,23 +57,11 @@ def test_label_equal_value_int32_batched(conn):
 def test_label_adversarial():
     # spiral, checkerboard, comb: long union chains and many diagonal-only contacts
     H = W = 96
-    spiral = np.zeros((H, W), np.uint8)
-    y = x = 0; dy, dx = 0, 1; lo_y, hi_y, lo_x, hi_x = 0, H - 1, 0, W - 1
-    for _ in range(H * W):
-        spiral[y, x] = 1
-        ny, nx = y + dy, x + dx
-        if not (lo_y <= ny <= hi_y and lo_x <= nx <= hi_x):
-            if (dy, dx) == (0, 1): lo_y += 2
-            elif (dy, dx) == (1, 0): hi_x -= 2
-            elif (dy, dx) == (0, -1): hi_y -= 2
-            else: lo_x += 2
-            dy, dx = dx, -dy
-            ny, nx = y + dy, x + dx
-            if not (lo_y - 0 <= ny <= hi_y and lo_x <= nx <= hi_x):
-                break
-        y, x = ny, nx
-    checker = (np.indices((H, W)).sum(0) % 2).astype(np.uint8)
-    comb = np.zeros((H, W), np.uint8); comb[::2, :] = 1; comb[:, 0] = 1
+    spiral = T.spiral(H, W)
+    assert sk.label(spiral, connectivity=1).max() == 1 and spiral.sum() >= 0.45 * H * W and spiral[:, 0].sum() > 1, \
+        "one 4-connected spiral that turns at every corner and covers half the tile"
+    checker = (T.checkerboard(H, W) == 2).astype(np.uint8)
+    comb = T.comb(W, H).T.copy()                       # teeth along rows, spine down the last column
     for name, m in (("spiral", spiral), ("checker", checker), ("comb", comb)):
         for conn in (1, 2):
             _diff(ops.label(m, connectivity=conn), sk.label(m, connectivity=conn), "%s conn %d" % (name, conn))
