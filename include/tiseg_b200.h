@@ -34,6 +34,15 @@ extern "C" {
 #define TISEG_ERR_NOGPU 3  /* no CUDA device: there is no CPU fallback                        */
 #define TISEG_ERR_LIMIT 4  /* a data-dependent limit was exceeded (instance id out of range)  */
 
+/* Element type of the network outputs handed to a *_typed entry (logits, distance / HV / foreground maps, direction and
+ * point heads).  All network inputs of one call share it.  Half-precision inputs are converted to fp32 as they are loaded
+ * and the arithmetic after the load is the fp32 path's, so a call fed fp16 / bf16 returns the bits the same call returns
+ * for the fp32 upcast of its inputs, at half the input bytes (a host buffer crosses PCIe at 2 B per element).  Outputs
+ * keep their types: probabilities and means stay fp32.  Another code returns TISEG_ERR_ARG. */
+#define TISEG_DTYPE_F32 0
+#define TISEG_DTYPE_F16 1
+#define TISEG_DTYPE_BF16 2
+
 typedef struct tiseg_ctx tiseg_ctx;
 
 /* ---- context -------------------------------------------------------------------------------- */
@@ -62,6 +71,9 @@ int tiseg_timing_report(tiseg_ctx* ctx, char* buf, int cap);
  * (first maximum wins, like torch.argmax). */
 int tiseg_softmax_argmax(tiseg_ctx* ctx, const float* logits, int N, int T, int C, int H, int W,
                          float* prob, uint8_t* cls);
+/* the same with logits of element type `dtype` (TISEG_DTYPE_*); tiseg_softmax_argmax is this with TISEG_DTYPE_F32 */
+int tiseg_softmax_argmax_typed(tiseg_ctx* ctx, int dtype, const void* logits, int N, int T, int C, int H, int W,
+                               float* prob, uint8_t* cls);
 
 /* ---- the step before A1, fused: window stitch + TTA reverse + softmax + mean + argmax -------------------------
  * Replaces split_inference's canvas (base.py:255-295), reverse_tta_transform (base.py:365-381) and the softmax /
@@ -74,12 +86,17 @@ long long tiseg_tta_input_elems(int T, int C, int H, int W, const int* rotate_de
 int tiseg_softmax_argmax_tta(tiseg_ctx* ctx, const float* logits, int N, int T, int C, int H, int W,
                              const int* rotate_degrees, const int* flips, int window, int overlap,
                              float* prob, uint8_t* cls);
+int tiseg_softmax_argmax_tta_typed(tiseg_ctx* ctx, int dtype, const void* logits, int N, int T, int C, int H, int W,
+                                   const int* rotate_degrees, const int* flips, int window, int overlap,
+                                   float* prob, uint8_t* cls);
 
 /* The plain (no softmax) TTA mean of a regression head with the same stitch + reverse-transform indexing:
  * `sum(dist_logit_list) / len(dist_logit_list)` of dist.py:398-410; hovernet.py:406 keeps variant 0 only (T = 1).
  * maps laid out like the logits of tiseg_softmax_argmax_tta; mean_out [N, C, H, W]. */
 int tiseg_tta_mean(tiseg_ctx* ctx, const float* maps, int N, int T, int C, int H, int W, const int* rotate_degrees,
                    const int* flips, int window, int overlap, float* mean_out);
+int tiseg_tta_mean_typed(tiseg_ctx* ctx, int dtype, const void* maps, int N, int T, int C, int H, int W,
+                         const int* rotate_degrees, const int* flips, int window, int overlap, float* mean_out);
 
 /* ---- A5 / A6 / A15: connected-component labelling ---------------------------------------------
  * skimage.measure.label(img, background=bg, connectivity=conn) (unet.py:85, dist.py:107,123,
@@ -146,6 +163,9 @@ int tiseg_postproc_dist(tiseg_ctx* ctx, const float* dist, int N, int H, int W, 
  * lamb > 0 runs an iterative reconstruction that synchronises with the host between sweeps. */
 int tiseg_postproc_dist_lambda(tiseg_ctx* ctx, const float* dist, int N, int H, int W, int lamb, int32_t* inst_out,
                                int32_t* markers_out, int32_t* ws_out);
+/* dist of element type `dtype` (TISEG_DTYPE_*): the distance map is read once, by the step that truncates it to levels */
+int tiseg_postproc_dist_lambda_typed(tiseg_ctx* ctx, int dtype, const void* dist, int N, int H, int W, int lamb,
+                                     int32_t* inst_out, int32_t* markers_out, int32_t* ws_out);
 
 /* ---- A9: skimage.morphology.reconstruction(seed, mask, method='erosion') on uint8 images, 3x3 footprint
  * (dist.py:56).  seed is clamped from below by mask.  Synchronises with the host between sweeps. */
@@ -160,6 +180,11 @@ int tiseg_reconstruction_erosion_u8(tiseg_ctx* ctx, const uint8_t* seed, const u
  * dist fp64 (the flooded image), marker int32. */
 int tiseg_postproc_hover(tiseg_ctx* ctx, const float* fore_map, const float* hv_map, int N, int H, int W,
                          int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out, int32_t* marker_out);
+/* fore_map and hv_map of element type `dtype` (TISEG_DTYPE_*); with scale_factor 2 the resize reads them and the chain
+ * after it runs on fp32 as above */
+int tiseg_postproc_hover_typed(tiseg_ctx* ctx, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
+                               int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
+                               int32_t* marker_out);
 
 /* ---- A12: CDNet direction-guided refinement ----------------------------------------------------------------
  * generate_direction_differential_map(dir_map, 9) (tiseg/models/utils/direct_diff_map.py:95-167):
@@ -172,6 +197,10 @@ int tiseg_ddm(tiseg_ctx* ctx, const uint8_t* dir_map, int N, int H, int W, float
 int tiseg_cdnet_refine(tiseg_ctx* ctx, const float* sem_logits, const float* dir_logits, const float* point_logits,
                        int N, int T, int C, int D, int H, int W, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
                        uint8_t* dir_map_out, float* dd_out);
+/* the three heads of element type `dtype` (TISEG_DTYPE_*); the outputs are as above (sem_prob_out stays fp32) */
+int tiseg_cdnet_refine_typed(tiseg_ctx* ctx, int dtype, const void* sem_logits, const void* dir_logits,
+                             const void* point_logits, int N, int T, int C, int D, int H, int W, int if_ddm,
+                             float* sem_prob_out, uint8_t* cls_out, uint8_t* dir_map_out, float* dd_out);
 
 /* _ddm_enhencement alone, IN PLACE on sem_prob [N,C,H,W]: mode 0 = CDNet (cdnet.py:354-367), mode 1 = MultiTaskCDNet
  * (multi_task_cdnet.py:548-564).  dd [N,H,W] mean DDM, point [N,H,W] TTA-mean point map (channel 0 of point_logit). */
@@ -188,6 +217,11 @@ int tiseg_mtcdnet_refine(tiseg_ctx* ctx, const float* tc_logits, const float* se
                          const float* point_logits, int N, int T, int Ctc, int Csem, int D, int H, int W, int if_ddm,
                          float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
                          uint8_t* dir_map_out, float* dd_out);
+/* the four heads of element type `dtype` (TISEG_DTYPE_*); the outputs are as above */
+int tiseg_mtcdnet_refine_typed(tiseg_ctx* ctx, int dtype, const void* tc_logits, const void* sem_logits,
+                               const void* dir_logits, const void* point_logits, int N, int T, int Ctc, int Csem, int D,
+                               int H, int W, int if_ddm, float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out,
+                               uint8_t* sem_cls_out, uint8_t* dir_map_out, float* dd_out);
 
 /* ---- A13: align_foreground (tiseg/models/utils/postprocess.py:123-155) -----------------------------------
  * Ordered multi-source BFS growing the labels of `pred` into `foreground` (8-neighbourhood, first claimant

@@ -27,11 +27,15 @@ SIGNATURES = {
     "tiseg_timing_enable": [_vp, _i],
     "tiseg_timing_report": [_vp, ctypes.c_char_p, _i],
     "tiseg_softmax_argmax": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
+    "tiseg_softmax_argmax_typed": [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_tta_input_elems": [_i, _i, _i, _i, _vp, _i, _i],
     "tiseg_softmax_argmax_tta": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp],
+    "tiseg_softmax_argmax_tta_typed": [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp],
     "tiseg_tta_mean": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp],
+    "tiseg_tta_mean_typed": [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp],
     "tiseg_ddm_enhance": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i],
     "tiseg_mtcdnet_refine": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tiseg_mtcdnet_refine_typed": [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp],
     "tiseg_pair_metrics_bin_iou": [_vp, _vp, _vp, _i, _i, _i, ctypes.c_double, _vp, _vp],
     "tiseg_pair_metrics_bin_u16gt": [_vp, _vp, _vp, _i, _i, _i, ctypes.c_double, _vp, _vp],
     "tiseg_label": [_vp, _vp, _i, _i, _i, ctypes.c_int32, _i, _vp, _vp],
@@ -47,10 +51,13 @@ SIGNATURES = {
     "tiseg_watershed_f64": [_vp, _vp, _vp, _vp, _i, _i, _i, _vp],
     "tiseg_postproc_dist": [_vp, _vp, _i, _i, _i, _vp, _vp, _vp],
     "tiseg_postproc_dist_lambda": [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp],
+    "tiseg_postproc_dist_lambda_typed": [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp],
     "tiseg_reconstruction_erosion_u8": [_vp, _vp, _vp, _i, _i, _i, _vp],
     "tiseg_postproc_hover": [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
+    "tiseg_postproc_hover_typed": [_vp, _i, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_ddm": [_vp, _vp, _i, _i, _i, _vp],
     "tiseg_cdnet_refine": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
+    "tiseg_cdnet_refine_typed": [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_align_foreground": [_vp, _vp, _vp, _i, _i, _i, _i],
     "tiseg_postproc_multitask": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_pair_metrics_bin": [_vp, _vp, _vp, _i, _i, _i, _vp, _vp],
@@ -250,6 +257,28 @@ def as_input(a, dtype):
     if a.dtype == np.bool_ and np.dtype(dtype) == np.uint8:
         a = a.view(np.uint8)
     return np.ascontiguousarray(a, dtype=dtype)
+
+
+# element type codes of the network outputs a *_typed entry reads (TISEG_DTYPE_* in tiseg_b200.h)
+DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
+
+
+def _half_code(a):
+    if is_torch(a):
+        import torch
+        return {torch.float16: DTYPE_F16, torch.bfloat16: DTYPE_BF16}.get(a.dtype, DTYPE_F32)
+    return DTYPE_F16 if isinstance(a, np.ndarray) and a.dtype == np.float16 else DTYPE_F32
+
+
+def net_inputs(*arrays):
+    """Network outputs of one call -> (arrays, dtype code).  fp16 / bf16 tensors (CUDA or CPU) and numpy float16 arrays are
+    kept in their dtype, made C-contiguous, when every array of the call shares it: the library converts them to fp32 as
+    it loads them (half the bytes read and staged, the same results as their fp32 upcast).  Anything else, mixed dtypes
+    included, is converted to fp32 like ``as_input`` does (code DTYPE_F32)."""
+    codes = {_half_code(a) for a in arrays}
+    if len(codes) == 1 and DTYPE_F32 not in codes:
+        return tuple(a.contiguous() if is_torch(a) else np.ascontiguousarray(a) for a in arrays), codes.pop()
+    return tuple(as_input(a, np.float32) for a in arrays), DTYPE_F32
 
 
 _device_out = threading.local()

@@ -5,13 +5,16 @@
 //                       dir[:,0] *= sem[:,0] -> argmax -> DDM, mean DDM, _ddm_enhencement (cdnet.py:354-367), argmax.
 // The reference does this with ~60 ATen launches per TTA variant (8 torch.roll temporaries); here the DDM is one
 // wrap-around 3x3 stencil on the uint8 direction map plus a per-tile max/min reduction.
+// The head outputs may be fp32, fp16 or bf16 (TI): the kernels that read them convert at the load; the probabilities,
+// DDM and point mean the library makes from them are fp32.
 #include <cfloat>
 
 #include "common.cuh"
 
 namespace tiseg {
 
-int softmax_argmax_dev(tiseg_ctx* c, const Geom& g, const float* d_in, int T, int C, float* d_prob, uint8_t* d_cls);
+template <class TI>
+int softmax_argmax_dev(tiseg_ctx* c, const Geom& g, const TI* d_in, int T, int C, float* d_prob, uint8_t* d_cls);   // softmax.cu
 
 // label -> (vertical, horizontal) unit-step vector, direct_diff_map.py:7
 __constant__ float c_dir9[9][2] = {{0, 0}, {0, -1}, {-1, -1}, {-1, 0}, {-1, 1}, {0, 1}, {1, 1}, {1, 0}, {1, -1}};
@@ -95,22 +98,22 @@ k_ddm_mean(Geom g, const uint8_t* __restrict__ lv, const int* __restrict__ mm, i
 
 // per variant: softmax over the D direction channels, channel 0 scaled by the mean background probability,
 // argmax (first maximum).  Four pixels per thread, every logit read once (128-bit loads), exp evaluated once.
-template <int DMAX>
+template <class TI, int DMAX>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_dir_map(long long P, const float* __restrict__ dir_logits, const float* __restrict__ sem_prob, int T, int D, int C,
+k_dir_map(long long P, const TI* __restrict__ dir_logits, const float* __restrict__ sem_prob, int T, int D, int C,
           uint8_t* __restrict__ dir_map, bool vec) {
     const int n = blockIdx.y;
     const long long i = flat4_index();
     if (i >= P) return;
     const Pack4<float> s0 = ld4(sem_prob + ((long long)n * C) * P, i, P, vec);
     for (int t = 0; t < T; ++t) {
-        const float* src = dir_logits + ((long long)n * T + t) * D * P;
+        const TI* src = dir_logits + ((long long)n * T + t) * D * P;
         Pack4<float> x[DMAX];
         float m[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
 #pragma unroll
         for (int d = 0; d < DMAX; ++d)
             if (d < D) {
-                x[d] = ld4(src + d * P, i, P, vec);
+                x[d] = ld4f(src + d * P, i, P, vec);
 #pragma unroll
                 for (int k = 0; k < 4; ++k) m[k] = fmaxf(m[k], x[d].v[k]);
             }
@@ -151,14 +154,15 @@ __global__ void k_key_init(int* k, int n) {
 }
 
 // point = sum_t point_t / T and its per-tile maximum
+template <class TI>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_point_mean(Geom g, const float* __restrict__ point_logits, int T, float* __restrict__ pmean, int* pmax_key) {
+k_point_mean(Geom g, const TI* __restrict__ point_logits, int T, float* __restrict__ pmean, int* pmax_key) {
     Pix px;
     if (!warp_pixel(g, px)) return;
     float acc = -INFINITY;
     if (px.ok) {
         for (int t = 0; t < T; ++t) {
-            float v = point_logits[((long long)px.n * T + t) * g.P + px.idx];
+            float v = to_f32(point_logits[((long long)px.n * T + t) * g.P + px.idx]);
             acc = t == 0 ? v : acc + v;
         }
         acc = acc / (float)T;
@@ -238,9 +242,34 @@ int tiseg_ddm(tiseg_ctx* c, const uint8_t* dir_map, int N, int H, int W, float* 
     return end_call(c);
 }
 
-int tiseg_cdnet_refine(tiseg_ctx* c, const float* sem_logits, const float* dir_logits, const float* point_logits,
-                       int N, int T, int C, int D, int H, int W, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
-                       uint8_t* dir_map_out, float* dd_out) {
+}  // extern "C"
+
+// the refinement after the front kernels: per-variant direction maps from dir_all on, TI = element type of the heads
+template <class TI>
+static int cdnet_refine_run(tiseg_ctx* c, const Geom& g, const TI* d_sem, const TI* d_dir, const TI* d_pt, int T, int C, int D,
+                            int if_ddm, float* d_prob, uint8_t* d_cls, float* d_dd, uint8_t* dir_all, float* pmean, int* pmax) {
+    const int N = g.N;
+    // softmax + TTA mean of the semantic head: the K1 kernel
+    TISEG_TRY(softmax_argmax_dev(c, g, d_sem, T, C, d_prob, nullptr));
+    {
+        const bool v4 = (g.P % 4 == 0) && aligned_x4<TI>(d_dir) && aligned16(d_prob) && (((uintptr_t)dir_all) & 3) == 0;
+        const dim3 fg(flat4_grid(g.P), (unsigned)N);
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dir_map<9>"), (k_dir_map<TI, 9>), fg, TISEG_THREADS, 0, (long long)g.P, d_dir, d_prob, T, D, C,
+                        dir_all, v4);     // D == 9 is checked by the caller
+    }
+    TISEG_TRY(ddm_dev(c, g, dir_all, T, d_dd));
+    TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_point_mean"), k_point_mean<TI>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
+    TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_prob, C, d_dd, pmean, pmax, if_ddm, 0, d_cls);
+    return TISEG_OK;
+}
+
+extern "C" {
+
+int tiseg_cdnet_refine_typed(tiseg_ctx* c, int dtype, const void* sem_logits, const void* dir_logits, const void* point_logits,
+                             int N, int T, int C, int D, int H, int W, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
+                             uint8_t* dir_map_out, float* dd_out) {
+    TISEG_TRY(check_dtype(dtype, "tiseg_cdnet_refine"));
     if (!c || !sem_logits || !dir_logits || !point_logits || T <= 0 || C < 2 || C > 16 || D != 9) {
         set_error("tiseg_cdnet_refine: bad argument (2 <= C <= 16, D == 9)");
         return TISEG_ERR_ARG;
@@ -249,9 +278,10 @@ int tiseg_cdnet_refine(tiseg_ctx* c, const float* sem_logits, const float* dir_l
     begin_call(c);
     Geom g = make_geom(N, H, W);
     size_t total = (size_t)N * g.P;
-    const float* d_sem = in(c, sem_logits, total * T * C);
-    const float* d_dir = in(c, dir_logits, total * T * D);
-    const float* d_pt = in(c, point_logits, total * T);
+    const size_t eb = dtype_bytes(dtype);
+    const void* d_sem = in_ptr(c, sem_logits, total * T * C * eb);
+    const void* d_dir = in_ptr(c, dir_logits, total * T * D * eb);
+    const void* d_pt = in_ptr(c, point_logits, total * T * eb);
     float* d_prob = sem_prob_out ? tiseg::out(c, sem_prob_out, total * C) : ws<float>(c, total * C);
     uint8_t* d_cls = cls_out ? tiseg::out(c, cls_out, total) : nullptr;
     float* d_dd = dd_out ? tiseg::out(c, dd_out, total) : ws<float>(c, total);
@@ -259,17 +289,11 @@ int tiseg_cdnet_refine(tiseg_ctx* c, const float* sem_logits, const float* dir_l
     float* pmean = ws<float>(c, total);
     int* pmax = ws<int>(c, (size_t)N);
     if (!d_sem || !d_dir || !d_pt || !d_prob || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
-    // softmax + TTA mean of the semantic head: the K1 kernel
-    TISEG_TRY(softmax_argmax_dev(c, g, d_sem, T, C, d_prob, nullptr));
-    {
-        const bool v4 = (g.P % 4 == 0) && aligned16(d_dir, d_prob) && (((uintptr_t)dir_all) & 3) == 0;
-        const dim3 fg(flat4_grid(g.P), (unsigned)N);
-        TISEG_LAUNCH(c, k_dir_map<9>, fg, TISEG_THREADS, 0, (long long)g.P, d_dir, d_prob, T, D, C, dir_all, v4);     // D == 9 is checked above
-    }
-    TISEG_TRY(ddm_dev(c, g, dir_all, T, d_dd));
-    TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
-    TISEG_LAUNCH(c, k_point_mean, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
-    TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_prob, C, d_dd, pmean, pmax, if_ddm, 0, d_cls);
+    TISEG_TRY(with_dtype(dtype, [&](auto z) {
+        using TI = decltype(z);
+        return cdnet_refine_run(c, g, (const TI*)d_sem, (const TI*)d_dir, (const TI*)d_pt, T, C, D, if_ddm, d_prob, d_cls, d_dd,
+                                dir_all, pmean, pmax);
+    }));
     if (dir_map_out) {
         // dir_map_list[0] of every tile (cdnet.py:217)
         uint8_t* d_dm = tiseg::out(c, dir_map_out, total);
@@ -277,6 +301,13 @@ int tiseg_cdnet_refine(tiseg_ctx* c, const float* sem_logits, const float* dir_l
         TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
     }
     return end_call(c);
+}
+
+int tiseg_cdnet_refine(tiseg_ctx* c, const float* sem_logits, const float* dir_logits, const float* point_logits,
+                       int N, int T, int C, int D, int H, int W, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
+                       uint8_t* dir_map_out, float* dd_out) {
+    return tiseg_cdnet_refine_typed(c, TISEG_DTYPE_F32, sem_logits, dir_logits, point_logits, N, T, C, D, H, W, if_ddm, sem_prob_out,
+                                    cls_out, dir_map_out, dd_out);
 }
 
 int tiseg_ddm_enhance(tiseg_ctx* c, float* sem_prob, const float* dd, const float* point, int N, int C, int H, int W, int mode) {
@@ -295,7 +326,7 @@ int tiseg_ddm_enhance(tiseg_ctx* c, float* sem_prob, const float* dd, const floa
     int* pmax = ws<int>(c, (size_t)N);
     if (!d_prob || !d_dd || !d_pt || !pmean || !pmax) return TISEG_ERR_CUDA;
     TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
-    TISEG_LAUNCH(c, k_point_mean, warp_grid(g), TISEG_THREADS, 0, g, d_pt, 1, pmean, pmax);
+    TISEG_LAUNCH_AS(c, "k_point_mean", k_point_mean<float>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, 1, pmean, pmax);
     TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_prob, C, d_dd, pmean, pmax, 1, mode, (uint8_t*)nullptr);
     return end_call(c);
 }
@@ -306,8 +337,9 @@ namespace tiseg {
 // use_regression (multi_task_cdnet.py:304-315): the direction head is ONE channel, an angle in radians.  Per variant:
 // clamp to [0, 2 pi], degrees, (180, 360] -> (-180, 0], class = 1 + bin of align_angle with eight angles
 // (direction_calculation.py:60-73); background (first maximum of the mean three-class probabilities is class 0) -> 0.
+template <class TI>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_reg_dir_map(Geom g, const float* __restrict__ reg, const float* __restrict__ tc_prob, int T, int C, uint8_t* __restrict__ dir_map) {
+k_reg_dir_map(Geom g, const TI* __restrict__ reg, const float* __restrict__ tc_prob, int T, int C, uint8_t* __restrict__ dir_map) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
     const float* tp = tc_prob + (long long)px.n * C * g.P + px.idx;
@@ -316,7 +348,7 @@ k_reg_dir_map(Geom g, const float* __restrict__ reg, const float* __restrict__ t
     for (int k = 1; k < C; ++k) if (tp[(long long)k * g.P] > best) { best = tp[(long long)k * g.P]; bg = false; }
     for (int t = 0; t < T; ++t) {
         const long long tile = (long long)px.n * T + t;
-        float a = reg[tile * g.P + px.idx];
+        float a = to_f32(reg[tile * g.P + px.idx]);
         if (a < 0.f) a = 0.f;
         if (a > 6.28318548202514648f) a = 6.28318548202514648f;
         float deg = (a * 180.f) / 3.14159274101257324f;
@@ -331,12 +363,41 @@ k_reg_dir_map(Geom g, const float* __restrict__ reg, const float* __restrict__ t
 }
 }  // namespace tiseg
 
+// the refinement after the staging, TI = element type of the heads
+template <class TI>
+static int mtcdnet_refine_run(tiseg_ctx* c, const Geom& g, const TI* d_tc, const TI* d_sem, const TI* d_dir, const TI* d_pt, int T,
+                              int Ctc, int Csem, int D, int if_ddm, float* d_tcp, uint8_t* d_tcc, float* d_semp, uint8_t* d_semc,
+                              float* d_dd, uint8_t* dir_all, float* pmean, int* pmax) {
+    const int N = g.N;
+    const size_t total = (size_t)N * g.P;
+    // softmax + TTA mean of the three-class and of the semantic head (multi_task_cdnet.py:283-294)
+    TISEG_TRY(softmax_argmax_dev(c, g, d_tc, T, Ctc, d_tcp, nullptr));
+    if (d_semp || d_semc) {
+        float* sp = d_semp;
+        if (!sp && T > 1) { sp = ws<float>(c, total * Csem); if (!sp) return TISEG_ERR_CUDA; }      // (T == 1: streaming argmax)
+        TISEG_TRY(softmax_argmax_dev(c, g, d_sem, T, Csem, sp, d_semc));
+    }
+    if (D == 1) {   // use_regression: the angle head -> classes (:304-315)
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_reg_dir_map"), k_reg_dir_map<TI>, warp_grid(g), TISEG_THREADS, 0, g, d_dir, d_tcp, T, Ctc, dir_all);
+    } else {   // per variant: dir[:, 0] *= tc[:, 0]; argmax; DDM (:318-322)
+        const bool v4 = (g.P % 4 == 0) && aligned_x4<TI>(d_dir) && aligned16(d_tcp) && (((uintptr_t)dir_all) & 3) == 0;
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dir_map<9>"), (k_dir_map<TI, 9>), dim3(flat4_grid(g.P), (unsigned)N), TISEG_THREADS, 0,
+                        (long long)g.P, d_dir, d_tcp, T, D, Ctc, dir_all, v4);
+    }
+    TISEG_TRY(ddm_dev(c, g, dir_all, T, d_dd));
+    TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_point_mean"), k_point_mean<TI>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
+    TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_tcp, Ctc, d_dd, pmean, pmax, if_ddm, 1, d_tcc);
+    return TISEG_OK;
+}
+
 extern "C" {
 
-int tiseg_mtcdnet_refine(tiseg_ctx* c, const float* tc_logits, const float* sem_logits, const float* dir_logits,
-                         const float* point_logits, int N, int T, int Ctc, int Csem, int D, int H, int W, int if_ddm,
-                         float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
-                         uint8_t* dir_map_out, float* dd_out) {
+int tiseg_mtcdnet_refine_typed(tiseg_ctx* c, int dtype, const void* tc_logits, const void* sem_logits, const void* dir_logits,
+                               const void* point_logits, int N, int T, int Ctc, int Csem, int D, int H, int W, int if_ddm,
+                               float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
+                               uint8_t* dir_map_out, float* dd_out) {
+    TISEG_TRY(check_dtype(dtype, "tiseg_mtcdnet_refine"));
     if (!c || !tc_logits || !sem_logits || !dir_logits || !point_logits || T <= 0 || Ctc < 2 || Ctc > 16 || Csem < 1 ||
         Csem > 16 || (D != 9 && D != 1)) {
         set_error("tiseg_mtcdnet_refine: bad argument (2 <= Ctc <= 16, 1 <= Csem <= 16, D == 9, or D == 1: the regression head)");
@@ -346,10 +407,11 @@ int tiseg_mtcdnet_refine(tiseg_ctx* c, const float* tc_logits, const float* sem_
     begin_call(c);
     Geom g = make_geom(N, H, W);
     const size_t total = (size_t)N * g.P;
-    const float* d_tc = in(c, tc_logits, total * T * Ctc);
-    const float* d_sem = in(c, sem_logits, total * T * Csem);
-    const float* d_dir = in(c, dir_logits, total * T * D);
-    const float* d_pt = in(c, point_logits, total * T);
+    const size_t eb = dtype_bytes(dtype);
+    const void* d_tc = in_ptr(c, tc_logits, total * T * Ctc * eb);
+    const void* d_sem = in_ptr(c, sem_logits, total * T * Csem * eb);
+    const void* d_dir = in_ptr(c, dir_logits, total * T * D * eb);
+    const void* d_pt = in_ptr(c, point_logits, total * T * eb);
     float* d_tcp = tc_prob_out ? tiseg::out(c, tc_prob_out, total * Ctc) : ws<float>(c, total * Ctc);
     uint8_t* d_tcc = tc_cls_out ? tiseg::out(c, tc_cls_out, total) : nullptr;
     float* d_semp = sem_prob_out ? tiseg::out(c, sem_prob_out, total * Csem) : nullptr;
@@ -359,29 +421,25 @@ int tiseg_mtcdnet_refine(tiseg_ctx* c, const float* tc_logits, const float* sem_
     float* pmean = ws<float>(c, total);
     int* pmax = ws<int>(c, (size_t)N);
     if (!d_tc || !d_sem || !d_dir || !d_pt || !d_tcp || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
-    // softmax + TTA mean of the three-class and of the semantic head (multi_task_cdnet.py:283-294)
-    TISEG_TRY(softmax_argmax_dev(c, g, d_tc, T, Ctc, d_tcp, nullptr));
-    if (d_semp || d_semc) {
-        float* sp = d_semp;
-        if (!sp && T > 1) { sp = ws<float>(c, total * Csem); if (!sp) return TISEG_ERR_CUDA; }      // (T == 1: streaming argmax)
-        TISEG_TRY(softmax_argmax_dev(c, g, d_sem, T, Csem, sp, d_semc));
-    }
-    if (D == 1) {   // use_regression: the angle head -> classes (:304-315)
-        TISEG_LAUNCH(c, k_reg_dir_map, warp_grid(g), TISEG_THREADS, 0, g, d_dir, d_tcp, T, Ctc, dir_all);
-    } else {   // per variant: dir[:, 0] *= tc[:, 0]; argmax; DDM (:318-322)
-        const bool v4 = (g.P % 4 == 0) && aligned16(d_dir, d_tcp) && (((uintptr_t)dir_all) & 3) == 0;
-        TISEG_LAUNCH(c, k_dir_map<9>, dim3(flat4_grid(g.P), (unsigned)N), TISEG_THREADS, 0, (long long)g.P, d_dir, d_tcp, T, D, Ctc, dir_all, v4);
-    }
-    TISEG_TRY(ddm_dev(c, g, dir_all, T, d_dd));
-    TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
-    TISEG_LAUNCH(c, k_point_mean, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
-    TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_tcp, Ctc, d_dd, pmean, pmax, if_ddm, 1, d_tcc);
+    TISEG_TRY(with_dtype(dtype, [&](auto z) {
+        using TI = decltype(z);
+        return mtcdnet_refine_run(c, g, (const TI*)d_tc, (const TI*)d_sem, (const TI*)d_dir, (const TI*)d_pt, T, Ctc, Csem, D, if_ddm,
+                                  d_tcp, d_tcc, d_semp, d_semc, d_dd, dir_all, pmean, pmax);
+    }));
     if (dir_map_out) {
         uint8_t* d_dm = tiseg::out(c, dir_map_out, total);
         if (!d_dm) return TISEG_ERR_CUDA;
         TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
     }
     return end_call(c);
+}
+
+int tiseg_mtcdnet_refine(tiseg_ctx* c, const float* tc_logits, const float* sem_logits, const float* dir_logits,
+                         const float* point_logits, int N, int T, int Ctc, int Csem, int D, int H, int W, int if_ddm,
+                         float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
+                         uint8_t* dir_map_out, float* dd_out) {
+    return tiseg_mtcdnet_refine_typed(c, TISEG_DTYPE_F32, tc_logits, sem_logits, dir_logits, point_logits, N, T, Ctc, Csem, D, H, W,
+                                      if_ddm, tc_prob_out, tc_cls_out, sem_prob_out, sem_cls_out, dir_map_out, dd_out);
 }
 
 }  // extern "C"

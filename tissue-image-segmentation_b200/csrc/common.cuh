@@ -5,6 +5,8 @@
 // horizontal segment of one row (coalesced 128-byte int32 or 32-byte uint8 requests); the warp-level
 // run primitives (ballot / clz) below are what the CCL, histogram and area kernels build on.
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string>
@@ -256,6 +258,73 @@ __device__ __forceinline__ void st4(T* __restrict__ p, long long i, long long to
     }
 }
 __device__ __forceinline__ long long flat4_index() { return ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4; }
+
+// ---- network outputs in fp32, fp16 or bf16 (TISEG_DTYPE_*) ---------------------------------------------------------
+// Kernels that read a network output are templated on its element type and convert at the load; everything after the
+// load is fp32 arithmetic.  fp16 -> fp32 and bf16 -> fp32 are exact, so a half input gives the bits of its fp32 upcast.
+template <> struct __align__(8) Pack4<__half> { __half v[4]; };
+template <> struct __align__(8) Pack4<__nv_bfloat16> { __nv_bfloat16 v[4]; };
+template <class T> struct InType;
+template <> struct InType<float> { static constexpr int code = TISEG_DTYPE_F32; };
+template <> struct InType<__half> { static constexpr int code = TISEG_DTYPE_F16; };
+template <> struct InType<__nv_bfloat16> { static constexpr int code = TISEG_DTYPE_BF16; };
+// timing name of a launch: the fp32 instantiation keeps the plain kernel name, the half ones carry the dtype
+#define TISEG_IN_NAME(T, name) \
+    (::tiseg::InType<T>::code == TISEG_DTYPE_F32 ? name : ::tiseg::InType<T>::code == TISEG_DTYPE_F16 ? name ":f16" : name ":bf16")
+// four consecutive elements of a network output are 16 B in fp32, 8 B in half precision
+template <class T> inline bool aligned_x4(const void* p) { return (((uintptr_t)p) & (4 * sizeof(T) - 1)) == 0; }
+inline int check_dtype(int dtype, const char* where) {
+    if (dtype == TISEG_DTYPE_F32 || dtype == TISEG_DTYPE_F16 || dtype == TISEG_DTYPE_BF16) return TISEG_OK;
+    set_error(std::string(where) + ": unknown dtype code " + std::to_string(dtype) + " (0 fp32, 1 fp16, 2 bf16)");
+    return TISEG_ERR_ARG;
+}
+inline size_t dtype_bytes(int dtype) { return dtype == TISEG_DTYPE_F32 ? 4 : 2; }
+// call fn(T()) with T the element type of the dtype code (checked beforehand with check_dtype)
+template <class F> inline int with_dtype(int dtype, F&& fn) {
+    if (dtype == TISEG_DTYPE_F16) return fn(__half());
+    if (dtype == TISEG_DTYPE_BF16) return fn(__nv_bfloat16());
+    return fn(0.f);
+}
+
+__device__ __forceinline__ float to_f32(float x) { return x; }
+__device__ __forceinline__ float to_f32(__half x) { return __half2float(x); }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 x) { return __bfloat162float(x); }
+__device__ __forceinline__ float2 to_f32(float2 x) { return x; }
+__device__ __forceinline__ float2 to_f32(__half2 x) { return __half22float2(x); }
+__device__ __forceinline__ float2 to_f32(__nv_bfloat162 x) { return __bfloat1622float2(x); }
+template <class T> struct Pair;                        // two interleaved channels (an HWC map of two)
+template <> struct Pair<float> { typedef float2 type; };
+template <> struct Pair<__half> { typedef __half2 type; };
+template <> struct Pair<__nv_bfloat16> { typedef __nv_bfloat162 type; };
+
+// ld4 of a network output, converted to fp32 (`vec`: the pointer is aligned to four elements)
+__device__ __forceinline__ Pack4<float> ld4f(const float* __restrict__ p, long long i, long long total, bool vec) {
+    return ld4(p, i, total, vec);
+}
+template <class T>
+__device__ __forceinline__ Pack4<float> ld4f(const T* __restrict__ p, long long i, long long total, bool vec) {
+    Pack4<float> r;
+    if (vec && i + 3 < total) {
+        const Pack4<T> h = *reinterpret_cast<const Pack4<T>*>(p + i);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) r.v[k] = to_f32(h.v[k]);
+    } else {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) r.v[k] = i + k < total ? to_f32(p[i + k]) : 0.f;
+    }
+    return r;
+}
+// four aligned consecutive elements, converted to fp32
+__device__ __forceinline__ void ld4f_aligned(const float* p, float (&x)[4]) {
+    const float4 u = *reinterpret_cast<const float4*>(p);
+    x[0] = u.x; x[1] = u.y; x[2] = u.z; x[3] = u.w;
+}
+template <class T>
+__device__ __forceinline__ void ld4f_aligned(const T* p, float (&x)[4]) {
+    const Pack4<T> h = *reinterpret_cast<const Pack4<T>*>(p);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) x[k] = to_f32(h.v[k]);
+}
 
 // Given the ballot of "this lane continues the run of the lane to its left" (bit 0 of the segment may be
 // set when the run continues from the previous segment), the lane at which my run starts inside the segment.

@@ -16,10 +16,11 @@
 namespace tiseg {
 
 // level image + the F plane of the mask b = (I < 255): one warp = 128 columns x DP_ROWS rows, four pixels per thread and
-// row, all loads of the thread issued before the first is used
+// row, all loads of the thread issued before the first is used.  The distance map may be fp32, fp16 or bf16 (TI); it is
+// converted to fp32 as it is loaded.
 #define DP_ROWS 4
-template <bool FULL>
-__device__ __forceinline__ void dp_rows(const Geom& g, const float* __restrict__ dt, uint8_t* __restrict__ It, unsigned* __restrict__ Ft,
+template <bool FULL, class TI>
+__device__ __forceinline__ void dp_rows(const Geom& g, const TI* __restrict__ dt, uint8_t* __restrict__ It, unsigned* __restrict__ Ft,
                                         int lane, int x, int y0) {
     const int W = g.W;
     float d[DP_ROWS][4];
@@ -29,10 +30,10 @@ __device__ __forceinline__ void dp_rows(const Geom& g, const float* __restrict__
         d[r][0] = d[r][1] = d[r][2] = d[r][3] = 0.f;
         if (y < g.H) {                               // (uniform)
             const int ro = y * W + x;
-            if (FULL) { const float4 t = *reinterpret_cast<const float4*>(dt + ro); d[r][0] = t.x; d[r][1] = t.y; d[r][2] = t.z; d[r][3] = t.w; }
+            if (FULL) ld4f_aligned(dt + ro, d[r]);
             else {
 #pragma unroll
-                for (int k = 0; k < 4; ++k) if (x + k < W) d[r][k] = dt[ro + k];
+                for (int k = 0; k < 4; ++k) if (x + k < W) d[r][k] = to_f32(dt[ro + k]);
             }
         }
     }
@@ -65,15 +66,16 @@ __device__ __forceinline__ void dp_rows(const Geom& g, const float* __restrict__
         if ((lane & 7) == 0 && seg < g.SEG) Ft[y * g.SEG + seg] = word;
     }
 }
+template <class TI>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_dist_prep(Geom g, const float* __restrict__ dist, uint8_t* __restrict__ I, unsigned* __restrict__ F, bool vec) {
+k_dist_prep(Geom g, const TI* __restrict__ dist, uint8_t* __restrict__ I, unsigned* __restrict__ F, bool vec) {
     const int lane = threadIdx.x & 31;
     const int strips = (g.W + 127) >> 7, chunks = (g.H + DP_ROWS - 1) / DP_ROWS;
     const long long wi = (long long)blockIdx.x * TISEG_WARPS_PER_BLOCK + (threadIdx.x >> 5);
     if (wi >= (long long)strips * chunks) return;
     const int ch = (int)(wi / strips), strip = (int)(wi - (long long)ch * strips), n = blockIdx.y;
     // (tile bases as opaque register pairs + 32-bit offsets: one IMAD.WIDE per access)
-    const float* dt = dist + (long long)n * g.P;
+    const TI* dt = dist + (long long)n * g.P;
     uint8_t* It = I + (long long)n * g.P;
     unsigned* Ft = F + (long long)n * g.H * g.SEG;
     asm volatile("" : "+l"(dt)); asm volatile("" : "+l"(It)); asm volatile("" : "+l"(Ft));
@@ -579,7 +581,8 @@ k_wsl_remove(Geom g, const int32_t* __restrict__ lab, const unsigned* __restrict
 
 int h_reconstruction_erosion_dev(tiseg_ctx* c, const Geom& g, const uint8_t* img, int h, uint8_t* out);   // recon.cu
 
-int postproc_dist_dev(tiseg_ctx* c, const Geom& g, const float* dist, int lamb, int32_t* inst, int32_t* markers_out,
+// dist: the distance map, of element type `dtype` (TISEG_DTYPE_*)
+int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, int lamb, int32_t* inst, int32_t* markers_out,
                       int32_t* ws_out) {
     int N = g.N, KS = g.P + 1;
     size_t total = (size_t)N * g.P;
@@ -616,11 +619,14 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, const float* dist, int lamb, 
     int* ndense = dense + N;
     TISEG_TRY(zero(c, marea, (2 * (size_t)N + 2) * sizeof(int)));
 
-    {
+    TISEG_TRY(with_dtype(dtype, [&](auto z) {
+        using TI = decltype(z);
         const long long warps = (long long)((g.W + 127) / 128) * ((g.H + DP_ROWS - 1) / DP_ROWS);
-        TISEG_LAUNCH(c, k_dist_prep, dim3((unsigned)((warps + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK), (unsigned)N),
-                     TISEG_THREADS, 0, g, dist, I0, mbits, (g.W % 4 == 0) && aligned16(dist) && (((uintptr_t)I0) & 3) == 0);
-    }
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dist_prep"), k_dist_prep<TI>,
+                        dim3((unsigned)((warps + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK), (unsigned)N), TISEG_THREADS, 0,
+                        g, (const TI*)dist, I0, mbits, (g.W % 4 == 0) && aligned_x4<TI>(dist) && (((uintptr_t)I0) & 3) == 0);
+        return TISEG_OK;
+    }));
     // Hrecons (dist.py:120): the identity for the lambda = 0.0 the reference hard-codes (dist.py:281); a real
     // H-minima reconstruction otherwise.  Markers and flood levels come from it, the mask b from the image itself.
     if (lamb > 0) {
@@ -709,18 +715,24 @@ extern "C" int tiseg_postproc_dist(tiseg_ctx* c, const float* dist, int N, int H
     return tiseg_postproc_dist_lambda(c, dist, N, H, W, 0, inst_out, markers_out, ws_out);
 }
 
-extern "C" int tiseg_postproc_dist_lambda(tiseg_ctx* c, const float* dist, int N, int H, int W, int lamb,
-                                          int32_t* inst_out, int32_t* markers_out, int32_t* ws_out) {
+extern "C" int tiseg_postproc_dist_lambda_typed(tiseg_ctx* c, int dtype, const void* dist, int N, int H, int W, int lamb,
+                                                int32_t* inst_out, int32_t* markers_out, int32_t* ws_out) {
+    TISEG_TRY(check_dtype(dtype, "tiseg_postproc_dist"));
     if (!c || !dist || !inst_out || lamb < 0 || lamb > 255) { set_error("tiseg_postproc_dist: bad argument (0 <= lambda <= 255)"); return TISEG_ERR_ARG; }
     TISEG_TRY(check_geom(N, H, W));
     begin_call(c);
     Geom g = make_geom(N, H, W);
     size_t total = (size_t)N * g.P;
-    const float* d_dist = in(c, dist, total);
+    const void* d_dist = in_ptr(c, dist, total * dtype_bytes(dtype));
     int32_t* d_inst = tiseg::out(c, inst_out, total);
     int32_t* d_mk = markers_out ? tiseg::out(c, markers_out, total) : nullptr;
     int32_t* d_ws = ws_out ? tiseg::out(c, ws_out, total) : nullptr;
     if (!d_dist || !d_inst) return TISEG_ERR_CUDA;
-    TISEG_TRY(postproc_dist_dev(c, g, d_dist, lamb, d_inst, d_mk, d_ws));
+    TISEG_TRY(postproc_dist_dev(c, g, dtype, d_dist, lamb, d_inst, d_mk, d_ws));
     return end_call(c);
+}
+
+extern "C" int tiseg_postproc_dist_lambda(tiseg_ctx* c, const float* dist, int N, int H, int W, int lamb,
+                                          int32_t* inst_out, int32_t* markers_out, int32_t* ws_out) {
+    return tiseg_postproc_dist_lambda_typed(c, TISEG_DTYPE_F32, dist, N, H, W, lamb, inst_out, markers_out, ws_out);
 }

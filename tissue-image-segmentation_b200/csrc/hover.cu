@@ -11,6 +11,8 @@
 //             BORDER_REFLECT_101
 //   GaussianBlur 3x3 on fp64: row pass (a/4 + b/2) + c/4, column pass b/2 + (a + c)/4
 // (--fmad=false for the whole library; fma() is written out where OpenCV contracts.)
+// The foreground and HV maps may be fp32, fp16 or bf16 (TI): the kernels that read them convert at the load, so the chain
+// sees the fp32 values of the inputs either way.
 #include <cfloat>
 
 #include "ccl.cuh"
@@ -49,10 +51,11 @@ __global__ void k_mm_init(long long* mm, int n) {
 }
 
 // min / max of the two HWC channels of the HV map (eight pixels per thread before the warp reduction)
+template <class TI>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_hv_minmax(Geom g, const float2* __restrict__ hv, long long* mm /* [N, 2 channels, 2] */) {
+k_hv_minmax(Geom g, const typename Pair<TI>::type* __restrict__ hv, long long* mm /* [N, 2 channels, 2] */) {
     const int n = blockIdx.y;
-    const float2* t = hv + (long long)n * g.P;
+    const typename Pair<TI>::type* t = hv + (long long)n * g.P;
     float lx = INFINITY, hx = -INFINITY, ly = INFINITY, hy = -INFINITY;
     bool any = false;
     const long long i0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x);
@@ -61,7 +64,7 @@ k_hv_minmax(Geom g, const float2* __restrict__ hv, long long* mm /* [N, 2 channe
     for (int k = 0; k < 8; ++k) {
         const long long i = i0 + k * stride;
         if (i < g.P) {
-            const float2 v = t[i];
+            const float2 v = to_f32(t[i]);
             lx = fminf(lx, v.x); hx = fmaxf(hx, v.x); ly = fminf(ly, v.y); hy = fmaxf(hy, v.y);
             any = true;
         }
@@ -80,13 +83,14 @@ __device__ __forceinline__ NormCoef norm_coef(const long long* mm) {
     return c;
 }
 
+template <class TI>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_hv_normalize(Geom g, const float2* __restrict__ hv, const long long* __restrict__ mm, float* __restrict__ hdir,
+k_hv_normalize(Geom g, const typename Pair<TI>::type* __restrict__ hv, const long long* __restrict__ mm, float* __restrict__ hdir,
                float* __restrict__ vdir) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
     NormCoef ch = norm_coef(mm + (long long)px.n * 4), cv = norm_coef(mm + (long long)px.n * 4 + 2);
-    float2 v = hv[px.base + px.idx];
+    float2 v = to_f32(hv[px.base + px.idx]);
     hdir[px.base + px.idx] = (float)fma((double)v.x, ch.a, ch.b);
     vdir[px.base + px.idx] = (float)fma((double)v.y, cv.a, cv.b);
 }
@@ -166,10 +170,11 @@ k_sobel_col(Geom g, const double* __restrict__ rowbuf, double* __restrict__ out,
     warp_minmax_commit(lo, hi, live, mm + (long long)n * 2);
 }
 
-__global__ void k_threshold_ge(Geom g, const float* __restrict__ x, float thr, uint8_t* __restrict__ out) {
+template <class TI>
+__global__ void k_threshold_ge(Geom g, const TI* __restrict__ x, float thr, uint8_t* __restrict__ out) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
-    out[px.base + px.idx] = x[px.base + px.idx] >= thr;
+    out[px.base + px.idx] = to_f32(x[px.base + px.idx]) >= thr;
 }
 
 // hovernet.py:343-353: overall, dist (before the blur) and the raw marker mask
@@ -266,7 +271,9 @@ k_ellipse5(Geom g, const uint8_t* __restrict__ src, uint8_t* __restrict__ out, b
     }
 }
 
-int postproc_hover_dev(tiseg_ctx* c, const Geom& g, const float* fore, const float* hv, int obj_size, int32_t* inst,
+// fore [N,H,W] and hv [N,H,W,2] of element type TI
+template <class TI>
+int postproc_hover_dev(tiseg_ctx* c, const Geom& g, const TI* fore, const TI* hv, int obj_size, int32_t* inst,
                        uint8_t* blb_out, double* dist_out, int32_t* marker_out) {
     int N = g.N;
     size_t total = (size_t)N * g.P;
@@ -285,15 +292,16 @@ int postproc_hover_dev(tiseg_ctx* c, const Geom& g, const float* fore, const flo
     if (!m0 || !blb || !hdir || !vdir || !rowb || !sobh || !sobv || !dist || !dpre || !mk0 || !mk1 || !lab || !markers || !mm || !par || !rank)
         return TISEG_ERR_CUDA;
     long long* mm_hv = mm; long long* mm_sh = mm + (size_t)N * 4; long long* mm_sv = mm + (size_t)N * 6;
-    const float2* hv2 = (const float2*)hv;
+    const typename Pair<TI>::type* hv2 = (const typename Pair<TI>::type*)hv;
 
     // blb = (fore >= 0.5) -> 4-connected components -> drop < 10 px (hovernet.py:294-298)
-    TISEG_LAUNCH(c, k_threshold_ge, warp_grid(g), TISEG_THREADS, 0, g, fore, 0.5f, m0);
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_threshold_ge"), k_threshold_ge<TI>, warp_grid(g), TISEG_THREADS, 0, g, fore, 0.5f, m0);
     TISEG_TRY(remove_small_mask(c, g, m0, 10, 1, blb));
     // normalised H / V maps
     TISEG_LAUNCH(c, k_mm_init, (4 * N + 255) / 256, 256, 0, mm, 4 * N);
-    TISEG_LAUNCH(c, k_hv_minmax, dim3((unsigned)((g.P + 8 * TISEG_THREADS - 1) / (8 * TISEG_THREADS)), (unsigned)N), TISEG_THREADS, 0, g, hv2, mm_hv);
-    TISEG_LAUNCH(c, k_hv_normalize, warp_grid(g), TISEG_THREADS, 0, g, hv2, mm_hv, hdir, vdir);
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_hv_minmax"), k_hv_minmax<TI>, dim3((unsigned)((g.P + 8 * TISEG_THREADS - 1) / (8 * TISEG_THREADS)), (unsigned)N),
+                    TISEG_THREADS, 0, g, hv2, mm_hv);
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_hv_normalize"), k_hv_normalize<TI>, warp_grid(g), TISEG_THREADS, 0, g, hv2, mm_hv, hdir, vdir);
     // Sobel(h_dir, dx=1): derivative along x, smoothing along y;  Sobel(v_dir, dy=1): the transpose
     const dim3 rg((unsigned)(((long long)((g.W + 3) / 4) * g.H + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N);
     const dim3 cg((unsigned)(((long long)((g.H + 3) / 4) * g.W + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N);
@@ -339,20 +347,20 @@ __device__ __forceinline__ float up2_mix(float x0, float x1, float a) {
     if (LERP) return fmaf(a, __fsub_rn(x1, x0), x0);
     return __fadd_rn(__fmul_rn(x0, __fsub_rn(1.f, a)), __fmul_rn(x1, a));
 }
-template <int CN, bool LERP>
+template <class TI, int CN, bool LERP>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_resize_up2(Geom gd, int H, int W, const float* __restrict__ src, float* __restrict__ dst) {
+k_resize_up2(Geom gd, int H, int W, const TI* __restrict__ src, float* __restrict__ dst) {
     Pix px;
     if (!warp_pixel(gd, px) || !px.ok) return;
     int y0, y1, x0, x1;
     float ay, ax;
     up2_coord(px.y, H, y0, y1, ay);
     up2_coord(px.x, W, x0, x1, ax);
-    const float* t = src + (long long)px.n * H * W * CN;
+    const TI* t = src + (long long)px.n * H * W * CN;
 #pragma unroll
     for (int ch = 0; ch < CN; ++ch) {
-        const float h0 = up2_mix<LERP>(t[((long long)y0 * W + x0) * CN + ch], t[((long long)y0 * W + x1) * CN + ch], ax);
-        const float h1 = up2_mix<LERP>(t[((long long)y1 * W + x0) * CN + ch], t[((long long)y1 * W + x1) * CN + ch], ax);
+        const float h0 = up2_mix<LERP>(to_f32(t[((long long)y0 * W + x0) * CN + ch]), to_f32(t[((long long)y0 * W + x1) * CN + ch]), ax);
+        const float h1 = up2_mix<LERP>(to_f32(t[((long long)y1 * W + x0) * CN + ch]), to_f32(t[((long long)y1 * W + x1) * CN + ch]), ax);
         dst[(px.base + px.idx) * CN + ch] = up2_mix<LERP>(h0, h1, ay);
     }
 }
@@ -368,9 +376,30 @@ k_resize_down2_nearest(Geom g, const int32_t* __restrict__ src, int32_t* __restr
 
 using namespace tiseg;
 
-extern "C" int tiseg_postproc_hover(tiseg_ctx* c, const float* fore_map, const float* hv_map, int N, int H, int W,
-                                    int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
-                                    int32_t* marker_out) {
+template <class TI>
+static int postproc_hover_entry(tiseg_ctx* c, const void* fore_map, const void* hv_map, const Geom& g, const Geom& gs,
+                                int scale_factor, int32_t* d_inst, uint8_t* d_blb, double* d_dist, int32_t* d_mk) {
+    const TI* d_fore = (const TI*)fore_map;
+    const TI* d_hv = (const TI*)hv_map;
+    if (scale_factor == 1) return postproc_hover_dev(c, g, d_fore, d_hv, 10, d_inst, d_blb, d_dist, d_mk);
+    const size_t stotal = (size_t)gs.N * gs.P;
+    float* fore2 = ws<float>(c, stotal);
+    float* hv2 = ws<float>(c, stotal * 2);
+    int32_t* inst2 = ws<int32_t>(c, stotal);
+    if (!fore2 || !hv2 || !inst2) return TISEG_ERR_CUDA;
+    const int H = g.H, W = g.W;
+    if (H >= 2 && W >= 2) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_resize_up2<1, true>)"), (k_resize_up2<TI, 1, true>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_fore, fore2);
+    else                  TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_resize_up2<1, false>)"), (k_resize_up2<TI, 1, false>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_fore, fore2);
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_resize_up2<2, false>)"), (k_resize_up2<TI, 2, false>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_hv, hv2);
+    TISEG_TRY(postproc_hover_dev(c, gs, (const float*)fore2, (const float*)hv2, 10, inst2, d_blb, d_dist, d_mk));
+    TISEG_LAUNCH(c, k_resize_down2_nearest, warp_grid(g), TISEG_THREADS, 0, g, inst2, d_inst);
+    return TISEG_OK;
+}
+
+extern "C" int tiseg_postproc_hover_typed(tiseg_ctx* c, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
+                                          int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
+                                          int32_t* marker_out) {
+    TISEG_TRY(check_dtype(dtype, "tiseg_postproc_hover"));
     if (!c || !fore_map || !hv_map || !inst_out) { set_error("tiseg_postproc_hover: bad argument"); return TISEG_ERR_ARG; }
     if (scale_factor != 1 && scale_factor != 2) {
         set_error("tiseg_postproc_hover: scale_factor must be 1 or 2 (the values of the reference configs)");
@@ -381,25 +410,22 @@ extern "C" int tiseg_postproc_hover(tiseg_ctx* c, const float* fore_map, const f
     Geom g = make_geom(N, H, W);
     Geom gs = make_geom(N, H * scale_factor, W * scale_factor);          // the resolution the pipeline runs at
     size_t total = (size_t)N * g.P, stotal = (size_t)N * gs.P;
-    const float* d_fore = in(c, fore_map, total);
-    const float* d_hv = in(c, hv_map, total * 2);
+    const void* d_fore = in_ptr(c, fore_map, total * dtype_bytes(dtype));
+    const void* d_hv = in_ptr(c, hv_map, total * 2 * dtype_bytes(dtype));
     int32_t* d_inst = tiseg::out(c, inst_out, total);
     uint8_t* d_blb = blb_out ? tiseg::out(c, blb_out, stotal) : nullptr;
     double* d_dist = dist_out ? tiseg::out(c, dist_out, stotal) : nullptr;
     int32_t* d_mk = marker_out ? tiseg::out(c, marker_out, stotal) : nullptr;
     if (!d_fore || !d_hv || !d_inst) return TISEG_ERR_CUDA;
-    if (scale_factor == 1) {
-        TISEG_TRY(postproc_hover_dev(c, g, d_fore, d_hv, 10, d_inst, d_blb, d_dist, d_mk));
-        return end_call(c);
-    }
-    float* fore2 = ws<float>(c, stotal);
-    float* hv2 = ws<float>(c, stotal * 2);
-    int32_t* inst2 = ws<int32_t>(c, stotal);
-    if (!fore2 || !hv2 || !inst2) return TISEG_ERR_CUDA;
-    if (H >= 2 && W >= 2) TISEG_LAUNCH(c, (k_resize_up2<1, true>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_fore, fore2);
-    else                  TISEG_LAUNCH(c, (k_resize_up2<1, false>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_fore, fore2);
-    TISEG_LAUNCH(c, (k_resize_up2<2, false>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_hv, hv2);
-    TISEG_TRY(postproc_hover_dev(c, gs, fore2, hv2, 10, inst2, d_blb, d_dist, d_mk));
-    TISEG_LAUNCH(c, k_resize_down2_nearest, warp_grid(g), TISEG_THREADS, 0, g, inst2, d_inst);
+    TISEG_TRY(with_dtype(dtype, [&](auto z) {
+        return postproc_hover_entry<decltype(z)>(c, d_fore, d_hv, g, gs, scale_factor, d_inst, d_blb, d_dist, d_mk);
+    }));
     return end_call(c);
+}
+
+extern "C" int tiseg_postproc_hover(tiseg_ctx* c, const float* fore_map, const float* hv_map, int N, int H, int W,
+                                    int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
+                                    int32_t* marker_out) {
+    return tiseg_postproc_hover_typed(c, TISEG_DTYPE_F32, fore_map, hv_map, N, H, W, scale_factor, inst_out, blb_out, dist_out,
+                                      marker_out);
 }

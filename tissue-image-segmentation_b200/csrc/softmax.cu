@@ -4,13 +4,14 @@
 //
 // fp32 arithmetic in the same order as the reference expression: e = exp(x - max), s = e_0 + e_1 + ...,
 // p = e / s, acc += p per variant, acc / T.  One thread per pixel, channel planes read coalesced.
+// The logits may be fp32, fp16 or bf16 (TI = the element type); they are converted to fp32 as they are loaded.
 #include "common.cuh"
 
 namespace tiseg {
 
-template <int CMAX>
+template <class TI, int CMAX>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_softmax_argmax(long long P, const float* __restrict__ logits, int T, int C, float* __restrict__ prob,
+k_softmax_argmax(long long P, const TI* __restrict__ logits, int T, int C, float* __restrict__ prob,
                  uint8_t* __restrict__ cls, bool vec) {
     // one thread = 4 consecutive pixels of one tile (blockIdx.y): float4 per channel plane, uchar4 out
     const int n = blockIdx.y;
@@ -18,13 +19,13 @@ k_softmax_argmax(long long P, const float* __restrict__ logits, int T, int C, fl
     if (i >= P) return;
     float acc[CMAX][4];
     for (int t = 0; t < T; ++t) {
-        const float* src = logits + ((long long)n * T + t) * C * P;
+        const TI* src = logits + ((long long)n * T + t) * C * P;
         Pack4<float> x[CMAX];
         float m[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
 #pragma unroll
         for (int c = 0; c < CMAX; ++c)
             if (c < C) {
-                x[c] = ld4(src + c * P, i, P, vec);
+                x[c] = ld4f(src + c * P, i, P, vec);
 #pragma unroll
                 for (int k = 0; k < 4; ++k) m[k] = fmaxf(m[k], x[c].v[k]);
             }
@@ -69,16 +70,16 @@ k_softmax_argmax(long long P, const float* __restrict__ logits, int T, int C, fl
 // under expf's 2-ulp error and two roundings of 6e-8 cannot close that gap, so the probabilities are strictly ordered
 // like the logits.  Pixels with a runner-up inside 1e-6 (or a NaN) are re-evaluated with the exact arithmetic of
 // k_softmax_argmax (same expf, same summation order, first maximum).
-template <int CMAX>
+template <class TI, int CMAX>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_argmax_logits(long long P, const float* __restrict__ logits, int C, uint8_t* __restrict__ cls, bool vec) {
+k_argmax_logits(long long P, const TI* __restrict__ logits, int C, uint8_t* __restrict__ cls, bool vec) {
     const int n = blockIdx.y;
     const long long i = flat4_index();
     if (i >= P) return;
-    const float* src = logits + (long long)n * C * P;
+    const TI* src = logits + (long long)n * C * P;
     Pack4<float> x[CMAX];
 #pragma unroll
-    for (int c = 0; c < CMAX; ++c) if (c < C) x[c] = ld4(src + c * P, i, P, vec);
+    for (int c = 0; c < CMAX; ++c) if (c < C) x[c] = ld4f(src + c * P, i, P, vec);
     Pack4<uint8_t> best;
     float bv[4];
 #pragma unroll
@@ -122,22 +123,23 @@ k_argmax_logits(long long P, const float* __restrict__ logits, int C, uint8_t* _
 
 // The same for exactly two classes (every binary nuclei model), written for the instruction issue rate: 32-bit tile-local
 // offsets from opaque tile bases, no class loop.  The generic kernel spends ~35 instructions per pixel on index arithmetic
-// and dead class slots and ran at 60 % of the HBM rate; this one is bound by the two 4-byte reads per pixel.
+// and dead class slots and ran at 60 % of the HBM rate; this one is bound by the two reads per pixel (4 B each in fp32).
+template <class TI>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_argmax_logits2(int P, const float* __restrict__ logits, uint8_t* __restrict__ cls, bool vec) {
+k_argmax_logits2(int P, const TI* __restrict__ logits, uint8_t* __restrict__ cls, bool vec) {
     const int i = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (i >= P) return;
-    const float* a = logits + (long long)blockIdx.y * 2 * P;
+    const TI* a = logits + (long long)blockIdx.y * 2 * P;
     uint8_t* o = cls + (long long)blockIdx.y * P;
     asm volatile("" : "+l"(a)); asm volatile("" : "+l"(o));
     __builtin_assume(__isGlobal(a)); __builtin_assume(__isGlobal(o));
     float x0[4], x1[4];
     if (vec) {
-        const float4 u = *reinterpret_cast<const float4*>(a + i), v = *reinterpret_cast<const float4*>(a + P + i);
-        x0[0] = u.x; x0[1] = u.y; x0[2] = u.z; x0[3] = u.w; x1[0] = v.x; x1[1] = v.y; x1[2] = v.z; x1[3] = v.w;
+        ld4f_aligned(a + i, x0);
+        ld4f_aligned(a + P + i, x1);
     } else {
 #pragma unroll
-        for (int k = 0; k < 4; ++k) { x0[k] = i + k < P ? a[i + k] : 0.f; x1[k] = i + k < P ? a[P + i + k] : 1.f; }
+        for (int k = 0; k < 4; ++k) { x0[k] = i + k < P ? to_f32(a[i + k]) : 0.f; x1[k] = i + k < P ? to_f32(a[P + i + k]) : 1.f; }
     }
     unsigned best = 0u;
     bool near = false;
@@ -171,23 +173,28 @@ k_argmax_logits2(int P, const float* __restrict__ logits, uint8_t* __restrict__ 
     }
 }
 
-int softmax_argmax_dev(tiseg_ctx* c, const Geom& g, const float* d_in, int T, int C, float* d_prob, uint8_t* d_cls) {
+// (the fp32 launches keep their plain timing names; the half-precision ones carry the dtype, TISEG_IN_NAME)
+template <class TI>
+int softmax_argmax_dev(tiseg_ctx* c, const Geom& g, const TI* d_in, int T, int C, float* d_prob, uint8_t* d_cls) {
     const long long P = g.P;
-    const bool vec = (P % 4 == 0) && aligned16(d_in, d_prob) && (((uintptr_t)d_cls) & 3) == 0;
+    const bool vec = (P % 4 == 0) && aligned_x4<TI>(d_in) && aligned16(d_prob) && (((uintptr_t)d_cls) & 3) == 0;
     dim3 grid(flat4_grid(P), (unsigned)g.N);
     if (T == 1 && !d_prob) {
-        if (C == 2) TISEG_LAUNCH(c, k_argmax_logits2, grid, TISEG_THREADS, 0, (int)P, d_in, d_cls, vec);
-        else if (C <= 2) TISEG_LAUNCH(c, k_argmax_logits<2>, grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
-        else if (C <= 4) TISEG_LAUNCH(c, k_argmax_logits<4>, grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
-        else if (C <= 8) TISEG_LAUNCH(c, k_argmax_logits<8>, grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
-        else TISEG_LAUNCH(c, k_argmax_logits<16>, grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
+        if (C == 2) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_argmax_logits2"), k_argmax_logits2<TI>, grid, TISEG_THREADS, 0, (int)P, d_in, d_cls, vec);
+        else if (C <= 2) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_argmax_logits<2>"), (k_argmax_logits<TI, 2>), grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
+        else if (C <= 4) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_argmax_logits<4>"), (k_argmax_logits<TI, 4>), grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
+        else if (C <= 8) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_argmax_logits<8>"), (k_argmax_logits<TI, 8>), grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
+        else TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_argmax_logits<16>"), (k_argmax_logits<TI, 16>), grid, TISEG_THREADS, 0, P, d_in, C, d_cls, vec);
         return TISEG_OK;
     }
-    if (C <= 4) TISEG_LAUNCH(c, k_softmax_argmax<4>, grid, TISEG_THREADS, 0, P, d_in, T, C, d_prob, d_cls, vec);
-    else if (C <= 8) TISEG_LAUNCH(c, k_softmax_argmax<8>, grid, TISEG_THREADS, 0, P, d_in, T, C, d_prob, d_cls, vec);
-    else TISEG_LAUNCH(c, k_softmax_argmax<16>, grid, TISEG_THREADS, 0, P, d_in, T, C, d_prob, d_cls, vec);
+    if (C <= 4) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_softmax_argmax<4>"), (k_softmax_argmax<TI, 4>), grid, TISEG_THREADS, 0, P, d_in, T, C, d_prob, d_cls, vec);
+    else if (C <= 8) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_softmax_argmax<8>"), (k_softmax_argmax<TI, 8>), grid, TISEG_THREADS, 0, P, d_in, T, C, d_prob, d_cls, vec);
+    else TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_softmax_argmax<16>"), (k_softmax_argmax<TI, 16>), grid, TISEG_THREADS, 0, P, d_in, T, C, d_prob, d_cls, vec);
     return TISEG_OK;
 }
+template int softmax_argmax_dev<float>(tiseg_ctx*, const Geom&, const float*, int, int, float*, uint8_t*);
+template int softmax_argmax_dev<__half>(tiseg_ctx*, const Geom&, const __half*, int, int, float*, uint8_t*);
+template int softmax_argmax_dev<__nv_bfloat16>(tiseg_ctx*, const Geom&, const __nv_bfloat16*, int, int, float*, uint8_t*);
 
 // ---- the step before K1, fused into its load indexing (SURVEY §8f rank 2) ------------------------------------------
 // The reference stitches the half-overlap window outputs of every TTA variant into a canvas (base.py:255-295), undoes
@@ -239,9 +246,9 @@ __device__ __forceinline__ long long window_source(const TtaPlan& p, int C, int 
 
 // SOFTMAX = false: the plain mean of the reverse-transformed variants, what the reference does with its regression heads
 // (`sum(dist_logit_list) / len(dist_logit_list)`, dist.py:398-410; hovernet.py:406 keeps variant 0 only, i.e. T = 1)
-template <int CMAX, bool SOFTMAX>
+template <class TI, int CMAX, bool SOFTMAX>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_softmax_argmax_tta(Geom g, const float* __restrict__ in, TtaPlan plan, int C, float* __restrict__ prob,
+k_softmax_argmax_tta(Geom g, const TI* __restrict__ in, TtaPlan plan, int C, float* __restrict__ prob,
                      uint8_t* __restrict__ cls) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
@@ -250,10 +257,10 @@ k_softmax_argmax_tta(Geom g, const float* __restrict__ in, TtaPlan plan, int C, 
         int sy, sx, Ht, Wt;
         tta_source(plan, t, g.H, g.W, px.y, px.x, sy, sx, Ht, Wt);
         long long cs;
-        const float* src = in + (long long)px.n * plan.tile_stride + plan.off[t] + window_source(plan, C, Ht, Wt, sy, sx, cs);
+        const TI* src = in + (long long)px.n * plan.tile_stride + plan.off[t] + window_source(plan, C, Ht, Wt, sy, sx, cs);
         float xv[CMAX], m = -INFINITY;
 #pragma unroll
-        for (int c = 0; c < CMAX; ++c) if (c < C) { xv[c] = src[c * cs]; m = fmaxf(m, xv[c]); }
+        for (int c = 0; c < CMAX; ++c) if (c < C) { xv[c] = to_f32(src[c * cs]); m = fmaxf(m, xv[c]); }
         if (SOFTMAX) {
             float sum = 0.f;
 #pragma unroll
@@ -301,7 +308,22 @@ extern "C" long long tiseg_tta_input_elems(int T, int C, int H, int W, const int
     return n;
 }
 
-static int tta_entry(tiseg_ctx* c, const float* logits, int N, int T, int C, int H, int W, const int* rotate_degrees,
+template <class TI>
+static int tta_launch(tiseg_ctx* c, const Geom& g, const TI* d_in, const TtaPlan& plan, int C, float* d_prob, uint8_t* d_cls,
+                      bool softmax) {
+    if (softmax) {
+        if (C <= 4) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<4, true>)"), (k_softmax_argmax_tta<TI, 4, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
+        else if (C <= 8) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<8, true>)"), (k_softmax_argmax_tta<TI, 8, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
+        else TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<16, true>)"), (k_softmax_argmax_tta<TI, 16, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
+    } else {
+        if (C <= 4) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<4, false>)"), (k_softmax_argmax_tta<TI, 4, false>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
+        else if (C <= 8) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<8, false>)"), (k_softmax_argmax_tta<TI, 8, false>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
+        else TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<16, false>)"), (k_softmax_argmax_tta<TI, 16, false>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
+    }
+    return TISEG_OK;
+}
+
+static int tta_entry(tiseg_ctx* c, int dtype, const void* logits, int N, int T, int C, int H, int W, const int* rotate_degrees,
                      const int* flips, int window, int overlap, float* prob, uint8_t* cls, bool softmax) {
     if (!c || !logits || !rotate_degrees || !flips || T <= 0 || T > 16 || C <= 0 || C > 16 || (!prob && !cls) ||
         window < 0 || (window > 0 && (overlap < 0 || overlap >= window))) {
@@ -324,36 +346,42 @@ static int tta_entry(tiseg_ctx* c, const float* logits, int N, int T, int C, int
     begin_call(c);
     Geom g = make_geom(N, H, W);
     size_t total = (size_t)N * g.P;
-    const float* d_in = in(c, logits, (size_t)N * (size_t)off);
+    const void* d_in = in_ptr(c, logits, (size_t)N * (size_t)off * dtype_bytes(dtype));
     float* d_prob = prob ? tiseg::out(c, prob, total * C) : nullptr;
     uint8_t* d_cls = cls ? tiseg::out(c, cls, total) : nullptr;
     if (!d_in) return TISEG_ERR_CUDA;
-    if (softmax) {
-        if (C <= 4) TISEG_LAUNCH(c, (k_softmax_argmax_tta<4, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
-        else if (C <= 8) TISEG_LAUNCH(c, (k_softmax_argmax_tta<8, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
-        else TISEG_LAUNCH(c, (k_softmax_argmax_tta<16, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
-    } else {
-        if (C <= 4) TISEG_LAUNCH(c, (k_softmax_argmax_tta<4, false>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
-        else if (C <= 8) TISEG_LAUNCH(c, (k_softmax_argmax_tta<8, false>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
-        else TISEG_LAUNCH(c, (k_softmax_argmax_tta<16, false>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
-    }
+    TISEG_TRY(with_dtype(dtype, [&](auto z) { return tta_launch(c, g, (const decltype(z)*)d_in, plan, C, d_prob, d_cls, softmax); }));
     return end_call(c);
+}
+
+extern "C" int tiseg_softmax_argmax_tta_typed(tiseg_ctx* c, int dtype, const void* logits, int N, int T, int C, int H, int W,
+                                              const int* rotate_degrees, const int* flips, int window, int overlap,
+                                              float* prob, uint8_t* cls) {
+    TISEG_TRY(check_dtype(dtype, "tiseg_softmax_argmax_tta"));
+    return tta_entry(c, dtype, logits, N, T, C, H, W, rotate_degrees, flips, window, overlap, prob, cls, true);
 }
 
 extern "C" int tiseg_softmax_argmax_tta(tiseg_ctx* c, const float* logits, int N, int T, int C, int H, int W,
                                         const int* rotate_degrees, const int* flips, int window, int overlap,
                                         float* prob, uint8_t* cls) {
-    return tta_entry(c, logits, N, T, C, H, W, rotate_degrees, flips, window, overlap, prob, cls, true);
+    return tiseg_softmax_argmax_tta_typed(c, TISEG_DTYPE_F32, logits, N, T, C, H, W, rotate_degrees, flips, window, overlap, prob, cls);
+}
+
+extern "C" int tiseg_tta_mean_typed(tiseg_ctx* c, int dtype, const void* maps, int N, int T, int C, int H, int W,
+                                    const int* rotate_degrees, const int* flips, int window, int overlap, float* mean_out) {
+    TISEG_TRY(check_dtype(dtype, "tiseg_tta_mean"));
+    if (!mean_out) { set_error("tiseg_tta_mean: null output"); return TISEG_ERR_ARG; }
+    return tta_entry(c, dtype, maps, N, T, C, H, W, rotate_degrees, flips, window, overlap, mean_out, nullptr, false);
 }
 
 extern "C" int tiseg_tta_mean(tiseg_ctx* c, const float* maps, int N, int T, int C, int H, int W, const int* rotate_degrees,
                               const int* flips, int window, int overlap, float* mean_out) {
-    if (!mean_out) { set_error("tiseg_tta_mean: null output"); return TISEG_ERR_ARG; }
-    return tta_entry(c, maps, N, T, C, H, W, rotate_degrees, flips, window, overlap, mean_out, nullptr, false);
+    return tiseg_tta_mean_typed(c, TISEG_DTYPE_F32, maps, N, T, C, H, W, rotate_degrees, flips, window, overlap, mean_out);
 }
 
-extern "C" int tiseg_softmax_argmax(tiseg_ctx* c, const float* logits, int N, int T, int C, int H, int W,
-                                    float* prob, uint8_t* cls) {
+extern "C" int tiseg_softmax_argmax_typed(tiseg_ctx* c, int dtype, const void* logits, int N, int T, int C, int H, int W,
+                                          float* prob, uint8_t* cls) {
+    TISEG_TRY(check_dtype(dtype, "tiseg_softmax_argmax"));
     if (!c || !logits || T <= 0 || C <= 0 || C > 16 || (!prob && !cls)) {
         set_error("tiseg_softmax_argmax: bad argument (1 <= C <= 16)");
         return TISEG_ERR_ARG;
@@ -362,10 +390,15 @@ extern "C" int tiseg_softmax_argmax(tiseg_ctx* c, const float* logits, int N, in
     begin_call(c);
     Geom g = make_geom(N, H, W);
     size_t total = (size_t)N * g.P;
-    const float* d_in = in(c, logits, total * T * C);
+    const void* d_in = in_ptr(c, logits, total * T * C * dtype_bytes(dtype));
     float* d_prob = prob ? tiseg::out(c, prob, total * C) : nullptr;
     uint8_t* d_cls = cls ? tiseg::out(c, cls, total) : nullptr;
     if (!d_in) return TISEG_ERR_CUDA;
-    TISEG_TRY(softmax_argmax_dev(c, g, d_in, T, C, d_prob, d_cls));
+    TISEG_TRY(with_dtype(dtype, [&](auto z) { return softmax_argmax_dev(c, g, (const decltype(z)*)d_in, T, C, d_prob, d_cls); }));
     return end_call(c);
+}
+
+extern "C" int tiseg_softmax_argmax(tiseg_ctx* c, const float* logits, int N, int T, int C, int H, int W,
+                                    float* prob, uint8_t* cls) {
+    return tiseg_softmax_argmax_typed(c, TISEG_DTYPE_F32, logits, N, T, C, H, W, prob, cls);
 }

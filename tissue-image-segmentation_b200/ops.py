@@ -7,7 +7,7 @@ kind.  Names follow the scipy / scikit-image calls the reference makes (SURVEY.m
 import numpy as np
 
 from . import _lib
-from ._lib import as_input, batched, empty_like_kind, get_ctx, ptr
+from ._lib import as_input, batched, empty_like_kind, get_ctx, net_inputs, ptr
 from ._lib import is_torch as _lib_is_torch
 
 
@@ -33,16 +33,17 @@ def _inplace_arg(a, dtype, what):
 
 
 def softmax_argmax(logits, want_prob=False):
-    """A1.  logits ``[T, C, H, W]`` / ``[N, T, C, H, W]`` fp32 (T = TTA variants) ->
-    class map uint8 (and the TTA-mean probabilities ``[.., C, H, W]`` when ``want_prob``)."""
-    x = as_input(logits, np.float32)
+    """A1.  logits ``[T, C, H, W]`` / ``[N, T, C, H, W]`` fp32, fp16 or bf16 (T = TTA variants) ->
+    class map uint8 (and the fp32 TTA-mean probabilities ``[.., C, H, W]`` when ``want_prob``).  Half-precision logits
+    are read as they are (2 B per element) and give the outputs of their fp32 upcast, bit for bit."""
+    (x,), dt = net_inputs(logits)
     single = x.ndim == 4
     if single:
         x = x[None]
     N, T, C, H, W = x.shape
     cls = empty_like_kind(x, (N, H, W), np.uint8)
     prob = empty_like_kind(x, (N, C, H, W), np.float32) if want_prob else None
-    get_ctx(_dev(x)).call("tiseg_softmax_argmax", ptr(x), N, T, C, H, W, ptr(prob), ptr(cls))
+    get_ctx(_dev(x)).call("tiseg_softmax_argmax_typed", dt, ptr(x), N, T, C, H, W, ptr(prob), ptr(cls))
     if single:
         cls, prob = cls[0], (prob[0] if want_prob else None)
     return (cls, prob) if want_prob else cls
@@ -151,16 +152,18 @@ def watershed(image, markers, mask=None):
 
 
 def postproc_dist(dist, debug=False, lamb=0):
-    """A8.  dist fp32 -> inst int32 (and, with ``debug``, the marker and raw-flood maps).  ``lamb`` is the first
-    argument of ``dynamic_watershed_alias`` (dist.py:114); the reference's test path passes 0.0 (dist.py:281)."""
-    x, was2d = batched(as_input(dist, np.float32))
+    """A8.  dist fp32, fp16 or bf16 -> inst int32 (and, with ``debug``, the marker and raw-flood maps).  ``lamb`` is the
+    first argument of ``dynamic_watershed_alias`` (dist.py:114); the reference's test path passes 0.0 (dist.py:281).
+    A half-precision map gives the outputs of its fp32 upcast."""
+    (x,), dt = net_inputs(dist)
+    x, was2d = batched(x)
     N, H, W = x.shape
     if int(lamb) != lamb:
         raise ValueError("lamb must be an integer number of grey levels")
     inst = empty_like_kind(x, (N, H, W), np.int32)
     mk = empty_like_kind(x, (N, H, W), np.int32) if debug else None
     ws = empty_like_kind(x, (N, H, W), np.int32) if debug else None
-    get_ctx(_dev(x)).call("tiseg_postproc_dist_lambda", ptr(x), N, H, W, int(lamb), ptr(inst), ptr(mk), ptr(ws))
+    get_ctx(_dev(x)).call("tiseg_postproc_dist_lambda_typed", dt, ptr(x), N, H, W, int(lamb), ptr(inst), ptr(mk), ptr(ws))
     if debug:
         return _unbatch(inst, was2d), _unbatch(mk, was2d), _unbatch(ws, was2d)
     return _unbatch(inst, was2d)
@@ -228,10 +231,9 @@ def ddm(dir_map):
 
 def cdnet_refine(sem_logits, dir_logits, point_logits, if_ddm=True):
     """A12: CDNet.inference tail.  sem_logits [N,T,C,H,W], dir_logits [N,T,9,H,W], point_logits [N,T,1,H,W]
-    (or without the leading N) -> dict(sem_prob [N,C,H,W], cls uint8, dir_map uint8, dd fp32)."""
-    s = as_input(sem_logits, np.float32)
-    d = as_input(dir_logits, np.float32)
-    p = as_input(point_logits, np.float32)
+    (or without the leading N), all fp32 or all fp16 / bf16 (read as they are; the outputs are those of their fp32 upcast)
+    -> dict(sem_prob [N,C,H,W] fp32, cls uint8, dir_map uint8, dd fp32)."""
+    (s, d, p), dt = net_inputs(sem_logits, dir_logits, point_logits)
     single = s.ndim == 4
     if single:
         s, d, p = s[None], d[None], p[None]
@@ -241,7 +243,7 @@ def cdnet_refine(sem_logits, dir_logits, point_logits, if_ddm=True):
     cls = empty_like_kind(s, (N, H, W), np.uint8)
     dm = empty_like_kind(s, (N, H, W), np.uint8)
     dd = empty_like_kind(s, (N, H, W), np.float32)
-    get_ctx(_dev(s)).call("tiseg_cdnet_refine", ptr(s), ptr(d), ptr(p), N, T, C, D, H, W, 1 if if_ddm else 0,
+    get_ctx(_dev(s)).call("tiseg_cdnet_refine_typed", dt, ptr(s), ptr(d), ptr(p), N, T, C, D, H, W, 1 if if_ddm else 0,
                           ptr(prob), ptr(cls), ptr(dm), ptr(dd))
     out = dict(sem_prob=prob, cls=cls, dir_map=dm, dd=dd)
     return {k: v[0] for k, v in out.items()} if single else out
@@ -267,12 +269,9 @@ def ddm_enhance(sem_prob, dd_map, point_map, mode=0):
 def mtcdnet_refine(tc_logits, sem_logits, dir_logits, point_logits, if_ddm=True, want_sem_prob=False):
     """MultiTaskCDNet.inference tail (multi_task_cdnet.py:262-330).  tc_logits [N,T,Ctc,H,W], sem_logits [N,T,Csem,H,W],
     dir_logits [N,T,9,H,W] (or [N,T,1,H,W]: the angle head of use_regression = True), point_logits [N,T,1,H,W] (or without
-    the leading N) ->
-    dict(tc_prob, tc_cls, sem_cls, dir_map, dd[, sem_prob])."""
-    t = as_input(tc_logits, np.float32)
-    s = as_input(sem_logits, np.float32)
-    d = as_input(dir_logits, np.float32)
-    p = as_input(point_logits, np.float32)
+    the leading N), all fp32 or all fp16 / bf16 (read as they are; the outputs are those of their fp32 upcast) ->
+    dict(tc_prob, tc_cls, sem_cls, dir_map, dd[, sem_prob]), probabilities and dd fp32."""
+    (t, s, d, p), dt = net_inputs(tc_logits, sem_logits, dir_logits, point_logits)
     single = t.ndim == 4
     if single:
         t, s, d, p = t[None], s[None], d[None], p[None]
@@ -284,7 +283,7 @@ def mtcdnet_refine(tc_logits, sem_logits, dir_logits, point_logits, if_ddm=True,
     semp = empty_like_kind(t, (N, Csem, H, W), np.float32) if want_sem_prob else None
     dm = empty_like_kind(t, (N, H, W), np.uint8)
     dd = empty_like_kind(t, (N, H, W), np.float32)
-    get_ctx(_dev(t)).call("tiseg_mtcdnet_refine", ptr(t), ptr(s), ptr(d), ptr(p), N, T, Ctc, Csem, D, H, W, 1 if if_ddm else 0,
+    get_ctx(_dev(t)).call("tiseg_mtcdnet_refine_typed", dt, ptr(t), ptr(s), ptr(d), ptr(p), N, T, Ctc, Csem, D, H, W, 1 if if_ddm else 0,
                           ptr(tcp), ptr(tcc), ptr(semp), ptr(semc), ptr(dm), ptr(dd))
     out = dict(tc_prob=tcp, tc_cls=tcc, sem_cls=semc, dir_map=dm, dd=dd)
     if want_sem_prob:
@@ -314,10 +313,11 @@ def postproc_multitask(inner, sem, max_class, edge_id=None, time=20):
 
 
 def postproc_hover(fore_map, hv_map, scale_factor=1, debug=False):
-    """A11: hover_post_proc.  fore_map [N,H,W] fp32, hv_map [N,H,W,2] fp32 -> inst int32 (with ``debug`` also
-    the blb mask, the flooded fp64 image and the markers)."""
-    f, was2d = batched(as_input(fore_map, np.float32))
-    hv = as_input(hv_map, np.float32)
+    """A11: hover_post_proc.  fore_map [N,H,W], hv_map [N,H,W,2], both fp32 or both fp16 / bf16 (read as they are; the
+    outputs are those of their fp32 upcast) -> inst int32 (with ``debug`` also the blb mask, the flooded fp64 image and
+    the markers)."""
+    (f, hv), dt = net_inputs(fore_map, hv_map)
+    f, was2d = batched(f)
     if hv.ndim == 3:
         hv = hv[None]
     N, H, W = f.shape
@@ -328,7 +328,7 @@ def postproc_hover(fore_map, hv_map, scale_factor=1, debug=False):
     blb = empty_like_kind(f, (N, H * sf, W * sf), np.uint8) if debug else None
     dist = empty_like_kind(f, (N, H * sf, W * sf), np.float64) if debug else None
     mk = empty_like_kind(f, (N, H * sf, W * sf), np.int32) if debug else None
-    get_ctx(_dev(f)).call("tiseg_postproc_hover", ptr(f), ptr(hv), N, H, W, int(scale_factor), ptr(inst), ptr(blb),
+    get_ctx(_dev(f)).call("tiseg_postproc_hover_typed", dt, ptr(f), ptr(hv), N, H, W, int(scale_factor), ptr(inst), ptr(blb),
                           ptr(dist), ptr(mk))
     if debug:
         return tuple(_unbatch(x, was2d) for x in (inst, blb, dist, mk))
@@ -376,14 +376,16 @@ def softmax_argmax_tta(variants, rotate_degrees, flip_directions, ori_hw, window
     ``variants``: one array per TTA variant, in the reference's loop order (rotate_degrees outer, flip_directions
     inner; pass the flattened lists), each the raw network output on the TRANSFORMED image: [N, C, Ht, Wt] for whole
     inference (``window = 0``) or [N, M, C, window, window] for split inference.  ``ori_hw`` = (H, W) of the image.
-    Returns the class map [N, H, W] uint8 (and the mean probabilities [N, C, H, W] with ``want_prob``)."""
+    The variants may be fp32, or all fp16 / bf16: they are packed and read in their dtype, and the outputs are those of
+    their fp32 upcast.  Returns the class map [N, H, W] uint8 (and the fp32 mean probabilities [N, C, H, W] with
+    ``want_prob``)."""
     import ctypes
     from . import _lib
     T = len(variants)
     if not (T == len(rotate_degrees) == len(flip_directions)):
         raise ValueError("one rotate_degree and one flip_direction per variant")
     H, W = int(ori_hw[0]), int(ori_hw[1])
-    vs = [as_input(v, np.float32) for v in variants]
+    vs, dt = net_inputs(*variants)
     N = int(vs[0].shape[0])
     C = int(vs[0].shape[1] if window == 0 else vs[0].shape[2])
     rots = (ctypes.c_int * T)(*[int(r) for r in rotate_degrees])
@@ -398,7 +400,7 @@ def softmax_argmax_tta(variants, rotate_degrees, flip_directions, ori_hw, window
         packed = np.ascontiguousarray(np.concatenate([v.reshape(N, -1) for v in vs], axis=1))
     cls = empty_like_kind(packed, (N, H, W), np.uint8)
     prob = empty_like_kind(packed, (N, C, H, W), np.float32) if want_prob else None
-    get_ctx(_dev(packed)).call("tiseg_softmax_argmax_tta", ptr(packed), N, T, C, H, W, rots, flips, int(window),
+    get_ctx(_dev(packed)).call("tiseg_softmax_argmax_tta_typed", dt, ptr(packed), N, T, C, H, W, rots, flips, int(window),
                                int(overlap), ptr(prob), ptr(cls))
     return (cls, prob) if want_prob else cls
 
@@ -406,13 +408,13 @@ def softmax_argmax_tta(variants, rotate_degrees, flip_directions, ori_hw, window
 def tta_mean(variants, rotate_degrees, flip_directions, ori_hw, window=0, overlap=0):
     """Window stitch + TTA reverse + PLAIN mean of a regression head (dist.py:398-410: ``sum(dist_logit_list) /
     len(dist_logit_list)``; hovernet.py:406 keeps ``hv_logit_list[0]``: pass that one variant).  Arguments as
-    ``softmax_argmax_tta``.  -> [N, C, H, W] fp32."""
+    ``softmax_argmax_tta`` (fp32, or all fp16 / bf16).  -> [N, C, H, W] fp32."""
     import ctypes
     T = len(variants)
     if not (T == len(rotate_degrees) == len(flip_directions)):
         raise ValueError("one rotate_degree and one flip_direction per variant")
     H, W = int(ori_hw[0]), int(ori_hw[1])
-    vs = [as_input(v, np.float32) for v in variants]
+    vs, dt = net_inputs(*variants)
     N = int(vs[0].shape[0])
     C = int(vs[0].shape[1] if window == 0 else vs[0].shape[2])
     rots = (ctypes.c_int * T)(*[int(r) for r in rotate_degrees])
@@ -426,7 +428,7 @@ def tta_mean(variants, rotate_degrees, flip_directions, ori_hw, window=0, overla
     else:
         packed = np.ascontiguousarray(np.concatenate([v.reshape(N, -1) for v in vs], axis=1))
     out = empty_like_kind(packed, (N, C, H, W), np.float32)
-    get_ctx(_dev(packed)).call("tiseg_tta_mean", ptr(packed), N, T, C, H, W, rots, flips, int(window), int(overlap), ptr(out))
+    get_ctx(_dev(packed)).call("tiseg_tta_mean_typed", dt, ptr(packed), N, T, C, H, W, rots, flips, int(window), int(overlap), ptr(out))
     return out
 
 
