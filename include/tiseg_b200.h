@@ -172,19 +172,27 @@ int tiseg_postproc_dist_lambda_typed(tiseg_ctx* ctx, int dtype, const void* dist
 int tiseg_reconstruction_erosion_u8(tiseg_ctx* ctx, const uint8_t* seed, const uint8_t* mask, int N, int H, int W,
                                     uint8_t* out);
 
-/* ---- A11: HoVer-Net post-process (hovernet.py:283-365, hover_post_proc; fx = 1) ------------------------------
+/* ---- A11: HoVer-Net post-process (hovernet.py:283-365, hover_post_proc(fore_map, hv_map, fx, scale_factor)) ----
  * fore_map [N,H,W] fp32 (softmax channel 1 of the foreground head), hv_map [N,H,W,2] fp32 HWC (horizontal,
  * vertical) as the reference passes them after permute(0,2,3,1).  scale_factor: 1 (the MoNuSeg / CoNSeP configs)
  * or 2 (the CoNIC config: cv2.resize x2 bilinear in, the whole chain at 2H x 2W, INTER_NEAREST back).
  * inst_out [N,H,W] int32.  Optional debug outputs (NULL to skip), at the SCALED size [N, sH, sW]: blb uint8,
- * dist fp64 (the flooded image), marker int32. */
+ * dist fp64 (the flooded image), marker int32.  This entry runs fx = 1 (Sobel ksize 21, marker obj_size 10). */
 int tiseg_postproc_hover(tiseg_ctx* ctx, const float* fore_map, const float* hv_map, int N, int H, int W,
                          int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out, int32_t* marker_out);
 /* fore_map and hv_map of element type `dtype` (TISEG_DTYPE_*); with scale_factor 2 the resize reads them and the chain
- * after it runs on fp32 as above */
+ * after it runs on fp32 as above.  fx = 1: tiseg_postproc_hover_ex with ksize 21 and obj_size 10. */
 int tiseg_postproc_hover_typed(tiseg_ctx* ctx, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
                                int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
                                int32_t* marker_out);
+/* Any fx of the reference, given as the two integers it derives from fx: ksize = int(20 * fx + 1), the Sobel kernel
+ * size (odd, 1..31: the sizes cv2.Sobel accepts; ksize 1 is the 3-tap derivative without smoothing), and
+ * obj_size = ceil(10 * fx^2), the size below which a marker is dropped (>= 0; 0 and 1 drop none).  The blb mask keeps
+ * its fixed min_size 10, as in the reference.  TISEG_ERR_ARG for an even or out-of-range ksize, a negative obj_size
+ * or a scale_factor other than 1 or 2. */
+int tiseg_postproc_hover_ex(tiseg_ctx* ctx, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
+                            int scale_factor, int ksize, int obj_size, int32_t* inst_out, uint8_t* blb_out,
+                            double* dist_out, int32_t* marker_out);
 
 /* ---- A12: CDNet direction-guided refinement ----------------------------------------------------------------
  * generate_direction_differential_map(dir_map, 9) (tiseg/models/utils/direct_diff_map.py:95-167):

@@ -55,6 +55,7 @@ SIGNATURES = {
     "tiseg_reconstruction_erosion_u8": [_vp, _vp, _vp, _i, _i, _i, _vp],
     "tiseg_postproc_hover": [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_postproc_hover_typed": [_vp, _i, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
+    "tiseg_postproc_hover_ex": [_vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_ddm": [_vp, _vp, _i, _i, _i, _vp],
     "tiseg_cdnet_refine": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_cdnet_refine_typed": [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],

@@ -1,14 +1,15 @@
-// K8 — HoVer-Net post-process (tiseg/models/segmentors/hovernet.py:283-365, hover_post_proc with fx = 1,
-// scale_factor = 1).
+// K8 — HoVer-Net post-process (tiseg/models/segmentors/hovernet.py:283-365, hover_post_proc(fore_map, hv_map, fx,
+// scale_factor)).  fx enters as two integers: the Sobel ksize = int(20 * fx + 1), odd in 1..31 (21 at fx = 1), and the
+// marker obj_size = ceil(10 * fx^2) (10 at fx = 1); scale_factor is 1 or 2.
 //
-// The float chain (cv2.normalize -> cv2.Sobel ksize 21 CV_64F -> cv2.normalize -> max -> thresholds ->
+// The float chain (cv2.normalize -> cv2.Sobel ksize k CV_64F -> cv2.normalize -> max -> thresholds ->
 // cv2.GaussianBlur 3x3) feeds two thresholds (>= 0.5, >= 0.4) and a watershed on the blurred map, so a 1-ulp
 // difference can flip an integer output.  The kernels therefore reproduce OpenCV's arithmetic ORDER, not just
 // its formulas (SURVEY.md Appendix A.2, re-derived in tests/cv_recipes.py and checked against cv2 bit for bit):
 //   normalize (-> CV_32F): a = (float)(1/(max-min)); b = 0.f - (float)(min * a); dst = (float)fma(x, a, b) in fp64
-//   Sobel 21: integer binomial kernels; row pass = sequential taps in fp64; column pass = centre tap, then
-//             k[10+t] * (R[+t] +/- R[-t]), t = 1..10, multiply and add rounded separately (no FMA);
-//             BORDER_REFLECT_101
+//   Sobel k:  integer kernels of cv2.getDerivKernels; row pass = sequential taps in fp64; column pass = centre tap,
+//             then k[r+t] * (R[+t] +/- R[-t]), t = 1..r, multiply and add rounded separately (no FMA);
+//             BORDER_REFLECT_101, reflected again while outside (images smaller than the radius r)
 //   GaussianBlur 3x3 on fp64: row pass (a/4 + b/2) + c/4, column pass b/2 + (a + c)/4
 // (--fmad=false for the whole library; fma() is written out where OpenCV contracts.)
 // The foreground and HV maps may be fp32, fp16 or bf16 (TI): the kernels that read them convert at the load, so the chain
@@ -21,10 +22,30 @@
 
 namespace tiseg {
 
-__constant__ double c_smooth21[21] = {1, 20, 190, 1140, 4845, 15504, 38760, 77520, 125970, 167960, 184756,
-                                      167960, 125970, 77520, 38760, 15504, 4845, 1140, 190, 20, 1};
-__constant__ double c_deriv21[21] = {-1, -18, -152, -798, -2907, -7752, -15504, -23256, -25194, -16796, 0,
-                                     16796, 25194, 23256, 15504, 7752, 2907, 798, 152, 18, 1};
+// cv2.getDerivKernels, indexed by tap radius r: smoothing = binomial row 2r; derivative (r >= 1) = binomial row 2r-1
+// convolved with [-1, 1].  ksize k uses radius k / 2 for both passes, except ksize 1: derivative [-1, 0, 1] (radius 1),
+// smoothing [1] (radius 0).  The largest coefficient, C(30, 15), is below 2^28, so every row product of an fp32 source
+// is exact in fp64.
+constexpr int SOBEL_RMAX = 15;                                  // ksize 31, the largest cv2.Sobel accepts
+struct SobelTaps {
+    double smooth[SOBEL_RMAX + 1][2 * SOBEL_RMAX + 1];
+    double deriv[SOBEL_RMAX + 1][2 * SOBEL_RMAX + 1];
+};
+constexpr SobelTaps make_sobel_taps() {
+    SobelTaps k{};
+    for (int r = 0; r <= SOBEL_RMAX; ++r) {
+        long long b[2 * SOBEL_RMAX + 1] = {1};                 // binomial row, built up to 2r
+        for (int n = 1; n <= 2 * r; ++n) {
+            if (n == 2 * r) {
+                for (int i = 0; i <= 2 * r; ++i) k.deriv[r][i] = (double)((i > 0 ? b[i - 1] : 0) - (i < n ? b[i] : 0));
+            }
+            for (int i = n; i > 0; --i) b[i] += b[i - 1];
+        }
+        for (int i = 0; i <= 2 * r; ++i) k.smooth[r][i] = (double)b[i];
+    }
+    return k;
+}
+__constant__ SobelTaps c_sobel = make_sobel_taps();
 
 __device__ __forceinline__ long long dkey(double d) {       // monotone double -> int64 (for atomicMax / atomicMin)
     long long b = __double_as_longlong(d);
@@ -101,41 +122,45 @@ __device__ __forceinline__ int reflect101(int i, int n) {
     return i;
 }
 
-// row pass: fp32 source -> fp64, 21 sequential taps along x.  One thread = four adjacent outputs: the 24 source values
-// they share are read once (reflected only at the image sides); every output keeps OpenCV's tap order.
-template <bool DERIV>
+// row pass: fp32 source -> fp64, 2R+1 sequential taps along x.  One thread = four adjacent outputs: the 2R+4 source
+// values they share are read once (reflected only at the image sides); every output keeps OpenCV's tap order.
+template <bool DERIV, int R>
 __global__ void __launch_bounds__(TISEG_THREADS)
 k_sobel_row(Geom g, const float* __restrict__ src, double* __restrict__ out) {
+    constexpr int NV = 2 * R + 4;
     const int W4 = (g.W + 3) >> 2;
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= (long long)W4 * g.H) return;
     const int y = (int)(t / W4), x = (int)(t - (long long)y * W4) * 4, n = blockIdx.y;
     const float* row = src + (long long)n * g.P + (long long)y * g.W;
     double* orow = out + (long long)n * g.P + (long long)y * g.W;
-    const double* k = DERIV ? c_deriv21 : c_smooth21;
-    double v[24];
-    if (x >= 10 && x + 13 < g.W) {
+    const double* k = DERIV ? c_sobel.deriv[R] : c_sobel.smooth[R];
+    double v[NV];
+    if (x >= R && x + 3 + R < g.W) {
 #pragma unroll
-        for (int j = 0; j < 24; ++j) v[j] = (double)row[x - 10 + j];
+        for (int j = 0; j < NV; ++j) v[j] = (double)row[x - R + j];
     } else {
 #pragma unroll
-        for (int j = 0; j < 24; ++j) v[j] = (double)row[reflect101(x - 10 + j, g.W)];
+        for (int j = 0; j < NV; ++j) v[j] = (double)row[reflect101(x - R + j, g.W)];
     }
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
         if (x + q >= g.W) break;
         double s = k[0] * v[q];
 #pragma unroll
-        for (int tt = 1; tt < 21; ++tt) s = s + k[tt] * v[q + tt];
+        for (int tt = 1; tt <= 2 * R; ++tt) s = s + k[tt] * v[q + tt];
         orow[x + q] = s;
     }
 }
 
 // column pass (symmetric pairing, separate multiply and add) + min / max of the result.  One thread = four
-// vertically adjacent outputs of one column (24 row values read once, each read coalesced over the warp).
-template <bool DERIV>
-__global__ void __launch_bounds__(TISEG_THREADS)
+// vertically adjacent outputs of one column (2R+4 row values read once, each read coalesced over the warp).
+// The bound of one block per SM lets ptxas give the pass the registers it needs: with the plain bound it stopped at an
+// occupancy step (48, 64 or 80 registers) and spilled 8-32 bytes at radii 4 and 7-11.
+template <bool DERIV, int R>
+__global__ void __launch_bounds__(TISEG_THREADS, 1)
 k_sobel_col(Geom g, const double* __restrict__ rowbuf, double* __restrict__ out, long long* mm /* [N, 2] */) {
+    constexpr int NV = 2 * R + 4;
     const int H4 = (g.H + 3) >> 2;
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const bool live = t < (long long)H4 * g.W;
@@ -144,23 +169,23 @@ k_sobel_col(Geom g, const double* __restrict__ rowbuf, double* __restrict__ out,
     if (live) {
         const int y = (int)(t / g.W) * 4, x = (int)(t - (long long)(y >> 2) * g.W);
         const double* col = rowbuf + (long long)n * g.P + x;
-        const double* k = DERIV ? c_deriv21 : c_smooth21;
-        double v[24];
-        if (y >= 10 && y + 13 < g.H) {
+        const double* k = DERIV ? c_sobel.deriv[R] : c_sobel.smooth[R];
+        double v[NV];
+        if (y >= R && y + 3 + R < g.H) {
 #pragma unroll
-            for (int j = 0; j < 24; ++j) v[j] = col[(long long)(y - 10 + j) * g.W];
+            for (int j = 0; j < NV; ++j) v[j] = col[(long long)(y - R + j) * g.W];
         } else {
 #pragma unroll
-            for (int j = 0; j < 24; ++j) v[j] = col[(long long)reflect101(y - 10 + j, g.H) * g.W];
+            for (int j = 0; j < NV; ++j) v[j] = col[(long long)reflect101(y - R + j, g.H) * g.W];
         }
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             if (y + q >= g.H) break;
-            double acc = DERIV ? 0.0 : __dmul_rn(k[10], v[q + 10]);
+            double acc = DERIV ? 0.0 : __dmul_rn(k[R], v[q + R]);
 #pragma unroll
-            for (int d = 1; d <= 10; ++d) {
-                const double pair = DERIV ? __dsub_rn(v[q + 10 + d], v[q + 10 - d]) : __dadd_rn(v[q + 10 + d], v[q + 10 - d]);
-                acc = __dadd_rn(acc, __dmul_rn(k[10 + d], pair));
+            for (int d = 1; d <= R; ++d) {
+                const double pair = DERIV ? __dsub_rn(v[q + R + d], v[q + R - d]) : __dadd_rn(v[q + R + d], v[q + R - d]);
+                acc = __dadd_rn(acc, __dmul_rn(k[R + d], pair));
             }
             out[(long long)n * g.P + (long long)(y + q) * g.W + x] = acc;
             lo = q == 0 ? acc : fmin(lo, acc);
@@ -168,6 +193,36 @@ k_sobel_col(Geom g, const double* __restrict__ rowbuf, double* __restrict__ out,
         }
     }
     warp_minmax_commit(lo, hi, live, mm + (long long)n * 2);
+}
+
+// Host dispatch of one pass on its tap radius r: a chain of instantiations from the smallest radius (1 for a derivative
+// pass, 0 for a smoothing pass) to SOBEL_RMAX.  Timing names "k_sobel_row<DERIV, R>" / "k_sobel_col<DERIV, R>".
+inline std::string sobel_name(const char* pass, bool deriv, int r) {
+    return std::string(pass) + (deriv ? "<true, " : "<false, ") + std::to_string(r) + ">";
+}
+inline int sobel_bad_radius(int r) {
+    set_error("hover Sobel: no kernel of tap radius " + std::to_string(r));
+    return TISEG_ERR_ARG;
+}
+template <bool DERIV, int R = (DERIV ? 1 : 0)>
+int sobel_row(tiseg_ctx* c, int r, const Geom& g, dim3 grid, const float* src, double* out) {
+    if (r != R) {
+        if constexpr (R < SOBEL_RMAX) return sobel_row<DERIV, R + 1>(c, r, g, grid, src, out);
+        else return sobel_bad_radius(r);
+    }
+    static const std::string name = sobel_name("k_sobel_row", DERIV, R);
+    TISEG_LAUNCH_AS(c, name.c_str(), (k_sobel_row<DERIV, R>), grid, TISEG_THREADS, 0, g, src, out);
+    return TISEG_OK;
+}
+template <bool DERIV, int R = (DERIV ? 1 : 0)>
+int sobel_col(tiseg_ctx* c, int r, const Geom& g, dim3 grid, const double* rowbuf, double* out, long long* mm) {
+    if (r != R) {
+        if constexpr (R < SOBEL_RMAX) return sobel_col<DERIV, R + 1>(c, r, g, grid, rowbuf, out, mm);
+        else return sobel_bad_radius(r);
+    }
+    static const std::string name = sobel_name("k_sobel_col", DERIV, R);
+    TISEG_LAUNCH_AS(c, name.c_str(), (k_sobel_col<DERIV, R>), grid, TISEG_THREADS, 0, g, rowbuf, out, mm);
+    return TISEG_OK;
 }
 
 template <class TI>
@@ -271,9 +326,9 @@ k_ellipse5(Geom g, const uint8_t* __restrict__ src, uint8_t* __restrict__ out, b
     }
 }
 
-// fore [N,H,W] and hv [N,H,W,2] of element type TI
+// fore [N,H,W] and hv [N,H,W,2] of element type TI; ksize odd in 1..31
 template <class TI>
-int postproc_hover_dev(tiseg_ctx* c, const Geom& g, const TI* fore, const TI* hv, int obj_size, int32_t* inst,
+int postproc_hover_dev(tiseg_ctx* c, const Geom& g, const TI* fore, const TI* hv, int ksize, int obj_size, int32_t* inst,
                        uint8_t* blb_out, double* dist_out, int32_t* marker_out) {
     int N = g.N;
     size_t total = (size_t)N * g.P;
@@ -302,13 +357,15 @@ int postproc_hover_dev(tiseg_ctx* c, const Geom& g, const TI* fore, const TI* hv
     TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_hv_minmax"), k_hv_minmax<TI>, dim3((unsigned)((g.P + 8 * TISEG_THREADS - 1) / (8 * TISEG_THREADS)), (unsigned)N),
                     TISEG_THREADS, 0, g, hv2, mm_hv);
     TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_hv_normalize"), k_hv_normalize<TI>, warp_grid(g), TISEG_THREADS, 0, g, hv2, mm_hv, hdir, vdir);
-    // Sobel(h_dir, dx=1): derivative along x, smoothing along y;  Sobel(v_dir, dy=1): the transpose
+    // Sobel(h_dir, dx=1): derivative along x, smoothing along y;  Sobel(v_dir, dy=1): the transpose.  Tap radii of
+    // the two kernels of cv2.getDerivKernels(ksize): ksize / 2, except ksize 1 = derivative [-1, 0, 1] and smoothing [1].
+    const int rd = ksize == 1 ? 1 : ksize / 2, rs = ksize / 2;
     const dim3 rg((unsigned)(((long long)((g.W + 3) / 4) * g.H + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N);
     const dim3 cg((unsigned)(((long long)((g.H + 3) / 4) * g.W + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N);
-    TISEG_LAUNCH(c, k_sobel_row<true>, rg, TISEG_THREADS, 0, g, hdir, rowb);
-    TISEG_LAUNCH(c, k_sobel_col<false>, cg, TISEG_THREADS, 0, g, rowb, sobh, mm_sh);
-    TISEG_LAUNCH(c, k_sobel_row<false>, rg, TISEG_THREADS, 0, g, vdir, rowb);
-    TISEG_LAUNCH(c, k_sobel_col<true>, cg, TISEG_THREADS, 0, g, rowb, sobv, mm_sv);
+    TISEG_TRY(sobel_row<true>(c, rd, g, rg, hdir, rowb));
+    TISEG_TRY(sobel_col<false>(c, rs, g, cg, rowb, sobh, mm_sh));
+    TISEG_TRY(sobel_row<false>(c, rs, g, rg, vdir, rowb));
+    TISEG_TRY(sobel_col<true>(c, rd, g, cg, rowb, sobv, mm_sv));
     // energy, thresholds, blurred distance
     TISEG_LAUNCH(c, k_hover_energy, warp_grid(g), TISEG_THREADS, 0, g, sobh, sobv, mm_sh, mm_sv, blb, dpre, mk0);
     TISEG_LAUNCH(c, k_gauss3_row, warp_grid(g), TISEG_THREADS, 0, g, dpre, rowb);
@@ -378,10 +435,11 @@ using namespace tiseg;
 
 template <class TI>
 static int postproc_hover_entry(tiseg_ctx* c, const void* fore_map, const void* hv_map, const Geom& g, const Geom& gs,
-                                int scale_factor, int32_t* d_inst, uint8_t* d_blb, double* d_dist, int32_t* d_mk) {
+                                int scale_factor, int ksize, int obj_size, int32_t* d_inst, uint8_t* d_blb, double* d_dist,
+                                int32_t* d_mk) {
     const TI* d_fore = (const TI*)fore_map;
     const TI* d_hv = (const TI*)hv_map;
-    if (scale_factor == 1) return postproc_hover_dev(c, g, d_fore, d_hv, 10, d_inst, d_blb, d_dist, d_mk);
+    if (scale_factor == 1) return postproc_hover_dev(c, g, d_fore, d_hv, ksize, obj_size, d_inst, d_blb, d_dist, d_mk);
     const size_t stotal = (size_t)gs.N * gs.P;
     float* fore2 = ws<float>(c, stotal);
     float* hv2 = ws<float>(c, stotal * 2);
@@ -391,18 +449,27 @@ static int postproc_hover_entry(tiseg_ctx* c, const void* fore_map, const void* 
     if (H >= 2 && W >= 2) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_resize_up2<1, true>)"), (k_resize_up2<TI, 1, true>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_fore, fore2);
     else                  TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_resize_up2<1, false>)"), (k_resize_up2<TI, 1, false>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_fore, fore2);
     TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_resize_up2<2, false>)"), (k_resize_up2<TI, 2, false>), warp_grid(gs), TISEG_THREADS, 0, gs, H, W, d_hv, hv2);
-    TISEG_TRY(postproc_hover_dev(c, gs, (const float*)fore2, (const float*)hv2, 10, inst2, d_blb, d_dist, d_mk));
+    TISEG_TRY(postproc_hover_dev(c, gs, (const float*)fore2, (const float*)hv2, ksize, obj_size, inst2, d_blb, d_dist, d_mk));
     TISEG_LAUNCH(c, k_resize_down2_nearest, warp_grid(g), TISEG_THREADS, 0, g, inst2, d_inst);
     return TISEG_OK;
 }
 
-extern "C" int tiseg_postproc_hover_typed(tiseg_ctx* c, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
-                                          int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
-                                          int32_t* marker_out) {
+extern "C" int tiseg_postproc_hover_ex(tiseg_ctx* c, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
+                                       int scale_factor, int ksize, int obj_size, int32_t* inst_out, uint8_t* blb_out,
+                                       double* dist_out, int32_t* marker_out) {
     TISEG_TRY(check_dtype(dtype, "tiseg_postproc_hover"));
     if (!c || !fore_map || !hv_map || !inst_out) { set_error("tiseg_postproc_hover: bad argument"); return TISEG_ERR_ARG; }
     if (scale_factor != 1 && scale_factor != 2) {
-        set_error("tiseg_postproc_hover: scale_factor must be 1 or 2 (the values of the reference configs)");
+        set_error("tiseg_postproc_hover: scale_factor must be 1 or 2 (the values of the reference configs), got " +
+                  std::to_string(scale_factor));
+        return TISEG_ERR_ARG;
+    }
+    if (ksize < 1 || ksize > 2 * SOBEL_RMAX + 1 || ksize % 2 == 0) {       // what cv2.Sobel refuses (and -1, Scharr)
+        set_error("tiseg_postproc_hover: ksize must be odd and in 1..31 (cv2.Sobel), got " + std::to_string(ksize));
+        return TISEG_ERR_ARG;
+    }
+    if (obj_size < 0) {
+        set_error("tiseg_postproc_hover: obj_size must be >= 0, got " + std::to_string(obj_size));
         return TISEG_ERR_ARG;
     }
     TISEG_TRY(check_geom(N, H * scale_factor, W * scale_factor));
@@ -418,9 +485,18 @@ extern "C" int tiseg_postproc_hover_typed(tiseg_ctx* c, int dtype, const void* f
     int32_t* d_mk = marker_out ? tiseg::out(c, marker_out, stotal) : nullptr;
     if (!d_fore || !d_hv || !d_inst) return TISEG_ERR_CUDA;
     TISEG_TRY(with_dtype(dtype, [&](auto z) {
-        return postproc_hover_entry<decltype(z)>(c, d_fore, d_hv, g, gs, scale_factor, d_inst, d_blb, d_dist, d_mk);
+        return postproc_hover_entry<decltype(z)>(c, d_fore, d_hv, g, gs, scale_factor, ksize, obj_size, d_inst, d_blb, d_dist,
+                                                 d_mk);
     }));
     return end_call(c);
+}
+
+// fx = 1 of the reference: ksize 21, obj_size 10
+extern "C" int tiseg_postproc_hover_typed(tiseg_ctx* c, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
+                                          int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
+                                          int32_t* marker_out) {
+    return tiseg_postproc_hover_ex(c, dtype, fore_map, hv_map, N, H, W, scale_factor, 21, 10, inst_out, blb_out, dist_out,
+                                   marker_out);
 }
 
 extern "C" int tiseg_postproc_hover(tiseg_ctx* c, const float* fore_map, const float* hv_map, int N, int H, int W,

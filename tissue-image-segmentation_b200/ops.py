@@ -4,6 +4,8 @@ Every function takes numpy arrays (host buffers; the library stages them) or CUD
 (zero-copy, stream-ordered) shaped ``[H, W]`` or batched ``[N, H, W]`` and returns arrays of the same
 kind.  Names follow the scipy / scikit-image calls the reference makes (SURVEY.md §8a).
 """
+import math
+
 import numpy as np
 
 from . import _lib
@@ -312,10 +314,14 @@ def postproc_multitask(inner, sem, max_class, edge_id=None, time=20):
     return _unbatch(canvas, was2d), _unbatch(inst, was2d)
 
 
-def postproc_hover(fore_map, hv_map, scale_factor=1, debug=False):
+def postproc_hover(fore_map, hv_map, scale_factor=1, debug=False, fx=1):
     """A11: hover_post_proc.  fore_map [N,H,W], hv_map [N,H,W,2], both fp32 or both fp16 / bf16 (read as they are; the
     outputs are those of their fp32 upcast) -> inst int32 (with ``debug`` also the blb mask, the flooded fp64 image and
-    the markers)."""
+    the markers).  ``fx`` sets the Sobel kernel size and the marker size threshold with the reference's expressions
+    (hovernet.py:283-365): ``fx = 0.5`` runs the chain on 20x data at its native size.  An fx whose ksize cv2.Sobel
+    refuses (even, or above 31: fx 0.05, 0.25, 0.75, >= 1.6, ...) raises TisegError, as the reference raises cv2.error."""
+    # clamped to int32, so that an absurd fx reaches the library's range check instead of wrapping in ctypes
+    ksize, obj_size = [max(-2 ** 31, min(v, 2 ** 31 - 1)) for v in (int((20 * fx) + 1), math.ceil(10 * (fx ** 2)))]
     (f, hv), dt = net_inputs(fore_map, hv_map)
     f, was2d = batched(f)
     if hv.ndim == 3:
@@ -328,8 +334,8 @@ def postproc_hover(fore_map, hv_map, scale_factor=1, debug=False):
     blb = empty_like_kind(f, (N, H * sf, W * sf), np.uint8) if debug else None
     dist = empty_like_kind(f, (N, H * sf, W * sf), np.float64) if debug else None
     mk = empty_like_kind(f, (N, H * sf, W * sf), np.int32) if debug else None
-    get_ctx(_dev(f)).call("tiseg_postproc_hover_typed", dt, ptr(f), ptr(hv), N, H, W, int(scale_factor), ptr(inst), ptr(blb),
-                          ptr(dist), ptr(mk))
+    get_ctx(_dev(f)).call("tiseg_postproc_hover_ex", dt, ptr(f), ptr(hv), N, H, W, int(scale_factor), ksize, obj_size, ptr(inst),
+                          ptr(blb), ptr(dist), ptr(mk))
     if debug:
         return tuple(_unbatch(x, was2d) for x in (inst, blb, dist, mk))
     return _unbatch(inst, was2d)

@@ -186,9 +186,7 @@ class HoverNet:
         self.test_cfg = dict(test_cfg or {})
 
     def hover_post_proc(self, fore_map, hv_map, fx=1, scale_factor=1):
-        if fx != 1:
-            raise NotImplementedError("hover_post_proc: only fx = 1 (ksize 21) is implemented")
-        return ops.postproc_hover(fore_map, hv_map, scale_factor=scale_factor)
+        return ops.postproc_hover(fore_map, hv_map, scale_factor=scale_factor, fx=fx)
 
     def inference_tail(self, sem_variants, hv_variants, fore_variants, ori_hw, window=0, overlap=0):
         """hovernet.py:367-414 after the CNN -> (sem class map [N,H,W], hv map [N,H,W,2] of variant 0 — the reference
