@@ -1,5 +1,5 @@
 """Per-kernel CUDA-event times of the DIST step on the bench batch (plain launches), plus the wall time of the step.
-    python scripts/step_times.py [batch]      env: whatever switches the library reads (TISEG_PAIR_LEGACY, ...)"""
+    python scripts/step_times.py [batch]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch

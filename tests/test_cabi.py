@@ -89,3 +89,16 @@ def test_reference_signatures():
     assert [k for k in inspect.signature(S.MultiTaskCDNet.__init__).parameters][1:] == ["num_classes", "num_angles", "test_cfg", "if_ddm",
                                                                                        "use_regression"]
 
+
+
+def test_library_reads_no_environment():
+    """The CUDA library's results and launches depend on its arguments alone: no source under csrc/ reads an environment
+    variable, so nothing set in a user's shell or a job profile can switch a stage to another implementation."""
+    csrc = os.path.join(ROOT, "tissue-image-segmentation_b200", "csrc")
+    found = []
+    for dirpath, _, files in os.walk(csrc):
+        for f in files:
+            path = os.path.join(dirpath, f)
+            with open(path, encoding="utf-8", errors="replace") as fh:
+                found += ["%s:%d" % (os.path.relpath(path, ROOT), i + 1) for i, line in enumerate(fh) if "getenv" in line]
+    assert not found, "environment reads in the library: " + ", ".join(found)

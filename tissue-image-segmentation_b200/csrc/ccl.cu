@@ -1,7 +1,5 @@
 // K3 — connected-component labelling entry points (tiseg_label*, tiseg_re_instance) and the
 // non-template parts of the CCL toolbox declared in ccl.cuh.
-#include <cstdlib>
-
 #include <cooperative_groups.h>
 #include "ccl.cuh"
 
@@ -53,94 +51,6 @@ __global__ void __launch_bounds__(TISEG_THREADS) k_ccl_flatten(Geom g, int* par,
     }
 }
 
-// selected pixels per row: one warp per row sums the popcounts of the row's words (one coalesced request per 32 segments)
-template <bool LISTED>
-__global__ void __launch_bounds__(TISEG_THREADS)
-k_rank_rowtot(Geom g, const unsigned* __restrict__ bits, int* __restrict__ rowpre) {
-    const int y = blockIdx.x * TISEG_WARPS_PER_BLOCK + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (y >= g.H) return;
-    FOR_TILES(LISTED, g, n) {
-        const unsigned* b = bits + ((long long)n * g.H + y) * g.SEG;
-        int v = 0;
-        for (int k = lane; k < g.SEG; k += 32) v += __popc(b[k]);
-#pragma unroll
-        for (int d = 16; d; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
-        if (lane == 0) rowpre[(long long)n * g.H + y] = v;
-    }
-}
-
-// one block per tile: exclusive scan of the row totals in place.
-// rowpre[n, y] = selected pixels in the rows above y; counts[n] = total.
-template <bool LISTED>
-__global__ void __launch_bounds__(1024) k_rank_rowscan(Geom g, int* __restrict__ rowpre, int* counts) {
-    __shared__ int wsum[32];
-    __shared__ int carry;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    FOR_TILES_OF(LISTED, g, (int)blockIdx.x, n) {
-    int* rp = rowpre + (long long)n * g.H;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (int base = 0; base < g.H; base += 1024) {
-        const int y = base + threadIdx.x;
-        const int v = y < g.H ? rp[y] : 0;
-        int incl = v;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            int t = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= d) incl += t;
-        }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        if (warp == 0) {
-            int w = wsum[lane], wi = w;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                int t = __shfl_up_sync(0xffffffffu, wi, d);
-                if (lane >= d) wi += t;
-            }
-            wsum[lane] = wi - w;                       // exclusive prefix of the warp totals
-        }
-        __syncthreads();
-        const int c0 = carry;
-        if (y < g.H) rp[y] = c0 + wsum[warp] + incl - v;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry = c0 + wsum[31] + incl;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0 && counts) counts[n] = carry;
-    __syncthreads();
-    }
-}
-
-// one warp per row, lane = row segment: warp scan of the popcounts, then one store per selected pixel
-template <bool LISTED>
-__global__ void __launch_bounds__(TISEG_THREADS)
-k_rank_place_bits(Geom g, const unsigned* __restrict__ bits, const int* __restrict__ rowpre, int* __restrict__ rank) {
-    const int y = blockIdx.x * TISEG_WARPS_PER_BLOCK + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (y >= g.H) return;
-    FOR_TILES(LISTED, g, n) {
-    int run = rowpre[(long long)n * g.H + y];
-    int* out = rank + (long long)n * g.P + (long long)y * g.W;
-    for (int c0 = 0; c0 < g.SEG; c0 += 32) {
-        const int seg = c0 + lane;
-        unsigned m = seg < g.SEG ? bits[((long long)n * g.H + y) * g.SEG + seg] : 0u;
-        int incl = __popc(m);
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            int t = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= d) incl += t;
-        }
-        int k = run + incl - __popc(m);
-        while (m) {
-            const int bit = __ffs(m) - 1;
-            m &= m - 1;
-            out[seg * 32 + bit] = ++k;
-        }
-        run += __shfl_sync(0xffffffffu, incl, 31);
-    }
-    }
-}
-
 // out = par >= 0 ? rank[par] : 0, four pixels per thread
 template <bool LISTED>
 __global__ void __launch_bounds__(TISEG_THREADS)
@@ -178,11 +88,12 @@ int ccl_flatten(tiseg_ctx* c, const Geom& g, int* par) {
     return TISEG_OK;
 }
 
-// The three passes above in ONE launch.  A tile belongs to a thread-block CLUSTER of RF_CTAS 1024-thread CTAs (a tile
-// per CTA left 84 of the 148 SMs idle on a 64-tile batch): every CTA ranks a quarter of the rows — row totals (one warp
-// per row, four rows of loads in flight), block scan over its rows, placement — and the CTAs exchange their totals
-// through distributed shared memory: the ranks of CTA r start after the set bits of CTAs 0 .. r-1.  The bitmap of a
-// tile is P / 8 bytes (125 KB at 1000^2): the second read comes from L1 / L2.
+// rank[n, pixel] = 1-based raster rank of each set bit of bits[n] (written at the set bits only); counts[n] = set bits
+// (may be null).  A tile belongs to a thread-block CLUSTER of RF_CTAS 1024-thread CTAs (a tile per CTA left 84 of the 148
+// SMs idle on a 64-tile batch): every CTA ranks a quarter of the rows — row totals (one warp per row, four rows of loads
+// in flight), block scan over its rows, placement (one warp per row: warp scan over the row's words, one store per set
+// bit) — and the CTAs exchange their totals through distributed shared memory: the ranks of CTA r start after the set
+// bits of CTAs 0 .. r-1.  The bitmap of a tile is P / 8 bytes (125 KB at 1000^2): the second read comes from L1 / L2.
 #define RF_ROWS 4096                    // rows scanned per round (4 per thread)
 #define RF_CTAS 4
 template <bool LISTED>
@@ -301,18 +212,7 @@ k_rank_fused(Geom g, const unsigned* __restrict__ bits, int* __restrict__ rank, 
 }
 
 int rank_from_bits(tiseg_ctx* c, const Geom& g, const unsigned* bits, int* rank, int* counts) {
-    static const bool split = getenv("TISEG_RANK_SPLIT") != nullptr;       // the three-launch form, for comparison
-    if (!split) {
-        TISEG_LAUNCH_TILES(c, k_rank_fused, g, grid_tiles(g) * RF_CTAS, 1024, 0, g, bits, rank, counts);
-        return TISEG_OK;
-    }
-    int* rowpre = ws<int>(c, (size_t)g.N * g.H);
-    if (!rowpre) return TISEG_ERR_CUDA;
-    TISEG_LAUNCH_TILES(c, k_rank_rowtot, g, dim3((g.H + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK, grid_tiles(g)), TISEG_THREADS, 0,
-                       g, bits, rowpre);
-    TISEG_LAUNCH_TILES(c, k_rank_rowscan, g, grid_tiles(g), 1024, 0, g, rowpre, counts);
-    TISEG_LAUNCH_TILES(c, k_rank_place_bits, g, dim3((g.H + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK, grid_tiles(g)), TISEG_THREADS, 0,
-                 g, bits, rowpre, rank);
+    TISEG_LAUNCH_TILES(c, k_rank_fused, g, grid_tiles(g) * RF_CTAS, 1024, 0, g, bits, rank, counts);
     return TISEG_OK;
 }
 

@@ -328,8 +328,8 @@ int ccl_build(tiseg_ctx* c, const Geom& g, Img img, int conn, int* par) {
 // rank[gi] = 1-based raster rank among the selected pixels of its tile (written only where selected);
 // counts[n] = number selected (may be null).
 // The selection is first reduced to a BITMAP, one 32-bit ballot word per row segment (bits[n, y, seg]); ranking then
-// touches P/32 words instead of P pixels: k_rank_rowscan (one CTA per tile: popcount per row, exclusive scan over
-// the rows) and k_rank_place_bits (one warp per row: warp scan over the row's words, one store per selected pixel).
+// touches P/32 words instead of P pixels: k_rank_fused (one cluster of CTAs per tile: popcount per row, exclusive scan
+// over the rows, then one warp per row: warp scan over the row's words, one store per selected pixel).
 struct SelRoot {                // roots of a flattened forest
     const int* par;
     __device__ __forceinline__ bool operator()(long long gi, int idx) const { return par[gi] == idx; }

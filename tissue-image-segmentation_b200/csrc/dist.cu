@@ -19,6 +19,7 @@ namespace tiseg {
 // row, all loads of the thread issued before the first is used.  The distance map may be fp32, fp16 or bf16 (TI); it is
 // converted to fp32 as it is loaded.
 #define DP_ROWS 4
+#define PB_ROWS_PER_WARP 32     // rows per warp band of k_plateau_bits (a multiple of 4)
 template <bool FULL, class TI>
 __device__ __forceinline__ void dp_rows(const Geom& g, const TI* __restrict__ dt, uint8_t* __restrict__ It, unsigned* __restrict__ Ft,
                                         int lane, int x, int y0) {
@@ -587,8 +588,6 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
     int N = g.N, KS = g.P + 1;
     size_t total = (size_t)N * g.P;
     const size_t nwords = (size_t)N * g.H * g.SEG;
-    static const bool seq_flood = getenv("TISEG_FLOOD_SEQ") != nullptr || getenv("TISEG_DEBUG_FLOOD") != nullptr ||
-                                  getenv("TISEG_FLOOD_VARIANT") != nullptr;        // (the lane-per-blob flood keeps no `first`)
     uint8_t* I0 = ws<uint8_t>(c, total);
     uint8_t* I = I0;
     uint8_t* low = ws<uint8_t>(c, total);
@@ -644,11 +643,10 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
     // markers: regional-minimum plateaus (8-connected, equal value) of I below 255, via the candidate pixels
     const dim3 word_grid((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N);
     {
-        static int PB_ROWS = 0;                  // rows per warp band (multiple of 4); TISEG_PB_ROWS for experiments
-        if (!PB_ROWS) { const char* e = getenv("TISEG_PB_ROWS"); PB_ROWS = e ? atoi(e) : 32; if (PB_ROWS < 4 || PB_ROWS % 4) PB_ROWS = 32; }
-        const long long warps = (long long)(((g.W + 3) / 4 + 23) / 24) * ((g.H + PB_ROWS - 1) / PB_ROWS);
+        const long long warps = (long long)(((g.W + 3) / 4 + 23) / 24) * ((g.H + PB_ROWS_PER_WARP - 1) / PB_ROWS_PER_WARP);
         TISEG_LAUNCH(c, k_plateau_bits, dim3((unsigned)((warps + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK), (unsigned)N),
-                     TISEG_THREADS, 0, g, I, cbits, bbits, par, low, (g.W % 4 == 0) && (((uintptr_t)I) & 3) == 0, PB_ROWS);
+                     TISEG_THREADS, 0, g, I, cbits, bbits, par, low, (g.W % 4 == 0) && (((uintptr_t)I) & 3) == 0,
+                     PB_ROWS_PER_WARP);
     }
     const BitPlanes cand = {cbits, nullptr, nullptr, nullptr, nullptr};
     // (a plateau with a pixel that touches an equal-valued non-candidate is not a regional minimum: low[root] = 1, set
@@ -660,7 +658,7 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
     // every marker pixel lies inside the mask b = (I < 255), so the markers are the flood's seed map as they are
     // (the flood writes inside the mask only and the passes below read inside it only: the full map is zero-filled just
     //  when the caller asked for it)
-    if (ws_out || markers_out || seq_flood) TISEG_TRY(zero(c, wsl, total * sizeof(int32_t)));
+    if (ws_out || markers_out) TISEG_TRY(zero(c, wsl, total * sizeof(int32_t)));
     TISEG_LAUNCH(c, k_marker_scatter, word_grid, TISEG_THREADS, 0, g, cbits, par, low, rank, wsl, mask, bpar, brank, b, seed_blob, sbits);
     if (markers_out) TISEG_CHECK(cudaMemcpyAsync(markers_out, wsl, total * sizeof(int32_t), cudaMemcpyDeviceToDevice, c->stream));
     // blobs with one marker label are filled, the others flooded in the (value, age) order
@@ -673,17 +671,12 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
     // background is 0 unless the mask covers more than half of a tile (then the histogram decides, on those tiles only)
     TISEG_TRY(zero(c, nflagged, sizeof(int)));
     TISEG_TRY(zero(c, fbits, (size_t)N * g.H * g.SEG * sizeof(unsigned)));
-    if (seq_flood) {
-        TISEG_LAUNCH(c, k_ws_hist<false>, quad_grid(g), TISEG_THREADS, 0, g, wsl, hist, first, KS, (g.W % 4 == 0) && aligned16(wsl));
-        TISEG_LAUNCH(c, k_pick_bg, N, 256, 0, hist, KS, nmark, g.P, bg, flagged, nflagged, (const int*)nullptr, (const int*)nullptr);
-    } else {
-        TISEG_LAUNCH(c, k_mask_area, dim3(8, N), TISEG_THREADS, 0, g, mbits, marea);
-        TISEG_LAUNCH(c, k_dense_tiles, (N + 255) / 256, 256, 0, marea, N, g.P, bg, dense, ndense);
-        Geom gd = listed_geom(g, dense, ndense);
-        TISEG_TRY(label_clean_listed(c, g, dense, ndense, mbits, wsl));    // (the histogram reads whole tiles)
-        TISEG_LAUNCH(c, k_ws_hist<true>, dim3(quad_grid(g).x, 1), TISEG_THREADS, 0, gd, wsl, hist, first, KS, (g.W % 4 == 0) && aligned16(wsl));
-        TISEG_LAUNCH(c, k_pick_bg, N, 256, 0, hist, KS, nmark, g.P, bg, flagged, nflagged, (const int*)dense, (const int*)ndense);
-    }
+    TISEG_LAUNCH(c, k_mask_area, dim3(8, N), TISEG_THREADS, 0, g, mbits, marea);
+    TISEG_LAUNCH(c, k_dense_tiles, (N + 255) / 256, 256, 0, marea, N, g.P, bg, dense, ndense);
+    Geom gd = listed_geom(g, dense, ndense);
+    TISEG_TRY(label_clean_listed(c, g, dense, ndense, mbits, wsl));    // (the histogram reads whole tiles)
+    TISEG_LAUNCH(c, k_ws_hist<true>, dim3(quad_grid(g).x, 1), TISEG_THREADS, 0, gd, wsl, hist, first, KS, (g.W % 4 == 0) && aligned16(wsl));
+    TISEG_LAUNCH(c, k_pick_bg, N, 256, 0, hist, KS, nmark, g.P, bg, flagged, nflagged, (const int*)dense, (const int*)ndense);
     //   background 0 (every tile but degenerate ones): ids = rank of each region's first pixel; watershed lines
     //   are found on the flood labels themselves (the renumbering is a bijection)
     TISEG_LAUNCH(c, k_first_bits, dim3(8, N), 256, 0, g, first, KS, nmark, fbits);

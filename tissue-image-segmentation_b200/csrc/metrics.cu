@@ -93,58 +93,7 @@ __global__ void k_inst_init(InstState s, int areas) {
     }
 }
 
-// one pass over the two relabelled maps: areas by id + pair table.  AREAS = false, BIG = true is the redo into the
-// always-sufficient table: a persistent grid that does nothing unless the first pass overflowed.
-template <bool BIG>
-__device__ __forceinline__ void pair_accumulate_strip(const Geom& g, const Strip& st, const int* __restrict__ par_g,
-                                                      const int* __restrict__ rank_g, const int* __restrict__ par_p,
-                                                      const int* __restrict__ rank_p, const InstState& s,
-                                                      const PairTabView& t, int* overflow) {
-    int a[STRIP_R], b[STRIP_R];
-#pragma unroll
-    for (int r = 0; r < STRIP_R; ++r) {
-        int y = st.y0 + r;
-        bool ok = st.okx && y < g.H;
-        a[r] = ok ? par_g[st.base + (long long)y * g.W + st.x] : -1;
-        b[r] = ok ? par_p[st.base + (long long)y * g.W + st.x] : -1;
-    }
-    bool any = false;
-#pragma unroll
-    for (int r = 0; r < STRIP_R; ++r) any |= a[r] >= 0 || b[r] >= 0;
-    if (!__ballot_sync(0xffffffffu, any)) return;            // (uniform) a strip of background on both sides
-    int gid[STRIP_R], pid[STRIP_R];
-#pragma unroll
-    for (int r = 0; r < STRIP_R; ++r) {
-        gid[r] = a[r] >= 0 ? rank_g[st.base + a[r]] : 0;
-        pid[r] = b[r] >= 0 ? rank_p[st.base + b[r]] : 0;
-    }
-    const long long o = (long long)st.n * s.KS;
-#pragma unroll
-    for (int r = 0; r < STRIP_R; ++r) {
-        int gl = __shfl_up_sync(0xffffffffu, gid[r], 1), pl = __shfl_up_sync(0xffffffffu, pid[r], 1);
-        bool first = st.lane == 0;
-        bool cg = !first && gid[r] == gl, cp = !first && pid[r] == pl;
-        unsigned mg = __ballot_sync(0xffffffffu, cg);
-        unsigned mp = __ballot_sync(0xffffffffu, cp);
-        unsigned mb = mg & mp;                              // both continue => the pair continues
-        if (!BIG) {
-            if (gid[r] && !cg) atomicAdd(&s.area_g[o + gid[r]], run_end_lane(mg, st.lane) - st.lane + 1);
-            if (pid[r] && !cp) atomicAdd(&s.area_p[o + pid[r]], run_end_lane(mp, st.lane) - st.lane + 1);
-        }
-        if (gid[r] && pid[r] && !(cg && cp))
-            pair_add(t, st.n, gid[r], pid[r], run_end_lane(mb, st.lane) - st.lane + 1, overflow);
-    }
-}
-
-__global__ void __launch_bounds__(TISEG_THREADS)
-k_pair_accumulate(Geom g, const int* __restrict__ par_g, const int* __restrict__ rank_g,
-                  const int* __restrict__ par_p, const int* __restrict__ rank_p, InstState s, PairTab t) {
-    Strip st;
-    if (!warp_strip(g, st)) return;
-    pair_accumulate_strip<false>(g, st, par_g, rank_g, par_p, rank_p, s, t.small, t.overflow);
-}
-
-// the redo (persistent grid; exits at once unless the small table overflowed)
+// clears the always-sufficient table for the redo (persistent grid; exits at once unless the small table overflowed)
 __global__ void __launch_bounds__(TISEG_THREADS) k_pair_zero_big(PairTab t, PairTab u, int N) {
     if (!*t.overflow) return;
     const long long total = (long long)N * t.big.cap;
@@ -153,26 +102,9 @@ __global__ void __launch_bounds__(TISEG_THREADS) k_pair_zero_big(PairTab t, Pair
         if (u.big.key != t.big.key) { u.big.key[i] = 0ull; u.big.cnt[i] = 0; }
     }
 }
-__global__ void __launch_bounds__(TISEG_THREADS)
-k_pair_accumulate_big(Geom g, const int* __restrict__ par_g, const int* __restrict__ rank_g,
-                      const int* __restrict__ par_p, const int* __restrict__ rank_p, InstState s, PairTab t, int* lost) {
-    if (!*t.overflow) return;
-    const int chunks = (g.H + STRIP_R - 1) / STRIP_R;
-    const long long wpt = (long long)g.SEG * chunks, total = wpt * g.N;
-    const int lane = threadIdx.x & 31;
-    for (long long w = (long long)blockIdx.x * TISEG_WARPS_PER_BLOCK + (threadIdx.x >> 5); w < total;
-         w += (long long)gridDim.x * TISEG_WARPS_PER_BLOCK) {
-        Strip st;
-        const int n = (int)(w / wpt), wl = (int)(w - (long long)n * wpt), ch = wl / g.SEG;
-        st.lane = lane; st.seg = wl - ch * g.SEG; st.y0 = ch * STRIP_R; st.n = n;
-        st.x = st.seg * 32 + lane; st.okx = st.x < g.W; st.base = (long long)n * g.P;
-        pair_accumulate_strip<true>(g, st, par_g, rank_g, par_p, rank_p, s, t.big, lost);
-    }
-}
-
 
 // =====================================================================================================================
-// Pair table from bit planes (the default path of tiseg_pair_metrics_*; bitccl.cuh).
+// Pair table from bit planes (tiseg_pair_metrics_*; bitccl.cuh).
 //
 // measure.label of both maps (inst_metrics.py:12-13) only serves to IDENTIFY the components the pair matrix is indexed
 // by; no per-pixel label map is needed.  Both instance maps are read ONCE (k_eqbits, 4 B/px each) into equality bit
@@ -643,21 +575,7 @@ __global__ void k_inst_class_pick(const int* __restrict__ hist, int C, int VM, u
     }
 }
 
-// class of every connected component = class of the instance value at its root pixel
-__global__ void k_comp_class(Geom g, const int32_t* __restrict__ inst, const int* __restrict__ par,
-                             const int* __restrict__ rank, const uint8_t* __restrict__ cls_inst, int VM, int C,
-                             uint8_t* cls_comp, int KS, int* ncomp) {
-    Pix px;
-    if (!warp_pixel(g, px) || !px.ok) return;
-    long long i = px.base + px.idx;
-    if (par[i] != px.idx) return;
-    int v = inst[i];
-    int cls = (v > 0 && v < VM) ? cls_inst[(long long)px.n * VM + v] : 0;
-    cls_comp[(long long)px.n * KS + rank[i]] = (uint8_t)cls;
-    atomicAdd(&ncomp[px.n * C + cls], 1);
-}
-
-// the same from the bitmap of the (final) roots instead of a per-pixel forest
+// class of every connected component = class of the instance value at its root pixel (from the bitmap of the roots)
 __global__ void __launch_bounds__(TISEG_THREADS)
 k_comp_class_bits(Geom g, const int32_t* __restrict__ inst, const unsigned* __restrict__ rootbits, const int* __restrict__ rank,
                   const uint8_t* __restrict__ cls_inst, int VM, int C, uint8_t* cls_comp, int KS, int* ncomp) {
@@ -686,18 +604,17 @@ struct PairWork {              // everything one evaluation shares: forests, ids
     double* scratch;
 };
 
-// Roots of the two labellings, however they were produced: rank (raster-order id) valid at the root pixels, and either
-// a flattened per-pixel forest (legacy path) or the bitmap of the roots (fused path).
+// Roots of the two labellings: rank (raster-order id) valid at the root pixels, and the bitmap of the roots.
 struct PairRoots {
-    const int* par_g; const int* rank_g; const int* par_p; const int* rank_p;      // par_* NULL on the fused path
-    const unsigned* bits_g; const unsigned* bits_p;                                 // NULL on the legacy path
+    const int* rank_g; const int* rank_p;
+    const unsigned* bits_g; const unsigned* bits_p;
 };
 
 static int pair_state_alloc(tiseg_ctx* c, const Geom& g, PairWork& w, int** ng, int** np, int** overflow) {
     const int N = g.N, KS = g.P + 1;
     const size_t ks = (size_t)N * KS;
     InstState& s = w.s;
-    *ng = ws<int>(c, (size_t)2 * N); *np = *ng ? *ng + N : nullptr;       // contiguous: the fused path ranks 2N tiles at once
+    *ng = ws<int>(c, (size_t)2 * N); *np = *ng ? *ng + N : nullptr;       // contiguous: pair_table_build ranks 2N tiles at once
     s.area_g = ws<int>(c, ks); s.area_p = ws<int>(c, ks);
     s.best = ws<unsigned long long>(c, ks); s.bestp = ws<int>(c, ks);
     s.used = ws<uint8_t>(c, ks); s.pqiou = ws<double>(c, ks);
@@ -724,40 +641,9 @@ static int pair_tab_alloc(tiseg_ctx* c, const Geom& g, PairTab& t, int* overflow
     return zero(c, t.small.cnt, cb);
 }
 
-// legacy path (TISEG_PAIR_LEGACY=1): per-pixel forests of both maps, flattened, then one pass over both for the table
-static int pair_table_build_legacy(tiseg_ctx* c, const Geom& g, const int32_t* d_pred, const int32_t* d_gt, PairWork& w,
-                                   PairRoots* roots) {
-    int N = g.N;
-    size_t total = (size_t)N * g.P;
-    int* par_g = ws<int>(c, total); int* rank_g = ws<int>(c, total);
-    int* par_p = ws<int>(c, total); int* rank_p = ws<int>(c, total);
-    int *ng, *np, *overflow;
-    if (!par_g || !rank_g || !par_p || !rank_p) return TISEG_ERR_CUDA;
-    TISEG_TRY(pair_state_alloc(c, g, w, &ng, &np, &overflow));
-    InstState& s = w.s;
-    // measure.label(inst.copy()) on both maps (inst_metrics.py:12-13): equal-value, 8-connected, background 0
-    TISEG_TRY(ccl_build(c, g, ImgEqI32{d_gt, 0}, 2, par_g));
-    TISEG_TRY(rank_roots(c, g, par_g, rank_g, ng));
-    TISEG_TRY(ccl_build(c, g, ImgEqI32{d_pred, 0}, 2, par_p));
-    TISEG_TRY(rank_roots(c, g, par_p, rank_p, np));
-    // the small table first; the always-sufficient one is zeroed and filled by a persistent grid that exits at once
-    // unless the first pass raised the overflow flag (a pathological input)
-    PairTab& t = w.t;
-    TISEG_TRY(pair_tab_alloc(c, g, t, overflow));
-    TISEG_TRY(zero(c, overflow, sizeof(int)));
-    TISEG_LAUNCH(c, k_inst_init, dim3(16, N), 256, 0, s, 1);
-    TISEG_LAUNCH(c, k_pair_accumulate, strip_grid(g), TISEG_THREADS, 0, g, par_g, rank_g, par_p, rank_p, s, t);
-    TISEG_LAUNCH(c, k_pair_zero_big, c->sm_count * 8, TISEG_THREADS, 0, t, t, N);
-    TISEG_LAUNCH(c, k_pair_accumulate_big, c->sm_count * 8, TISEG_THREADS, 0, g, par_g, rank_g, par_p, rank_p, s, t, c->d_err + 1);
-    if (roots) *roots = PairRoots{par_g, rank_g, par_p, rank_p, nullptr, nullptr};
-    return TISEG_OK;
-}
-
-// default path: bit planes (see the comment above k_pair_bits)
+// from bit planes (see the comment above k_pair_bits)
 static int pair_table_build(tiseg_ctx* c, const Geom& g, const int32_t* d_pred, const int32_t* d_gt, PairWork& w,
                             PairRoots* roots, const uint16_t* d_gt16 = nullptr) {
-    static const bool legacy = getenv("TISEG_PAIR_LEGACY") != nullptr;
-    if (legacy && !d_gt16) return pair_table_build_legacy(c, g, d_pred, d_gt, w, roots);
     const int N = g.N;
     const size_t total = (size_t)N * g.P, words = (size_t)N * g.H * g.SEG;
     BitPlanesW pw;
@@ -790,7 +676,7 @@ static int pair_table_build(tiseg_ctx* c, const Geom& g, const int32_t* d_pred, 
     // a pathological input overflowed the small table: clear the always-sufficient one and redo (idle otherwise)
     TISEG_LAUNCH(c, k_pair_zero_big, c->sm_count * 8, TISEG_THREADS, 0, t, t, N);
     TISEG_LAUNCH(c, k_pair_bits<true>, wgrid, TISEG_THREADS, 0, g, p, par, rank, s, t, c->d_err + 1);
-    if (roots) *roots = PairRoots{nullptr, rank, nullptr, rank + total, fbits, fbits + words};
+    if (roots) *roots = PairRoots{rank, rank + total, fbits, fbits + words};
     return TISEG_OK;
 }
 
@@ -818,9 +704,9 @@ static int pair_eval(tiseg_ctx* c, const Geom& g, PairWork& w, const uint8_t* cl
 }
 
 // class of every component of one side (pred or gt)
-static int side_classes(tiseg_ctx* c, const Geom& g, const int32_t* inst, const uint8_t* sem, const int* par,
-                        const int* rank, const unsigned* rootbits, int C, int VM, uint8_t** cls_comp_out, int** ncomp_out,
-                        int** ninst_out, int* bad) {
+static int side_classes(tiseg_ctx* c, const Geom& g, const int32_t* inst, const uint8_t* sem, const int* rank,
+                        const unsigned* rootbits, int C, int VM, uint8_t** cls_comp_out, int** ncomp_out, int** ninst_out,
+                        int* bad) {
     int N = g.N, KS = g.P + 1;
     int* hist = ws<int>(c, (size_t)N * VM * (C + 1));
     uint8_t* cls_inst = ws<uint8_t>(c, (size_t)N * VM);
@@ -836,11 +722,8 @@ static int side_classes(tiseg_ctx* c, const Geom& g, const int32_t* inst, const 
     TISEG_LAUNCH(c, k_zero_class_hist, dim3(8, N), 256, 0, hist, C, VM, maxid);
     TISEG_LAUNCH(c, k_inst_class_hist, warp_grid(g), TISEG_THREADS, 0, g, inst, sem, C, VM, hist, bad);
     TISEG_LAUNCH(c, k_inst_class_pick, dim3(8, N), 256, 0, hist, C, VM, cls_inst, ninst, maxid);
-    if (rootbits)
-        TISEG_LAUNCH(c, k_comp_class_bits, dim3((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N),
-                     TISEG_THREADS, 0, g, inst, rootbits, rank, cls_inst, VM, C, cls_comp, KS, ncomp);
-    else
-        TISEG_LAUNCH(c, k_comp_class, warp_grid(g), TISEG_THREADS, 0, g, inst, par, rank, cls_inst, VM, C, cls_comp, KS, ncomp);
+    TISEG_LAUNCH(c, k_comp_class_bits, dim3((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N),
+                 TISEG_THREADS, 0, g, inst, rootbits, rank, cls_inst, VM, C, cls_comp, KS, ncomp);
     *cls_comp_out = cls_comp; *ncomp_out = ncomp; *ninst_out = ninst;
     return TISEG_OK;
 }
@@ -961,9 +844,9 @@ int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const 
         uint8_t *cls_g, *cls_p;
         ClassInfo ci;
         int *a, *b;
-        TISEG_TRY(side_classes(c, g, d_gi, d_gs, rt.par_g, rt.rank_g, rt.bits_g, C, VM, &cls_g, &a, &b, bad));
+        TISEG_TRY(side_classes(c, g, d_gi, d_gs, rt.rank_g, rt.bits_g, C, VM, &cls_g, &a, &b, bad));
         ci.ncomp_g = a; ci.ninst_g = b;
-        TISEG_TRY(side_classes(c, g, d_pi, d_ps, rt.par_p, rt.rank_p, rt.bits_p, C, VM, &cls_p, &a, &b, bad));
+        TISEG_TRY(side_classes(c, g, d_pi, d_ps, rt.rank_p, rt.bits_p, C, VM, &cls_p, &a, &b, bad));
         ci.ncomp_p = a; ci.ninst_p = b;
         TISEG_TRY(pair_eval(c, g, w, cls_g, cls_p, C, ci, first, d_aji, d_pq));
     }
@@ -994,7 +877,6 @@ int tiseg_sem_counts(tiseg_ctx* c, const uint8_t* pred, const uint8_t* gt, int N
         gx = (unsigned)(want < most ? want : most);
         if (gx < 1) gx = 1;
     }
-    if (getenv("TISEG_SEM_GX")) gx = (unsigned)atoi(getenv("TISEG_SEM_GX"));
     bool vec = (g.P % 4 == 0) && ((((uintptr_t)d_pred) | ((uintptr_t)d_gt)) & 3) == 0;
     TISEG_LAUNCH(c, k_sem_counts, dim3(gx, N), TISEG_THREADS, 0, (long long)g.P, d_pred, d_gt, C, ignore_index,
                  (unsigned long long*)d_counts, (unsigned long long*)d_valid, vec);

@@ -1,9 +1,7 @@
-// K6 — ordered marker-controlled watershed: blob bookkeeping, the uint8 bucket flood, the fp64 heap flood
-// and the tiseg_watershed_* entry points.  See watershed.cuh for the algorithm statement.
+// K6 — ordered marker-controlled watershed: blob bookkeeping, the warp-cooperative uint8 flood, the ranked fp64
+// bucket flood with its heap fallback, and the tiseg_watershed_* entry points.  See watershed.cuh for the algorithm
+// statement.
 #include "watershed.cuh"
-
-#include <cstdio>
-#include <cstdlib>
 
 namespace tiseg {
 
@@ -127,43 +125,28 @@ k_ws_seed(long long total, const int32_t* __restrict__ markers, const int* __res
     st4(out, i, total, vec, o);
 }
 
-// ---- uint8 levels: FIFO buckets ---------------------------------------------------------------------------
+// ---- work lists and staging, shared by the uint8 and the ranked fp64 flood -----------------------------------------
 // A blob's flood is a chain of dependent steps (pop -> look at 4 neighbours -> push), so its speed is the latency
 // of the memory it runs in and the number of floods in flight.  Every blob is therefore STAGED into shared memory
-// first: the bounding box plus a one-pixel frame (no bounds checks in the flood), 4 bytes per cell — one 16-bit field
-// that holds the level until the cell is labelled and its FIFO link afterwards (the level is dead by then), and the
-// local index of the seed pixel whose label the cell inherits (u16) — flooded there, and written back with batched
-// loads/stores.
+// first: the bounding box plus a one-pixel frame (no bounds checks in the flood), flooded there, and written back with
+// batched loads/stores.
 //
-// One persistent kernel (one CTA per SM), fed from work lists sorted by size class so that long floods start first:
-//  * multi-slot floods — the workhorse.  Every warp owns an arena of shared memory that is cut into 1..SLOTS equal
-//    slots according to the size class it is working on; the warp stages one blob per slot cooperatively, links the
-//    seeds into their buckets in raster order (match_any), then LANE s FLOODS SLOT s: up to SLOTS independent floods
-//    advance per warp instruction.  Buckets are indexed by (level mod 32): a blob qualifies if its levels span < 32
-//    values (a distance map inside a nucleus does); the head and tail of the current level live in registers.
-//    Default geometry: 12 warps x 4224-cell arenas x 16 slots (other geometries behind TISEG_FLOOD_VARIANT).  A blob
-//    whose seeds all carry one label is simply filled (a 4-connected blob is flooded completely from any seed).
-//  * general floods — framed boxes beyond the arena, or level spans >= 32: one blob per CTA at a time, staged by all
-//    warps into one 45056-cell slice with all 256 buckets.  The first sm_count/12 CTAs start with this list so the
-//    largest blobs begin at t = 0; every CTA helps with it after the multi-slot work.  Level-span overflows found
-//    while flooding go to a second list drained by a second (normally empty) launch.  Only boxes beyond 45056
-//    cells are flooded in global memory.
+// Both floods (k_ws_flood_par, k_ws_flood_ranked) are persistent kernels (one CTA per SM) fed from work lists sorted by
+// size class so that long floods start first.  Framed boxes beyond a warp arena go to a general list, staged by a whole
+// CTA: the largest blobs begin at t = 0.  Only boxes beyond that CTA-wide slice are flooded in global memory.
 #define WS_NOTIN 0xFFFFu
 #define WS_UNLAB 0xFFFEu
 #define WS_END 0xFFFFu
 
-#define WM_R 32                 // levels per multi-slot flood (buckets indexed by level mod WM_R)
 #define WS_MAXCLS 16            // most slots per warp arena (= number of size classes)
-#define WG_CAP 45056            // cells of the single-blob slice of the general path
-#define WG_SMEM_BYTES ((size_t)WG_CAP * 5 + 1024)
 extern __shared__ __align__(16) unsigned char ws_smem[];
 
 // Work lists of one batch.  An item is (tile << 32) | blob id.  Size class c = blobs whose framed box fits a slot of
 // arena / (c + 1) cells but no smaller one, so class 0 holds the largest blobs and is drained first.
 struct FloodWork {
     long long* items;   // classes 0..slots-1, contiguous, class c at offset[c] .. offset[c] + count[c]
-    long long* gen;     // general list, filled by k_flood_scatter: boxes beyond the arena
-    long long* ovf;     // overflow list, filled by the flood kernel: level spans >= WM_R; drained by a second launch
+    long long* gen;     // general list: boxes beyond the warp arena
+    long long* ovf;     // ranked flood only: blobs too large to rank or stage, flooded by k_ws_flood_f64
     int* count;         // [WS_MAXCLS]
     int* offset;        // [WS_MAXCLS]
     int* fill;          // [WS_MAXCLS] scatter cursors
@@ -271,10 +254,8 @@ int label_clean_listed(tiseg_ctx* c, const Geom& g, const int* list, const int* 
 // floor(j / wp) for j * wp < 2^32 with magic = 0xFFFFFFFF / wp + 1
 __device__ __forceinline__ int fdiv(int j, unsigned magic) { return (int)__umulhi((unsigned)j, magic); }
 
-// Copy the framed box of a blob into shared memory: lab = own index (seed), UNLAB (in the blob), NOTIN; lvl = level.
-// `tid`/`nthr`: the cooperating threads (a warp or a CTA); eight cells per thread are loaded before any is used.
-// Per-thread by-products (the caller reduces them if it wants them): the range [lmn, lmx] of the seed labels seen and
-// the lowest seed cell — a blob whose seeds all carry ONE label needs no ordered flood at all.
+// Per-thread by-products of staging a blob (the caller reduces them if it wants them): the range [lmn, lmx] of the seed
+// labels seen and the lowest seed cell — a blob whose seeds all carry ONE label needs no ordered flood at all.
 struct SeedStats { int lmn, lmx, jseed; };
 // membership of a staged cell (see BlobMember in watershed.cuh)
 struct InForest {
@@ -296,8 +277,15 @@ struct InMask {
         return ((word >> (x & 31)) & 1u) && seed_blob[gi] == bid;
     }
 };
-template <class IT, class LT, class MB>
-__device__ __forceinline__ SeedStats stage_copy(int tid, int nthr, int W, const IT* __restrict__ I, const MB mb,
+
+// ---- helpers of the ranked fp64 flood: FIFO buckets, one lane per staged blob -----------------------------------------
+// A staged cell takes 4 bytes: the local index of the seed cell whose label it inherits (u16), and one 16-bit field that
+// holds the level until the cell is labelled and its FIFO link afterwards (the level is dead by then).
+//
+// Copy the framed box of a blob into shared memory: lab = own index (seed), UNLAB (in the blob), NOTIN; lvl = level.
+// `tid`/`nthr`: the cooperating threads (a warp or a CTA); eight cells per thread are loaded before any is used.
+template <class IT, class LT>
+__device__ __forceinline__ SeedStats stage_copy(int tid, int nthr, int W, const IT* __restrict__ I, const InForest mb,
                                                 const int32_t* __restrict__ o, int root,
                                                 int y0, int x0, int w, int h, unsigned short* lab, LT* lvl) {
     SeedStats st; st.lmn = 0x7fffffff; st.lmx = 0; st.jseed = 0x7fffffff;
@@ -316,14 +304,13 @@ __device__ __forceinline__ SeedStats stage_copy(int tid, int nthr, int W, const 
         int tpv[8], ov[8];
         IT iv[8];
 #pragma unroll
-        for (int u = 0; u < 8; ++u) { tpv[u] = mb.load(gi[u]); iv[u] = I[gi[u]]; ov[u] = MB::kMasked ? 0 : o[gi[u]]; }
+        for (int u = 0; u < 8; ++u) { tpv[u] = mb.load(gi[u]); iv[u] = I[gi[u]]; ov[u] = o[gi[u]]; }
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
             const int j = j0 + u * nthr + tid;
             if (j < cells) {
                 const bool inblob = in[u] && mb.in(tpv[u]);
-                const int gy = gi[u] / W, gx = gi[u] - gy * W;
-                const bool seed = inblob && mb.seed(gi[u], MB::kMasked ? mb.seed_word(gy, gx) : 0u, gx, ov[u]);
+                const bool seed = inblob && mb.seed(gi[u], 0u, 0, ov[u]);
                 lab[j] = (unsigned short)(inblob ? (seed ? (unsigned)j : WS_UNLAB) : WS_NOTIN);
                 lvl[j] = (LT)iv[u];
                 if (seed) { st.lmn = min(st.lmn, ov[u]); st.lmx = max(st.lmx, ov[u]); st.jseed = min(st.jseed, j); }
@@ -469,7 +456,8 @@ __device__ __forceinline__ void stage_writeback(int tid, int nthr, int W, int32_
     }
 }
 
-// The same flood in global memory (framed bounding box too large for shared memory); head/tail are int[256].
+// The sequential uint8 flood of one blob in global memory, by one lane (framed bounding box too large for shared
+// memory): 256 FIFO buckets, head/tail are int[256], the links live in `nx`.
 template <class MB>
 __device__ __forceinline__ void flood_blob_global(int lane, int W, int H, const uint8_t* __restrict__ I,
                                                   const MB mb, int32_t* o, int* nx, int root, int y0,
@@ -539,188 +527,11 @@ __device__ __forceinline__ void flood_blob_global(int lane, int W, int H, const 
     __syncwarp();
 }
 
-struct BucketAll { __device__ __forceinline__ int operator()(int v) const { return v; } };
-template <int SLOTS> struct BucketSlot {    // heads of one level are contiguous over the slots of the warp
-    int s;
-    __device__ __forceinline__ int operator()(int v) const { return ((v & (WM_R - 1)) * SLOTS) + s; }
-};
-
-// General path: one blob per CTA at a time, staged by all warps into one WG_CAP-cell slice with all 256 buckets.
-template <bool MASKED>
-__device__ __forceinline__ void general_drain(const Geom& g, const uint8_t* __restrict__ image, const BlobMember& bm,
-                                              const BlobInfo& b, const long long* list, int count, int* cursor, int* next,
-                                              int* gheads, int32_t* out) {
-    __shared__ int s_item;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    unsigned short* lab = reinterpret_cast<unsigned short*>(ws_smem);
-    unsigned short* nxs = lab + WG_CAP;
-    unsigned short* head = nxs + WG_CAP;
-    unsigned short* tail = head + 256;
-    unsigned char* lvl = reinterpret_cast<unsigned char*>(tail + 256);
-    const int W = g.W, H = g.H;
-    for (;;) {
-        __syncthreads();
-        if (threadIdx.x == 0) s_item = atomicAdd(cursor, 1);
-        __syncthreads();
-        const int k = s_item;
-        if (k >= count) break;
-        const long long item = list[k];
-        const int n = (int)(item >> 32), bid = (int)(item & 0xffffffffll);
-        const long long base = (long long)n * g.P, ko = (long long)n * b.KS;
-        const uint8_t* I = image + base;
-        int32_t* o = out + base;
-        const int root = b.root[ko + bid];
-        const int y0 = root / W, y1 = b.ymax[ko + bid], x0 = b.xmin[ko + bid], x1 = b.xmax[ko + bid];
-        const int w = x1 - x0 + 1, h = y1 - y0 + 1;
-        const long long cells = (long long)(w + 2) * (h + 2);
-        const InForest inf = {bm.par + base, root};
-        const InMask inm = {MASKED ? bm.mask_img + base : nullptr, MASKED ? bm.seed_blob + base : nullptr,
-                                MASKED ? bm.seed_bits + (long long)n * g.H * g.SEG : nullptr, g.SEG, bid};
-        if (cells > WG_CAP) {         // does not fit: the same flood in global memory, by one lane
-            if (warp == 0) {
-                if (MASKED) flood_blob_global(lane, W, H, I, inm, o, next + base, root, y0, y1, x0, x1,
-                                              gheads + (size_t)blockIdx.x * 512, gheads + (size_t)blockIdx.x * 512 + 256);
-                else flood_blob_global(lane, W, H, I, inf, o, next + base, root, y0, y1, x0, x1,
-                                       gheads + (size_t)blockIdx.x * 512, gheads + (size_t)blockIdx.x * 512 + 256);
-            }
-            continue;
-        }
-        for (int i = threadIdx.x; i < 256; i += blockDim.x) { head[i] = (unsigned short)WS_END; tail[i] = (unsigned short)WS_END; }
-        if (MASKED) stage_copy(threadIdx.x, blockDim.x, W, I, inm, o, root, y0, x0, w, h, lab, lvl);
-        else stage_copy(threadIdx.x, blockDim.x, W, I, inf, o, root, y0, x0, w, h, lab, lvl);
-        __syncthreads();
-        if (warp == 0) {
-            int vmin, vmax, vsmin;
-            link_seeds(lane, (int)cells, lab, nxs, lvl, head, tail, BucketAll{}, vmin, vmax, vsmin);
-            __syncwarp();
-            if (lane == 0 && vsmin <= vmax) lane_flood(w + 2, vsmin, vmax, lab, nxs, lvl, head, tail, BucketAll{});
-        }
-        __syncthreads();
-        stage_writeback(threadIdx.x, blockDim.x, W, o, y0, x0, w, h, lab);
-    }
-}
-
-// The flood kernel.  CTAs below `gen_first` start with the general list (the few largest blobs begin at t = 0), every
-// CTA then drains the multi-slot classes from the largest to the smallest (`do_multi`), and finally helps with what
-// is left of the general list.
-template <int WARPS, int ARENA, int SLOTS, bool PROF, bool MASKED>
-__global__ void __launch_bounds__(32 * WARPS, 1)
-k_ws_flood_u8(Geom g, const uint8_t* __restrict__ image, BlobMember bm, BlobInfo b, FloodWork wk,
-              int* next, int* gheads, int32_t* out, int gen_first, int do_multi, long long* prof) {
-    constexpr size_t WARP_BYTES = (size_t)ARENA * 4 + (size_t)WM_R * SLOTS * 4;
-    if (!do_multi) {       // second launch: what the first one found too wide in levels
-        general_drain<MASKED>(g, image, bm, b, wk.ovf, wk.ngen[1], wk.gcursor + 1, next, gheads, out);
-        return;
-    }
-    const int ngen = wk.ngen[0];
-    if ((int)blockIdx.x < min(gen_first, ngen) && ngen > 0) general_drain<MASKED>(g, image, bm, b, wk.gen, ngen, wk.gcursor, next, gheads, out);
-    {
-        __syncthreads();
-        const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-        long long t_stage = 0, t_flood = 0, t_wb = 0, t0 = 0, t_all = PROF ? clock64() : 0, iters = 0;
-        unsigned char* wbase = ws_smem + (size_t)warp * WARP_BYTES;
-        unsigned short* lab = reinterpret_cast<unsigned short*>(wbase);
-        unsigned short* nxs = lab + ARENA;
-        unsigned short* head = nxs + ARENA;
-        unsigned short* tail = head + WM_R * SLOTS;
-        // 4 bytes per cell: the level of a cell is dead once the cell is labelled and its FIFO link only lives after
-        // that, so both sit in the same 16-bit field (every reader below takes the level before it writes the link)
-        unsigned short* lvl = nxs;
-        const int W = g.W;
-        for (int cls = 0; cls < SLOTS; ++cls) {
-            const int cap = ARENA / (cls + 1), slots = cls + 1;
-            const int cnt = wk.count[cls];
-            const long long* list = wk.items + wk.offset[cls];
-            for (;;) {
-                int k0 = 0;
-                if (lane == 0) k0 = atomicAdd(&wk.cursor[cls], slots);
-                k0 = __shfl_sync(FULL, k0, 0);
-                if (k0 >= cnt) break;
-                const int m = min(slots, cnt - k0);
-                // lane s < m holds the description of the blob in slot s
-                int mn = 0, mroot = 0, my0 = 0, mx0 = 0, mw = 0, mh = 0, mbid = 0;
-                if (lane < m) {
-                    const long long item = list[k0 + lane];
-                    mn = (int)(item >> 32);
-                    mbid = (int)(item & 0xffffffffll);
-                    const long long ko = (long long)mn * b.KS;
-                    mroot = b.root[ko + mbid];
-                    my0 = mroot / W; mx0 = b.xmin[ko + mbid];
-                    mw = b.xmax[ko + mbid] - mx0 + 1; mh = b.ymax[ko + mbid] - my0 + 1;
-                }
-                for (int i = lane; i < WM_R * SLOTS; i += 32) { head[i] = (unsigned short)WS_END; tail[i] = (unsigned short)WS_END; }
-                if (PROF) t0 = clock64();
-                unsigned single = 0;                                           // slots whose blob has one marker label
-                for (int s = 0; s < m; ++s) {
-                    const int n = __shfl_sync(FULL, mn, s), root = __shfl_sync(FULL, mroot, s), bid = __shfl_sync(FULL, mbid, s);
-                    const int y0 = __shfl_sync(FULL, my0, s), x0 = __shfl_sync(FULL, mx0, s);
-                    const int w = __shfl_sync(FULL, mw, s), h = __shfl_sync(FULL, mh, s);
-                    const long long base = (long long)n * g.P;
-                    if (MASKED) {       // (blobs with a single marker never get here: nothing to short-cut)
-                        const InMask inm = {bm.mask_img + base, bm.seed_blob + base, bm.seed_bits + (long long)n * g.H * g.SEG, g.SEG, bid};
-                        stage_copy(lane, 32, W, image + base, inm, out + base, root, y0, x0, w, h, lab + s * cap, lvl + s * cap);
-                    } else {
-                        const InForest inf = {bm.par + base, root};
-                        const SeedStats st = stage_copy(lane, 32, W, image + base, inf, out + base, root, y0, x0, w, h,
-                                                        lab + s * cap, lvl + s * cap);
-                        __syncwarp();
-                        if (fill_if_single_marker(lane, st, (w + 2) * (h + 2), lab + s * cap)) single |= 1u << s;
-                    }
-                }
-                __syncwarp();
-                int lmin = WS_LVL_NONE, lmax = -1, smin = WS_LVL_NONE;        // of slot `lane`
-                for (int s = 0; s < m; ++s) {
-                    if ((single >> s) & 1u) continue;                          // nothing to flood in this slot
-                    const int w = __shfl_sync(FULL, mw, s), h = __shfl_sync(FULL, mh, s);
-                    int vmin, vmax, vsmin;
-                    link_seeds(lane, (w + 2) * (h + 2), lab + s * cap, nxs + s * cap, lvl + s * cap, head, tail,
-                               BucketSlot<SLOTS>{s}, vmin, vmax, vsmin);
-                    if (lane == s) { lmin = vmin; lmax = vmax; smin = vsmin; }
-                }
-                __syncwarp();
-                if (PROF) { long long t = clock64(); t_stage += t - t0; t0 = t; }
-                // ---- the floods: lane s floods slot s
-                const bool overflow = lane < m && lmax - lmin >= WM_R;
-                if (overflow) wk.ovf[atomicAdd(wk.ngen + 1, 1)] = list[k0 + lane];
-                const unsigned ovf = __ballot_sync(FULL, overflow);
-                {
-                    int pops = 0;
-                    if (lane < m && !overflow && smin <= lmax)
-                        pops = lane_flood(mw + 2, smin, lmax, lab + lane * cap, nxs + lane * cap, lvl + lane * cap, head, tail,
-                                          BucketSlot<SLOTS>{lane});
-                    if (PROF) {
-#pragma unroll
-                        for (int d = 16; d; d >>= 1) pops = max(pops, __shfl_xor_sync(FULL, pops, d));
-                        iters += pops;
-                    }
-                }
-                __syncwarp();
-                if (PROF) { long long t = clock64(); t_flood += t - t0; t0 = t; }
-                // ---- write back
-                for (int s = 0; s < m; ++s) {
-                    if ((ovf >> s) & 1u) continue;
-                    const int n = __shfl_sync(FULL, mn, s);
-                    const int y0 = __shfl_sync(FULL, my0, s), x0 = __shfl_sync(FULL, mx0, s);
-                    const int w = __shfl_sync(FULL, mw, s), h = __shfl_sync(FULL, mh, s);
-                    stage_writeback(lane, 32, W, out + (long long)n * g.P, y0, x0, w, h, lab + s * cap);
-                }
-                __syncwarp();
-                if (PROF) t_wb += clock64() - t0;
-            }
-        }
-        if (PROF && lane == 0) {
-            long long* p = prof + ((size_t)blockIdx.x * WARPS + warp) * 5;
-            p[0] = t_stage; p[1] = t_flood; p[2] = t_wb; p[3] = clock64() - t_all; p[4] = iters;
-        }
-    }
-    if (ngen > 0) general_drain<MASKED>(g, image, bm, b, wk.gen, ngen, wk.gcursor, next, gheads, out);
-}
-
 // ---- uint8 levels, warp-cooperative flood ---------------------------------------------------------------------------------
-// The lane-per-blob flood above advances one pixel per ~500 cycles and blob, so a cluster of touching nuclei (a blob of
-// 2-3 thousand pixels) alone lasts as long as the whole kernel (profiles/r2_flood_debug.txt: mean 0.73 M cycles per
-// warp, max 1.04 M).  Here ONE WARP floods one blob and pops up to 32 pixels of the current level per step, with exactly
-// the sequential result:
+// A flood by one lane (as in lane_flood) advances one pixel per ~500 cycles and blob, so a cluster of touching nuclei (a
+// blob of 2-3 thousand pixels) alone would last as long as the whole kernel (profiles/r2_flood_debug.txt: mean 0.73 M
+// cycles per warp, max 1.04 M).  Here ONE WARP floods one blob and pops up to 32 pixels of the current level per step,
+// with exactly the sequential result:
 //   * queues are ARRAYS: every cell is pushed at most once, so level v never receives more entries than the blob has
 //     cells of level v; the staging pass counts them and the queue storage is cut into one segment per level.  The
 //     first B <= 32 entries e_0 .. e_{B-1} of the current level are read by lanes 0 .. B-1.
@@ -952,9 +763,8 @@ __device__ __forceinline__ void wp_writeback(int tid, int nthr, int W, int32_t* 
 template <bool MASKED>
 __global__ void __launch_bounds__(32 * WP_WARPS, 1)
 k_ws_flood_par(Geom g, const uint8_t* __restrict__ image, BlobMember bm, BlobInfo b, FloodWork wk, int* next, int* gheads,
-               int32_t* out, long long* prof) {
+               int32_t* out) {
     __shared__ int s_item;
-    long long t_gen = 0, t_stage = 0, t_prep = 0, t_flood = 0, t_wb = 0, t0 = 0, t_all = prof ? clock64() : 0;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int W = g.W, H = g.H;
     // ---- blobs beyond one warp arena: the whole CTA stages, one warp floods (largest first: they start at t = 0)
@@ -1005,7 +815,6 @@ k_ws_flood_par(Geom g, const uint8_t* __restrict__ image, BlobMember bm, BlobInf
         }
         __syncthreads();
     }
-    if (prof) t_gen = clock64() - t_all;
     // ---- one blob per warp, size classes from the largest to the smallest
     const bool big = warp < WP_BIG_WARPS;
     const int arena = big ? WP_ARENA : WP_SMALL_ARENA;
@@ -1033,7 +842,6 @@ k_ws_flood_par(Geom g, const uint8_t* __restrict__ image, BlobMember bm, BlobInf
             const int cells = (w + 2) * (h + 2);
             for (int i = lane; i < 128; i += 32) cnt32[i] = 0u;
             __syncwarp();
-            if (prof) t0 = clock64();
             bool flood = true;
             if (MASKED) {
                 const InMask inm = {bm.mask_img + base, bm.seed_blob + base, bm.seed_bits + (long long)n * g.H * g.SEG, g.SEG, bid};
@@ -1056,29 +864,21 @@ k_ws_flood_par(Geom g, const uint8_t* __restrict__ image, BlobMember bm, BlobInf
                 }
             }
             __syncwarp();
-            if (prof) { const long long t = clock64(); t_stage += t - t0; t0 = t; }
             if (flood) {
                 const int smin = wp_prepare(lane, cells, cell, Q, head, tail, cnt32);
-                if (prof) { const long long t = clock64(); t_prep += t - t0; t0 = t; }
                 if (smin < 256) wp_flood(lane, w + 2, cell, Q, head, tail, smin);
             }
             __syncwarp();
-            if (prof) { const long long t = clock64(); t_flood += t - t0; t0 = t; }
             wp_writeback(lane, 32, W, out + base, y0, x0, w, h, cell, b.first ? b.first + ko : nullptr);
             __syncwarp();
-            if (prof) t_wb += clock64() - t0;
         }
-    }
-    if (prof && lane == 0) {
-        long long* p = prof + ((size_t)blockIdx.x * WP_WARPS + warp) * 6;
-        p[0] = t_gen; p[1] = t_stage; p[2] = t_prep; p[3] = t_flood; p[4] = t_wb; p[5] = clock64() - t_all;
     }
 }
 
-// ---- fp64 values, fast path: per-blob dense ranks + the same bucket flood ---------------------------------------------
+// ---- fp64 values, fast path: per-blob dense ranks + a bucket flood in shared memory ------------------------------------
 // The (value, age) order of the flood only compares values INSIDE one blob, so the fp64 image can be replaced, blob
 // by blob, by the dense rank of each pixel's value among the blob's distinct values (equal doubles -> equal rank):
-// the flood then runs on small integers with FIFO buckets in shared memory exactly like the uint8 case, instead of
+// the flood then runs on small integers with FIFO buckets in shared memory (stage_copy .. stage_writeback), instead of
 // a binary heap in global memory.  Ranking = one bitonic sort of the blob's values in shared memory (k_rank_blobs),
 // a flag-and-scan for the distinct values, and a binary search per pixel.  Blobs whose framed box exceeds WR_GEN_CAP
 // cells or whose area exceeds WR_SORT_MAX keep the heap flood (k_ws_flood_f64).
@@ -1228,7 +1028,7 @@ __device__ __forceinline__ void general_drain_ranked(const Geom& g, const unsign
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     unsigned short* lab = reinterpret_cast<unsigned short*>(ws_smem);
     unsigned short* nxs = lab + WR_GEN_CAP;
-    unsigned short* lvl = nxs;                       // level and FIFO link share a field, as in k_ws_flood_u8
+    unsigned short* lvl = nxs;                       // level and FIFO link share a field (see stage_copy)
     unsigned short* head = nxs + WR_GEN_CAP;
     unsigned short* tail = head + WR_GEN_CAP;
     const int W = g.W;
@@ -1373,25 +1173,18 @@ __device__ __forceinline__ HeapItem heap_pop(HeapItem* h, int& sz) {
     return top;
 }
 
-// `list` == NULL: every blob of tile blockIdx.y (queue[n] is the cursor); else the listed blobs only (persistent grid)
+// one warp per listed blob, list[0 .. *nlist) (persistent grid; `cursor` hands out the items)
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_ws_flood_f64(Geom g, const double* __restrict__ image, const int* __restrict__ par, BlobInfo b, int* queue,
+k_ws_flood_f64(Geom g, const double* __restrict__ image, const int* __restrict__ par, BlobInfo b, int* cursor,
                const long long* __restrict__ list, const int* __restrict__ nlist, HeapItem* heap, int32_t* out) {
     const int lane = threadIdx.x & 31;
     const int W = g.W, H = g.H;
     for (;;) {
-        int n = blockIdx.y, bid = 0;
-        if (list) {
-            int k = 0;
-            if (lane == 0) k = atomicAdd(queue, 1);
-            k = __shfl_sync(FULL, k, 0);
-            if (k >= *nlist) break;
-            n = (int)(list[k] >> 32); bid = (int)(list[k] & 0xffffffffll);
-        } else {
-            if (lane == 0) bid = atomicAdd(&queue[n], 1) + 1;
-            bid = __shfl_sync(FULL, bid, 0);
-            if (bid > b.count[n]) break;
-        }
+        int k = 0;
+        if (lane == 0) k = atomicAdd(cursor, 1);
+        k = __shfl_sync(FULL, k, 0);
+        if (k >= *nlist) break;
+        const int n = (int)(list[k] >> 32), bid = (int)(list[k] & 0xffffffffll);
         const long long base = (long long)n * g.P, ko = (long long)n * b.KS;
         const double* I = image + base;
         const int* tp = par + base;
@@ -1464,62 +1257,6 @@ int blobs_describe(tiseg_ctx* c, const Geom& g, const int* par, const int* rank,
     return TISEG_OK;
 }
 
-static inline int flood_blocks(tiseg_ctx* c, int N) {
-    // persistent-style grid: enough warps to fill the chip several times over, split evenly over tiles
-    int per_tile = (c->sm_count * 8 * 4 + N - 1) / N;
-    if (per_tile < 1) per_tile = 1;
-    if (per_tile > 512) per_tile = 512;
-    return per_tile;
-}
-
-template <int WARPS, int ARENA, int SLOTS, bool MASKED>
-static int flood_launch(tiseg_ctx* c, const Geom& g, const uint8_t* image, const BlobMember& par, const BlobInfo& b,
-                        FloodWork wk, int* next, int* gheads, int32_t* out, int* ints, bool debug) {
-    static_assert(SLOTS <= WS_MAXCLS, "slots");
-    constexpr size_t MULTI = (size_t)WARPS * ((size_t)ARENA * 4 + (size_t)WM_R * SLOTS * 4);
-    constexpr size_t SMEM = MULTI > WG_SMEM_BYTES ? MULTI : WG_SMEM_BYTES;
-    static_assert(SMEM + 64 <= 232448, "shared memory");
-    TISEG_LAUNCH(c, k_flood_count, dim3(8, g.N), 256, 0, b, g.W, wk, ARENA, SLOTS);
-    TISEG_LAUNCH(c, k_flood_offsets, 1, 32, 0, wk);
-    TISEG_LAUNCH(c, k_flood_scatter, dim3(8, g.N), 256, 0, b, g.W, wk, ARENA, SLOTS, 0ll, (int*)nullptr);
-    static bool attr_set = false;
-    if (!attr_set) {
-        TISEG_CHECK(cudaFuncSetAttribute(k_ws_flood_u8<WARPS, ARENA, SLOTS, false, MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
-        TISEG_CHECK(cudaFuncSetAttribute(k_ws_flood_u8<WARPS, ARENA, SLOTS, true, MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
-        attr_set = true;
-    }
-    const int gen_first = c->sm_count >= 8 ? c->sm_count / 4 : 1;     // at most this many CTAs, one per listed blob
-    long long* prof = nullptr;
-    if (debug) {
-        prof = ws<long long>(c, (size_t)c->sm_count * WARPS * 5);
-        if (!prof) return TISEG_ERR_CUDA;
-        TISEG_LAUNCH_AS(c, "k_ws_flood_u8", (k_ws_flood_u8<WARPS, ARENA, SLOTS, true, MASKED>), c->sm_count, 32 * WARPS, SMEM, g,
-                        image, par, b, wk, next, gheads, out, gen_first, 1, prof);
-    } else {
-        TISEG_LAUNCH_AS(c, "k_ws_flood_u8", (k_ws_flood_u8<WARPS, ARENA, SLOTS, false, MASKED>), c->sm_count, 32 * WARPS, SMEM, g,
-                        image, par, b, wk, next, gheads, out, gen_first, 1, prof);
-    }
-    // blobs found too wide in levels after the other CTAs had left the general list; exits at once if there are none
-    TISEG_LAUNCH_AS(c, "k_ws_flood_u8(level-span overflow)", (k_ws_flood_u8<WARPS, ARENA, SLOTS, false, MASKED>), c->sm_count,
-                    32 * WARPS, SMEM, g, image, par, b, wk, next, gheads, out, 0, 0, nullptr);
-    if (debug) {                                  // work-list census on stderr (synchronises; diagnostics only)
-        int h[WK_INTS];
-        TISEG_CHECK(cudaMemcpyAsync(h, ints, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
-        TISEG_CHECK(cudaStreamSynchronize(c->stream));
-        fprintf(stderr, "[tiseg flood] warps %d arena %d slots %d | N=%d classes:", WARPS, ARENA, SLOTS, g.N);
-        for (int k = 0; k < SLOTS; ++k) fprintf(stderr, " %d", h[k]);
-        fprintf(stderr, " | general: %d, level-span overflow: %d\n", h[4 * WS_MAXCLS], h[4 * WS_MAXCLS + 1]);
-        std::vector<long long> hp((size_t)c->sm_count * WARPS * 5);
-        TISEG_CHECK(cudaMemcpy(hp.data(), prof, hp.size() * sizeof(long long), cudaMemcpyDeviceToHost));
-        long long sum[5] = {0, 0, 0, 0, 0}, mx[5] = {0, 0, 0, 0, 0};
-        for (size_t i = 0; i < hp.size(); ++i) { sum[i % 5] += hp[i]; if (hp[i] > mx[i % 5]) mx[i % 5] = hp[i]; }
-        const double nw = (double)c->sm_count * WARPS;
-        fprintf(stderr, "[tiseg flood] per-warp cycles mean (max): stage %.0f (%lld) flood %.0f (%lld) writeback %.0f (%lld) total %.0f (%lld); flood steps %.0f (%lld)\n",
-                sum[0] / nw, mx[0], sum[1] / nw, mx[1], sum[2] / nw, mx[2], sum[3] / nw, mx[3], sum[4] / nw, mx[4]);
-    }
-    return TISEG_OK;
-}
-
 template <bool MASKED>
 static int watershed_u8_any(tiseg_ctx* c, const Geom& g, const uint8_t* image, const BlobMember& bm, const BlobInfo& b, int32_t* out) {
     const int N = g.N;
@@ -1527,64 +1264,34 @@ static int watershed_u8_any(tiseg_ctx* c, const Geom& g, const uint8_t* image, c
     FloodWork wk;
     wk.items = ws<long long>(c, max_blobs);
     wk.gen = ws<long long>(c, max_blobs);
-    wk.ovf = ws<long long>(c, max_blobs);
+    wk.ovf = nullptr;
     int* ints = ws<int>(c, WK_INTS + 2 * (size_t)N + 1);
     int* next = ws<int>(c, (size_t)N * g.P);
     int* gheads = ws<int>(c, (size_t)c->sm_count * 512);
-    if (!wk.items || !wk.gen || !wk.ovf || !ints || !next || !gheads) return TISEG_ERR_CUDA;
+    if (!wk.items || !wk.gen || !ints || !next || !gheads) return TISEG_ERR_CUDA;
     wk.count = ints; wk.offset = ints + WS_MAXCLS; wk.fill = ints + 2 * WS_MAXCLS; wk.cursor = ints + 3 * WS_MAXCLS;
     wk.ngen = ints + 4 * WS_MAXCLS; wk.gcursor = wk.ngen + 2;
     int* huge = ints + WK_INTS;                 // tiles with a blob that is flooded in global memory
     TISEG_TRY(zero(c, ints, (WK_INTS + 2 * (size_t)N + 1) * sizeof(int)));
-    static const bool debug = getenv("TISEG_DEBUG_FLOOD") != nullptr;
-    static const int variant = getenv("TISEG_FLOOD_VARIANT") ? atoi(getenv("TISEG_FLOOD_VARIANT")) : 0;
-    static const bool sequential = getenv("TISEG_FLOOD_SEQ") != nullptr || debug || variant != 0;
-    if (!sequential) {            // warp-cooperative flood (default)
-        static_assert(WP_SMEM_BYTES + 64 <= 232448, "shared memory");
-        TISEG_LAUNCH(c, k_flood_count, dim3(8, g.N), 256, 0, b, g.W, wk, WP_ARENA, WS_MAXCLS);
-        TISEG_LAUNCH(c, k_flood_offsets, 1, 32, 0, wk);
-        TISEG_LAUNCH(c, k_flood_scatter, dim3(8, g.N), 256, 0, b, g.W, wk, WP_ARENA, WS_MAXCLS, (long long)WP_GEN_CAP, MASKED ? huge : (int*)nullptr);
-        // mask mode: the label map holds the seeds and is otherwise unwritten; the flood in global memory reads it
-        if (MASKED) {
-            Geom gh = listed_geom(g, huge + N, huge + 2 * N);
-            const BitPlanes mp = {const_cast<unsigned*>(bm.mask_bits), nullptr, nullptr, nullptr, nullptr};
-            TISEG_LAUNCH(c, k_huge_clean, dim3((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), 1), TISEG_THREADS, 0,
-                         gh, mp, bm.bpar, bm.brank, b, bm.seed_bits, (long long)WP_GEN_CAP, out);
-        }
-        static bool attr_set = false;
-        if (!attr_set) {
-            TISEG_CHECK(cudaFuncSetAttribute(k_ws_flood_par<MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WP_SMEM_BYTES));
-            attr_set = true;
-        }
-        static const bool par_prof = getenv("TISEG_PROF_FLOOD") != nullptr;
-        long long* prof = nullptr;
-        if (par_prof) { prof = ws<long long>(c, (size_t)c->sm_count * WP_WARPS * 6); if (!prof) return TISEG_ERR_CUDA; }
-        TISEG_LAUNCH_AS(c, "k_ws_flood_par", (k_ws_flood_par<MASKED>), c->sm_count, 32 * WP_WARPS, WP_SMEM_BYTES, g, image, bm, b,
-                        wk, next, gheads, out, prof);
-        if (par_prof) {                           // diagnostics only (synchronises)
-            int hh[WK_INTS];
-            TISEG_CHECK(cudaMemcpyAsync(hh, ints, sizeof(hh), cudaMemcpyDeviceToHost, c->stream));
-            std::vector<long long> hp((size_t)c->sm_count * WP_WARPS * 6);
-            TISEG_CHECK(cudaMemcpyAsync(hp.data(), prof, hp.size() * sizeof(long long), cudaMemcpyDeviceToHost, c->stream));
-            TISEG_CHECK(cudaStreamSynchronize(c->stream));
-            fprintf(stderr, "[tiseg flood par] N=%d classes:", g.N);
-            for (int k = 0; k < WS_MAXCLS; ++k) fprintf(stderr, " %d", hh[k]);
-            fprintf(stderr, " | general: %d\n", hh[4 * WS_MAXCLS]);
-            long long sum[6] = {0, 0, 0, 0, 0, 0}, mx[6] = {0, 0, 0, 0, 0, 0};
-            for (size_t i = 0; i < hp.size(); ++i) { sum[i % 6] += hp[i]; if (hp[i] > mx[i % 6]) mx[i % 6] = hp[i]; }
-            const double nw = (double)c->sm_count * WP_WARPS;
-            fprintf(stderr, "[tiseg flood par] per-warp cycles mean (max): general %.0f (%lld) stage %.0f (%lld) prepare %.0f (%lld) flood %.0f (%lld) writeback %.0f (%lld) total %.0f (%lld)\n",
-                    sum[0] / nw, mx[0], sum[1] / nw, mx[1], sum[2] / nw, mx[2], sum[3] / nw, mx[3], sum[4] / nw, mx[4], sum[5] / nw, mx[5]);
-        }
-        return TISEG_OK;
+    static_assert(WP_SMEM_BYTES + 64 <= 232448, "shared memory");
+    TISEG_LAUNCH(c, k_flood_count, dim3(8, g.N), 256, 0, b, g.W, wk, WP_ARENA, WS_MAXCLS);
+    TISEG_LAUNCH(c, k_flood_offsets, 1, 32, 0, wk);
+    TISEG_LAUNCH(c, k_flood_scatter, dim3(8, g.N), 256, 0, b, g.W, wk, WP_ARENA, WS_MAXCLS, (long long)WP_GEN_CAP, MASKED ? huge : (int*)nullptr);
+    // mask mode: the label map holds the seeds and is otherwise unwritten; the flood in global memory reads it
+    if (MASKED) {
+        Geom gh = listed_geom(g, huge + N, huge + 2 * N);
+        const BitPlanes mp = {const_cast<unsigned*>(bm.mask_bits), nullptr, nullptr, nullptr, nullptr};
+        TISEG_LAUNCH(c, k_huge_clean, dim3((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), 1), TISEG_THREADS, 0,
+                     gh, mp, bm.bpar, bm.brank, b, bm.seed_bits, (long long)WP_GEN_CAP, out);
     }
-    switch (variant) {            // lane-per-blob flood; arena geometries kept for tuning on other blob-size distributions
-        case 1: return flood_launch<13, 3840, 16, MASKED>(c, g, image, bm, b, wk, next, gheads, out, ints, debug);
-        case 2: return flood_launch<12, 4096, 16, MASKED>(c, g, image, bm, b, wk, next, gheads, out, ints, debug);
-        case 3: return flood_launch<10, 5120, 16, MASKED>(c, g, image, bm, b, wk, next, gheads, out, ints, debug);
-        case 4: return flood_launch<12, 4224, 12, MASKED>(c, g, image, bm, b, wk, next, gheads, out, ints, debug);
-        default: return flood_launch<12, 4224, 16, MASKED>(c, g, image, bm, b, wk, next, gheads, out, ints, debug);
+    static bool attr_set = false;
+    if (!attr_set) {
+        TISEG_CHECK(cudaFuncSetAttribute(k_ws_flood_par<MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WP_SMEM_BYTES));
+        attr_set = true;
     }
+    TISEG_LAUNCH_AS(c, "k_ws_flood_par", (k_ws_flood_par<MASKED>), c->sm_count, 32 * WP_WARPS, WP_SMEM_BYTES, g, image, bm, b,
+                    wk, next, gheads, out);
+    return TISEG_OK;
 }
 
 int watershed_u8_dev(tiseg_ctx* c, const Geom& g, const uint8_t* image, const int* par, const int* rank,
@@ -1628,17 +1335,8 @@ int watershed_f64_dev(tiseg_ctx* c, const Geom& g, const double* image, const in
                       const BlobInfo& b, int32_t* out) {
     (void)rank;
     const int N = g.N;
-    static const bool heap_only = getenv("TISEG_F64_HEAP") != nullptr;       // the global-memory heap flood for everything
     HeapItem* heap = ws<HeapItem>(c, (size_t)N * g.P);
     if (!heap || !b.off) return TISEG_ERR_CUDA;
-    if (heap_only) {
-        int* queue = ws<int>(c, (size_t)N);
-        if (!queue) return TISEG_ERR_CUDA;
-        TISEG_TRY(zero(c, queue, (size_t)N * sizeof(int)));
-        TISEG_LAUNCH(c, k_ws_flood_f64, dim3(flood_blocks(c, N), N), TISEG_THREADS, 0, g, image, par, b, queue,
-                     (const long long*)nullptr, (const int*)nullptr, heap, out);
-        return TISEG_OK;
-    }
     // ranked levels per blob, then the bucket flood in shared memory
     constexpr int WARPS = 7, ARENA = 3840, SLOTS = 16;
     constexpr size_t MULTI = (size_t)WARPS * ARENA * 8, GEN = (size_t)WR_GEN_CAP * 8;

@@ -9,10 +9,14 @@
 // global order to one blob is the order of that blob flooded alone.  One warp owns one blob at a time
 // (dynamic work queue per tile), so parallelism comes from the ~10^3 blobs per 1000^2 tile times the tiles
 // of the batch.
-//   uint8 images (DIST):   256 FIFO buckets (head/tail in shared memory, links in a global `next` array)
-//                          reproduce the (value, age) heap order exactly.
-//   fp64 images (HoVer):   per-blob binary heap keyed (value, age) in a global arena slice sized by the
-//                          blob's area.
+//   uint8 images (DIST):   k_ws_flood_par stages each blob in shared memory, and one warp floods it from one
+//                          array queue per level, popping up to 32 entries of the current level per step with
+//                          the sequential result.  A blob too large for shared memory is flooded in global
+//                          memory by one lane (flood_blob_global: 256 FIFO buckets, links in a global `next`).
+//   fp64 images (HoVer):   k_rank_blobs replaces each blob's values by their dense ranks, then k_ws_flood_ranked
+//                          floods the staged blob from FIFO buckets in shared memory, one lane per blob.  A blob
+//                          too large to rank or stage is flooded by k_ws_flood_f64: a binary heap keyed
+//                          (value, age) in a global arena slice sized by the blob's area.
 #pragma once
 #include "bitccl.cuh"
 #include "ccl.cuh"
