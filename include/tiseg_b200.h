@@ -17,7 +17,7 @@
  * A call with a host output synchronises anyway and reports them itself; a call with device outputs only returns
  * before execution, and the error is reported by the next call on the context that synchronises (any call with a
  * host output, or tiseg_synchronize).  No call decides anything on the host in the middle of its kernels, except
- * tiseg_reconstruction_erosion_u8 / tiseg_postproc_dist_lambda with lamb > 0 (iteration to a fixed point).
+ * tiseg_reconstruction_erosion_u8 / tiseg_postproc_dist_lambda_typed with lamb > 0 (iteration to a fixed point).
  */
 #ifndef TISEG_B200_H
 #define TISEG_B200_H
@@ -34,11 +34,13 @@ extern "C" {
 #define TISEG_ERR_NOGPU 3  /* no CUDA device: there is no CPU fallback                        */
 #define TISEG_ERR_LIMIT 4  /* a data-dependent limit was exceeded (instance id out of range)  */
 
-/* Element type of the network outputs handed to a *_typed entry (logits, distance / HV / foreground maps, direction and
- * point heads).  All network inputs of one call share it.  Half-precision inputs are converted to fp32 as they are loaded
- * and the arithmetic after the load is the fp32 path's, so a call fed fp16 / bf16 returns the bits the same call returns
- * for the fp32 upcast of its inputs, at half the input bytes (a host buffer crosses PCIe at 2 B per element).  Outputs
- * keep their types: probabilities and means stay fp32.  Another code returns TISEG_ERR_ARG. */
+/* Element type of the network outputs (logits, distance / HV / foreground maps, direction and point heads) handed to
+ * the entries whose second argument is `dtype`: tiseg_softmax_argmax_typed, tiseg_softmax_argmax_tta_typed,
+ * tiseg_tta_mean_typed, tiseg_postproc_dist_lambda_typed, tiseg_postproc_hover_ex, tiseg_cdnet_refine_typed and
+ * tiseg_mtcdnet_refine_typed.  All network inputs of one call share it.  Half-precision inputs are converted to fp32 as
+ * they are loaded and the arithmetic after the load is the fp32 path's, so a call fed fp16 / bf16 returns the bits the
+ * same call returns for the fp32 upcast of its inputs, at half the input bytes (a host buffer crosses PCIe at 2 B per
+ * element).  Outputs keep their types: probabilities and means stay fp32.  Another code returns TISEG_ERR_ARG. */
 #define TISEG_DTYPE_F32 0
 #define TISEG_DTYPE_F16 1
 #define TISEG_DTYPE_BF16 2
@@ -67,11 +69,8 @@ int tiseg_timing_report(tiseg_ctx* ctx, char* buf, int cap);
 /* ---- A1: softmax / TTA mean / argmax ---------------------------------------------------------
  * tiseg/models/segmentors/base.py:321-339 (F.softmax per TTA variant, sum/len, resize == identity
  * at ori_hw) followed by `sem_logit.argmax(dim=1)` (unet.py:62, dist.py:266, hovernet.py:271).
- * logits [N, T, C, H, W] fp32; prob [N, C, H, W] fp32 or NULL; cls [N, H, W] uint8 or NULL
- * (first maximum wins, like torch.argmax). */
-int tiseg_softmax_argmax(tiseg_ctx* ctx, const float* logits, int N, int T, int C, int H, int W,
-                         float* prob, uint8_t* cls);
-/* the same with logits of element type `dtype` (TISEG_DTYPE_*); tiseg_softmax_argmax is this with TISEG_DTYPE_F32 */
+ * logits [N, T, C, H, W] of element type `dtype` (TISEG_DTYPE_*); prob [N, C, H, W] fp32 or NULL; cls [N, H, W] uint8
+ * or NULL (first maximum wins, like torch.argmax). */
 int tiseg_softmax_argmax_typed(tiseg_ctx* ctx, int dtype, const void* logits, int N, int T, int C, int H, int W,
                                float* prob, uint8_t* cls);
 
@@ -83,18 +82,13 @@ int tiseg_softmax_argmax_typed(tiseg_ctx* ctx, int dtype, const void* logits, in
  * (window = 0; (Ht, Wt) = (W, H) for 90/270 degrees) or its windows [My*Mx, C, window, window] in the row-major
  * order split_inference visits them.  tiseg_tta_input_elems gives the elements per tile.  H, W: the original image. */
 long long tiseg_tta_input_elems(int T, int C, int H, int W, const int* rotate_degrees, int window, int overlap);
-int tiseg_softmax_argmax_tta(tiseg_ctx* ctx, const float* logits, int N, int T, int C, int H, int W,
-                             const int* rotate_degrees, const int* flips, int window, int overlap,
-                             float* prob, uint8_t* cls);
 int tiseg_softmax_argmax_tta_typed(tiseg_ctx* ctx, int dtype, const void* logits, int N, int T, int C, int H, int W,
                                    const int* rotate_degrees, const int* flips, int window, int overlap,
                                    float* prob, uint8_t* cls);
 
 /* The plain (no softmax) TTA mean of a regression head with the same stitch + reverse-transform indexing:
  * `sum(dist_logit_list) / len(dist_logit_list)` of dist.py:398-410; hovernet.py:406 keeps variant 0 only (T = 1).
- * maps laid out like the logits of tiseg_softmax_argmax_tta; mean_out [N, C, H, W]. */
-int tiseg_tta_mean(tiseg_ctx* ctx, const float* maps, int N, int T, int C, int H, int W, const int* rotate_degrees,
-                   const int* flips, int window, int overlap, float* mean_out);
+ * maps laid out like the logits of tiseg_softmax_argmax_tta_typed; mean_out [N, C, H, W]. */
 int tiseg_tta_mean_typed(tiseg_ctx* ctx, int dtype, const void* maps, int N, int T, int C, int H, int W,
                          const int* rotate_degrees, const int* flips, int window, int overlap, float* mean_out);
 
@@ -154,16 +148,12 @@ int tiseg_watershed_f64(tiseg_ctx* ctx, const double* image, const int32_t* mark
                         int N, int H, int W, int32_t* out);
 
 /* ---- A8: DIST postprocess (dist.py:275-284 -> dynamic_watershed_alias :114-129) ---------------------
- * dist [N,H,W] fp32 raw distance-head output; inst_out [N,H,W] int32 (the reference returns int64
- * with the same values).  Optional debug outputs (NULL to skip): markers int32, ws int32 (raw flood). */
-int tiseg_postproc_dist(tiseg_ctx* ctx, const float* dist, int N, int H, int W, int32_t* inst_out,
-                        int32_t* markers_out, int32_t* ws_out);
-/* The same with the paper's p1 ("lamb" of dynamic_watershed_alias, dist.py:114; the reference's test path passes 0.0,
- * dist.py:281): markers and flood levels come from Hrecons = reconstruction_by_erosion(min(255, I + lamb), I).
- * lamb > 0 runs an iterative reconstruction that synchronises with the host between sweeps. */
-int tiseg_postproc_dist_lambda(tiseg_ctx* ctx, const float* dist, int N, int H, int W, int lamb, int32_t* inst_out,
-                               int32_t* markers_out, int32_t* ws_out);
-/* dist of element type `dtype` (TISEG_DTYPE_*): the distance map is read once, by the step that truncates it to levels */
+ * dist [N,H,W] raw distance-head output of element type `dtype` (TISEG_DTYPE_*), read once, by the step that truncates
+ * it to levels; inst_out [N,H,W] int32 (the reference returns int64 with the same values).  Optional debug outputs
+ * (NULL to skip): markers int32, ws int32 (raw flood).  lamb is the paper's p1 ("lamb" of dynamic_watershed_alias,
+ * dist.py:114; the reference's test path passes 0.0, dist.py:281): markers and flood levels come from
+ * Hrecons = reconstruction_by_erosion(min(255, I + lamb), I).  lamb > 0 runs an iterative reconstruction that
+ * synchronises with the host between sweeps. */
 int tiseg_postproc_dist_lambda_typed(tiseg_ctx* ctx, int dtype, const void* dist, int N, int H, int W, int lamb,
                                      int32_t* inst_out, int32_t* markers_out, int32_t* ws_out);
 
@@ -173,23 +163,17 @@ int tiseg_reconstruction_erosion_u8(tiseg_ctx* ctx, const uint8_t* seed, const u
                                     uint8_t* out);
 
 /* ---- A11: HoVer-Net post-process (hovernet.py:283-365, hover_post_proc(fore_map, hv_map, fx, scale_factor)) ----
- * fore_map [N,H,W] fp32 (softmax channel 1 of the foreground head), hv_map [N,H,W,2] fp32 HWC (horizontal,
- * vertical) as the reference passes them after permute(0,2,3,1).  scale_factor: 1 (the MoNuSeg / CoNSeP configs)
- * or 2 (the CoNIC config: cv2.resize x2 bilinear in, the whole chain at 2H x 2W, INTER_NEAREST back).
+ * fore_map [N,H,W] (softmax channel 1 of the foreground head), hv_map [N,H,W,2] HWC (horizontal, vertical) as the
+ * reference passes them after permute(0,2,3,1), both of element type `dtype` (TISEG_DTYPE_*); with scale_factor 2 the
+ * resize reads them and the chain after it runs on fp32.  scale_factor: 1 (the MoNuSeg / CoNSeP configs) or 2 (the
+ * CoNIC config: cv2.resize x2 bilinear in, the whole chain at 2H x 2W, INTER_NEAREST back).
  * inst_out [N,H,W] int32.  Optional debug outputs (NULL to skip), at the SCALED size [N, sH, sW]: blb uint8,
- * dist fp64 (the flooded image), marker int32.  This entry runs fx = 1 (Sobel ksize 21, marker obj_size 10). */
-int tiseg_postproc_hover(tiseg_ctx* ctx, const float* fore_map, const float* hv_map, int N, int H, int W,
-                         int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out, int32_t* marker_out);
-/* fore_map and hv_map of element type `dtype` (TISEG_DTYPE_*); with scale_factor 2 the resize reads them and the chain
- * after it runs on fp32 as above.  fx = 1: tiseg_postproc_hover_ex with ksize 21 and obj_size 10. */
-int tiseg_postproc_hover_typed(tiseg_ctx* ctx, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
-                               int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
-                               int32_t* marker_out);
-/* Any fx of the reference, given as the two integers it derives from fx: ksize = int(20 * fx + 1), the Sobel kernel
+ * dist fp64 (the flooded image), marker int32.
+ * fx is given as the two integers the reference derives from it: ksize = int(20 * fx + 1), the Sobel kernel
  * size (odd, 1..31: the sizes cv2.Sobel accepts; ksize 1 is the 3-tap derivative without smoothing), and
- * obj_size = ceil(10 * fx^2), the size below which a marker is dropped (>= 0; 0 and 1 drop none).  The blb mask keeps
- * its fixed min_size 10, as in the reference.  TISEG_ERR_ARG for an even or out-of-range ksize, a negative obj_size
- * or a scale_factor other than 1 or 2. */
+ * obj_size = ceil(10 * fx^2), the size below which a marker is dropped (>= 0; 0 and 1 drop none); the reference's
+ * default fx = 1 is ksize 21, obj_size 10.  The blb mask keeps its fixed min_size 10, as in the reference.
+ * TISEG_ERR_ARG for an even or out-of-range ksize, a negative obj_size or a scale_factor other than 1 or 2. */
 int tiseg_postproc_hover_ex(tiseg_ctx* ctx, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
                             int scale_factor, int ksize, int obj_size, int32_t* inst_out, uint8_t* blb_out,
                             double* dist_out, int32_t* marker_out);
@@ -199,13 +183,10 @@ int tiseg_postproc_hover_ex(tiseg_ctx* ctx, int dtype, const void* fore_map, con
  * dir_map [N,H,W] uint8 (0 = background, 1..8 directions) -> dd [N,H,W] fp32 in {0, 0.5, 1}. */
 int tiseg_ddm(tiseg_ctx* ctx, const uint8_t* dir_map, int N, int H, int W, float* dd);
 /* The tail of CDNet.inference after the CNN (cdnet.py:183-217) including _ddm_enhencement (:354-367):
- * sem_logits [N,T,C,H,W], dir_logits [N,T,D=9,H,W], point_logits [N,T,1,H,W] raw fp32 head outputs of the T
- * TTA variants.  Outputs (any may be NULL): sem_prob_out [N,C,H,W] refined probabilities, cls_out [N,H,W]
- * their argmax, dir_map_out [N,H,W] direction map of variant 0, dd_out [N,H,W] mean DDM. */
-int tiseg_cdnet_refine(tiseg_ctx* ctx, const float* sem_logits, const float* dir_logits, const float* point_logits,
-                       int N, int T, int C, int D, int H, int W, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
-                       uint8_t* dir_map_out, float* dd_out);
-/* the three heads of element type `dtype` (TISEG_DTYPE_*); the outputs are as above (sem_prob_out stays fp32) */
+ * sem_logits [N,T,C,H,W], dir_logits [N,T,D=9,H,W], point_logits [N,T,1,H,W] raw head outputs of the T TTA
+ * variants, of element type `dtype` (TISEG_DTYPE_*).  Outputs (any may be NULL): sem_prob_out [N,C,H,W] refined fp32
+ * probabilities, cls_out [N,H,W] their argmax, dir_map_out [N,H,W] direction map of variant 0, dd_out [N,H,W] mean
+ * DDM. */
 int tiseg_cdnet_refine_typed(tiseg_ctx* ctx, int dtype, const void* sem_logits, const void* dir_logits,
                              const void* point_logits, int N, int T, int C, int D, int H, int W, int if_ddm,
                              float* sem_prob_out, uint8_t* cls_out, uint8_t* dir_map_out, float* dd_out);
@@ -218,14 +199,10 @@ int tiseg_ddm_enhance(tiseg_ctx* ctx, float* sem_prob, const float* dd, const fl
  * is 1 + the class of the clamped angle with eight angles, 0 on the background of the mean tc map, :304-315): softmax +
  * TTA mean of the three-class (tc) and semantic heads, TTA mean of the point head, per variant dir[:,0] *= tc[:,0] ->
  * argmax -> DDM, mean DDM, its own _ddm_enhencement (:548-564) on the tc probabilities.  tc_logits [N,T,Ctc,H,W],
- * sem_logits [N,T,Csem,H,W], dir_logits [N,T,9,H,W], point_logits [N,T,1,H,W].  Outputs (any may be NULL): tc_prob_out
- * [N,Ctc,H,W] refined, tc_cls_out / sem_cls_out [N,H,W] the argmax maps postprocess consumes (:209-213), sem_prob_out
- * [N,Csem,H,W], dir_map_out [N,H,W] direction map of variant 0, dd_out [N,H,W]. */
-int tiseg_mtcdnet_refine(tiseg_ctx* ctx, const float* tc_logits, const float* sem_logits, const float* dir_logits,
-                         const float* point_logits, int N, int T, int Ctc, int Csem, int D, int H, int W, int if_ddm,
-                         float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
-                         uint8_t* dir_map_out, float* dd_out);
-/* the four heads of element type `dtype` (TISEG_DTYPE_*); the outputs are as above */
+ * sem_logits [N,T,Csem,H,W], dir_logits [N,T,9,H,W], point_logits [N,T,1,H,W], the four heads of element type `dtype`
+ * (TISEG_DTYPE_*).  Outputs (any may be NULL): tc_prob_out [N,Ctc,H,W] refined, tc_cls_out / sem_cls_out [N,H,W] the
+ * argmax maps postprocess consumes (:209-213), sem_prob_out [N,Csem,H,W], dir_map_out [N,H,W] direction map of
+ * variant 0, dd_out [N,H,W]. */
 int tiseg_mtcdnet_refine_typed(tiseg_ctx* ctx, int dtype, const void* tc_logits, const void* sem_logits,
                                const void* dir_logits, const void* point_logits, int N, int T, int Ctc, int Csem, int D,
                                int H, int W, int if_ddm, float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out,
@@ -246,11 +223,9 @@ int tiseg_postproc_multitask(tiseg_ctx* ctx, const uint8_t* inner, const uint8_t
 /* ---- A16 / A17: pre_eval_bin_aji + pre_eval_bin_pq (inst_metrics.py:10-92, 138-229) ---------------
  * pred / gt [N,H,W] int32 instance maps with arbitrary ids (the relabelling the reference does with
  * re_instance + measure.label is done inside).  aji [N,2] fp64 = (overall_inter, overall_union);
- * pq [N,4] fp64 = (tp, fp, fn, iou_sum).  Either output may be NULL.  match_iou is the reference default 0.5 (the
- * Hungarian branch for match_iou < 0.5 is reached by no caller of the reference and is not built). */
-int tiseg_pair_metrics_bin(tiseg_ctx* ctx, const int32_t* pred, const int32_t* gt, int N, int H, int W,
-                           double* aji, double* pq);
-/* the same with pre_eval_bin_pq's match_iou (>= 0.5; a pair matches when iou > match_iou, inst_metrics.py:197-203) */
+ * pq [N,4] fp64 = (tp, fp, fn, iou_sum).  Either output may be NULL.  match_iou is pre_eval_bin_pq's (reference
+ * default 0.5; a pair matches when iou > match_iou, inst_metrics.py:197-203); it must be >= 0.5 (the Hungarian branch
+ * for match_iou < 0.5 is reached by no caller of the reference and is not built). */
 int tiseg_pair_metrics_bin_iou(tiseg_ctx* ctx, const int32_t* pred, const int32_t* gt, int N, int H, int W, double match_iou,
                                double* aji, double* pq);
 /* the same with the ground truth shipped as uint16 (ids below 65536: every dataset the reference converts,
@@ -263,7 +238,7 @@ int tiseg_pair_metrics_bin_u16gt(tiseg_ctx* ctx, const int32_t* pred, const uint
  * pre_eval_pq (inst_metrics.py:95-135, 232-280), and optionally the binary records, from ONE pair table.
  * *_inst int32 (ids < max(H*W+1, 65536)), *_sem uint8, C = number of classes incl. background.
  * aji [N,C,2], pq [N,C,4] fp64 with slot 0 = the reference's class-0 slot (dropped by reduce_zero_label);
- * bin_aji [N,2], bin_pq [N,4] as tiseg_pair_metrics_bin.  Any output may be NULL. */
+ * bin_aji [N,2], bin_pq [N,4] as tiseg_pair_metrics_bin_iou with match_iou 0.5.  Any output may be NULL. */
 int tiseg_pair_metrics_multiclass(tiseg_ctx* ctx, const int32_t* pred_inst, const uint8_t* pred_sem,
                                   const int32_t* gt_inst, const uint8_t* gt_sem, int N, int H, int W, int C,
                                   double* aji, double* pq, double* bin_aji, double* bin_pq);

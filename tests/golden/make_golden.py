@@ -480,7 +480,7 @@ def main():
 
     # ---- BaseSegmentor.inference (base.py:255-381): window canvas + TTA + reverse + softmax + mean, from source.
     # `self.calculate` is a recorder that returns seeded logits for every window it is asked for; the recorded windows
-    # are what the fused kernel (tiseg_softmax_argmax_tta) is given.
+    # are what the fused kernel (tiseg_softmax_argmax_tta_typed) is given.
     import torch.nn.functional as F
     benv = {"torch": torch, "F": F, "resize": None}
     b_inference = ref_method("tiseg/models/segmentors/base.py", "BaseSegmentor", "inference", benv)

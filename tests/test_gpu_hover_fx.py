@@ -110,14 +110,13 @@ def _call(name, fore, hv, sf, *extra):
     return inst, blb, dist, mk
 
 
-def test_fx_1_is_the_typed_entry():
+def test_fx_1_is_ksize_21_obj_size_10():
     maps = [_maps(250, 131, 40 + j) for j in range(2)]
     fore, hv = np.stack([m[0] for m in maps]), np.stack([m[1] for m in maps])
     for sf in (1, 2):
-        typed = _call("tiseg_postproc_hover_typed", fore, hv, sf)
-        _same(_call("tiseg_postproc_hover_ex", fore, hv, sf, 21, 10), typed, "ex(21, 10) scale %d" % sf)
-        _same(ops.postproc_hover(fore, hv, scale_factor=sf, debug=True, fx=1), typed, "fx=1 scale %d" % sf)
-        _same(ops.postproc_hover(fore, hv, scale_factor=sf, debug=True), typed, "default fx scale %d" % sf)
+        ex = _call("tiseg_postproc_hover_ex", fore, hv, sf, 21, 10)
+        _same(ops.postproc_hover(fore, hv, scale_factor=sf, debug=True, fx=1), ex, "fx=1 vs ex(21, 10) scale %d" % sf)
+        _same(ops.postproc_hover(fore, hv, scale_factor=sf, debug=True), ex, "default fx vs ex(21, 10) scale %d" % sf)
 
 
 def test_reference_api_hover_post_proc():

@@ -747,7 +747,7 @@ def test_label_makers_degenerate_geometry():
 
 
 def test_postproc_dist_matches_reference_source_golden():
-    """tiseg_postproc_dist vs the outputs of the reference's own dist.py source text (tests/golden/dist_ref.npz)."""
+    """tiseg_postproc_dist_lambda_typed vs the outputs of the reference's own dist.py source text (tests/golden/dist_ref.npz)."""
     m = np.load(os.path.join(G, "dist_ref.npz"))
     for j in range(4):
         _diff(ops.postproc_dist(m["d%d_in" % j]), m["d%d_out" % j], "dist inst (reference source golden %d)" % j)

@@ -26,15 +26,11 @@ SIGNATURES = {
     "tiseg_build_hash": [],
     "tiseg_timing_enable": [_vp, _i],
     "tiseg_timing_report": [_vp, ctypes.c_char_p, _i],
-    "tiseg_softmax_argmax": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_softmax_argmax_typed": [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_tta_input_elems": [_i, _i, _i, _i, _vp, _i, _i],
-    "tiseg_softmax_argmax_tta": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp],
     "tiseg_softmax_argmax_tta_typed": [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp],
-    "tiseg_tta_mean": [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp],
     "tiseg_tta_mean_typed": [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp],
     "tiseg_ddm_enhance": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i],
-    "tiseg_mtcdnet_refine": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp],
     "tiseg_mtcdnet_refine_typed": [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp],
     "tiseg_pair_metrics_bin_iou": [_vp, _vp, _vp, _i, _i, _i, ctypes.c_double, _vp, _vp],
     "tiseg_pair_metrics_bin_u16gt": [_vp, _vp, _vp, _i, _i, _i, ctypes.c_double, _vp, _vp],
@@ -49,19 +45,13 @@ SIGNATURES = {
     "tiseg_postproc_unet": [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp],
     "tiseg_watershed_u8": [_vp, _vp, _vp, _vp, _i, _i, _i, _vp],
     "tiseg_watershed_f64": [_vp, _vp, _vp, _vp, _i, _i, _i, _vp],
-    "tiseg_postproc_dist": [_vp, _vp, _i, _i, _i, _vp, _vp, _vp],
-    "tiseg_postproc_dist_lambda": [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp],
     "tiseg_postproc_dist_lambda_typed": [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp],
     "tiseg_reconstruction_erosion_u8": [_vp, _vp, _vp, _i, _i, _i, _vp],
-    "tiseg_postproc_hover": [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
-    "tiseg_postproc_hover_typed": [_vp, _i, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_postproc_hover_ex": [_vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_ddm": [_vp, _vp, _i, _i, _i, _vp],
-    "tiseg_cdnet_refine": [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_cdnet_refine_typed": [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_align_foreground": [_vp, _vp, _vp, _i, _i, _i, _i],
     "tiseg_postproc_multitask": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
-    "tiseg_pair_metrics_bin": [_vp, _vp, _vp, _i, _i, _i, _vp, _vp],
     "tiseg_pair_metrics_multiclass": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_sem_counts": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_assign_sem_class": [_vp, _vp, _vp, _i, _i, _i, _i, _vp],
@@ -260,7 +250,7 @@ def as_input(a, dtype):
     return np.ascontiguousarray(a, dtype=dtype)
 
 
-# element type codes of the network outputs a *_typed entry reads (TISEG_DTYPE_* in tiseg_b200.h)
+# element type codes of the network outputs an entry with a dtype argument reads (TISEG_DTYPE_* in tiseg_b200.h)
 DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
 
 

@@ -1,6 +1,7 @@
 // K9 — CDNet direction-guided refinement.
 //   tiseg_ddm           generate_direction_differential_map (tiseg/models/utils/direct_diff_map.py:95-167), 9 classes
-//   tiseg_cdnet_refine  the tail of CDNet.inference after the CNN (tiseg/models/segmentors/cdnet.py:183-217):
+//   tiseg_cdnet_refine_typed
+//                       the tail of CDNet.inference after the CNN (tiseg/models/segmentors/cdnet.py:183-217):
 //                       softmax + TTA mean of the semantic head, TTA mean of the point head, per variant
 //                       dir[:,0] *= sem[:,0] -> argmax -> DDM, mean DDM, _ddm_enhencement (cdnet.py:354-367), argmax.
 // The reference does this with ~60 ATen launches per TTA variant (8 torch.roll temporaries); here the DDM is one
@@ -269,9 +270,9 @@ extern "C" {
 int tiseg_cdnet_refine_typed(tiseg_ctx* c, int dtype, const void* sem_logits, const void* dir_logits, const void* point_logits,
                              int N, int T, int C, int D, int H, int W, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
                              uint8_t* dir_map_out, float* dd_out) {
-    TISEG_TRY(check_dtype(dtype, "tiseg_cdnet_refine"));
+    TISEG_TRY(check_dtype(dtype, "tiseg_cdnet_refine_typed"));
     if (!c || !sem_logits || !dir_logits || !point_logits || T <= 0 || C < 2 || C > 16 || D != 9) {
-        set_error("tiseg_cdnet_refine: bad argument (2 <= C <= 16, D == 9)");
+        set_error("tiseg_cdnet_refine_typed: bad argument (2 <= C <= 16, D == 9)");
         return TISEG_ERR_ARG;
     }
     TISEG_TRY(check_geom(N * T, H, W));
@@ -301,13 +302,6 @@ int tiseg_cdnet_refine_typed(tiseg_ctx* c, int dtype, const void* sem_logits, co
         TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
     }
     return end_call(c);
-}
-
-int tiseg_cdnet_refine(tiseg_ctx* c, const float* sem_logits, const float* dir_logits, const float* point_logits,
-                       int N, int T, int C, int D, int H, int W, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
-                       uint8_t* dir_map_out, float* dd_out) {
-    return tiseg_cdnet_refine_typed(c, TISEG_DTYPE_F32, sem_logits, dir_logits, point_logits, N, T, C, D, H, W, if_ddm, sem_prob_out,
-                                    cls_out, dir_map_out, dd_out);
 }
 
 int tiseg_ddm_enhance(tiseg_ctx* c, float* sem_prob, const float* dd, const float* point, int N, int C, int H, int W, int mode) {
@@ -397,10 +391,10 @@ int tiseg_mtcdnet_refine_typed(tiseg_ctx* c, int dtype, const void* tc_logits, c
                                const void* point_logits, int N, int T, int Ctc, int Csem, int D, int H, int W, int if_ddm,
                                float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
                                uint8_t* dir_map_out, float* dd_out) {
-    TISEG_TRY(check_dtype(dtype, "tiseg_mtcdnet_refine"));
+    TISEG_TRY(check_dtype(dtype, "tiseg_mtcdnet_refine_typed"));
     if (!c || !tc_logits || !sem_logits || !dir_logits || !point_logits || T <= 0 || Ctc < 2 || Ctc > 16 || Csem < 1 ||
         Csem > 16 || (D != 9 && D != 1)) {
-        set_error("tiseg_mtcdnet_refine: bad argument (2 <= Ctc <= 16, 1 <= Csem <= 16, D == 9, or D == 1: the regression head)");
+        set_error("tiseg_mtcdnet_refine_typed: bad argument (2 <= Ctc <= 16, 1 <= Csem <= 16, D == 9, or D == 1: the regression head)");
         return TISEG_ERR_ARG;
     }
     TISEG_TRY(check_geom(N * T, H, W));
@@ -432,14 +426,6 @@ int tiseg_mtcdnet_refine_typed(tiseg_ctx* c, int dtype, const void* tc_logits, c
         TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
     }
     return end_call(c);
-}
-
-int tiseg_mtcdnet_refine(tiseg_ctx* c, const float* tc_logits, const float* sem_logits, const float* dir_logits,
-                         const float* point_logits, int N, int T, int Ctc, int Csem, int D, int H, int W, int if_ddm,
-                         float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
-                         uint8_t* dir_map_out, float* dd_out) {
-    return tiseg_mtcdnet_refine_typed(c, TISEG_DTYPE_F32, tc_logits, sem_logits, dir_logits, point_logits, N, T, Ctc, Csem, D, H, W,
-                                      if_ddm, tc_prob_out, tc_cls_out, sem_prob_out, sem_cls_out, dir_map_out, dd_out);
 }
 
 }  // extern "C"

@@ -260,7 +260,7 @@ const char* tiseg_last_error(void) { return tiseg::g_err.c_str(); }
 
 long long tiseg_launch_count(tiseg_ctx* c) { return c ? c->launches : 0; }
 
-int tiseg_version(void) { return 200; }
+int tiseg_version(void) { return 300; }
 
 #ifndef TISEG_SRC_HASH
 #define TISEG_SRC_HASH "unknown"

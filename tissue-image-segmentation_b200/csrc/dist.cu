@@ -700,18 +700,10 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
 
 using namespace tiseg;
 
-extern "C" int tiseg_postproc_dist_lambda(tiseg_ctx* c, const float* dist, int N, int H, int W, int lamb,
-                                          int32_t* inst_out, int32_t* markers_out, int32_t* ws_out);
-
-extern "C" int tiseg_postproc_dist(tiseg_ctx* c, const float* dist, int N, int H, int W, int32_t* inst_out,
-                                   int32_t* markers_out, int32_t* ws_out) {
-    return tiseg_postproc_dist_lambda(c, dist, N, H, W, 0, inst_out, markers_out, ws_out);
-}
-
 extern "C" int tiseg_postproc_dist_lambda_typed(tiseg_ctx* c, int dtype, const void* dist, int N, int H, int W, int lamb,
                                                 int32_t* inst_out, int32_t* markers_out, int32_t* ws_out) {
-    TISEG_TRY(check_dtype(dtype, "tiseg_postproc_dist"));
-    if (!c || !dist || !inst_out || lamb < 0 || lamb > 255) { set_error("tiseg_postproc_dist: bad argument (0 <= lambda <= 255)"); return TISEG_ERR_ARG; }
+    TISEG_TRY(check_dtype(dtype, "tiseg_postproc_dist_lambda_typed"));
+    if (!c || !dist || !inst_out || lamb < 0 || lamb > 255) { set_error("tiseg_postproc_dist_lambda_typed: bad argument (0 <= lambda <= 255)"); return TISEG_ERR_ARG; }
     TISEG_TRY(check_geom(N, H, W));
     begin_call(c);
     Geom g = make_geom(N, H, W);
@@ -723,9 +715,4 @@ extern "C" int tiseg_postproc_dist_lambda_typed(tiseg_ctx* c, int dtype, const v
     if (!d_dist || !d_inst) return TISEG_ERR_CUDA;
     TISEG_TRY(postproc_dist_dev(c, g, dtype, d_dist, lamb, d_inst, d_mk, d_ws));
     return end_call(c);
-}
-
-extern "C" int tiseg_postproc_dist_lambda(tiseg_ctx* c, const float* dist, int N, int H, int W, int lamb,
-                                          int32_t* inst_out, int32_t* markers_out, int32_t* ws_out) {
-    return tiseg_postproc_dist_lambda_typed(c, TISEG_DTYPE_F32, dist, N, H, W, lamb, inst_out, markers_out, ws_out);
 }

@@ -457,19 +457,19 @@ static int postproc_hover_entry(tiseg_ctx* c, const void* fore_map, const void* 
 extern "C" int tiseg_postproc_hover_ex(tiseg_ctx* c, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
                                        int scale_factor, int ksize, int obj_size, int32_t* inst_out, uint8_t* blb_out,
                                        double* dist_out, int32_t* marker_out) {
-    TISEG_TRY(check_dtype(dtype, "tiseg_postproc_hover"));
-    if (!c || !fore_map || !hv_map || !inst_out) { set_error("tiseg_postproc_hover: bad argument"); return TISEG_ERR_ARG; }
+    TISEG_TRY(check_dtype(dtype, "tiseg_postproc_hover_ex"));
+    if (!c || !fore_map || !hv_map || !inst_out) { set_error("tiseg_postproc_hover_ex: bad argument"); return TISEG_ERR_ARG; }
     if (scale_factor != 1 && scale_factor != 2) {
-        set_error("tiseg_postproc_hover: scale_factor must be 1 or 2 (the values of the reference configs), got " +
+        set_error("tiseg_postproc_hover_ex: scale_factor must be 1 or 2 (the values of the reference configs), got " +
                   std::to_string(scale_factor));
         return TISEG_ERR_ARG;
     }
     if (ksize < 1 || ksize > 2 * SOBEL_RMAX + 1 || ksize % 2 == 0) {       // what cv2.Sobel refuses (and -1, Scharr)
-        set_error("tiseg_postproc_hover: ksize must be odd and in 1..31 (cv2.Sobel), got " + std::to_string(ksize));
+        set_error("tiseg_postproc_hover_ex: ksize must be odd and in 1..31 (cv2.Sobel), got " + std::to_string(ksize));
         return TISEG_ERR_ARG;
     }
     if (obj_size < 0) {
-        set_error("tiseg_postproc_hover: obj_size must be >= 0, got " + std::to_string(obj_size));
+        set_error("tiseg_postproc_hover_ex: obj_size must be >= 0, got " + std::to_string(obj_size));
         return TISEG_ERR_ARG;
     }
     TISEG_TRY(check_geom(N, H * scale_factor, W * scale_factor));
@@ -489,19 +489,4 @@ extern "C" int tiseg_postproc_hover_ex(tiseg_ctx* c, int dtype, const void* fore
                                                  d_mk);
     }));
     return end_call(c);
-}
-
-// fx = 1 of the reference: ksize 21, obj_size 10
-extern "C" int tiseg_postproc_hover_typed(tiseg_ctx* c, int dtype, const void* fore_map, const void* hv_map, int N, int H, int W,
-                                          int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
-                                          int32_t* marker_out) {
-    return tiseg_postproc_hover_ex(c, dtype, fore_map, hv_map, N, H, W, scale_factor, 21, 10, inst_out, blb_out, dist_out,
-                                   marker_out);
-}
-
-extern "C" int tiseg_postproc_hover(tiseg_ctx* c, const float* fore_map, const float* hv_map, int N, int H, int W,
-                                    int scale_factor, int32_t* inst_out, uint8_t* blb_out, double* dist_out,
-                                    int32_t* marker_out) {
-    return tiseg_postproc_hover_typed(c, TISEG_DTYPE_F32, fore_map, hv_map, N, H, W, scale_factor, inst_out, blb_out, dist_out,
-                                      marker_out);
 }

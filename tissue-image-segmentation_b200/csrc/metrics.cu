@@ -1,6 +1,7 @@
 // K12 / K13 — evaluation kernels: GT x pred pair-overlap histogram -> AJI and PQ, semantic counts.
 //
-//   tiseg_pair_metrics_bin  replaces pre_eval_bin_aji + pre_eval_bin_pq (tiseg/utils/inst_metrics.py:10-92,
+//   tiseg_pair_metrics_bin_iou
+//                           replaces pre_eval_bin_aji + pre_eval_bin_pq (tiseg/utils/inst_metrics.py:10-92,
 //                           138-229) including the measure.label relabelling they start with.
 //   tiseg_sem_counts        replaces pre_eval_all_semantic_metric (tiseg/utils/sem_metrics.py:16-53).
 //
@@ -771,28 +772,10 @@ int tiseg_assign_sem_class(tiseg_ctx* c, const int32_t* inst, const uint8_t* sem
     return end_call(c);
 }
 
-int tiseg_pair_metrics_bin(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, int N, int H, int W,
-                           double* aji, double* pq) {
-    return tiseg_pair_metrics_bin_iou(c, pred, gt, N, H, W, 0.5, aji, pq);
-}
-
-static int pair_metrics_bin_any(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, const uint16_t* gt16, int N, int H, int W,
-                                double match_iou, double* aji, double* pq);
-
-int tiseg_pair_metrics_bin_iou(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, int N, int H, int W, double match_iou,
-                               double* aji, double* pq) {
-    return pair_metrics_bin_any(c, pred, gt, nullptr, N, H, W, match_iou, aji, pq);
-}
-
-int tiseg_pair_metrics_bin_u16gt(tiseg_ctx* c, const int32_t* pred, const uint16_t* gt, int N, int H, int W, double match_iou,
-                                 double* aji, double* pq) {
-    return pair_metrics_bin_any(c, pred, nullptr, gt, N, H, W, match_iou, aji, pq);
-}
-
 static int pair_metrics_bin_any(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, const uint16_t* gt16, int N, int H, int W,
                                 double match_iou, double* aji, double* pq) {
     if (!c || !pred || (!gt && !gt16) || !(match_iou >= 0.5)) {
-        set_error("tiseg_pair_metrics_bin: bad argument (match_iou >= 0.5: below it the reference switches to Hungarian matching)");
+        set_error("tiseg_pair_metrics_bin_iou: bad argument (match_iou >= 0.5: below it the reference switches to Hungarian matching)");
         return TISEG_ERR_ARG;
     }
     TISEG_TRY(check_geom(N, H, W));
@@ -810,6 +793,16 @@ static int pair_metrics_bin_any(tiseg_ctx* c, const int32_t* pred, const int32_t
     ClassInfo ci = {nullptr, nullptr, nullptr, nullptr};
     TISEG_TRY(pair_eval(c, g, w, nullptr, nullptr, 2, ci, true, d_aji, d_pq, match_iou));
     return end_call(c);
+}
+
+int tiseg_pair_metrics_bin_iou(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, int N, int H, int W, double match_iou,
+                               double* aji, double* pq) {
+    return pair_metrics_bin_any(c, pred, gt, nullptr, N, H, W, match_iou, aji, pq);
+}
+
+int tiseg_pair_metrics_bin_u16gt(tiseg_ctx* c, const int32_t* pred, const uint16_t* gt, int N, int H, int W, double match_iou,
+                                 double* aji, double* pq) {
+    return pair_metrics_bin_any(c, pred, nullptr, gt, N, H, W, match_iou, aji, pq);
 }
 
 int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const uint8_t* pred_sem,

@@ -327,7 +327,7 @@ static int tta_entry(tiseg_ctx* c, int dtype, const void* logits, int N, int T, 
                      const int* flips, int window, int overlap, float* prob, uint8_t* cls, bool softmax) {
     if (!c || !logits || !rotate_degrees || !flips || T <= 0 || T > 16 || C <= 0 || C > 16 || (!prob && !cls) ||
         window < 0 || (window > 0 && (overlap < 0 || overlap >= window))) {
-        set_error("tiseg_softmax_argmax_tta: bad argument (1 <= T, C <= 16, 0 <= overlap < window)");
+        set_error("tiseg_softmax_argmax_tta_typed: bad argument (1 <= T, C <= 16, 0 <= overlap < window)");
         return TISEG_ERR_ARG;
     }
     TISEG_TRY(check_geom(N, H, W));
@@ -335,7 +335,7 @@ static int tta_entry(tiseg_ctx* c, int dtype, const void* logits, int N, int T, 
     plan.T = T; plan.window = window; plan.overlap = overlap;
     long long off = 0;
     for (int t = 0; t < T; ++t) {
-        if (rotate_degrees[t] % 90 != 0 || flips[t] < 0 || flips[t] > 3) { set_error("tiseg_softmax_argmax_tta: bad transform"); return TISEG_ERR_ARG; }
+        if (rotate_degrees[t] % 90 != 0 || flips[t] < 0 || flips[t] > 3) { set_error("tiseg_softmax_argmax_tta_typed: bad transform"); return TISEG_ERR_ARG; }
         plan.rot[t] = ((rotate_degrees[t] / 90) % 4 + 4) % 4;
         plan.flip[t] = flips[t];
         plan.off[t] = off;
@@ -357,33 +357,22 @@ static int tta_entry(tiseg_ctx* c, int dtype, const void* logits, int N, int T, 
 extern "C" int tiseg_softmax_argmax_tta_typed(tiseg_ctx* c, int dtype, const void* logits, int N, int T, int C, int H, int W,
                                               const int* rotate_degrees, const int* flips, int window, int overlap,
                                               float* prob, uint8_t* cls) {
-    TISEG_TRY(check_dtype(dtype, "tiseg_softmax_argmax_tta"));
+    TISEG_TRY(check_dtype(dtype, "tiseg_softmax_argmax_tta_typed"));
     return tta_entry(c, dtype, logits, N, T, C, H, W, rotate_degrees, flips, window, overlap, prob, cls, true);
-}
-
-extern "C" int tiseg_softmax_argmax_tta(tiseg_ctx* c, const float* logits, int N, int T, int C, int H, int W,
-                                        const int* rotate_degrees, const int* flips, int window, int overlap,
-                                        float* prob, uint8_t* cls) {
-    return tiseg_softmax_argmax_tta_typed(c, TISEG_DTYPE_F32, logits, N, T, C, H, W, rotate_degrees, flips, window, overlap, prob, cls);
 }
 
 extern "C" int tiseg_tta_mean_typed(tiseg_ctx* c, int dtype, const void* maps, int N, int T, int C, int H, int W,
                                     const int* rotate_degrees, const int* flips, int window, int overlap, float* mean_out) {
-    TISEG_TRY(check_dtype(dtype, "tiseg_tta_mean"));
-    if (!mean_out) { set_error("tiseg_tta_mean: null output"); return TISEG_ERR_ARG; }
+    TISEG_TRY(check_dtype(dtype, "tiseg_tta_mean_typed"));
+    if (!mean_out) { set_error("tiseg_tta_mean_typed: null output"); return TISEG_ERR_ARG; }
     return tta_entry(c, dtype, maps, N, T, C, H, W, rotate_degrees, flips, window, overlap, mean_out, nullptr, false);
-}
-
-extern "C" int tiseg_tta_mean(tiseg_ctx* c, const float* maps, int N, int T, int C, int H, int W, const int* rotate_degrees,
-                              const int* flips, int window, int overlap, float* mean_out) {
-    return tiseg_tta_mean_typed(c, TISEG_DTYPE_F32, maps, N, T, C, H, W, rotate_degrees, flips, window, overlap, mean_out);
 }
 
 extern "C" int tiseg_softmax_argmax_typed(tiseg_ctx* c, int dtype, const void* logits, int N, int T, int C, int H, int W,
                                           float* prob, uint8_t* cls) {
-    TISEG_TRY(check_dtype(dtype, "tiseg_softmax_argmax"));
+    TISEG_TRY(check_dtype(dtype, "tiseg_softmax_argmax_typed"));
     if (!c || !logits || T <= 0 || C <= 0 || C > 16 || (!prob && !cls)) {
-        set_error("tiseg_softmax_argmax: bad argument (1 <= C <= 16)");
+        set_error("tiseg_softmax_argmax_typed: bad argument (1 <= C <= 16)");
         return TISEG_ERR_ARG;
     }
     TISEG_TRY(check_geom(N, H, W));
@@ -396,9 +385,4 @@ extern "C" int tiseg_softmax_argmax_typed(tiseg_ctx* c, int dtype, const void* l
     if (!d_in) return TISEG_ERR_CUDA;
     TISEG_TRY(with_dtype(dtype, [&](auto z) { return softmax_argmax_dev(c, g, (const decltype(z)*)d_in, T, C, d_prob, d_cls); }));
     return end_call(c);
-}
-
-extern "C" int tiseg_softmax_argmax(tiseg_ctx* c, const float* logits, int N, int T, int C, int H, int W,
-                                    float* prob, uint8_t* cls) {
-    return tiseg_softmax_argmax_typed(c, TISEG_DTYPE_F32, logits, N, T, C, H, W, prob, cls);
 }
