@@ -98,3 +98,90 @@ def diagonal_contact(kind, k=1, anti=False):
     ((y - 1, x - 1), (y, x)) by default, down-left ((y - 1, x), (y, x - 1)) with ``anti``."""
     y, x = boundary_point(kind, k)
     return ((y - 1, x), (y, x - 1)) if anti else ((y - 1, x - 1), (y, x))
+
+
+# --------------------------------------------------------------------------- single blobs with an exact bounding box
+# for the size limits of the watershed's floods (csrc/watershed.cu), which pick a flood by the blob's bounding box framed
+# by one pixel, (h + 2) (w + 2) cells, and by its area.  tests/test_gpu_watershed.py checks their claims on the CPU.
+BLOB_SHAPES = ("box", "frame", "serpentine", "stairs", "holes")
+
+
+def framed_boxes(cells):
+    """every (h, w) whose framed box (h + 2) (w + 2) holds exactly `cells` cells, from one row to one column"""
+    return [(d - 2, cells // d - 2) for d in range(3, cells // 3 + 1) if cells % d == 0]
+
+
+def cells_at_most(limit):
+    """the largest framed-box size <= limit (a prime has no box)"""
+    c = limit
+    while not framed_boxes(c):
+        c -= 1
+    return c
+
+
+def cells_above(limit):
+    """the smallest framed-box size > limit"""
+    c = limit + 1
+    while not framed_boxes(c):
+        c += 1
+    return c
+
+
+def box_for(cells, form="square"):
+    """(h, w) with (h + 2) (w + 2) == cells: "square" (closest to square), "flat" (closest to h : w = 1 : 8), "row"
+    (h = 1) or "col" (w = 1)"""
+    boxes = framed_boxes(cells)
+    assert boxes, "no framed box holds %d cells" % cells
+    if form in ("row", "col"):
+        hw = [b for b in boxes if (b[0] if form == "row" else b[1]) == 1]
+        assert hw, "%d cells: no %s of them" % (cells, form)
+        return hw[0]
+    ratio = 1.0 if form == "square" else 0.125
+    return min(boxes, key=lambda b: (abs(np.log(b[0] / b[1] / ratio)), b[0]))
+
+
+def blob(shape, h, w):
+    """One 4-connected blob whose bounding box is exactly h x w (uint8, 1 on the blob):
+      box         solid
+      frame       a one-pixel frame (solid when h or w <= 2)
+      serpentine  full rows every other row, joined at alternate ends: about half the box
+      stairs      a 4-connected monotone staircase from corner to corner: h + w - 1 pixels
+      holes       solid with 5 x 5 holes every 8 pixels, each holding a 3 x 3 island (marked 2: a blob of its own,
+                  one pixel clear of the host all round)"""
+    s = np.zeros((h, w), np.uint8)
+    if shape == "box":
+        s[:] = 1
+    elif shape == "frame":
+        s[:] = 1
+        if h > 2 and w > 2:
+            s[1:-1, 1:-1] = 0
+    elif shape == "serpentine":
+        s[0::2, :] = 1
+        for y in range(1, h, 2):
+            s[y, w - 1 if (y // 2) % 2 == 0 else 0] = 1
+    elif shape == "stairs":
+        y = x = 0
+        s[0, 0] = 1
+        while (y, x) != (h - 1, w - 1):
+            if x < w - 1 and (y == h - 1 or (x + 1) * h <= (y + 1) * w):
+                x += 1
+            else:
+                y += 1
+            s[y, x] = 1
+    elif shape == "holes":
+        s[:] = 1
+        for y0 in range(2, h - 6, 8):
+            for x0 in range(2, w - 6, 8):
+                s[y0:y0 + 5, x0:x0 + 5] = 0
+                s[y0 + 1:y0 + 4, x0 + 1:x0 + 4] = 2
+    else:
+        raise ValueError(shape)
+    return s
+
+
+def area_blob(area, w):
+    """`area` pixels filled in raster order over rows of width w: full rows and one partial row (bounding box
+    ceil(area / w) x w for area >= w)"""
+    s = np.zeros(((area + w - 1) // w, w), np.uint8)
+    s.ravel()[:area] = 1
+    return s
