@@ -736,6 +736,29 @@ def test_mixed_batch_equals_single_tiles(kind):
 
 
 @gpu
+def test_floods_on_two_devices_in_one_process():
+    """the floods raise their shared-memory limits per device: the u8 and fp64 floods and DIST's, from CUDA tensors on
+    cuda:0 and then on cuda:1 of one process (each op takes the context of its input's device)"""
+    import torch
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two CUDA devices")
+    batches = {kind: mixed_batch(kind) for kind in ("u8", "f64")}
+    want = {kind: [sk.watershed(*(a[j] for a in b)) for j in range(len(b[0]))] for kind, b in batches.items()}
+    d = dist_batch()
+    want_dist = [opp.dist_postprocess(None, d[j], literal=False)[1] for j in range(len(d))]
+    for dev in ("cuda:0", "cuda:1"):
+        for kind, b in batches.items():
+            got = ops.watershed(*[torch.from_numpy(a).to(dev) for a in b])
+            assert got.device == torch.device(dev)
+            for j in range(len(want[kind])):
+                _diff(got[j].cpu().numpy(), want[kind][j], "%s on %s, tile %d" % (kind, dev, j))
+        got = ops.postproc_dist(torch.from_numpy(d).to(dev))
+        assert got.device == torch.device(dev)
+        for j in range(len(d)):
+            _diff(got[j].cpu().numpy(), want_dist[j], "dist on %s, tile %d" % (dev, j))
+
+
+@gpu
 def test_hover_ranked_cta_and_heap():
     fore, hv, (want, dbg) = _hover_oracle()
     inst, blb, dist, mk = ops.postproc_hover(fore, hv, debug=True)

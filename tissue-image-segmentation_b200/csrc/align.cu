@@ -128,15 +128,12 @@ extern "C" {
 
 int tiseg_align_foreground(tiseg_ctx* c, int32_t* pred, const uint8_t* foreground, int N, int H, int W, int time) {
     if (!c || !pred || !foreground) { set_error("tiseg_align_foreground: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    int32_t* d_pred = (int32_t*)inout_ptr(c, pred, total * sizeof(int32_t));
-    const uint8_t* d_fg = in(c, foreground, total);
-    if (!d_pred || !d_fg) return TISEG_ERR_CUDA;
-    TISEG_TRY(align_foreground_dev(c, g, d_pred, d_fg, time));
-    return end_call(c);
+    Call call(c, "tiseg_align_foreground", N, H, W);
+    int32_t* d_pred = call.inout(pred, call.total);
+    const uint8_t* d_fg = call.in(foreground, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(align_foreground_dev(c, call.g, d_pred, d_fg, time));
+    return call.finish();
 }
 
 int tiseg_postproc_multitask(tiseg_ctx* c, const uint8_t* inner, const uint8_t* sem, int N, int H, int W,
@@ -145,20 +142,18 @@ int tiseg_postproc_multitask(tiseg_ctx* c, const uint8_t* inner, const uint8_t* 
         set_error("tiseg_postproc_multitask: bad argument");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_inner = in(c, inner, total);
-    const uint8_t* d_sem = in(c, sem, total);
-    uint8_t* d_canvas = tiseg::out(c, canvas_out, total);
-    int32_t* d_inst = tiseg::out(c, inst_out, total);
-    if (!d_inner || !d_sem || !d_canvas || !d_inst) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_postproc_multitask", N, H, W);
+    const uint8_t* d_inner = call.in(inner, call.total);
+    const uint8_t* d_sem = call.in(sem, call.total);
+    uint8_t* d_canvas = call.out(canvas_out, call.total);
+    int32_t* d_inst = call.out(inst_out, call.total);
+    TISEG_TRY(call.status());
+    const Geom& g = call.g;
     TISEG_TRY(sem_canvas_dev(c, g, d_sem, max_class, d_canvas));
     // measure.label(bin_pred, connectivity=1) with the edge class zeroed (multi_task_cunet.py:99-103)
     TISEG_TRY(ccl_label(c, g, ImgEqU8Drop{d_inner, edge_id}, 1, d_inst, nullptr));
     TISEG_TRY(align_foreground_dev(c, g, d_inst, d_canvas, time));
-    return end_call(c);
+    return call.finish();
 }
 
 }  // extern "C"

@@ -77,14 +77,13 @@ __global__ void __launch_bounds__(TISEG_THREADS) k_ccl_areas(Geom g, const int* 
     FOR_QUAD_RUNS(r, k, len) atomicAdd(&area[q.base + p[k]], (int)len);
 }
 
-int ccl_flatten(tiseg_ctx* c, const Geom& g, int* par) {
+int ccl_flatten(tiseg_ctx* c, const Geom& g, int* par, const unsigned** root_bits) {
     unsigned* bits = ws<unsigned>(c, (size_t)g.N * g.H * g.SEG);
     if (!bits) return TISEG_ERR_CUDA;
     TISEG_TRY(zero(c, bits, (size_t)g.N * g.H * g.SEG * sizeof(unsigned)));
     const dim3 qg((unsigned)(((long long)((g.W + 3) / 4) * g.H + TISEG_THREADS - 1) / TISEG_THREADS), grid_tiles(g));
     TISEG_LAUNCH_TILES(c, k_ccl_flatten, g, qg, TISEG_THREADS, 0, g, par, bits, (g.W % 4 == 0) && aligned16(par));
-    c->rootblk_par = par;             // rank_roots on this forest can skip its bitmap pass
-    c->rootblk = (int*)bits;
+    if (root_bits) *root_bits = bits;
     return TISEG_OK;
 }
 
@@ -216,16 +215,6 @@ int rank_from_bits(tiseg_ctx* c, const Geom& g, const unsigned* bits, int* rank,
     return TISEG_OK;
 }
 
-int rank_roots(tiseg_ctx* c, const Geom& g, const int* par, int* rank, int* counts) {
-    if (c->rootblk_par == par && c->rootblk) {
-        // the flatten pass already left the bitmap of the roots
-        const unsigned* bits = (const unsigned*)c->rootblk;
-        c->rootblk_par = nullptr;
-        return rank_from_bits(c, g, bits, rank, counts);
-    }
-    return rank_generic(c, g, SelRoot{par}, rank, counts);
-}
-
 int apply_rank(tiseg_ctx* c, const Geom& g, const int* par, const int* rank, int32_t* out) {
     const long long P = g.P;
     const bool vec = (P % 4 == 0) && aligned16(par, out);
@@ -266,43 +255,35 @@ extern "C" {
 int tiseg_label(tiseg_ctx* c, const int32_t* img, int N, int H, int W, int32_t background, int connectivity,
                 int32_t* out, int32_t* count) {
     if (!c || !img || !out || (connectivity != 1 && connectivity != 2)) { set_error("tiseg_label: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const int32_t* d_img = in(c, img, total);
-    int32_t* d_out = tiseg::out(c, out, total);
-    int32_t* d_cnt = count ? tiseg::out(c, count, (size_t)N) : nullptr;
-    if (!d_img || !d_out) return TISEG_ERR_CUDA;
-    TISEG_TRY(ccl_label(c, g, ImgEqI32{d_img, background}, connectivity, d_out, d_cnt));
-    return end_call(c);
+    Call call(c, "tiseg_label", N, H, W);
+    const int32_t* d_img = call.in(img, call.total);
+    int32_t* d_out = call.out(out, call.total);
+    int32_t* d_cnt = call.out(count, (size_t)N);
+    TISEG_TRY(call.status());
+    TISEG_TRY(ccl_label(c, call.g, ImgEqI32{d_img, background}, connectivity, d_out, d_cnt));
+    return call.finish();
 }
 
 int tiseg_label_u8(tiseg_ctx* c, const uint8_t* img, int N, int H, int W, int32_t background, int connectivity,
                    int32_t* out, int32_t* count) {
     if (!c || !img || !out || (connectivity != 1 && connectivity != 2)) { set_error("tiseg_label_u8: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_img = in(c, img, total);
-    int32_t* d_out = tiseg::out(c, out, total);
-    int32_t* d_cnt = count ? tiseg::out(c, count, (size_t)N) : nullptr;
-    if (!d_img || !d_out) return TISEG_ERR_CUDA;
-    TISEG_TRY(ccl_label(c, g, ImgEqU8{d_img, background}, connectivity, d_out, d_cnt));
-    return end_call(c);
+    Call call(c, "tiseg_label_u8", N, H, W);
+    const uint8_t* d_img = call.in(img, call.total);
+    int32_t* d_out = call.out(out, call.total);
+    int32_t* d_cnt = call.out(count, (size_t)N);
+    TISEG_TRY(call.status());
+    TISEG_TRY(ccl_label(c, call.g, ImgEqU8{d_img, background}, connectivity, d_out, d_cnt));
+    return call.finish();
 }
 
 int tiseg_re_instance(tiseg_ctx* c, const int32_t* img, int N, int H, int W, int32_t* out, int32_t* count) {
     if (!c || !img || !out) { set_error("tiseg_re_instance: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const int32_t* d_img = in(c, img, total);
-    int32_t* d_out = tiseg::out(c, out, total);
-    int32_t* d_cnt = count ? tiseg::out(c, count, (size_t)N) : nullptr;
-    if (!d_img || !d_out) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_re_instance", N, H, W);
+    const int32_t* d_img = call.in(img, call.total);
+    int32_t* d_out = call.out(out, call.total);
+    int32_t* d_cnt = call.out(count, (size_t)N);
+    TISEG_TRY(call.status());
+    const Geom& g = call.g;
     // value axis: ids are bounded by a generous multiple of the pixel count (instance ids never exceed it
     // in the reference's datasets); larger ids are reported as an argument error rather than mis-ranked
     int vmax = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
@@ -317,7 +298,7 @@ int tiseg_re_instance(tiseg_ctx* c, const int32_t* img, int N, int H, int W, int
     Geom gv = make_geom(N, vmax / 1024, 1024);
     TISEG_TRY(rank_generic(c, gv, SelFlagU8{seen}, vr, d_cnt));
     TISEG_LAUNCH(c, k_lookup_values, warp_grid(g), TISEG_THREADS, 0, g, d_img, vr, vmax, d_out);
-    return end_call(c);
+    return call.finish();
 }
 
 }  // extern "C"

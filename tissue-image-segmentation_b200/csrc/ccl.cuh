@@ -79,7 +79,7 @@ struct ImgNonZeroI32 {          // binary: non-zero int32
 //                 per 32 pixels and ran issue-bound at 3.4 IPC, profiles/r1_ccl_local_*.)
 //   k_ccl_border  only the pixels on tile borders (~4 %) merge across tiles with global atomicMin unions.
 //   k_ccl_flatten every pixel points at its global root (lowest flat index of the component = first pixel in
-//                 raster order); also leaves the bitmap of the roots for the id ranking that usually follows.
+//                 raster order); also writes the bitmap of the roots for the id ranking that usually follows.
 // =====================================================================================================
 #define CCL_WARPS 8                     // warps per tile CTA
 #define CCL_RPW 4                       // rows per warp
@@ -294,12 +294,12 @@ __global__ void __launch_bounds__(256) k_ccl_border(Geom g, Img img, int* par) {
     FOR_TILES(LISTED, g, n) ccl_border_one<Img, CONN>(g, img, par, n, blockIdx.x * blockDim.x + threadIdx.x);
 }
 
-// flatten + bitmap of the roots; defined in ccl.cu
-int ccl_flatten(tiseg_ctx* c, const Geom& g, int* par);
+// flatten; *root_bits (if wanted) = the bitmap of the roots [N, H, SEG], arena scratch of this call; defined in ccl.cu
+int ccl_flatten(tiseg_ctx* c, const Geom& g, int* par, const unsigned** root_bits);
 
-// build + flatten.  par: [N*P] int
+// build + flatten.  par: [N*P] int; root_bits: as for ccl_flatten
 template <class Img>
-int ccl_build(tiseg_ctx* c, const Geom& g, Img img, int conn, int* par) {
+int ccl_build(tiseg_ctx* c, const Geom& g, Img img, int conn, int* par, const unsigned** root_bits = nullptr) {
     const int tilesY = (g.H + CCL_TH - 1) / CCL_TH, tilesX = (g.W + CCL_TW - 1) / CCL_TW;
     dim3 lg((unsigned)(tilesX * tilesY), grid_tiles(g));
     const int nb = (tilesY - 1) * g.W + (tilesX - 1) * g.H * (conn == 2 ? 2 : 1);
@@ -319,21 +319,17 @@ int ccl_build(tiseg_ctx* c, const Geom& g, Img img, int conn, int* par) {
         TISEG_LAUNCH(c, (k_ccl_local<Img, 2, false>), lg, 32 * CCL_WARPS, 0, g, img, par, vec);
         if (nb > 0) TISEG_LAUNCH(c, (k_ccl_border<Img, 2, false>), dim3((nb + 255) / 256, g.N), 256, 0, g, img, par);
     }
-    return ccl_flatten(c, g, par);
+    return ccl_flatten(c, g, par, root_bits);
 }
 #endif
 
 // ---- raster-order ranks ------------------------------------------------------------------------
-// Selection is a functor  __device__ bool operator()(long long gi, int idx) const  (e.g. "is a root").
+// Selection is a functor  __device__ bool operator()(long long gi, int idx) const  (e.g. "flag is set").
 // rank[gi] = 1-based raster rank among the selected pixels of its tile (written only where selected);
 // counts[n] = number selected (may be null).
 // The selection is first reduced to a BITMAP, one 32-bit ballot word per row segment (bits[n, y, seg]); ranking then
 // touches P/32 words instead of P pixels: k_rank_fused (one cluster of CTAs per tile: popcount per row, exclusive scan
 // over the rows, then one warp per row: warp scan over the row's words, one store per selected pixel).
-struct SelRoot {                // roots of a flattened forest
-    const int* par;
-    __device__ __forceinline__ bool operator()(long long gi, int idx) const { return par[gi] == idx; }
-};
 struct SelFlagU8 {
     const uint8_t* f;
     __device__ __forceinline__ bool operator()(long long gi, int) const { return f[gi] != 0; }
@@ -371,8 +367,6 @@ int rank_generic(tiseg_ctx* c, const Geom& g, Sel sel, int* rank, int* counts) {
 }
 #endif
 
-// roots of a flattened forest: rank[root] = raster rank (1-based); counts[n] = K
-int rank_roots(tiseg_ctx* c, const Geom& g, const int* par, int* rank, int* counts);
 // out[gi] = par[gi] >= 0 ? rank[par[gi]] : 0
 int apply_rank(tiseg_ctx* c, const Geom& g, const int* par, const int* rank, int32_t* out);
 // area[root] = component size (this zeroes `area` itself; valid at root positions only)
@@ -386,8 +380,9 @@ int ccl_label(tiseg_ctx* c, const Geom& g, Img img, int conn, int32_t* out, int*
     int* par = ws<int>(c, total);
     int* rank = ws<int>(c, total);
     if (!par || !rank) return TISEG_ERR_CUDA;
-    TISEG_TRY(ccl_build(c, g, img, conn, par));
-    TISEG_TRY(rank_roots(c, g, par, rank, counts));
+    const unsigned* roots;
+    TISEG_TRY(ccl_build(c, g, img, conn, par, &roots));
+    TISEG_TRY(rank_from_bits(c, g, roots, rank, counts));
     TISEG_TRY(apply_rank(c, g, par, rank, out));
 #endif
     return TISEG_OK;

@@ -232,15 +232,12 @@ extern "C" {
 
 int tiseg_ddm(tiseg_ctx* c, const uint8_t* dir_map, int N, int H, int W, float* dd) {
     if (!c || !dir_map || !dd) { set_error("tiseg_ddm: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_dir = in(c, dir_map, total);
-    float* d_dd = tiseg::out(c, dd, total);
-    if (!d_dir || !d_dd) return TISEG_ERR_CUDA;
-    TISEG_TRY(ddm_dev(c, g, d_dir, 1, d_dd));
-    return end_call(c);
+    Call call(c, "tiseg_ddm", N, H, W);
+    const uint8_t* d_dir = call.in(dir_map, call.total);
+    float* d_dd = call.out(dd, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(ddm_dev(c, call.g, d_dir, 1, d_dd));
+    return call.finish();
 }
 
 }  // extern "C"
@@ -275,21 +272,22 @@ int tiseg_cdnet_refine_typed(tiseg_ctx* c, int dtype, const void* sem_logits, co
         set_error("tiseg_cdnet_refine_typed: bad argument (2 <= C <= 16, D == 9)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N * T, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const size_t eb = dtype_bytes(dtype);
-    const void* d_sem = in_ptr(c, sem_logits, total * T * C * eb);
-    const void* d_dir = in_ptr(c, dir_logits, total * T * D * eb);
-    const void* d_pt = in_ptr(c, point_logits, total * T * eb);
-    float* d_prob = sem_prob_out ? tiseg::out(c, sem_prob_out, total * C) : ws<float>(c, total * C);
-    uint8_t* d_cls = cls_out ? tiseg::out(c, cls_out, total) : nullptr;
-    float* d_dd = dd_out ? tiseg::out(c, dd_out, total) : ws<float>(c, total);
+    Call call(c, "tiseg_cdnet_refine_typed", N, H, W, T);
+    const Geom& g = call.g;
+    const size_t total = call.total, eb = dtype_bytes(dtype);
+    const void* d_sem = call.in_bytes(sem_logits, total * T * C * eb);
+    const void* d_dir = call.in_bytes(dir_logits, total * T * D * eb);
+    const void* d_pt = call.in_bytes(point_logits, total * T * eb);
+    float* d_prob = call.out(sem_prob_out, total * C);
+    uint8_t* d_cls = call.out(cls_out, total);
+    float* d_dd = call.out(dd_out, total);
+    TISEG_TRY(call.status());
+    if (!d_prob) d_prob = ws<float>(c, total * C);         // outputs the caller does not take: scratch
+    if (!d_dd) d_dd = ws<float>(c, total);
     uint8_t* dir_all = ws<uint8_t>(c, total * T);
     float* pmean = ws<float>(c, total);
     int* pmax = ws<int>(c, (size_t)N);
-    if (!d_sem || !d_dir || !d_pt || !d_prob || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
+    if (!d_prob || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
     TISEG_TRY(with_dtype(dtype, [&](auto z) {
         using TI = decltype(z);
         return cdnet_refine_run(c, g, (const TI*)d_sem, (const TI*)d_dir, (const TI*)d_pt, T, C, D, if_ddm, d_prob, d_cls, d_dd,
@@ -297,11 +295,11 @@ int tiseg_cdnet_refine_typed(tiseg_ctx* c, int dtype, const void* sem_logits, co
     }));
     if (dir_map_out) {
         // dir_map_list[0] of every tile (cdnet.py:217)
-        uint8_t* d_dm = tiseg::out(c, dir_map_out, total);
-        if (!d_dm) return TISEG_ERR_CUDA;
+        uint8_t* d_dm = call.out(dir_map_out, total);
+        TISEG_TRY(call.status());
         TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
     }
-    return end_call(c);
+    return call.finish();
 }
 
 int tiseg_ddm_enhance(tiseg_ctx* c, float* sem_prob, const float* dd, const float* point, int N, int C, int H, int W, int mode) {
@@ -309,20 +307,20 @@ int tiseg_ddm_enhance(tiseg_ctx* c, float* sem_prob, const float* dd, const floa
         set_error("tiseg_ddm_enhance: bad argument (2 <= C <= 16, mode 0 | 1)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    const size_t total = (size_t)N * g.P;
-    float* d_prob = (float*)inout_ptr(c, sem_prob, total * C * sizeof(float));
-    const float* d_dd = in(c, dd, total);
-    const float* d_pt = in(c, point, total);
+    Call call(c, "tiseg_ddm_enhance", N, H, W);
+    const Geom& g = call.g;
+    const size_t total = call.total;
+    float* d_prob = call.inout(sem_prob, total * C);
+    const float* d_dd = call.in(dd, total);
+    const float* d_pt = call.in(point, total);
+    TISEG_TRY(call.status());
     float* pmean = ws<float>(c, total);
     int* pmax = ws<int>(c, (size_t)N);
-    if (!d_prob || !d_dd || !d_pt || !pmean || !pmax) return TISEG_ERR_CUDA;
+    if (!pmean || !pmax) return TISEG_ERR_CUDA;
     TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
     TISEG_LAUNCH_AS(c, "k_point_mean", k_point_mean<float>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, 1, pmean, pmax);
     TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_prob, C, d_dd, pmean, pmax, 1, mode, (uint8_t*)nullptr);
-    return end_call(c);
+    return call.finish();
 }
 
 }  // extern "C"
@@ -397,35 +395,36 @@ int tiseg_mtcdnet_refine_typed(tiseg_ctx* c, int dtype, const void* tc_logits, c
         set_error("tiseg_mtcdnet_refine_typed: bad argument (2 <= Ctc <= 16, 1 <= Csem <= 16, D == 9, or D == 1: the regression head)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N * T, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    const size_t total = (size_t)N * g.P;
-    const size_t eb = dtype_bytes(dtype);
-    const void* d_tc = in_ptr(c, tc_logits, total * T * Ctc * eb);
-    const void* d_sem = in_ptr(c, sem_logits, total * T * Csem * eb);
-    const void* d_dir = in_ptr(c, dir_logits, total * T * D * eb);
-    const void* d_pt = in_ptr(c, point_logits, total * T * eb);
-    float* d_tcp = tc_prob_out ? tiseg::out(c, tc_prob_out, total * Ctc) : ws<float>(c, total * Ctc);
-    uint8_t* d_tcc = tc_cls_out ? tiseg::out(c, tc_cls_out, total) : nullptr;
-    float* d_semp = sem_prob_out ? tiseg::out(c, sem_prob_out, total * Csem) : nullptr;
-    uint8_t* d_semc = sem_cls_out ? tiseg::out(c, sem_cls_out, total) : nullptr;
-    float* d_dd = dd_out ? tiseg::out(c, dd_out, total) : ws<float>(c, total);
+    Call call(c, "tiseg_mtcdnet_refine_typed", N, H, W, T);
+    const Geom& g = call.g;
+    const size_t total = call.total, eb = dtype_bytes(dtype);
+    const void* d_tc = call.in_bytes(tc_logits, total * T * Ctc * eb);
+    const void* d_sem = call.in_bytes(sem_logits, total * T * Csem * eb);
+    const void* d_dir = call.in_bytes(dir_logits, total * T * D * eb);
+    const void* d_pt = call.in_bytes(point_logits, total * T * eb);
+    float* d_tcp = call.out(tc_prob_out, total * Ctc);
+    uint8_t* d_tcc = call.out(tc_cls_out, total);
+    float* d_semp = call.out(sem_prob_out, total * Csem);
+    uint8_t* d_semc = call.out(sem_cls_out, total);
+    float* d_dd = call.out(dd_out, total);
+    TISEG_TRY(call.status());
+    if (!d_tcp) d_tcp = ws<float>(c, total * Ctc);         // outputs the caller does not take: scratch
+    if (!d_dd) d_dd = ws<float>(c, total);
     uint8_t* dir_all = ws<uint8_t>(c, total * T);
     float* pmean = ws<float>(c, total);
     int* pmax = ws<int>(c, (size_t)N);
-    if (!d_tc || !d_sem || !d_dir || !d_pt || !d_tcp || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
+    if (!d_tcp || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
     TISEG_TRY(with_dtype(dtype, [&](auto z) {
         using TI = decltype(z);
         return mtcdnet_refine_run(c, g, (const TI*)d_tc, (const TI*)d_sem, (const TI*)d_dir, (const TI*)d_pt, T, Ctc, Csem, D, if_ddm,
                                   d_tcp, d_tcc, d_semp, d_semc, d_dd, dir_all, pmean, pmax);
     }));
     if (dir_map_out) {
-        uint8_t* d_dm = tiseg::out(c, dir_map_out, total);
-        if (!d_dm) return TISEG_ERR_CUDA;
+        uint8_t* d_dm = call.out(dir_map_out, total);
+        TISEG_TRY(call.status());
         TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
     }
-    return end_call(c);
+    return call.finish();
 }
 
 }  // extern "C"

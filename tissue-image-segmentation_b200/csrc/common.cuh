@@ -36,9 +36,10 @@ struct tiseg_ctx {
     // return before execution and leave them to the next call that synchronises (tiseg_synchronize included).
     int* d_err = nullptr;      // [2] device
     int* h_err = nullptr;      // [2] pinned host mirror
-    // root counts per block left behind by the last ccl_flatten (consumed by rank_roots on the same forest)
-    const int* rootblk_par = nullptr;
-    int* rootblk = nullptr;
+    // dynamic shared-memory limits of the flood kernels, raised once on this context's device (cudaFuncSetAttribute acts
+    // on the current device, so the flag belongs with the device and not with the process)
+    bool smem_flood_u8[2] = {false, false};    // k_ws_flood_par<false>, k_ws_flood_par<true>
+    bool smem_flood_f64 = false;               // k_rank_blobs<true>, k_ws_flood_ranked
     // optional per-kernel CUDA-event timing (bench.py's roofline leg); off by default
     bool timing = false;
     struct Timed { const char* name; cudaEvent_t a, b; };
@@ -52,21 +53,10 @@ void set_error(const std::string& msg);
 int fail(const char* where, cudaError_t e);
 
 // ---- call-scoped workspace -------------------------------------------------------------------
-void begin_call(tiseg_ctx* c);
-int end_call(tiseg_ctx* c);                       // flush pending D2H, sync if any host output
 int check_deferred(tiseg_ctx* c);                 // after a stream sync: report + clear kernel-raised errors
-void* ws_alloc(tiseg_ctx* c, size_t bytes);       // 256-byte aligned device scratch, valid until end_call
-bool is_device_ptr(const void* p);
-// input: device pointer returned as is; host pointer staged to the arena with an async H2D
-const void* in_ptr(tiseg_ctx* c, const void* p, size_t bytes);
-// output: device pointer returned as is; host pointer gets arena scratch + a pending D2H
-void* out_ptr(tiseg_ctx* c, void* p, size_t bytes);
-// in/out (mutated in place by the reference): staged in, copied back
-void* inout_ptr(tiseg_ctx* c, void* p, size_t bytes);
+void* ws_alloc(tiseg_ctx* c, size_t bytes);       // 256-byte aligned device scratch, valid until the next call
 
 template <class T> inline T* ws(tiseg_ctx* c, size_t n) { return (T*)ws_alloc(c, n * sizeof(T)); }
-template <class T> inline const T* in(tiseg_ctx* c, const T* p, size_t n) { return (const T*)in_ptr(c, p, n * sizeof(T)); }
-template <class T> inline T* out(tiseg_ctx* c, T* p, size_t n) { return p ? (T*)out_ptr(c, p, n * sizeof(T)) : nullptr; }
 
 int zero(tiseg_ctx* c, void* p, size_t bytes);
 // records the 'before' event of a timed launch and returns the 'after' event to record
@@ -121,13 +111,44 @@ inline unsigned flat4_grid(long long n) { return (unsigned)((n + 4 * TISEG_THREA
 inline bool aligned16(const void* a, const void* b = nullptr, const void* c = nullptr, const void* d = nullptr, const void* e = nullptr) {
     return ((((uintptr_t)a) | ((uintptr_t)b) | ((uintptr_t)c) | ((uintptr_t)d) | ((uintptr_t)e)) & 15) == 0;
 }
-inline int check_geom(int N, int H, int W) {
+inline int check_geom(long long N, int H, int W) {
     if (N <= 0 || H <= 0 || W <= 0 || N > 65535 || (long long)H * W >= (1ll << 30)) {
         set_error("bad tile geometry (need 1 <= N <= 65535, H*W < 2^30)");
         return TISEG_ERR_ARG;
     }
     return TISEG_OK;
 }
+
+// ---- one call of a C entry point --------------------------------------------------------------------------------
+//   Call call(c, "tiseg_x", N, H, W);        checks the context and the geometry, then resets the arena
+//   d_a = call.in(a, n); d_b = call.out(b, n);   device pointers pass through, host arguments are staged
+//   TISEG_TRY(call.status());                once, after the staging and before the first launch
+//   return call.finish();                    the copies back to host outputs, and the wait for them
+// in / out / inout return nullptr for a null argument and only then, so an optional argument cannot be mistaken for
+// a failed staging.  The first failure (bad geometry, workspace allocation, host-to-device copy) is recorded with its
+// message; nothing is staged after it, and every later argument comes back as given, which no launch may use before
+// status() is checked.  There is no destructor: a call that returns early leaves its pending copies to the next call,
+// which drops them.
+class Call {
+  public:
+    // `variants`: images per tile (test-time augmentation); the geometry check counts N * variants tiles
+    Call(tiseg_ctx* c, const char* name, int N, int H, int W, int variants = 1);
+    Geom g{};                   // of the N tiles (all zero if the geometry was refused)
+    size_t total = 0;           // N * H * W
+    template <class T> const T* in(const T* p, size_t n) { return (const T*)stage(const_cast<T*>(p), n * sizeof(T), true, false); }
+    const void* in_bytes(const void* p, size_t bytes) { return stage(const_cast<void*>(p), bytes, true, false); }
+    template <class T> T* out(T* p, size_t n) { return (T*)stage(p, n * sizeof(T), false, true); }
+    template <class T> T* inout(T* p, size_t n) { return (T*)stage(p, n * sizeof(T), true, true); }
+    int status() const;         // the recorded failure (its message becomes the last error), or TISEG_OK
+    int finish();               // status(), or: queue the copies back to host outputs and wait for them
+
+  private:
+    tiseg_ctx* c_;
+    int err_ = TISEG_OK;
+    std::string msg_;
+    void* stage(void* p, size_t bytes, bool to_device, bool to_host);
+    void* failed(void* p, int err);
+};
 
 #ifdef __CUDACC__
 struct Pix {

@@ -15,26 +15,6 @@ int fail(const char* where, cudaError_t e) {
     return TISEG_ERR_CUDA;
 }
 
-void begin_call(tiseg_ctx* c) {
-    cudaSetDevice(c->device);
-    // coalesce the arena if the previous call spilled into extra blocks
-    if (c->blocks.size() > 1) {
-        size_t total = 0;
-        for (auto& b : c->blocks) total += b.cap;
-        cudaStreamSynchronize(c->stream);
-        for (auto& b : c->blocks) cudaFree(b.p);
-        c->blocks.clear();
-        char* p = nullptr;
-        if (cudaMalloc(&p, total) == cudaSuccess) c->blocks.push_back({p, total});
-        else cudaGetLastError();
-    }
-    c->cur_block = 0;
-    c->cur_off = 0;
-    c->pending.clear();
-    c->rootblk_par = nullptr;
-    c->rootblk = nullptr;
-}
-
 void* ws_alloc(tiseg_ctx* c, size_t bytes) {
     bytes = (bytes + 255) & ~size_t(255);
     if (bytes == 0) bytes = 256;
@@ -61,7 +41,7 @@ void* ws_alloc(tiseg_ctx* c, size_t bytes) {
     return p;
 }
 
-bool is_device_ptr(const void* p) {
+static bool is_device_ptr(const void* p) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
         cudaGetLastError();
@@ -70,41 +50,61 @@ bool is_device_ptr(const void* p) {
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
-const void* in_ptr(tiseg_ctx* c, const void* p, size_t bytes) {
-    if (!p) return nullptr;
-    if (is_device_ptr(p)) return p;
-    void* d = ws_alloc(c, bytes);
-    if (!d) return nullptr;
-    if (cudaMemcpyAsync(d, p, bytes, cudaMemcpyHostToDevice, c->stream) != cudaSuccess) {
-        fail("H2D", cudaGetLastError());
-        return nullptr;
+Call::Call(tiseg_ctx* c, const char* name, int N, int H, int W, int variants) : c_(c) {
+    if (!c) {
+        err_ = TISEG_ERR_ARG;
+        msg_ = std::string(name) + ": null context";
+        return;
     }
-    return d;
-}
-
-void* out_ptr(tiseg_ctx* c, void* p, size_t bytes) {
-    if (!p) return nullptr;
-    if (is_device_ptr(p)) return p;
-    void* d = ws_alloc(c, bytes);
-    if (!d) return nullptr;
-    c->pending.push_back({p, d, bytes});
-    return d;
-}
-
-void* inout_ptr(tiseg_ctx* c, void* p, size_t bytes) {
-    if (!p) return nullptr;
-    if (is_device_ptr(p)) return p;
-    void* d = ws_alloc(c, bytes);
-    if (!d) return nullptr;
-    if (cudaMemcpyAsync(d, p, bytes, cudaMemcpyHostToDevice, c->stream) != cudaSuccess) {
-        fail("H2D", cudaGetLastError());
-        return nullptr;
+    if ((err_ = check_geom((long long)N * variants, H, W)) != TISEG_OK) {
+        msg_ = g_err;
+        return;
     }
-    c->pending.push_back({p, d, bytes});
+    cudaSetDevice(c->device);
+    // coalesce the arena if the previous call spilled into extra blocks
+    if (c->blocks.size() > 1) {
+        size_t total = 0;
+        for (auto& b : c->blocks) total += b.cap;
+        cudaStreamSynchronize(c->stream);
+        for (auto& b : c->blocks) cudaFree(b.p);
+        c->blocks.clear();
+        char* p = nullptr;
+        if (cudaMalloc(&p, total) == cudaSuccess) c->blocks.push_back({p, total});
+        else cudaGetLastError();
+    }
+    c->cur_block = 0;
+    c->cur_off = 0;
+    c->pending.clear();
+    g = make_geom(N, H, W);
+    total = (size_t)N * g.P;
+}
+
+void* Call::failed(void* p, int err) {
+    err_ = err;
+    msg_ = g_err;
+    return p;
+}
+
+// device pointers are returned as they are; a host argument gets arena scratch, filled with an async H2D if it is
+// read (to_device) and copied back by finish() if it is written (to_host)
+void* Call::stage(void* p, size_t bytes, bool to_device, bool to_host) {
+    if (!p || err_ != TISEG_OK || is_device_ptr(p)) return p;
+    void* d = ws_alloc(c_, bytes);
+    if (!d) return failed(p, TISEG_ERR_CUDA);
+    if (to_device && cudaMemcpyAsync(d, p, bytes, cudaMemcpyHostToDevice, c_->stream) != cudaSuccess)
+        return failed(p, fail("H2D", cudaGetLastError()));
+    if (to_host) c_->pending.push_back({p, d, bytes});
     return d;
 }
 
-int end_call(tiseg_ctx* c) {
+int Call::status() const {
+    if (err_ != TISEG_OK) set_error(msg_);
+    return err_;
+}
+
+int Call::finish() {
+    if (err_ != TISEG_OK) return status();
+    tiseg_ctx* c = c_;
     if (c->pending.empty()) return TISEG_OK;          // device outputs: stream-ordered, nothing to wait for
     for (auto& q : c->pending)
         TISEG_CHECK(cudaMemcpyAsync(q.host, q.dev, q.bytes, cudaMemcpyDeviceToHost, c->stream));

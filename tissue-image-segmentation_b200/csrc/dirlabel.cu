@@ -209,18 +209,18 @@ extern "C" int tiseg_direction_labels(tiseg_ctx* c, const int32_t* inst, int N, 
         set_error("tiseg_direction_labels: bad argument (2 <= num_angles <= 64; the weight map exists for 8 angles only)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    const size_t total = (size_t)N * g.P;
+    Call call(c, "tiseg_direction_labels", N, H, W);
+    const size_t total = call.total;
+    const int32_t* d_inst = call.in(inst, total);
+    float* d_dist = call.out(dist_out, total);
+    float* d_point = call.out(point_out, total);
+    uint8_t* d_dir = call.out(dir_out, total);
+    float* d_reg = call.out(reg_dir_out, total);
+    float* d_w = call.out(weight_out, total);
+    TISEG_TRY(call.status());
+    const Geom& g = call.g;
     const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
     const size_t nt = (size_t)N * VM;
-    const int32_t* d_inst = in(c, inst, total);
-    float* d_dist = tiseg::out(c, dist_out, total);
-    float* d_point = tiseg::out(c, point_out, total);
-    uint8_t* d_dir = tiseg::out(c, dir_out, total);
-    float* d_reg = tiseg::out(c, reg_dir_out, total);
-    float* d_w = tiseg::out(c, weight_out, total);
     DlTab t;
     t.VM = VM;
     t.best = ws<unsigned long long>(c, nt); t.center = ws<int>(c, nt); t.maxd = ws<unsigned long long>(c, nt);
@@ -229,9 +229,7 @@ extern "C" int tiseg_direction_labels(tiseg_ctx* c, const int32_t* inst, int N, 
     float* impulse = ws<float>(c, total);
     float* tmp = ws<float>(c, total);
     double* d_gw = ws<double>(c, (size_t)2 * gauss_radius + 1);
-    if (!d_inst || !d_dist || !d_point || !d_dir || !d_reg || !t.best || !t.center || !t.maxd || !cent || !dmap || !impulse ||
-        !tmp || !d_gw)
-        return TISEG_ERR_CUDA;
+    if (!t.best || !t.center || !t.maxd || !cent || !dmap || !impulse || !tmp || !d_gw) return TISEG_ERR_CUDA;
     // (the weights are host data: 2 * radius + 1 doubles, as scipy.ndimage._filters._gaussian_kernel1d returns them)
     TISEG_CHECK(cudaMemcpyAsync(d_gw, gauss_weights, ((size_t)2 * gauss_radius + 1) * sizeof(double), cudaMemcpyDefault, c->stream));
     DlDirs dirs;
@@ -250,5 +248,5 @@ extern "C" int tiseg_direction_labels(tiseg_ctx* c, const int32_t* inst, int N, 
         TISEG_TRY(ddm_dev(c, g, d_dir, 1, dd));
         TISEG_LAUNCH(c, k_dl_weight, warp_grid(g), TISEG_THREADS, 0, g, dd, d_dist, d_w);
     }
-    return end_call(c);
+    return call.finish();
 }

@@ -688,8 +688,9 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
                  (g.W % 4 == 0) && aligned16(wsl, inst));
     //   any other background: the general relabelling, on the listed tiles only (no blocks do anything otherwise)
     Geom gl = listed_geom(g, flagged, nflagged);
-    TISEG_TRY(ccl_build(c, gl, ImgEqI32TileBg{wsl, bg}, 2, par));
-    TISEG_TRY(rank_roots(c, gl, par, rank, nullptr));
+    const unsigned* roots;
+    TISEG_TRY(ccl_build(c, gl, ImgEqI32TileBg{wsl, bg}, 2, par, &roots));
+    TISEG_TRY(rank_from_bits(c, gl, roots, rank, nullptr));
     TISEG_TRY(apply_rank(c, gl, par, rank, arranged));
     TISEG_LAUNCH_AS(c, "k_wsl_remove<true>", (k_wsl_remove<true, 2>), dim3(px4_grid.x, 1), TISEG_THREADS, 0, gl, arranged, (const unsigned*)nullptr, (const int*)nullptr, 0, inst,
                  (g.W % 4 == 0) && aligned16(arranged, inst));
@@ -704,15 +705,12 @@ extern "C" int tiseg_postproc_dist_lambda_typed(tiseg_ctx* c, int dtype, const v
                                                 int32_t* inst_out, int32_t* markers_out, int32_t* ws_out) {
     TISEG_TRY(check_dtype(dtype, "tiseg_postproc_dist_lambda_typed"));
     if (!c || !dist || !inst_out || lamb < 0 || lamb > 255) { set_error("tiseg_postproc_dist_lambda_typed: bad argument (0 <= lambda <= 255)"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const void* d_dist = in_ptr(c, dist, total * dtype_bytes(dtype));
-    int32_t* d_inst = tiseg::out(c, inst_out, total);
-    int32_t* d_mk = markers_out ? tiseg::out(c, markers_out, total) : nullptr;
-    int32_t* d_ws = ws_out ? tiseg::out(c, ws_out, total) : nullptr;
-    if (!d_dist || !d_inst) return TISEG_ERR_CUDA;
-    TISEG_TRY(postproc_dist_dev(c, g, dtype, d_dist, lamb, d_inst, d_mk, d_ws));
-    return end_call(c);
+    Call call(c, "tiseg_postproc_dist_lambda_typed", N, H, W);
+    const void* d_dist = call.in_bytes(dist, call.total * dtype_bytes(dtype));
+    int32_t* d_inst = call.out(inst_out, call.total);
+    int32_t* d_mk = call.out(markers_out, call.total);
+    int32_t* d_ws = call.out(ws_out, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(postproc_dist_dev(c, call.g, dtype, d_dist, lamb, d_inst, d_mk, d_ws));
+    return call.finish();
 }

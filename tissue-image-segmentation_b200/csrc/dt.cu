@@ -100,28 +100,22 @@ extern "C" {
 
 int tiseg_distance_transform_edt(tiseg_ctx* c, const uint8_t* mask, int N, int H, int W, double* out) {
     if (!c || !mask || !out) { set_error("tiseg_distance_transform_edt: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_mask = in(c, mask, total);
-    double* d_out = tiseg::out(c, out, total);
-    if (!d_mask || !d_out) return TISEG_ERR_CUDA;
-    TISEG_TRY(distance_transform_dev(c, g, d_mask, 0, d_out, nullptr));
-    return end_call(c);
+    Call call(c, "tiseg_distance_transform_edt", N, H, W);
+    const uint8_t* d_mask = call.in(mask, call.total);
+    double* d_out = call.out(out, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(distance_transform_dev(c, call.g, d_mask, 0, d_out, nullptr));
+    return call.finish();
 }
 
 int tiseg_distance_transform_cdt(tiseg_ctx* c, const uint8_t* mask, int N, int H, int W, int32_t* out) {
     if (!c || !mask || !out) { set_error("tiseg_distance_transform_cdt: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_mask = in(c, mask, total);
-    int32_t* d_out = tiseg::out(c, out, total);
-    if (!d_mask || !d_out) return TISEG_ERR_CUDA;
-    TISEG_TRY(distance_transform_dev(c, g, d_mask, 1, nullptr, d_out));
-    return end_call(c);
+    Call call(c, "tiseg_distance_transform_cdt", N, H, W);
+    const uint8_t* d_mask = call.in(mask, call.total);
+    int32_t* d_out = call.out(out, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(distance_transform_dev(c, call.g, d_mask, 1, nullptr, d_out));
+    return call.finish();
 }
 
 }  // extern "C"

@@ -472,21 +472,19 @@ extern "C" int tiseg_postproc_hover_ex(tiseg_ctx* c, int dtype, const void* fore
         set_error("tiseg_postproc_hover_ex: obj_size must be >= 0, got " + std::to_string(obj_size));
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H * scale_factor, W * scale_factor));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    Geom gs = make_geom(N, H * scale_factor, W * scale_factor);          // the resolution the pipeline runs at
-    size_t total = (size_t)N * g.P, stotal = (size_t)N * gs.P;
-    const void* d_fore = in_ptr(c, fore_map, total * dtype_bytes(dtype));
-    const void* d_hv = in_ptr(c, hv_map, total * 2 * dtype_bytes(dtype));
-    int32_t* d_inst = tiseg::out(c, inst_out, total);
-    uint8_t* d_blb = blb_out ? tiseg::out(c, blb_out, stotal) : nullptr;
-    double* d_dist = dist_out ? tiseg::out(c, dist_out, stotal) : nullptr;
-    int32_t* d_mk = marker_out ? tiseg::out(c, marker_out, stotal) : nullptr;
-    if (!d_fore || !d_hv || !d_inst) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_postproc_hover_ex", N, H * scale_factor, W * scale_factor);   // the resolution the pipeline runs at
+    const size_t total = (size_t)N * H * W, stotal = call.total;
+    const void* d_fore = call.in_bytes(fore_map, total * dtype_bytes(dtype));
+    const void* d_hv = call.in_bytes(hv_map, total * 2 * dtype_bytes(dtype));
+    int32_t* d_inst = call.out(inst_out, total);
+    uint8_t* d_blb = call.out(blb_out, stotal);
+    double* d_dist = call.out(dist_out, stotal);
+    int32_t* d_mk = call.out(marker_out, stotal);
+    TISEG_TRY(call.status());
+    const Geom g = make_geom(N, H, W);
     TISEG_TRY(with_dtype(dtype, [&](auto z) {
-        return postproc_hover_entry<decltype(z)>(c, d_fore, d_hv, g, gs, scale_factor, ksize, obj_size, d_inst, d_blb, d_dist,
+        return postproc_hover_entry<decltype(z)>(c, d_fore, d_hv, g, call.g, scale_factor, ksize, obj_size, d_inst, d_blb, d_dist,
                                                  d_mk);
     }));
-    return end_call(c);
+    return call.finish();
 }

@@ -364,51 +364,49 @@ extern "C" {
 
 int tiseg_gen_hv_map(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, float* hv_out) {
     if (!c || !inst || !hv_out) { set_error("tiseg_gen_hv_map: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const int32_t* d_inst = in(c, inst, total);
-    float* d_hv = tiseg::out(c, hv_out, total * 2);
-    if (!d_inst || !d_hv) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_gen_hv_map", N, H, W);
+    const int32_t* d_inst = call.in(inst, call.total);
+    float* d_hv = call.out(hv_out, call.total * 2);
+    TISEG_TRY(call.status());
+    const Geom& g = call.g;
     InstBox b;
     TISEG_TRY(inst_tables(c, g, d_inst, b));
     TISEG_LAUNCH(c, k_hv_map, warp_grid(g), TISEG_THREADS, 0, g, d_inst, b, (float2*)d_hv);
-    return end_call(c);
+    return call.finish();
 }
 
 int tiseg_instance_distance_map(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, int inst_norm, float* dist_out) {
     if (!c || !inst || !dist_out) { set_error("tiseg_instance_distance_map: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
+    Call call(c, "tiseg_instance_distance_map", N, H, W);
+    const Geom& g = call.g;
+    const size_t total = call.total;
+    const int32_t* d_inst = call.in(inst, total);
+    float* d_out = call.out(dist_out, total);
+    TISEG_TRY(call.status());
     const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
-    const int32_t* d_inst = in(c, inst, total);
-    float* d_out = tiseg::out(c, dist_out, total);
     int* col = ws<int>(c, total); int* dist = ws<int>(c, total);
     int* maxd = ws<int>(c, (size_t)N * VM);
-    if (!d_inst || !d_out || !col || !dist || !maxd) return TISEG_ERR_CUDA;
+    if (!col || !dist || !maxd) return TISEG_ERR_CUDA;
     TISEG_TRY(zero(c, maxd, (size_t)N * VM * sizeof(int)));
     TISEG_LAUNCH(c, k_idm_columns, dim3((g.W + TISEG_THREADS - 1) / TISEG_THREADS, N), TISEG_THREADS, 0, g, d_inst, col);
     TISEG_LAUNCH(c, k_idm_rows, dim3(g.H, N), TISEG_THREADS, 0, g, d_inst, col, dist, maxd, VM);
     TISEG_LAUNCH(c, k_idm_finish, warp_grid(g), TISEG_THREADS, 0, g, d_inst, dist, maxd, VM, inst_norm, d_out);
-    return end_call(c);
+    return call.finish();
 }
 
 int tiseg_fix_inst(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, int32_t* out) {
     if (!c || !inst || !out) { set_error("tiseg_fix_inst: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    const size_t total = (size_t)N * g.P;
+    Call call(c, "tiseg_fix_inst", N, H, W);
+    const Geom& g = call.g;
+    const size_t total = call.total;
+    const int32_t* d_inst = call.in(inst, total);
+    int32_t* d_out = call.out(out, total);
+    TISEG_TRY(call.status());
     const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
-    const int32_t* d_inst = in(c, inst, total);
-    int32_t* d_out = tiseg::out(c, out, total);
     int* par = ws<int>(c, total); int* aux = ws<int>(c, total); int* lst = ws<int>(c, total);
     int32_t* kept = ws<int32_t>(c, total);
     int* cnt = ws<int>(c, (size_t)N * VM); int* base = ws<int>(c, (size_t)N * VM); int* vmax = ws<int>(c, N);
-    if (!d_inst || !d_out || !par || !aux || !lst || !kept || !cnt || !base || !vmax) return TISEG_ERR_CUDA;
+    if (!par || !aux || !lst || !kept || !cnt || !base || !vmax) return TISEG_ERR_CUDA;
     const unsigned fg = (unsigned)((total + TISEG_THREADS - 1) / TISEG_THREADS);
     // remove_small_objects(inst == id, 5): 4-connected pieces of equal id
     TISEG_TRY(ccl_build(c, g, ImgEqI32{d_inst, 0}, 1, par));
@@ -425,7 +423,7 @@ int tiseg_fix_inst(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, int32
     if (!newid) return TISEG_ERR_CUDA;
     TISEG_LAUNCH(c, k_fix_newid, warp_grid(g), TISEG_THREADS, 0, g, kept, par, base, cnt, lst, newid, VM);
     TISEG_TRY(apply_rank(c, g, par, newid, d_out));
-    return end_call(c);
+    return call.finish();
 }
 
 int tiseg_bound_label(tiseg_ctx* c, const uint8_t* sem, const int32_t* inst, int N, int H, int W, int edge_id,
@@ -435,42 +433,40 @@ int tiseg_bound_label(tiseg_ctx* c, const uint8_t* sem, const int32_t* inst, int
         set_error("tiseg_bound_label: bad argument");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    const size_t total = (size_t)N * g.P;
-    const uint8_t* d_sem = in(c, sem, total);
-    const int32_t* d_inst = in(c, inst, total);
-    uint8_t* d_so = sem_out ? tiseg::out(c, sem_out, total) : nullptr;
-    uint8_t* d_bo = tiseg::out(c, sem_w_bound_out, total);
-    if (!d_sem || !d_inst || !d_bo || (sem_out && !d_so)) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_bound_label", N, H, W);
+    const uint8_t* d_sem = call.in(sem, call.total);
+    const int32_t* d_inst = call.in(inst, call.total);
+    uint8_t* d_so = call.out(sem_out, call.total);
+    uint8_t* d_bo = call.out(sem_w_bound_out, call.total);
+    TISEG_TRY(call.status());
+    const Geom& g = call.g;
     TISEG_LAUNCH(c, k_bound_label, warp_grid(g), TISEG_THREADS, 0, g, d_sem, d_inst, edge_id, radius_dilate, radius_erode,
                  d_so, d_bo);
-    return end_call(c);
+    return call.finish();
 }
 
 int tiseg_unet_weight_map(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, double w0, double sigma,
                           int32_t* inner_out, double* wmap_out) {
     if (!c || !inst || !inner_out || !wmap_out || !(sigma > 0)) { set_error("tiseg_unet_weight_map: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    const size_t total = (size_t)N * g.P;
+    Call call(c, "tiseg_unet_weight_map", N, H, W);
+    const Geom& g = call.g;
+    const size_t total = call.total;
+    const int32_t* d_inst = call.in(inst, total);
+    int32_t* d_inner = call.out(inner_out, total);
+    double* d_w = call.out(wmap_out, total);
+    TISEG_TRY(call.status());
     const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
-    const int32_t* d_inst = in(c, inst, total);
-    int32_t* d_inner = tiseg::out(c, inner_out, total);
-    double* d_w = tiseg::out(c, wmap_out, total);
     uint8_t* seen = ws<uint8_t>(c, (size_t)N * VM);
     int* count = ws<int>(c, N);
     int4* col = ws<int4>(c, total);
-    if (!d_inst || !d_inner || !d_w || !seen || !count || !col) return TISEG_ERR_CUDA;
+    if (!seen || !count || !col) return TISEG_ERR_CUDA;
     TISEG_TRY(zero(c, seen, (size_t)N * VM));
     TISEG_TRY(zero(c, count, (size_t)N * sizeof(int)));
     TISEG_LAUNCH(c, k_unet_inner, warp_grid(g), TISEG_THREADS, 0, g, d_inst, d_inner, seen, VM, c->d_err);
     TISEG_LAUNCH(c, k_count_seen, dim3(32, N), 256, 0, seen, VM, count);
     TISEG_LAUNCH(c, k_unet_columns, dim3((g.W + TISEG_THREADS - 1) / TISEG_THREADS, N), TISEG_THREADS, 0, g, d_inner, col);
     TISEG_LAUNCH(c, k_unet_weight, dim3(g.H, N), TISEG_THREADS, 0, g, d_inner, col, count, w0, sigma, d_w);
-    return end_call(c);
+    return call.finish();
 }
 
 }  // extern "C"

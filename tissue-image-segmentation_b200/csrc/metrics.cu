@@ -756,20 +756,19 @@ extern "C" {
 
 int tiseg_assign_sem_class(tiseg_ctx* c, const int32_t* inst, const uint8_t* sem, int N, int H, int W, int C, uint8_t* table_out) {
     if (!c || !inst || !sem || !table_out || C < 2 || C > 64) { set_error("tiseg_assign_sem_class: bad argument (2 <= C <= 64)"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
+    Call call(c, "tiseg_assign_sem_class", N, H, W);
+    const Geom& g = call.g;
     const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
-    const int32_t* d_inst = in(c, inst, total);
-    const uint8_t* d_sem = in(c, sem, total);
-    uint8_t* d_tab = tiseg::out(c, table_out, (size_t)N * VM);
+    const int32_t* d_inst = call.in(inst, call.total);
+    const uint8_t* d_sem = call.in(sem, call.total);
+    uint8_t* d_tab = call.out(table_out, (size_t)N * VM);
+    TISEG_TRY(call.status());
     int* hist = ws<int>(c, (size_t)N * VM * (C + 1));
-    if (!d_inst || !d_sem || !d_tab || !hist) return TISEG_ERR_CUDA;
+    if (!hist) return TISEG_ERR_CUDA;
     TISEG_TRY(zero(c, hist, (size_t)N * VM * (C + 1) * sizeof(int)));
     TISEG_LAUNCH(c, k_inst_class_hist, warp_grid(g), TISEG_THREADS, 0, g, d_inst, d_sem, C, VM, hist, c->d_err);
     TISEG_LAUNCH(c, k_inst_class_table, dim3((VM + 255) / 256, N), 256, 0, hist, C, VM, d_tab);
-    return end_call(c);
+    return call.finish();
 }
 
 static int pair_metrics_bin_any(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, const uint16_t* gt16, int N, int H, int W,
@@ -778,21 +777,19 @@ static int pair_metrics_bin_any(tiseg_ctx* c, const int32_t* pred, const int32_t
         set_error("tiseg_pair_metrics_bin_iou: bad argument (match_iou >= 0.5: below it the reference switches to Hungarian matching)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const int32_t* d_pred = in(c, pred, total);
-    const int32_t* d_gt = gt ? in(c, gt, total) : nullptr;
-    const uint16_t* d_gt16 = gt16 ? in(c, gt16, total) : nullptr;
-    double* d_aji = aji ? tiseg::out(c, aji, 2 * (size_t)N) : nullptr;
-    double* d_pq = pq ? tiseg::out(c, pq, 4 * (size_t)N) : nullptr;
-    if (!d_pred || (!d_gt && !d_gt16)) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_pair_metrics_bin_iou", N, H, W);
+    const Geom& g = call.g;
+    const int32_t* d_pred = call.in(pred, call.total);
+    const int32_t* d_gt = call.in(gt, call.total);
+    const uint16_t* d_gt16 = call.in(gt16, call.total);
+    double* d_aji = call.out(aji, 2 * (size_t)N);
+    double* d_pq = call.out(pq, 4 * (size_t)N);
+    TISEG_TRY(call.status());
     PairWork w;
     TISEG_TRY(pair_table_build(c, g, d_pred, d_gt, w, nullptr, d_gt16));
     ClassInfo ci = {nullptr, nullptr, nullptr, nullptr};
     TISEG_TRY(pair_eval(c, g, w, nullptr, nullptr, 2, ci, true, d_aji, d_pq, match_iou));
-    return end_call(c);
+    return call.finish();
 }
 
 int tiseg_pair_metrics_bin_iou(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, int N, int H, int W, double match_iou,
@@ -812,19 +809,17 @@ int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const 
         set_error("tiseg_pair_metrics_multiclass: bad argument (2 <= C <= 64)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const int32_t* d_pi = in(c, pred_inst, total);
-    const uint8_t* d_ps = in(c, pred_sem, total);
-    const int32_t* d_gi = in(c, gt_inst, total);
-    const uint8_t* d_gs = in(c, gt_sem, total);
-    double* d_aji = aji ? tiseg::out(c, aji, 2 * (size_t)N * C) : nullptr;
-    double* d_pq = pq ? tiseg::out(c, pq, 4 * (size_t)N * C) : nullptr;
-    double* d_baji = bin_aji ? tiseg::out(c, bin_aji, 2 * (size_t)N) : nullptr;
-    double* d_bpq = bin_pq ? tiseg::out(c, bin_pq, 4 * (size_t)N) : nullptr;
-    if (!d_pi || !d_ps || !d_gi || !d_gs) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_pair_metrics_multiclass", N, H, W);
+    const Geom& g = call.g;
+    const int32_t* d_pi = call.in(pred_inst, call.total);
+    const uint8_t* d_ps = call.in(pred_sem, call.total);
+    const int32_t* d_gi = call.in(gt_inst, call.total);
+    const uint8_t* d_gs = call.in(gt_sem, call.total);
+    double* d_aji = call.out(aji, 2 * (size_t)N * C);
+    double* d_pq = call.out(pq, 4 * (size_t)N * C);
+    double* d_baji = call.out(bin_aji, 2 * (size_t)N);
+    double* d_bpq = call.out(bin_pq, 4 * (size_t)N);
+    TISEG_TRY(call.status());
     PairWork w;
     PairRoots rt;
     TISEG_TRY(pair_table_build(c, g, d_pi, d_gi, w, &rt));
@@ -843,21 +838,19 @@ int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const 
         ci.ncomp_p = a; ci.ninst_p = b;
         TISEG_TRY(pair_eval(c, g, w, cls_g, cls_p, C, ci, first, d_aji, d_pq));
     }
-    return end_call(c);
+    return call.finish();
 }
 
 int tiseg_sem_counts(tiseg_ctx* c, const uint8_t* pred, const uint8_t* gt, int N, int H, int W, int C,
                      int ignore_index, int64_t* counts, int64_t* valid) {
     if (!c || !pred || !gt || !counts || !valid || C <= 0 || C > SEM_MAXC) { set_error("tiseg_sem_counts: bad argument (C <= 64)"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_pred = in(c, pred, total);
-    const uint8_t* d_gt = in(c, gt, total);
-    int64_t* d_counts = tiseg::out(c, counts, (size_t)N * 5 * C);
-    int64_t* d_valid = tiseg::out(c, valid, (size_t)N);
-    if (!d_pred || !d_gt || !d_counts || !d_valid) return TISEG_ERR_CUDA;
+    Call call(c, "tiseg_sem_counts", N, H, W);
+    const Geom& g = call.g;
+    const uint8_t* d_pred = call.in(pred, call.total);
+    const uint8_t* d_gt = call.in(gt, call.total);
+    int64_t* d_counts = call.out(counts, (size_t)N * 5 * C);
+    int64_t* d_valid = call.out(valid, (size_t)N);
+    TISEG_TRY(call.status());
     TISEG_TRY(zero(c, d_counts, (size_t)N * 5 * C * sizeof(int64_t)));
     TISEG_TRY(zero(c, d_valid, (size_t)N * sizeof(int64_t)));
     unsigned gx = flat4_grid(g.P);
@@ -873,7 +866,7 @@ int tiseg_sem_counts(tiseg_ctx* c, const uint8_t* pred, const uint8_t* gt, int N
     bool vec = (g.P % 4 == 0) && ((((uintptr_t)d_pred) | ((uintptr_t)d_gt)) & 3) == 0;
     TISEG_LAUNCH(c, k_sem_counts, dim3(gx, N), TISEG_THREADS, 0, (long long)g.P, d_pred, d_gt, C, ignore_index,
                  (unsigned long long*)d_counts, (unsigned long long*)d_valid, vec);
-    return end_call(c);
+    return call.finish();
 }
 
 }  // extern "C"

@@ -276,8 +276,9 @@ int postproc_unet_dev(tiseg_ctx* c, const Geom& g, uint8_t* cls, int max_class, 
         TISEG_LAUNCH(c, k_keep_large, dim3(flat4_grid(g.P), N), TISEG_THREADS, 0, (long long)g.P, par, aux, 5, m2,
                      (g.P % 4 == 0) && aligned16(par) && (((uintptr_t)m2) & 3) == 0);
         // measure.label (8-connected, raster ids)
-        TISEG_TRY(ccl_build(c, g, ImgMaskU8{m2}, 2, par));
-        TISEG_TRY(rank_roots(c, g, par, aux, counts));
+        const unsigned* roots;
+        TISEG_TRY(ccl_build(c, g, ImgMaskU8{m2}, 2, par, &roots));
+        TISEG_TRY(rank_from_bits(c, g, roots, aux, counts));
         TISEG_TRY(apply_rank(c, g, par, aux, lab));
         // dilation(disk(radius)) + overwrite + cur bookkeeping
         TISEG_LAUNCH(c, k_zero_prefix_u8, dim3(8, N), 256, 0, seen, KS, counts);
@@ -304,59 +305,48 @@ extern "C" {
 
 int tiseg_fill_holes(tiseg_ctx* c, const uint8_t* mask, int N, int H, int W, uint8_t* out) {
     if (!c || !mask || !out) { set_error("tiseg_fill_holes: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_in = in(c, mask, total);
-    uint8_t* d_out = tiseg::out(c, out, total);
-    int* par = ws<int>(c, total);
-    if (!d_in || !d_out || !par) return TISEG_ERR_CUDA;
-    TISEG_TRY(ccl_build(c, g, ImgNotMaskU8{d_in}, 1, par));
-    TISEG_TRY(fill_from_complement_forest(c, g, par, d_out));
-    return end_call(c);
+    Call call(c, "tiseg_fill_holes", N, H, W);
+    const uint8_t* d_in = call.in(mask, call.total);
+    uint8_t* d_out = call.out(out, call.total);
+    TISEG_TRY(call.status());
+    int* par = ws<int>(c, call.total);
+    if (!par) return TISEG_ERR_CUDA;
+    TISEG_TRY(ccl_build(c, call.g, ImgNotMaskU8{d_in}, 1, par));
+    TISEG_TRY(fill_from_complement_forest(c, call.g, par, d_out));
+    return call.finish();
 }
 
 int tiseg_remove_small_objects(tiseg_ctx* c, const uint8_t* mask, int N, int H, int W, int min_size, int connectivity,
                                uint8_t* out) {
     if (!c || !mask || !out || (connectivity != 1 && connectivity != 2)) { set_error("tiseg_remove_small_objects: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_in = in(c, mask, total);
-    uint8_t* d_out = tiseg::out(c, out, total);
-    if (!d_in || !d_out) return TISEG_ERR_CUDA;
-    TISEG_TRY(remove_small_mask(c, g, d_in, min_size, connectivity, d_out));
-    return end_call(c);
+    Call call(c, "tiseg_remove_small_objects", N, H, W);
+    const uint8_t* d_in = call.in(mask, call.total);
+    uint8_t* d_out = call.out(out, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(remove_small_mask(c, call.g, d_in, min_size, connectivity, d_out));
+    return call.finish();
 }
 
 int tiseg_remove_small_labels(tiseg_ctx* c, const int32_t* lab, int N, int H, int W, int min_size, int32_t* out) {
     if (!c || !lab || !out) { set_error("tiseg_remove_small_labels: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const int32_t* d_in = in(c, lab, total);
-    int32_t* d_out = tiseg::out(c, out, total);
-    if (!d_in || !d_out) return TISEG_ERR_CUDA;
-    TISEG_TRY(remove_small_labels(c, g, d_in, min_size, d_out));
-    return end_call(c);
+    Call call(c, "tiseg_remove_small_labels", N, H, W);
+    const int32_t* d_in = call.in(lab, call.total);
+    int32_t* d_out = call.out(out, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(remove_small_labels(c, call.g, d_in, min_size, d_out));
+    return call.finish();
 }
 
 static int morph_entry(tiseg_ctx* c, const int32_t* lab, int N, int H, int W, int footprint, int radius, bool dil,
                        int32_t* out) {
     if (!c || !lab || !out || footprint < 0 || footprint > 1 || radius < 0 || radius > 3) { set_error("label morphology: bad argument (radius <= 3)"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const int32_t* d_in = in(c, lab, total);
-    int32_t* d_out = tiseg::out(c, out, total);
-    if (!d_in || !d_out) return TISEG_ERR_CUDA;
+    Call call(c, dil ? "tiseg_dilate_labels" : "tiseg_erode_labels", N, H, W);
+    const int32_t* d_in = call.in(lab, call.total);
+    int32_t* d_out = call.out(out, call.total);
+    TISEG_TRY(call.status());
     if (d_in == d_out) { set_error("label morphology cannot run in place"); return TISEG_ERR_ARG; }
-    TISEG_TRY(grey_morph(c, g, d_in, footprint, radius, dil, d_out));
-    return end_call(c);
+    TISEG_TRY(grey_morph(c, call.g, d_in, footprint, radius, dil, d_out));
+    return call.finish();
 }
 int tiseg_dilate_labels(tiseg_ctx* c, const int32_t* lab, int N, int H, int W, int footprint, int radius, int32_t* out) {
     return morph_entry(c, lab, N, H, W, footprint, radius, true, out);
@@ -371,18 +361,16 @@ int tiseg_postproc_unet(tiseg_ctx* c, uint8_t* cls, int N, int H, int W, int max
         set_error("tiseg_postproc_unet: bad argument (1 <= max_class <= 63, radius <= 3)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    bool mutate = edge_id >= 0 || kill;
-    uint8_t* d_cls = mutate ? (uint8_t*)inout_ptr(c, cls, total) : (uint8_t*)in_ptr(c, cls, total);
-    const uint8_t* d_kill = kill ? in(c, kill, total) : nullptr;
-    uint8_t* d_sem = tiseg::out(c, sem_out, total);
-    int32_t* d_inst = tiseg::out(c, inst_out, total);
-    if (!d_cls || !d_sem || !d_inst) return TISEG_ERR_CUDA;
-    TISEG_TRY(postproc_unet_dev(c, g, d_cls, max_class, radius, edge_id, d_kill, d_sem, d_inst));
-    return end_call(c);
+    Call call(c, "tiseg_postproc_unet", N, H, W);
+    const size_t total = call.total;
+    const bool mutate = edge_id >= 0 || kill;          // then the class map is edited in place (and copied back from host)
+    uint8_t* d_cls = mutate ? call.inout(cls, total) : const_cast<uint8_t*>(call.in(cls, total));
+    const uint8_t* d_kill = call.in(kill, total);
+    uint8_t* d_sem = call.out(sem_out, total);
+    int32_t* d_inst = call.out(inst_out, total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(postproc_unet_dev(c, call.g, d_cls, max_class, radius, edge_id, d_kill, d_sem, d_inst));
+    return call.finish();
 }
 
 }  // extern "C"

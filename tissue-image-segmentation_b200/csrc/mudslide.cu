@@ -188,21 +188,21 @@ using namespace tiseg;
 extern "C" int tiseg_mudslide_watershed(tiseg_ctx* c, const uint8_t* seg, uint8_t* dir_graph, const uint8_t* fore, int N, int H,
                                         int W, uint8_t* pred_out, uint8_t* boundary_out) {
     if (!c || !seg || !dir_graph || !fore || !pred_out || !boundary_out) { set_error("tiseg_mudslide_watershed: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_seg = in(c, seg, total);
-    uint8_t* d_dir = (uint8_t*)inout_ptr(c, dir_graph, total);
-    const uint8_t* d_fore = in(c, fore, total);
-    uint8_t* d_pred = tiseg::out(c, pred_out, total);
-    uint8_t* d_bnd = tiseg::out(c, boundary_out, total);
+    Call call(c, "tiseg_mudslide_watershed", N, H, W);
+    const Geom& g = call.g;
+    const size_t total = call.total;
+    const uint8_t* d_seg = call.in(seg, total);
+    uint8_t* d_dir = call.inout(dir_graph, total);
+    const uint8_t* d_fore = call.in(fore, total);
+    uint8_t* d_pred = call.out(pred_out, total);
+    uint8_t* d_bnd = call.out(boundary_out, total);
+    TISEG_TRY(call.status());
     uint8_t* m[10];
     for (auto& p : m) { p = ws<uint8_t>(c, total); if (!p) return TISEG_ERR_CUDA; }
     int* par = ws<int>(c, total); int* rank = ws<int>(c, total);
     int* level = ws<int>(c, total); int* vis = ws<int>(c, total); int* queue = ws<int>(c, total);
     int* work = ws<int>(c, (size_t)N);
-    if (!d_seg || !d_dir || !d_fore || !d_pred || !d_bnd || !par || !rank || !level || !vis || !queue || !work) return TISEG_ERR_CUDA;
+    if (!par || !rank || !level || !vis || !queue || !work) return TISEG_ERR_CUDA;
     uint8_t *segb = m[0], *segf = m[1], *foref = m[2], *forec = m[3], *segc = m[4], *contour = m[5], *small = m[6], *du = m[7], *tmp = m[8], *aux = m[9];
     // seg = fill_holes(seg); fore = remove_small_objects(fill_holes(fore), 20); seg[fore == 0] = 0; contour = fore ^ seg
     TISEG_LAUNCH(c, k_mud_binarise, warp_grid(g), TISEG_THREADS, 0, g, d_seg, segb);
@@ -237,5 +237,5 @@ extern "C" int tiseg_mudslide_watershed(tiseg_ctx* c, const uint8_t* seg, uint8_
     TISEG_LAUNCH(c, k_mud_levels_out, warp_grid(g), TISEG_THREADS, 0, g, level, segf, d_bnd);
     TISEG_TRY(remove_small_mask(c, g, segf, 15, 1, foref));
     TISEG_LAUNCH(c, k_mud_xor, warp_grid(g), TISEG_THREADS, 0, g, foref, small, d_pred);
-    return end_call(c);
+    return call.finish();
 }

@@ -99,15 +99,13 @@ using namespace tiseg;
 extern "C" int tiseg_reconstruction_erosion_u8(tiseg_ctx* c, const uint8_t* seed, const uint8_t* mask, int N, int H, int W,
                                                uint8_t* out) {
     if (!c || !seed || !mask || !out) { set_error("tiseg_reconstruction_erosion_u8: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const uint8_t* d_seed = in(c, seed, total);
-    const uint8_t* d_mask = in(c, mask, total);
-    uint8_t* d_out = tiseg::out(c, out, total);
-    if (!d_seed || !d_mask || !d_out) return TISEG_ERR_CUDA;
-    TISEG_LAUNCH(c, k_recon_seed, flat_grid((long long)total), TISEG_THREADS, 0, (long long)total, d_mask, d_seed, 0, d_out);
-    TISEG_TRY(reconstruction_erosion_dev(c, g, d_mask, d_out));
-    return end_call(c);
+    Call call(c, "tiseg_reconstruction_erosion_u8", N, H, W);
+    const long long total = (long long)call.total;
+    const uint8_t* d_seed = call.in(seed, total);
+    const uint8_t* d_mask = call.in(mask, total);
+    uint8_t* d_out = call.out(out, total);
+    TISEG_TRY(call.status());
+    TISEG_LAUNCH(c, k_recon_seed, flat_grid(total), TISEG_THREADS, 0, total, d_mask, d_seed, 0, d_out);
+    TISEG_TRY(reconstruction_erosion_dev(c, call.g, d_mask, d_out));
+    return call.finish();
 }

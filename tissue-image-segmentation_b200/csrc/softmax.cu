@@ -343,15 +343,13 @@ static int tta_entry(tiseg_ctx* c, int dtype, const void* logits, int N, int T, 
         off += tta_variant_elems(C, odd ? W : H, odd ? H : W, window, overlap);
     }
     plan.tile_stride = off;
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const void* d_in = in_ptr(c, logits, (size_t)N * (size_t)off * dtype_bytes(dtype));
-    float* d_prob = prob ? tiseg::out(c, prob, total * C) : nullptr;
-    uint8_t* d_cls = cls ? tiseg::out(c, cls, total) : nullptr;
-    if (!d_in) return TISEG_ERR_CUDA;
-    TISEG_TRY(with_dtype(dtype, [&](auto z) { return tta_launch(c, g, (const decltype(z)*)d_in, plan, C, d_prob, d_cls, softmax); }));
-    return end_call(c);
+    Call call(c, "tiseg_softmax_argmax_tta_typed", N, H, W);
+    const void* d_in = call.in_bytes(logits, (size_t)N * (size_t)off * dtype_bytes(dtype));
+    float* d_prob = call.out(prob, call.total * C);
+    uint8_t* d_cls = call.out(cls, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(with_dtype(dtype, [&](auto z) { return tta_launch(c, call.g, (const decltype(z)*)d_in, plan, C, d_prob, d_cls, softmax); }));
+    return call.finish();
 }
 
 extern "C" int tiseg_softmax_argmax_tta_typed(tiseg_ctx* c, int dtype, const void* logits, int N, int T, int C, int H, int W,
@@ -375,14 +373,11 @@ extern "C" int tiseg_softmax_argmax_typed(tiseg_ctx* c, int dtype, const void* l
         set_error("tiseg_softmax_argmax_typed: bad argument (1 <= C <= 16)");
         return TISEG_ERR_ARG;
     }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const void* d_in = in_ptr(c, logits, total * T * C * dtype_bytes(dtype));
-    float* d_prob = prob ? tiseg::out(c, prob, total * C) : nullptr;
-    uint8_t* d_cls = cls ? tiseg::out(c, cls, total) : nullptr;
-    if (!d_in) return TISEG_ERR_CUDA;
-    TISEG_TRY(with_dtype(dtype, [&](auto z) { return softmax_argmax_dev(c, g, (const decltype(z)*)d_in, T, C, d_prob, d_cls); }));
-    return end_call(c);
+    Call call(c, "tiseg_softmax_argmax_typed", N, H, W);
+    const void* d_in = call.in_bytes(logits, call.total * T * C * dtype_bytes(dtype));
+    float* d_prob = call.out(prob, call.total * C);
+    uint8_t* d_cls = call.out(cls, call.total);
+    TISEG_TRY(call.status());
+    TISEG_TRY(with_dtype(dtype, [&](auto z) { return softmax_argmax_dev(c, call.g, (const decltype(z)*)d_in, T, C, d_prob, d_cls); }));
+    return call.finish();
 }

@@ -1284,10 +1284,9 @@ static int watershed_u8_any(tiseg_ctx* c, const Geom& g, const uint8_t* image, c
         TISEG_LAUNCH(c, k_huge_clean, dim3((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), 1), TISEG_THREADS, 0,
                      gh, mp, bm.bpar, bm.brank, b, bm.seed_bits, (long long)WP_GEN_CAP, out);
     }
-    static bool attr_set = false;
-    if (!attr_set) {
+    if (!c->smem_flood_u8[MASKED]) {
         TISEG_CHECK(cudaFuncSetAttribute(k_ws_flood_par<MASKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WP_SMEM_BYTES));
-        attr_set = true;
+        c->smem_flood_u8[MASKED] = true;
     }
     TISEG_LAUNCH_AS(c, "k_ws_flood_par", (k_ws_flood_par<MASKED>), c->sm_count, 32 * WP_WARPS, WP_SMEM_BYTES, g, image, bm, b,
                     wk, next, gheads, out);
@@ -1354,12 +1353,11 @@ int watershed_f64_dev(tiseg_ctx* c, const Geom& g, const double* image, const in
     wk.count = ints; wk.offset = ints + WS_MAXCLS; wk.fill = ints + 2 * WS_MAXCLS; wk.cursor = ints + 3 * WS_MAXCLS;
     wk.ngen = ints + 4 * WS_MAXCLS; wk.gcursor = wk.ngen + 2;
     TISEG_TRY(zero(c, ints, WK_INTS * sizeof(int)));
-    static bool attr_set = false;
     constexpr size_t RK_SMALL = (size_t)WR_SORT_SMALL * 10, RK_LARGE = (size_t)WR_SORT_MAX * 10;
-    if (!attr_set) {
+    if (!c->smem_flood_f64) {
         TISEG_CHECK(cudaFuncSetAttribute(k_rank_blobs<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_LARGE));
         TISEG_CHECK(cudaFuncSetAttribute((k_ws_flood_ranked<WARPS, ARENA, SLOTS>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
-        attr_set = true;
+        c->smem_flood_f64 = true;
     }
     TISEG_LAUNCH(c, k_blob_prefix, 1, 32, 0, b.count, N, prefix);
     TISEG_LAUNCH(c, k_rank_blobs<false>, c->sm_count * 16, 128, RK_SMALL, g, image, par, b, prefix, level);
@@ -1379,17 +1377,16 @@ template <class T>
 static int watershed_entry(tiseg_ctx* c, const T* image, const int32_t* markers, const uint8_t* mask, int N, int H,
                            int W, int32_t* out) {
     if (!c || !image || !markers || !out) { set_error("tiseg_watershed: bad argument"); return TISEG_ERR_ARG; }
-    TISEG_TRY(check_geom(N, H, W));
-    begin_call(c);
-    Geom g = make_geom(N, H, W);
-    size_t total = (size_t)N * g.P;
-    const T* d_img = in(c, image, total);
-    const int32_t* d_mk = in(c, markers, total);
-    const uint8_t* d_mask = mask ? in(c, mask, total) : nullptr;
-    int32_t* d_out = tiseg::out(c, out, total);
-    int* par = ws<int>(c, total);
-    int* rank = ws<int>(c, total);
-    if (!d_img || !d_mk || !d_out || !par || !rank) return TISEG_ERR_CUDA;
+    Call call(c, sizeof(T) == 8 ? "tiseg_watershed_f64" : "tiseg_watershed_u8", N, H, W);
+    const Geom& g = call.g;
+    const T* d_img = call.in(image, call.total);
+    const int32_t* d_mk = call.in(markers, call.total);
+    const uint8_t* d_mask = call.in(mask, call.total);
+    int32_t* d_out = call.out(out, call.total);
+    TISEG_TRY(call.status());
+    int* par = ws<int>(c, call.total);
+    int* rank = ws<int>(c, call.total);
+    if (!par || !rank) return TISEG_ERR_CUDA;
     BlobInfo b;
     constexpr bool F64 = sizeof(T) == 8;
     if (d_mask) TISEG_TRY(blobs_build(c, g, ImgMaskU8{d_mask}, par, rank, b, F64));
@@ -1397,7 +1394,7 @@ static int watershed_entry(tiseg_ctx* c, const T* image, const int32_t* markers,
     TISEG_TRY(ws_seed(c, g, d_mk, par, d_out));
     if constexpr (F64) TISEG_TRY(watershed_f64_dev(c, g, (const double*)d_img, par, rank, b, d_out));
     else               TISEG_TRY(watershed_u8_dev(c, g, (const uint8_t*)d_img, par, rank, b, d_out));
-    return end_call(c);
+    return call.finish();
 }
 
 }  // namespace tiseg

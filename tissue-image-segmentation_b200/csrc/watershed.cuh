@@ -109,10 +109,10 @@ int blobs_build(tiseg_ctx* c, const Geom& g, MaskImg mask, int* par, int* rank, 
     b.area = ws<int>(c, ks); b.off = want_offsets ? ws<int>(c, ks) : nullptr;
     b.KS = KS; b.count = count; b.lmin = nullptr; b.lmax = nullptr; b.first = nullptr;
     if (!count || !b.root || !b.ymax || !b.xmin || !b.xmax || !b.area || (want_offsets && !b.off)) return TISEG_ERR_CUDA;
-    TISEG_TRY(ccl_build(c, g, mask, conn, par));
-    const unsigned* root_bits = (const unsigned*)c->rootblk;      // left by the flatten; rank_roots consumes the same bitmap
-    TISEG_TRY(rank_roots(c, g, par, rank, count));
-    return blobs_describe(c, g, par, rank, root_bits, b, want_offsets);
+    const unsigned* roots;
+    TISEG_TRY(ccl_build(c, g, mask, conn, par, &roots));
+    TISEG_TRY(rank_from_bits(c, g, roots, rank, count));
+    return blobs_describe(c, g, par, rank, roots, b, want_offsets);
 }
 #endif
 
