@@ -242,12 +242,21 @@ int tiseg_pair_metrics_bin_u16gt(tiseg_ctx* ctx, const int32_t* pred, const uint
 int tiseg_pair_metrics_multiclass(tiseg_ctx* ctx, const int32_t* pred_inst, const uint8_t* pred_sem,
                                   const int32_t* gt_inst, const uint8_t* gt_sem, int N, int H, int W, int C,
                                   double* aji, double* pq, double* bin_aji, double* bin_pq);
+/* the same with the ground-truth instance map as uint16 (ids below 65536), read as it is by every kernel of the ground-truth
+ * side (equality planes, largest id, class histogram, component classes): 3 B/px of ground truth (instances + classes)
+ * instead of 5.  The results are those of the int32 upcast, bit for bit; the prediction stays int32. */
+int tiseg_pair_metrics_multiclass_u16gt(tiseg_ctx* ctx, const int32_t* pred_inst, const uint8_t* pred_sem,
+                                        const uint16_t* gt_inst, const uint8_t* gt_sem, int N, int H, int W, int C,
+                                        double* aji, double* pq, double* bin_aji, double* bin_pq);
 
 /* assign_sem_class_to_insts (datasets/utils/instance_semantic.py:68-93) as a table: table_out [N, VM] uint8 with
  * VM = max(H*W + 1, 65536); entry v = class of instance id v (first argmax over the classes >= 1 of its pixel counts,
  * 0 if it has no non-background pixel; id 0 is class 0), 255 = the id does not occur. */
 int tiseg_assign_sem_class(tiseg_ctx* ctx, const int32_t* inst, const uint8_t* sem, int N, int H, int W, int C,
                            uint8_t* table_out);
+/* the same for a uint16 instance map (read as it is; the table is that of the int32 upcast) */
+int tiseg_assign_sem_class_u16(tiseg_ctx* ctx, const uint16_t* inst, const uint8_t* sem, int N, int H, int W, int C,
+                               uint8_t* table_out);
 
 /* ---- A19: pre_eval_all_semantic_metric (sem_metrics.py:16-53) --------------------------------------
  * pred / gt [N,H,W] uint8; counts [N, 5, C] int64 = TP, FP, FN, Pred, GT per class (TN derived on the
@@ -276,11 +285,16 @@ int tiseg_distance_transform_cdt(tiseg_ctx* ctx, const uint8_t* mask, int N, int
  * instance map already passed through its _fix_inst: dist_out [N,H,W] fp32, divided by the instance maximum when
  * inst_norm != 0.  Instance ids must be < max(H*W+1, 65536) (deferred error otherwise). */
 int tiseg_gen_hv_map(tiseg_ctx* ctx, const int32_t* inst, int N, int H, int W, float* hv_out);
+/* gen_instance_hv_map of a uint16 instance map, read as it is: hv_out is that of the int32 upcast, bit for bit */
+int tiseg_gen_hv_map_u16(tiseg_ctx* ctx, const uint16_t* inst, int N, int H, int W, float* hv_out);
 int tiseg_instance_distance_map(tiseg_ctx* ctx, const int32_t* inst, int N, int H, int W, int inst_norm, float* dist_out);
 /* _fix_inst, the first step of every label maker (distance_map.py:41-57, bound_map.py:18-33, unet_map.py:36-51,
  * direction_map.py:17-32): per id drop the 4-connected pieces under 5 px, split into 8-connected pieces, renumber
  * 1..K in (id, raster order of the piece) order. */
 int tiseg_fix_inst(tiseg_ctx* ctx, const int32_t* inst, int N, int H, int W, int32_t* out);
+/* _fix_inst of a uint16 instance map: both labellings read the ids at 2 B/px; out is int32 and equals that of the int32
+ * upcast */
+int tiseg_fix_inst_u16(tiseg_ctx* ctx, const uint16_t* inst, int N, int H, int W, int32_t* out);
 /* BoundLabelMake.__call__ after _fix_inst (bound_map.py:62-88): sem_out = sem with unlabelled pixels zeroed (may be
  * NULL), sem_w_bound_out = sem_out with edge_id on dilation(diamond(radius_dilate)) & ~erosion(diamond(radius_erode))
  * of every instance. */

@@ -53,12 +53,16 @@ SIGNATURES = {
     "tiseg_align_foreground": [_vp, _vp, _vp, _i, _i, _i, _i],
     "tiseg_postproc_multitask": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_pair_metrics_multiclass": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
+    "tiseg_pair_metrics_multiclass_u16gt": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_sem_counts": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_assign_sem_class": [_vp, _vp, _vp, _i, _i, _i, _i, _vp],
+    "tiseg_assign_sem_class_u16": [_vp, _vp, _vp, _i, _i, _i, _i, _vp],
     "tiseg_mudslide_watershed": [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp],
     "tiseg_gen_hv_map": [_vp, _vp, _i, _i, _i, _vp],
+    "tiseg_gen_hv_map_u16": [_vp, _vp, _i, _i, _i, _vp],
     "tiseg_instance_distance_map": [_vp, _vp, _i, _i, _i, _i, _vp],
     "tiseg_fix_inst": [_vp, _vp, _i, _i, _i, _vp],
+    "tiseg_fix_inst_u16": [_vp, _vp, _i, _i, _i, _vp],
     "tiseg_unet_weight_map": [_vp, _vp, _i, _i, _i, ctypes.c_double, ctypes.c_double, _vp, _vp],
     "tiseg_direction_labels": [_vp, _vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp],
     "tiseg_bound_label": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],

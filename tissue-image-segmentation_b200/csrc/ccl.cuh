@@ -20,6 +20,12 @@ struct ImgEqI32 {               // equal-value components of an int32 image, `bg
     const int32_t* p; int bg;
     __device__ __forceinline__ bool operator()(int n, long long gi, int& v) const { v = p[gi]; return v != bg; }
 };
+struct ImgEqU16 {               // equal-value components of a uint16 image (instance ids below 65536), `bg` is background
+    const uint16_t* p; int bg;
+    __device__ __forceinline__ bool operator()(int n, long long gi, int& v) const { v = p[gi]; return v != bg; }
+};
+inline ImgEqI32 img_eq(const int32_t* p, int bg) { return ImgEqI32{p, bg}; }     // the functor of an instance map's id type
+inline ImgEqU16 img_eq(const uint16_t* p, int bg) { return ImgEqU16{p, bg}; }
 struct ImgEqU8 {                // equal-value components of a uint8 image, bg < 0 => no background
     const uint8_t* p; int bg;
     __device__ __forceinline__ bool operator()(int n, long long gi, int& v) const { v = p[gi]; return v != bg; }
@@ -109,6 +115,12 @@ __device__ __forceinline__ bool quad_i32(const int32_t* q, int (&b)[4]) {
     b[0] = w.x; b[1] = w.y; b[2] = w.z; b[3] = w.w;
     return true;
 }
+__device__ __forceinline__ bool quad_u16(const uint16_t* q, int (&b)[4]) {
+    if (((uintptr_t)q) & 7) return false;
+    const uint2 w = *reinterpret_cast<const uint2*>(q);
+    b[0] = w.x & 0xffffu; b[1] = w.x >> 16; b[2] = w.y & 0xffffu; b[3] = w.y >> 16;
+    return true;
+}
 #define TISEG_IMG_QUAD(Type, LOAD, PTR, FG, VAL)                                                                  \
     __device__ __forceinline__ void img_quad(const Type& img, int n, long long gi, int (&v)[4]) {                 \
         int b[4];                                                                                                 \
@@ -119,6 +131,7 @@ __device__ __forceinline__ bool quad_i32(const int32_t* q, int (&b)[4]) {
         }                                                                                                         \
     }
 TISEG_IMG_QUAD(ImgEqI32, quad_i32, img.p, b[k] != img.bg, b[k])
+TISEG_IMG_QUAD(ImgEqU16, quad_u16, img.p, b[k] != img.bg, b[k])
 TISEG_IMG_QUAD(ImgNonZeroI32, quad_i32, img.p, b[k] != 0, 1)
 TISEG_IMG_QUAD(ImgEqU8, quad_u8, img.p, b[k] != img.bg, b[k])
 TISEG_IMG_QUAD(ImgMaskU8, quad_u8, img.p, b[k] != 0, 1)

@@ -347,6 +347,22 @@ __device__ __forceinline__ void ld4f_aligned(const T* p, float (&x)[4]) {
     for (int k = 0; k < 4; ++k) x[k] = to_f32(h.v[k]);
 }
 
+// ---- instance maps in int32 or uint16 -----------------------------------------------------------------------------------
+// Kernels that read a ground-truth instance map are templated on its id type: int32, or uint16 (ids below 65536, which
+// every dataset the reference converts keeps to) read as it is, at half the bytes, and widened in registers.  A uint16 id
+// is below every id table's VM = max(H*W + 1, 65536), so it can never raise the "instance id out of range" error.
+// Timing name of a launch: the int32 instantiation keeps the plain kernel name, the uint16 one carries the type.
+#define TISEG_ID_NAME(T, name) (sizeof(T) == 2 ? name "<uint16_t>" : name)
+// four consecutive ids from an address aligned to four elements: one 16-byte load in int32, one 8-byte load in uint16
+__device__ __forceinline__ void ld_ids4(const int32_t* p, int (&v)[4]) {
+    const int4 q = *reinterpret_cast<const int4*>(p);
+    v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+}
+__device__ __forceinline__ void ld_ids4(const uint16_t* p, int (&v)[4]) {
+    const uint2 q = *reinterpret_cast<const uint2*>(p);
+    v[0] = q.x & 0xffffu; v[1] = q.x >> 16; v[2] = q.y & 0xffffu; v[3] = q.y >> 16;
+}
+
 // Given the ballot of "this lane continues the run of the lane to its left" (bit 0 of the segment may be
 // set when the run continues from the previous segment), the lane at which my run starts inside the segment.
 __device__ __forceinline__ int run_start_lane(unsigned cont, int lane) {

@@ -22,11 +22,14 @@ struct InstBox {
     int VM;
 };
 
+// The kernels that read a raw ground-truth instance map (gen_instance_hv_map, _fix_inst) are templated on its id type T,
+// int32 or uint16 (common.cuh); the maps they produce are int32 either way.
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_inst_stats(Geom g, const int32_t* __restrict__ inst, InstBox b, int* bad) {
+k_inst_stats(Geom g, const T* __restrict__ inst, InstBox b, int* bad) {
     Pix px;
     if (!warp_pixel(g, px)) return;
-    int v = px.ok ? inst[px.base + px.idx] : 0;
+    int v = px.ok ? (int)inst[px.base + px.idx] : 0;
     int vl = __shfl_up_sync(0xffffffffu, v, 1);
     bool cont = px.lane > 0 && v == vl;
     unsigned m = __ballot_sync(0xffffffffu, cont);
@@ -49,11 +52,12 @@ __global__ void k_inst_box_init(InstBox b, int N, int H, int W) {
 
 // hv_map.py:36-95 per pixel: crop box = bbox expanded by 2 (clipped); centre of mass of the crop rounded to a pixel;
 // x = (col - box_x0 + 1) - com_x; negative side divided by its most negative value, positive side by its largest.
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_hv_map(Geom g, const int32_t* __restrict__ inst, InstBox b, float2* __restrict__ hv) {
+k_hv_map(Geom g, const T* __restrict__ inst, InstBox b, float2* __restrict__ hv) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
-    const int v = inst[px.base + px.idx];
+    const int v = (int)inst[px.base + px.idx];
     float xv = 0.f, yv = 0.f;
     if (v > 0 && v < b.VM) {
         const long long o = (long long)px.n * b.VM + v;
@@ -141,23 +145,26 @@ k_idm_finish(Geom g, const int32_t* __restrict__ inst, const int* __restrict__ d
 // Per id: remove_small_objects(mask, 5) (4-connected pieces), measure.label (8-connected), ids handed out in
 // (id, raster order of the piece) order.  Two equal-value CCL passes do the per-id work for every id at once; the
 // new id of a piece = pieces of smaller ids (scan over the id axis) + its raster rank among the pieces of its id + 1.
+// The kept map has the id type of the input, so both labellings read the ids at the input's width.
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_fix_keep(long long total, long long P, const int32_t* __restrict__ inst, const int* __restrict__ par,
-           const int* __restrict__ area, int32_t* __restrict__ out) {
+k_fix_keep(long long total, long long P, const T* __restrict__ inst, const int* __restrict__ par,
+           const int* __restrict__ area, T* __restrict__ out) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     const int p = par[i];
-    out[i] = (p >= 0 && area[i - i % P + p] >= 5) ? inst[i] : 0;
+    out[i] = (p >= 0 && area[i - i % P + p] >= 5) ? inst[i] : (T)0;
 }
 // every root: slot within its id, max id per tile
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_fix_root_slots(Geom g, const int32_t* __restrict__ lab, const int* __restrict__ par, int* cnt, int* slot, int* vmax,
+k_fix_root_slots(Geom g, const T* __restrict__ lab, const int* __restrict__ par, int* cnt, int* slot, int* vmax,
                  int VM, int* bad) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
     const long long i = px.base + px.idx;
     if (par[i] != px.idx) return;
-    const int v = lab[i];
+    const int v = (int)lab[i];
     if (v < 0 || v >= VM) { *bad = 1; return; }
     slot[i] = atomicAdd(&cnt[(long long)px.n * VM + v], 1);
     atomicMax(&vmax[px.n], v);
@@ -192,23 +199,25 @@ __global__ void __launch_bounds__(1024) k_fix_scan(const int* __restrict__ cnt, 
         __syncthreads();
     }
 }
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_fix_list(Geom g, const int32_t* __restrict__ lab, const int* __restrict__ par, const int* __restrict__ base,
+k_fix_list(Geom g, const T* __restrict__ lab, const int* __restrict__ par, const int* __restrict__ base,
            const int* __restrict__ slot, int* __restrict__ lst, int VM) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
     const long long i = px.base + px.idx;
     if (par[i] != px.idx) return;
-    lst[px.base + base[(long long)px.n * VM + lab[i]] + slot[i]] = px.idx;
+    lst[px.base + base[(long long)px.n * VM + (int)lab[i]] + slot[i]] = px.idx;
 }
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_fix_newid(Geom g, const int32_t* __restrict__ lab, const int* __restrict__ par, const int* __restrict__ base,
+k_fix_newid(Geom g, const T* __restrict__ lab, const int* __restrict__ par, const int* __restrict__ base,
             const int* __restrict__ cnt, const int* __restrict__ lst, int* __restrict__ newid, int VM) {
     Pix px;
     if (!warp_pixel(g, px) || !px.ok) return;
     const long long i = px.base + px.idx;
     if (par[i] != px.idx) return;
-    const long long o = (long long)px.n * VM + lab[i];
+    const long long o = (long long)px.n * VM + (int)lab[i];
     const int b = base[o], k = cnt[o];
     int before = 0;
     for (int j = 0; j < k; ++j) before += lst[px.base + b + j] < px.idx;
@@ -344,7 +353,8 @@ k_unet_weight(Geom g, const int32_t* __restrict__ inner, const int4* __restrict_
     }
 }
 
-static int inst_tables(tiseg_ctx* c, const Geom& g, const int32_t* d_inst, InstBox& b) {
+template <class T>
+static int inst_tables(tiseg_ctx* c, const Geom& g, const T* d_inst, InstBox& b) {
     const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
     const size_t n = (size_t)g.N * VM;
     b.VM = VM;
@@ -352,8 +362,59 @@ static int inst_tables(tiseg_ctx* c, const Geom& g, const int32_t* d_inst, InstB
     b.sy = ws<unsigned long long>(c, n); b.sx = ws<unsigned long long>(c, n);
     if (!b.ymin || !b.ymax || !b.xmin || !b.xmax || !b.cnt || !b.sy || !b.sx) return TISEG_ERR_CUDA;
     TISEG_LAUNCH(c, k_inst_box_init, (unsigned)((n + 255) / 256), 256, 0, b, g.N, g.H, g.W);
-    TISEG_LAUNCH(c, k_inst_stats, warp_grid(g), TISEG_THREADS, 0, g, d_inst, b, c->d_err);
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_inst_stats"), k_inst_stats<T>, warp_grid(g), TISEG_THREADS, 0, g, d_inst, b, c->d_err);
     return TISEG_OK;
+}
+
+// the int32 / uint16 twins of the C entries below share these bodies
+template <class T>
+static int gen_hv_map_any(tiseg_ctx* c, const T* inst, int N, int H, int W, float* hv_out) {
+    if (!c || !inst || !hv_out) { set_error("tiseg_gen_hv_map: bad argument"); return TISEG_ERR_ARG; }
+    Call call(c, "tiseg_gen_hv_map", N, H, W);
+    const T* d_inst = call.in(inst, call.total);
+    float* d_hv = call.out(hv_out, call.total * 2);
+    TISEG_TRY(call.status());
+    const Geom& g = call.g;
+    InstBox b;
+    TISEG_TRY(inst_tables(c, g, d_inst, b));
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_hv_map"), k_hv_map<T>, warp_grid(g), TISEG_THREADS, 0, g, d_inst, b, (float2*)d_hv);
+    return call.finish();
+}
+
+template <class T>
+static int fix_inst_any(tiseg_ctx* c, const T* inst, int N, int H, int W, int32_t* out) {
+    if (!c || !inst || !out) { set_error("tiseg_fix_inst: bad argument"); return TISEG_ERR_ARG; }
+    Call call(c, "tiseg_fix_inst", N, H, W);
+    const Geom& g = call.g;
+    const size_t total = call.total;
+    const T* d_inst = call.in(inst, total);
+    int32_t* d_out = call.out(out, total);
+    TISEG_TRY(call.status());
+    const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
+    int* par = ws<int>(c, total); int* aux = ws<int>(c, total); int* lst = ws<int>(c, total);
+    T* kept = ws<T>(c, total);
+    int* cnt = ws<int>(c, (size_t)N * VM); int* base = ws<int>(c, (size_t)N * VM); int* vmax = ws<int>(c, N);
+    if (!par || !aux || !lst || !kept || !cnt || !base || !vmax) return TISEG_ERR_CUDA;
+    const unsigned fg = (unsigned)((total + TISEG_THREADS - 1) / TISEG_THREADS);
+    // remove_small_objects(inst == id, 5): 4-connected pieces of equal id
+    TISEG_TRY(ccl_build(c, g, img_eq(d_inst, 0), 1, par));
+    TISEG_TRY(ccl_areas(c, g, par, aux));
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_fix_keep"), k_fix_keep<T>, fg, TISEG_THREADS, 0, (long long)total, (long long)g.P, d_inst, par,
+                    aux, kept);
+    // measure.label(mask): 8-connected pieces of equal id
+    TISEG_TRY(ccl_build(c, g, img_eq((const T*)kept, 0), 2, par));
+    TISEG_TRY(zero(c, cnt, (size_t)N * VM * sizeof(int)));
+    TISEG_TRY(zero(c, vmax, (size_t)N * sizeof(int)));
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_fix_root_slots"), k_fix_root_slots<T>, warp_grid(g), TISEG_THREADS, 0, g, kept, par, cnt, aux,
+                    vmax, VM, c->d_err);
+    TISEG_LAUNCH(c, k_fix_scan, N, 1024, 0, cnt, base, vmax, VM);
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_fix_list"), k_fix_list<T>, warp_grid(g), TISEG_THREADS, 0, g, kept, par, base, aux, lst, VM);
+    int* newid = ws<int>(c, total);
+    if (!newid) return TISEG_ERR_CUDA;
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_fix_newid"), k_fix_newid<T>, warp_grid(g), TISEG_THREADS, 0, g, kept, par, base, cnt, lst, newid,
+                    VM);
+    TISEG_TRY(apply_rank(c, g, par, newid, d_out));
+    return call.finish();
 }
 
 }  // namespace tiseg
@@ -363,16 +424,11 @@ using namespace tiseg;
 extern "C" {
 
 int tiseg_gen_hv_map(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, float* hv_out) {
-    if (!c || !inst || !hv_out) { set_error("tiseg_gen_hv_map: bad argument"); return TISEG_ERR_ARG; }
-    Call call(c, "tiseg_gen_hv_map", N, H, W);
-    const int32_t* d_inst = call.in(inst, call.total);
-    float* d_hv = call.out(hv_out, call.total * 2);
-    TISEG_TRY(call.status());
-    const Geom& g = call.g;
-    InstBox b;
-    TISEG_TRY(inst_tables(c, g, d_inst, b));
-    TISEG_LAUNCH(c, k_hv_map, warp_grid(g), TISEG_THREADS, 0, g, d_inst, b, (float2*)d_hv);
-    return call.finish();
+    return gen_hv_map_any(c, inst, N, H, W, hv_out);
+}
+
+int tiseg_gen_hv_map_u16(tiseg_ctx* c, const uint16_t* inst, int N, int H, int W, float* hv_out) {
+    return gen_hv_map_any(c, inst, N, H, W, hv_out);
 }
 
 int tiseg_instance_distance_map(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, int inst_norm, float* dist_out) {
@@ -395,35 +451,11 @@ int tiseg_instance_distance_map(tiseg_ctx* c, const int32_t* inst, int N, int H,
 }
 
 int tiseg_fix_inst(tiseg_ctx* c, const int32_t* inst, int N, int H, int W, int32_t* out) {
-    if (!c || !inst || !out) { set_error("tiseg_fix_inst: bad argument"); return TISEG_ERR_ARG; }
-    Call call(c, "tiseg_fix_inst", N, H, W);
-    const Geom& g = call.g;
-    const size_t total = call.total;
-    const int32_t* d_inst = call.in(inst, total);
-    int32_t* d_out = call.out(out, total);
-    TISEG_TRY(call.status());
-    const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
-    int* par = ws<int>(c, total); int* aux = ws<int>(c, total); int* lst = ws<int>(c, total);
-    int32_t* kept = ws<int32_t>(c, total);
-    int* cnt = ws<int>(c, (size_t)N * VM); int* base = ws<int>(c, (size_t)N * VM); int* vmax = ws<int>(c, N);
-    if (!par || !aux || !lst || !kept || !cnt || !base || !vmax) return TISEG_ERR_CUDA;
-    const unsigned fg = (unsigned)((total + TISEG_THREADS - 1) / TISEG_THREADS);
-    // remove_small_objects(inst == id, 5): 4-connected pieces of equal id
-    TISEG_TRY(ccl_build(c, g, ImgEqI32{d_inst, 0}, 1, par));
-    TISEG_TRY(ccl_areas(c, g, par, aux));
-    TISEG_LAUNCH(c, k_fix_keep, fg, TISEG_THREADS, 0, (long long)total, (long long)g.P, d_inst, par, aux, kept);
-    // measure.label(mask): 8-connected pieces of equal id
-    TISEG_TRY(ccl_build(c, g, ImgEqI32{kept, 0}, 2, par));
-    TISEG_TRY(zero(c, cnt, (size_t)N * VM * sizeof(int)));
-    TISEG_TRY(zero(c, vmax, (size_t)N * sizeof(int)));
-    TISEG_LAUNCH(c, k_fix_root_slots, warp_grid(g), TISEG_THREADS, 0, g, kept, par, cnt, aux, vmax, VM, c->d_err);
-    TISEG_LAUNCH(c, k_fix_scan, N, 1024, 0, cnt, base, vmax, VM);
-    TISEG_LAUNCH(c, k_fix_list, warp_grid(g), TISEG_THREADS, 0, g, kept, par, base, aux, lst, VM);
-    int* newid = ws<int>(c, total);
-    if (!newid) return TISEG_ERR_CUDA;
-    TISEG_LAUNCH(c, k_fix_newid, warp_grid(g), TISEG_THREADS, 0, g, kept, par, base, cnt, lst, newid, VM);
-    TISEG_TRY(apply_rank(c, g, par, newid, d_out));
-    return call.finish();
+    return fix_inst_any(c, inst, N, H, W, out);
+}
+
+int tiseg_fix_inst_u16(tiseg_ctx* c, const uint16_t* inst, int N, int H, int W, int32_t* out) {
+    return fix_inst_any(c, inst, N, H, W, out);
 }
 
 int tiseg_bound_label(tiseg_ctx* c, const uint8_t* sem, const int32_t* inst, int N, int H, int W, int edge_id,

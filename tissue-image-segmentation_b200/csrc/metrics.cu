@@ -519,13 +519,14 @@ static int next_pow2(long long v) { int p = 1; while (p < v) p <<= 1; return p; 
 // ---- instance -> class assignment (assign_sem_class_to_insts, datasets/utils/instance_semantic.py:68-93) ----
 // hist[n, v, 0..C] = pixels of instance value v per semantic class (slot C collects out-of-range classes so
 // that the instance still exists); one atomic per in-segment run of equal (instance, class)
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_inst_class_hist(Geom g, const int32_t* __restrict__ inst, const uint8_t* __restrict__ sem, int C, int VM,
+k_inst_class_hist(Geom g, const T* __restrict__ inst, const uint8_t* __restrict__ sem, int C, int VM,
                   int* hist, int* bad) {
     Pix px;
     if (!warp_pixel(g, px)) return;
     int v = 0, c = 0;
-    if (px.ok) { v = inst[px.base + px.idx]; c = sem[px.base + px.idx]; if (c >= C) c = C; }
+    if (px.ok) { v = (int)inst[px.base + px.idx]; c = sem[px.base + px.idx]; if (c >= C) c = C; }
     int key = v * (C + 1) + c;
     int kl = __shfl_up_sync(0xffffffffu, key, 1);
     bool cont = px.lane > 0 && key == kl;
@@ -538,14 +539,17 @@ k_inst_class_hist(Geom g, const int32_t* __restrict__ inst, const uint8_t* __res
 
 // The class tables are addressed by instance id with a stride of VM = max(P + 1, 65536) entries per tile, but only the ids
 // that occur can be touched: the largest id of every tile is found first, and clearing / scanning stop there (a CoNIC
-// batch of 512 tiles has ~60 instances each: 1 GB of table shrinks to a few hundred KB of traffic).
-__global__ void __launch_bounds__(TISEG_THREADS) k_max_id(Geom g, const int32_t* __restrict__ inst, int* __restrict__ maxid) {
+// batch of 512 tiles has ~60 instances each: 1 GB of table shrinks to a few hundred KB of traffic).  Four ids per load
+// (16 B in int32, 8 B in uint16) when the tiles are aligned to four ids.
+template <class T>
+__global__ void __launch_bounds__(TISEG_THREADS) k_max_id(Geom g, const T* __restrict__ inst, int* __restrict__ maxid) {
     const int n = blockIdx.y;
-    const int32_t* t = inst + (long long)n * g.P;
+    const T* t = inst + (long long)n * g.P;
+    const bool vec = ((((uintptr_t)t) | (g.P * (unsigned long long)sizeof(T))) & (4 * sizeof(T) - 1)) == 0;
     int m = 0;
     for (long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4; i < g.P; i += (long long)gridDim.x * blockDim.x * 4) {
-        if (i + 3 < g.P && ((((uintptr_t)t) | (g.P * 4ull)) & 15) == 0) { const int4 q = *reinterpret_cast<const int4*>(t + i); m = max(max(m, max(q.x, q.y)), max(q.z, q.w)); }
-        else for (int k = 0; k < 4 && i + k < g.P; ++k) m = max(m, t[i + k]);
+        if (i + 3 < g.P && vec) { int q[4]; ld_ids4(t + i, q); m = max(max(m, max(q[0], q[1])), max(q[2], q[3])); }
+        else for (int k = 0; k < 4 && i + k < g.P; ++k) m = max(m, (int)t[i + k]);
     }
     m = __reduce_max_sync(0xffffffffu, m);
     if ((threadIdx.x & 31) == 0 && m > 0) atomicMax(&maxid[n], m);
@@ -577,8 +581,9 @@ __global__ void k_inst_class_pick(const int* __restrict__ hist, int C, int VM, u
 }
 
 // class of every connected component = class of the instance value at its root pixel (from the bitmap of the roots)
+template <class T>
 __global__ void __launch_bounds__(TISEG_THREADS)
-k_comp_class_bits(Geom g, const int32_t* __restrict__ inst, const unsigned* __restrict__ rootbits, const int* __restrict__ rank,
+k_comp_class_bits(Geom g, const T* __restrict__ inst, const unsigned* __restrict__ rootbits, const int* __restrict__ rank,
                   const uint8_t* __restrict__ cls_inst, int VM, int C, uint8_t* cls_comp, int KS, int* ncomp) {
     const long long words = (long long)g.H * g.SEG;
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -592,7 +597,7 @@ k_comp_class_bits(Geom g, const int32_t* __restrict__ inst, const unsigned* __re
         const int b = __ffs(m) - 1;
         m &= m - 1;
         const int idx = y * g.W + seg * 32 + b;
-        const int v = inst[base + idx];
+        const int v = (int)inst[base + idx];
         const int cls = (v > 0 && v < VM) ? cls_inst[(long long)n * VM + v] : 0;
         cls_comp[(long long)n * KS + rank[base + idx]] = (uint8_t)cls;
         atomicAdd(&ncomp[n * C + cls], 1);
@@ -642,9 +647,9 @@ static int pair_tab_alloc(tiseg_ctx* c, const Geom& g, PairTab& t, int* overflow
     return zero(c, t.small.cnt, cb);
 }
 
-// from bit planes (see the comment above k_pair_bits)
-static int pair_table_build(tiseg_ctx* c, const Geom& g, const int32_t* d_pred, const int32_t* d_gt, PairWork& w,
-                            PairRoots* roots, const uint16_t* d_gt16 = nullptr) {
+// from bit planes (see the comment above k_pair_bits); the ground truth is int32 or uint16 (T), the prediction int32
+template <class T>
+static int pair_table_build(tiseg_ctx* c, const Geom& g, const int32_t* d_pred, const T* d_gt, PairWork& w, PairRoots* roots) {
     const int N = g.N;
     const size_t total = (size_t)N * g.P, words = (size_t)N * g.H * g.SEG;
     BitPlanesW pw;
@@ -664,8 +669,8 @@ static int pair_table_build(tiseg_ctx* c, const Geom& g, const int32_t* d_pred, 
     const long long warps = (long long)((g.W + 255) / 256) * ((g.H + EQ_BAND - 1) / EQ_BAND);
     const dim3 eg((unsigned)((warps + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK), (unsigned)N);
     BitPlanesW pwp = {pw.F + words, pw.C + words, pw.EU + words, pw.EL + words, pw.ER + words};
-    if (d_gt16) TISEG_LAUNCH(c, k_eqbits<uint16_t>, eg, TISEG_THREADS, 0, g, d_gt16, pw, (g.W % 4 == 0) && (((uintptr_t)d_gt16) & 7) == 0);
-    else TISEG_LAUNCH(c, k_eqbits<int32_t>, eg, TISEG_THREADS, 0, g, d_gt, pw, (g.W % 4 == 0) && aligned16(d_gt));
+    TISEG_LAUNCH_AS(c, sizeof(T) == 2 ? "k_eqbits<uint16_t>" : "k_eqbits<int32_t>", k_eqbits<T>, eg, TISEG_THREADS, 0, g, d_gt, pw,
+                    (g.W % 4 == 0) && aligned_x4<T>(d_gt));
     TISEG_LAUNCH(c, k_eqbits<int32_t>, eg, TISEG_THREADS, 0, g, d_pred, pwp, (g.W % 4 == 0) && aligned16(d_pred));
     const BitPlanes p = as_const(pw);
     Geom g2 = make_geom(2 * N, g.H, g.W);                  // both maps as one batch: gt tiles, then pred tiles
@@ -704,8 +709,9 @@ static int pair_eval(tiseg_ctx* c, const Geom& g, PairWork& w, const uint8_t* cl
     return TISEG_OK;
 }
 
-// class of every component of one side (pred or gt)
-static int side_classes(tiseg_ctx* c, const Geom& g, const int32_t* inst, const uint8_t* sem, const int* rank,
+// class of every component of one side (pred or gt; T = the id type of that side's instance map)
+template <class T>
+static int side_classes(tiseg_ctx* c, const Geom& g, const T* inst, const uint8_t* sem, const int* rank,
                         const unsigned* rootbits, int C, int VM, uint8_t** cls_comp_out, int** ncomp_out, int** ninst_out,
                         int* bad) {
     int N = g.N, KS = g.P + 1;
@@ -719,11 +725,12 @@ static int side_classes(tiseg_ctx* c, const Geom& g, const int32_t* inst, const 
     TISEG_TRY(zero(c, ncomp, (size_t)N * C * sizeof(int)));
     TISEG_TRY(zero(c, ninst, (size_t)N * C * sizeof(int)));
     TISEG_TRY(zero(c, maxid, (size_t)N * sizeof(int)));
-    TISEG_LAUNCH(c, k_max_id, dim3(8, N), TISEG_THREADS, 0, g, inst, maxid);
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_max_id"), k_max_id<T>, dim3(8, N), TISEG_THREADS, 0, g, inst, maxid);
     TISEG_LAUNCH(c, k_zero_class_hist, dim3(8, N), 256, 0, hist, C, VM, maxid);
-    TISEG_LAUNCH(c, k_inst_class_hist, warp_grid(g), TISEG_THREADS, 0, g, inst, sem, C, VM, hist, bad);
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_inst_class_hist"), k_inst_class_hist<T>, warp_grid(g), TISEG_THREADS, 0, g, inst, sem, C, VM,
+                    hist, bad);
     TISEG_LAUNCH(c, k_inst_class_pick, dim3(8, N), 256, 0, hist, C, VM, cls_inst, ninst, maxid);
-    TISEG_LAUNCH(c, k_comp_class_bits, dim3((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N),
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_comp_class_bits"), k_comp_class_bits<T>, dim3((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N),
                  TISEG_THREADS, 0, g, inst, rootbits, rank, cls_inst, VM, C, cls_comp, KS, ncomp);
     *cls_comp_out = cls_comp; *ncomp_out = ncomp; *ninst_out = ninst;
     return TISEG_OK;
@@ -752,59 +759,51 @@ __global__ void k_inst_class_table(const int* __restrict__ hist, int C, int VM, 
     table[(long long)n * VM + v] = (uint8_t)cls;
 }
 
-extern "C" {
-
-int tiseg_assign_sem_class(tiseg_ctx* c, const int32_t* inst, const uint8_t* sem, int N, int H, int W, int C, uint8_t* table_out) {
+// the int32 / uint16 twins of the C entries below share these bodies (T = the id type of the ground-truth instance map)
+template <class T>
+static int assign_sem_class_any(tiseg_ctx* c, const T* inst, const uint8_t* sem, int N, int H, int W, int C, uint8_t* table_out) {
     if (!c || !inst || !sem || !table_out || C < 2 || C > 64) { set_error("tiseg_assign_sem_class: bad argument (2 <= C <= 64)"); return TISEG_ERR_ARG; }
     Call call(c, "tiseg_assign_sem_class", N, H, W);
     const Geom& g = call.g;
     const int VM = g.P + 1 < (1 << 16) ? (1 << 16) : g.P + 1;
-    const int32_t* d_inst = call.in(inst, call.total);
+    const T* d_inst = call.in(inst, call.total);
     const uint8_t* d_sem = call.in(sem, call.total);
     uint8_t* d_tab = call.out(table_out, (size_t)N * VM);
     TISEG_TRY(call.status());
     int* hist = ws<int>(c, (size_t)N * VM * (C + 1));
     if (!hist) return TISEG_ERR_CUDA;
     TISEG_TRY(zero(c, hist, (size_t)N * VM * (C + 1) * sizeof(int)));
-    TISEG_LAUNCH(c, k_inst_class_hist, warp_grid(g), TISEG_THREADS, 0, g, d_inst, d_sem, C, VM, hist, c->d_err);
+    TISEG_LAUNCH_AS(c, TISEG_ID_NAME(T, "k_inst_class_hist"), k_inst_class_hist<T>, warp_grid(g), TISEG_THREADS, 0, g, d_inst, d_sem, C,
+                    VM, hist, c->d_err);
     TISEG_LAUNCH(c, k_inst_class_table, dim3((VM + 255) / 256, N), 256, 0, hist, C, VM, d_tab);
     return call.finish();
 }
 
-static int pair_metrics_bin_any(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, const uint16_t* gt16, int N, int H, int W,
-                                double match_iou, double* aji, double* pq) {
-    if (!c || !pred || (!gt && !gt16) || !(match_iou >= 0.5)) {
+template <class T>
+static int pair_metrics_bin_any(tiseg_ctx* c, const int32_t* pred, const T* gt, int N, int H, int W, double match_iou, double* aji,
+                                double* pq) {
+    if (!c || !pred || !gt || !(match_iou >= 0.5)) {
         set_error("tiseg_pair_metrics_bin_iou: bad argument (match_iou >= 0.5: below it the reference switches to Hungarian matching)");
         return TISEG_ERR_ARG;
     }
     Call call(c, "tiseg_pair_metrics_bin_iou", N, H, W);
     const Geom& g = call.g;
     const int32_t* d_pred = call.in(pred, call.total);
-    const int32_t* d_gt = call.in(gt, call.total);
-    const uint16_t* d_gt16 = call.in(gt16, call.total);
+    const T* d_gt = call.in(gt, call.total);
     double* d_aji = call.out(aji, 2 * (size_t)N);
     double* d_pq = call.out(pq, 4 * (size_t)N);
     TISEG_TRY(call.status());
     PairWork w;
-    TISEG_TRY(pair_table_build(c, g, d_pred, d_gt, w, nullptr, d_gt16));
+    TISEG_TRY(pair_table_build(c, g, d_pred, d_gt, w, nullptr));
     ClassInfo ci = {nullptr, nullptr, nullptr, nullptr};
     TISEG_TRY(pair_eval(c, g, w, nullptr, nullptr, 2, ci, true, d_aji, d_pq, match_iou));
     return call.finish();
 }
 
-int tiseg_pair_metrics_bin_iou(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, int N, int H, int W, double match_iou,
-                               double* aji, double* pq) {
-    return pair_metrics_bin_any(c, pred, gt, nullptr, N, H, W, match_iou, aji, pq);
-}
-
-int tiseg_pair_metrics_bin_u16gt(tiseg_ctx* c, const int32_t* pred, const uint16_t* gt, int N, int H, int W, double match_iou,
-                                 double* aji, double* pq) {
-    return pair_metrics_bin_any(c, pred, nullptr, gt, N, H, W, match_iou, aji, pq);
-}
-
-int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const uint8_t* pred_sem,
-                                  const int32_t* gt_inst, const uint8_t* gt_sem, int N, int H, int W, int C,
-                                  double* aji, double* pq, double* bin_aji, double* bin_pq) {
+template <class T>
+static int pair_metrics_multiclass_any(tiseg_ctx* c, const int32_t* pred_inst, const uint8_t* pred_sem, const T* gt_inst,
+                                       const uint8_t* gt_sem, int N, int H, int W, int C, double* aji, double* pq, double* bin_aji,
+                                       double* bin_pq) {
     if (!c || !pred_inst || !pred_sem || !gt_inst || !gt_sem || C < 2 || C > 64) {
         set_error("tiseg_pair_metrics_multiclass: bad argument (2 <= C <= 64)");
         return TISEG_ERR_ARG;
@@ -813,7 +812,7 @@ int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const 
     const Geom& g = call.g;
     const int32_t* d_pi = call.in(pred_inst, call.total);
     const uint8_t* d_ps = call.in(pred_sem, call.total);
-    const int32_t* d_gi = call.in(gt_inst, call.total);
+    const T* d_gi = call.in(gt_inst, call.total);
     const uint8_t* d_gs = call.in(gt_sem, call.total);
     double* d_aji = call.out(aji, 2 * (size_t)N * C);
     double* d_pq = call.out(pq, 4 * (size_t)N * C);
@@ -839,6 +838,38 @@ int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const 
         TISEG_TRY(pair_eval(c, g, w, cls_g, cls_p, C, ci, first, d_aji, d_pq));
     }
     return call.finish();
+}
+
+extern "C" {
+
+int tiseg_assign_sem_class(tiseg_ctx* c, const int32_t* inst, const uint8_t* sem, int N, int H, int W, int C, uint8_t* table_out) {
+    return assign_sem_class_any(c, inst, sem, N, H, W, C, table_out);
+}
+
+int tiseg_assign_sem_class_u16(tiseg_ctx* c, const uint16_t* inst, const uint8_t* sem, int N, int H, int W, int C, uint8_t* table_out) {
+    return assign_sem_class_any(c, inst, sem, N, H, W, C, table_out);
+}
+
+int tiseg_pair_metrics_bin_iou(tiseg_ctx* c, const int32_t* pred, const int32_t* gt, int N, int H, int W, double match_iou,
+                               double* aji, double* pq) {
+    return pair_metrics_bin_any(c, pred, gt, N, H, W, match_iou, aji, pq);
+}
+
+int tiseg_pair_metrics_bin_u16gt(tiseg_ctx* c, const int32_t* pred, const uint16_t* gt, int N, int H, int W, double match_iou,
+                                 double* aji, double* pq) {
+    return pair_metrics_bin_any(c, pred, gt, N, H, W, match_iou, aji, pq);
+}
+
+int tiseg_pair_metrics_multiclass(tiseg_ctx* c, const int32_t* pred_inst, const uint8_t* pred_sem,
+                                  const int32_t* gt_inst, const uint8_t* gt_sem, int N, int H, int W, int C,
+                                  double* aji, double* pq, double* bin_aji, double* bin_pq) {
+    return pair_metrics_multiclass_any(c, pred_inst, pred_sem, gt_inst, gt_sem, N, H, W, C, aji, pq, bin_aji, bin_pq);
+}
+
+int tiseg_pair_metrics_multiclass_u16gt(tiseg_ctx* c, const int32_t* pred_inst, const uint8_t* pred_sem,
+                                        const uint16_t* gt_inst, const uint8_t* gt_sem, int N, int H, int W, int C,
+                                        double* aji, double* pq, double* bin_aji, double* bin_pq) {
+    return pair_metrics_multiclass_any(c, pred_inst, pred_sem, gt_inst, gt_sem, N, H, W, C, aji, pq, bin_aji, bin_pq);
 }
 
 int tiseg_sem_counts(tiseg_ctx* c, const uint8_t* pred, const uint8_t* gt, int N, int H, int W, int C,

@@ -128,9 +128,18 @@ class CustomDataset:
         """Same-shaped per-image arrays -> one batch (CUDA tensors stay on the device)."""
         if is_torch(arrs[0]):
             import torch
+            if dtype == np.uint16:
+                # stacked as int16 views (the same bits): torch implements few operators for uint16
+                return torch.stack([a.view(torch.int16) for a in arrs]).view(torch.uint16)
             tdt = {np.uint8: torch.uint8, np.int32: torch.int32}[dtype]
             return torch.stack([a for a in arrs]).to(tdt)
         return np.stack([np.asarray(a) for a in arrs]).astype(dtype, copy=False)
+
+    @staticmethod
+    def _inst_dtype(arrs):
+        """Batch dtype of a group of ground-truth instance maps: uint16 when every map of the group is uint16 (numpy or
+        torch; the kernels read it as it is, at half the bytes of int32), int32 otherwise."""
+        return np.uint16 if all(str(getattr(a, "dtype", "")) in ("uint16", "torch.uint16") for a in arrs) else np.int32
 
     def _groups(self, preds):
         by_shape = OrderedDict()
@@ -150,7 +159,7 @@ class CustomDataset:
             sem_p = self._stack([preds[k]['sem_pred'] for k in ks], np.uint8)
             inst_p = self._stack([preds[k]['inst_pred'] for k in ks], np.int32)
             sem_g = self._stack([sem_gts[k] for k in ks], np.uint8)        # CUDA-resident ground truth stays resident
-            inst_g = self._stack([inst_gts[k] for k in ks], np.int32)
+            inst_g = self._stack([inst_gts[k] for k in ks], self._inst_dtype([inst_gts[k] for k in ks]))
             sem_res = M.pre_eval_all_semantic_metric(sem_p, sem_g, C)
             # re_instance + measure.label of both maps happen inside the pair kernel (custom.py:272-277)
             aji, pq = ops.pair_metrics_bin(inst_p, inst_g)
@@ -174,7 +183,7 @@ class CustomDataset:
         if inst is not None and not isinstance(inst, (list, tuple)) and contiguous:
             return sem[indices[0]:indices[0] + len(indices)], inst[indices[0]:indices[0] + len(indices)]
         sg, ig = zip(*[self._load_gt(i) for i in indices])
-        return self._stack(list(sg), np.uint8), self._stack(list(ig), np.int32)
+        return self._stack(list(sg), np.uint8), self._stack(list(ig), self._inst_dtype(ig))
 
     def pre_eval_records(self, sem_pred, inst_pred, indices, check=True):
         """``pre_eval`` for a whole batch ``[n, H, W]`` without a Python loop over the images: returns ONE float64 array
@@ -330,7 +339,7 @@ class CoNICDataset(CustomDataset):
             sem_p = self._stack([preds[k]['sem_pred'] for k in ks], np.uint8)
             inst_p = self._stack([preds[k]['inst_pred'] for k in ks], np.int32)
             sem_g = self._stack([sem_gts[k] for k in ks], np.uint8)        # CUDA-resident ground truth stays resident
-            inst_g = self._stack([inst_gts[k] for k in ks], np.int32)
+            inst_g = self._stack([inst_gts[k] for k in ks], self._inst_dtype([inst_gts[k] for k in ks]))
             sem_res = M.pre_eval_all_semantic_metric(sem_p, sem_g, C)
             r = ops.pair_metrics_multiclass(inst_p, sem_p, inst_g, sem_g, C)
             aji, pq = _host(r['aji']).astype(np.float32), _host(r['pq']).astype(np.float32)

@@ -3,6 +3,7 @@
 Same class names, constructor arguments and ``data`` dict protocol as the reference (``DistanceLabelMake``:
 datasets/ops/distance_map.py:23-142, ``HVLabelMake``: hv_map.py:100-114, ``BoundLabelMake``: bound_map.py:6-89).
 ``UNetLabelMake``: unet_map.py:7-127, ``DirectionLabelMake``: direction_map.py:11-193 with ``to_center=True``).
+``data["inst_gt"]`` may be int32 or uint16; a uint16 map is read as it is and gives the same ``data`` dict.
 """
 import numpy as np
 

@@ -63,7 +63,7 @@ def _maps_from_id_lists(inst, id_list_per_class, num_classes):
     """The reference's ``{class: [instance ids]}`` form (what ``assign_sem_class_to_insts`` returns,
     instance_semantic.py:68-93) -> (instance map with unlisted ids removed, class map): every listed instance is painted
     with its class, so the device-side majority vote reproduces the dictionary exactly; ids that appear in no list do not
-    take part in the reference's sums at all (inst_metrics.py:103-131) and are zeroed."""
+    take part in the reference's sums at all (inst_metrics.py:103-131) and are zeroed.  A uint16 map stays uint16."""
     inst = np.asarray(_host(inst))
     top = int(inst.max()) if inst.size else 0
     lut = np.full(top + 2, -1, np.int64)
@@ -78,7 +78,8 @@ def _maps_from_id_lists(inst, id_list_per_class, num_classes):
                 lut[i] = int(cls)
     cls_of = lut[np.clip(inst, 0, top + 1)]
     keep = (cls_of >= 0) & (inst > 0)
-    return np.where(keep, inst, 0).astype(np.int32), np.where(keep, cls_of, 0).astype(np.uint8)
+    ids = np.uint16 if inst.dtype == np.uint16 else np.int32
+    return np.where(keep, inst, 0).astype(ids), np.where(keep, cls_of, 0).astype(np.uint8)
 
 
 def _multiclass(inst_pred, inst_gt, a, b, num_classes):

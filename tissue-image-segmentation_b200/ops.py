@@ -21,6 +21,14 @@ def _unbatch(out, was2d):
     return out[0] if was2d else out
 
 
+def _gt_ids(inst):
+    """A ground-truth instance map -> (C-contiguous array, is_uint16).  A uint16 map (numpy ``uint16`` or ``torch.uint16``;
+    ids below 65536, as in every dataset the reference converts) is taken as it is and read by the kernels at 2 B per
+    pixel, with the results of its int32 upcast; any other dtype is converted to int32."""
+    u16 = str(getattr(inst, "dtype", "")) in ("uint16", "torch.uint16")
+    return as_input(inst, np.uint16 if u16 else np.int32), u16
+
+
 def _inplace_arg(a, dtype, what):
     """Arguments the reference mutates in place are handed to the library as they are (no converted copy could carry
     the mutation back), so they must already be C-contiguous arrays of the exact dtype."""
@@ -176,8 +184,8 @@ def pair_metrics_bin(inst_pred, inst_gt, match_iou=0.5):
     ``match_iou`` >= 0.5: a pair counts as a PQ match when its IoU is greater (inst_metrics.py:197-203)."""
     p, was2d = batched(as_input(inst_pred, np.int32))
     # a uint16 ground truth (ids < 65536) is taken as it is: half the bytes to upload
-    gt16 = str(getattr(inst_gt, "dtype", "")) in ("uint16", "torch.uint16")
-    g, _ = batched(as_input(inst_gt, np.uint16 if gt16 else np.int32))
+    g, gt16 = _gt_ids(inst_gt)
+    g, _ = batched(g)
     if tuple(p.shape) != tuple(g.shape):
         raise ValueError("prediction / ground-truth shape mismatch: %r vs %r" % (tuple(p.shape), tuple(g.shape)))
     N, H, W = p.shape
@@ -203,9 +211,11 @@ def sem_counts(pred, gt, num_classes, ignore_index=255):
 
 def pair_metrics_multiclass(inst_pred, sem_pred, inst_gt, sem_gt, num_classes, want_bin=True):
     """A18 (+ A16/A17 from the same pair table).  -> dict(aji [N,C,2], pq [N,C,4], bin_aji [N,2], bin_pq [N,4])
-    fp64; slot 0 of the class axis is the reference's class-0 slot."""
+    fp64; slot 0 of the class axis is the reference's class-0 slot.  A uint16 ``inst_gt`` is read as it is (3 B/px of
+    ground truth with ``sem_gt`` instead of 5) and gives the results of its int32 upcast."""
     p, was2d = batched(as_input(inst_pred, np.int32))
-    g, _ = batched(as_input(inst_gt, np.int32))
+    g, gt16 = _gt_ids(inst_gt)
+    g, _ = batched(g)
     ps, _ = batched(as_input(sem_pred, np.uint8))
     gs, _ = batched(as_input(sem_gt, np.uint8))
     N, H, W = p.shape
@@ -214,7 +224,7 @@ def pair_metrics_multiclass(inst_pred, sem_pred, inst_gt, sem_gt, num_classes, w
     pq = empty_like_kind(p, (N, C, 4), np.float64)
     baji = empty_like_kind(p, (N, 2), np.float64) if want_bin else None
     bpq = empty_like_kind(p, (N, 4), np.float64) if want_bin else None
-    get_ctx(_dev(p)).call("tiseg_pair_metrics_multiclass", ptr(p), ptr(ps), ptr(g), ptr(gs), N, H, W, C,
+    get_ctx(_dev(p)).call("tiseg_pair_metrics_multiclass_u16gt" if gt16 else "tiseg_pair_metrics_multiclass", ptr(p), ptr(ps), ptr(g), ptr(gs), N, H, W, C,
                           ptr(aji), ptr(pq), ptr(baji), ptr(bpq))
     out = dict(aji=aji, pq=pq, bin_aji=baji, bin_pq=bpq)
     if was2d:
@@ -463,22 +473,25 @@ def mudslide_watershed(seg, dir_graph, fore):
 
 
 def assign_sem_class(inst, sem, num_classes):
-    """Class of every instance id as a table [N, VM] uint8 (255 = id absent); see ``metrics.assign_sem_class_to_insts``."""
-    x, was2d = batched(as_input(inst, np.int32))
+    """Class of every instance id as a table [N, VM] uint8 (255 = id absent); see ``metrics.assign_sem_class_to_insts``.
+    ``inst`` int32, or uint16 (read as it is)."""
+    x, u16 = _gt_ids(inst)
+    x, was2d = batched(x)
     sm, _ = batched(as_input(sem, np.uint8))
     N, H, W = x.shape
     VM = max(H * W + 1, 1 << 16)
     table = empty_like_kind(x, (N, VM), np.uint8)
-    get_ctx(_dev(x)).call("tiseg_assign_sem_class", ptr(x), ptr(sm), N, H, W, int(num_classes), ptr(table))
+    get_ctx(_dev(x)).call("tiseg_assign_sem_class_u16" if u16 else "tiseg_assign_sem_class", ptr(x), ptr(sm), N, H, W, int(num_classes), ptr(table))
     return table[0] if was2d else table
 
 
 def gen_instance_hv_map(inst):
-    """datasets/ops/hv_map.py:18-97.  inst [H,W] / [N,H,W] int -> [.., H, W, 2] fp32 (x map, y map)."""
-    x, was2d = batched(as_input(inst, np.int32))
+    """datasets/ops/hv_map.py:18-97.  inst [H,W] / [N,H,W] int (uint16 is read as it is) -> [.., H, W, 2] fp32 (x map, y map)."""
+    x, u16 = _gt_ids(inst)
+    x, was2d = batched(x)
     N, H, W = x.shape
     out = empty_like_kind(x, (N, H, W, 2), np.float32)
-    get_ctx(_dev(x)).call("tiseg_gen_hv_map", ptr(x), N, H, W, ptr(out))
+    get_ctx(_dev(x)).call("tiseg_gen_hv_map_u16" if u16 else "tiseg_gen_hv_map", ptr(x), N, H, W, ptr(out))
     return out[0] if was2d else out
 
 
@@ -493,11 +506,13 @@ def instance_distance_map(inst, inst_norm=True):
 
 
 def fix_inst(inst):
-    """``_fix_inst`` of the label makers (datasets/ops/distance_map.py:41-57 and its copies)."""
-    x, was2d = batched(as_input(inst, np.int32))
+    """``_fix_inst`` of the label makers (datasets/ops/distance_map.py:41-57 and its copies) -> int32.  A uint16 ``inst``
+    is read as it is."""
+    x, u16 = _gt_ids(inst)
+    x, was2d = batched(x)
     N, H, W = x.shape
     out = empty_like_kind(x, (N, H, W), np.int32)
-    get_ctx(_dev(x)).call("tiseg_fix_inst", ptr(x), N, H, W, ptr(out))
+    get_ctx(_dev(x)).call("tiseg_fix_inst_u16" if u16 else "tiseg_fix_inst", ptr(x), N, H, W, ptr(out))
     return _unbatch(out, was2d)
 
 
