@@ -275,7 +275,8 @@ __device__ __forceinline__ int bt_node_of(const unsigned (*sS)[BT_TWW], int row,
 
 // p: planes of `g.N` tile-batch entries; par [g.N, P]; lbits [g.N, H, SEG].  conn 1: 4-neighbourhood, 2: 8.
 // `bad` / `low` (may be null): a bit plane of flagged pixels; low[local root] = 1 for every tile component that holds one
-// (k_bitccl_resolve carries the flags on to the final roots).  `low` must be 0 at every node beforehand.
+// (k_bitccl_resolve carries the flags on to the final roots).  `low` is cleared at every node first (each tile clears its
+// own nodes before its first barrier); it is only meaningful at the nodes.
 template <int CONN>
 __global__ void __launch_bounds__(BT_THREADS)
 k_bitccl_tile(Geom g, BitPlanes p, int* __restrict__ par, unsigned* __restrict__ lbits, const unsigned* __restrict__ bad,
@@ -297,7 +298,13 @@ k_bitccl_tile(Geom g, BitPlanes p, int* __restrict__ par, unsigned* __restrict__
     const unsigned S = m.f & ~m.c;
     sS[r][w] = S;
     const int node0 = r * BT_TW + w * 32;
-    for (unsigned s = S; s; s &= s - 1) { const int b = __ffs(s) - 1; spar[node0 + b] = node0 + b; }
+    // the flags of the tile's own nodes start at 0 (they are raised after the second barrier, on nodes of this tile only)
+    uint8_t* lown = low ? low + (long long)n * g.P + (long long)y * g.W + seg * 32 : nullptr;
+    for (unsigned s = S; s; s &= s - 1) {
+        const int b = __ffs(s) - 1;
+        spar[node0 + b] = node0 + b;
+        if (lown) lown[b] = 0;
+    }
     __syncthreads();
     // unions with the row above; a pixel that continues its run and whose left neighbour already sits under the same
     // upper run needs none (rule of k_ccl_local)

@@ -2,11 +2,11 @@
 // with prepare_prob (:31-40), H_reconstruction_erosion (:43-57; lambda = 0.0 => identity), find_maxima
 // (:60-71), arrange_label (:101-111) and generate_wsl (:83-98).
 //
-//   d  = int32(clip(dist, 0, 255))             (truncation)             k_dist_prep
-//   I  = 255 - uint8(d);  b = d > 0.5  <=>  I < 255
+//   d  = int32(clip(dist, 0, 255))             (truncation)             k_dist_prep (one pass: I, the mask plane,
+//   I  = 255 - uint8(d);  b = d > 0.5  <=>  I < 255                      the marker candidates, the mask area)
 //   markers = label(recon_by_erosion(min(255, I+1), I) - I, masked by b)
 //           = 8-connected regional-minimum plateaus of I with value < 255, raster ids
-//                                                                       plateau CCL + k_plateau_lower + rank
+//                                                                       bit-plane CCL of the candidates + rank
 //   ws = watershed(I, markers, mask=b)                                   K6 (bucket flood)
 //   arranged = label(ws, background = most frequent value of ws)         k_ws_hist + k_pick_bg + CCL
 //   arranged[3x3 window holds >= 2 different non-zero labels] = 0        k_wsl_remove
@@ -15,87 +15,7 @@
 
 namespace tiseg {
 
-// level image + the F plane of the mask b = (I < 255): one warp = 128 columns x DP_ROWS rows, four pixels per thread and
-// row, all loads of the thread issued before the first is used.  The distance map may be fp32, fp16 or bf16 (TI); it is
-// converted to fp32 as it is loaded.
-#define DP_ROWS 4
-#define PB_ROWS_PER_WARP 32     // rows per warp band of k_plateau_bits (a multiple of 4)
-template <bool FULL, class TI>
-__device__ __forceinline__ void dp_rows(const Geom& g, const TI* __restrict__ dt, uint8_t* __restrict__ It, unsigned* __restrict__ Ft,
-                                        int lane, int x, int y0) {
-    const int W = g.W;
-    float d[DP_ROWS][4];
-#pragma unroll
-    for (int r = 0; r < DP_ROWS; ++r) {
-        const int y = y0 + r;
-        d[r][0] = d[r][1] = d[r][2] = d[r][3] = 0.f;
-        if (y < g.H) {                               // (uniform)
-            const int ro = y * W + x;
-            if (FULL) ld4f_aligned(dt + ro, d[r]);
-            else {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) if (x + k < W) d[r][k] = to_f32(dt[ro + k]);
-            }
-        }
-    }
-    const int seg = x >> 5, sh = (lane & 7) * 4;
-#pragma unroll
-    for (int r = 0; r < DP_ROWS; ++r) {
-        const int y = y0 + r;
-        if (y >= g.H) break;                         // (uniform)
-        const int ro = y * W + x;
-        unsigned pack = 0, nib = 0;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            float v = d[r][k];
-            if (v > 255.f) v = 255.f;      // dist.py:277-278 (comparisons are false for NaN, like numpy)
-            if (v < 0.f) v = 0.f;
-            const int t = (int)v;          // astype('int32'): truncation
-            const unsigned lv = (unsigned)(255 - (t & 255)) & 255u;
-            pack |= lv << (8 * k);
-            if ((FULL || x + k < W) && lv < 255u) nib |= 1u << k;
-        }
-        if (FULL) *reinterpret_cast<unsigned*>(It + ro) = pack;
-        else {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) if (x + k < W) It[ro + k] = (uint8_t)(pack >> (8 * k));
-        }
-        unsigned word = nib << sh;
-        word |= __shfl_xor_sync(0xffffffffu, word, 1);
-        word |= __shfl_xor_sync(0xffffffffu, word, 2);
-        word |= __shfl_xor_sync(0xffffffffu, word, 4);
-        if ((lane & 7) == 0 && seg < g.SEG) Ft[y * g.SEG + seg] = word;
-    }
-}
-template <class TI>
-__global__ void __launch_bounds__(TISEG_THREADS)
-k_dist_prep(Geom g, const TI* __restrict__ dist, uint8_t* __restrict__ I, unsigned* __restrict__ F, bool vec) {
-    const int lane = threadIdx.x & 31;
-    const int strips = (g.W + 127) >> 7, chunks = (g.H + DP_ROWS - 1) / DP_ROWS;
-    const long long wi = (long long)blockIdx.x * TISEG_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    if (wi >= (long long)strips * chunks) return;
-    const int ch = (int)(wi / strips), strip = (int)(wi - (long long)ch * strips), n = blockIdx.y;
-    // (tile bases as opaque register pairs + 32-bit offsets: one IMAD.WIDE per access)
-    const TI* dt = dist + (long long)n * g.P;
-    uint8_t* It = I + (long long)n * g.P;
-    unsigned* Ft = F + (long long)n * g.H * g.SEG;
-    asm volatile("" : "+l"(dt)); asm volatile("" : "+l"(It)); asm volatile("" : "+l"(Ft));
-    __builtin_assume(__isGlobal(dt)); __builtin_assume(__isGlobal(It)); __builtin_assume(__isGlobal(Ft));
-    if (vec && strip * 128 + 127 < g.W) dp_rows<true>(g, dt, It, Ft, lane, strip * 128 + lane * 4, ch * DP_ROWS);
-    else dp_rows<false>(g, dt, It, Ft, lane, strip * 128 + lane * 4, ch * DP_ROWS);
-}
-
-// pixels of the mask per tile (decides below whether the flood labels can outnumber the background)
-__global__ void __launch_bounds__(TISEG_THREADS) k_mask_area(Geom g, const unsigned* __restrict__ F, int* __restrict__ marea) {
-    const long long words = (long long)g.H * g.SEG;
-    const int n = blockIdx.y;
-    int a = 0;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < words; i += (long long)gridDim.x * blockDim.x)
-        a += __popc(F[(long long)n * words + i]);
-    a = __reduce_add_sync(0xffffffffu, a);
-    if ((threadIdx.x & 31) == 0 && a) atomicAdd(&marea[n], a);
-}
-
+// ---- the front: level image, mask plane, marker candidates --------------------------------------------------------------
 // Regional-minimum plateaus without labelling every plateau of the image.  A pixel is a CANDIDATE if its value is
 // below 255 and no 8-neighbour is strictly lower.  A plateau P (maximal 8-connected set of equal values) is a regional
 // minimum iff all its pixels are candidates.  Label the candidates only (equal value, 8-connected): if P is a
@@ -104,18 +24,12 @@ __global__ void __launch_bounds__(TISEG_THREADS) k_mask_area(Geom g, const unsig
 // equal-valued pixel outside C — which must be a non-candidate (a candidate would have joined C).  Hence:
 // minimum plateaus = candidate components without an "equal-valued non-candidate neighbour" flag.  On a distance map
 // the candidates are the few pixels around each nucleus centre.
-__device__ __forceinline__ unsigned ld_u8x4(const uint8_t* __restrict__ row, int x, int W, unsigned oob, bool vec) {
-    if (vec) return *reinterpret_cast<const unsigned*>(row + x);
-    unsigned r = 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) r |= (x + k < W ? (unsigned)row[x + k] : oob) << (8 * k);
-    return r;
-}
 // Candidates are a few percent of the pixels, so the plateau labelling works on one 32-bit word per 32-pixel row
-// segment (bits[n, y, seg]) and touches `par` / `low` only at the first pixel of each in-word run of candidates (the
-// nodes of the union-find).  Adjacent candidates always carry the same level (the higher one would have a lower
+// segment (bits[n, y, seg]).  Adjacent candidates always carry the same level (the higher one would have a lower
 // neighbour), so the labelling is binary.
-//   k_plateau_bits         candidate bitmap + bitmap of the candidates that touch an equal-valued non-candidate
+//   k_dist_prep            one pass over the distance map: level image I, mask plane, candidate bitmap, bitmap of the
+//                          candidates that touch an equal-valued non-candidate, mask pixels per tile
+//   (lambda > 0)           k_dist_prep without the candidates; k_plateau_bits takes them from the reconstructed image
 //   bitccl_build           8-connected components of the candidate bitmap (bitccl.cuh: union-find over runs)
 //   (bitccl_build)         low[root] = 1 for plateaus with a bad pixel; k_filter_root_bits drops them from the roots
 //   k_marker_scatter       the seed map (rank of the plateau's root on its pixels; zero elsewhere by memset)
@@ -128,18 +42,34 @@ __device__ __forceinline__ int run_start_of(unsigned w, int q) {       // first 
     return below ? 32 - __clz(below) : 0;
 }
 
-// Candidate and "bad candidate" bitmaps in one sweep.  With J = I where a pixel is NOT a candidate and 255 where it
-// is, a candidate p touches an equal-valued non-candidate iff min3x3(J)(p) == I(p) (every neighbour of a candidate is
-// >= it).  So both maps are 3x3 minima.  A thread owns four pixels of a row as two u16x2 words (pixels 0,1 / 2,3) so
-// that a three-way minimum of two pixels is ONE instruction (VIMNMX3.U16x2, __vimin3_u16x2); a warp walks down
-// PB_ROWS rows of a 32-thread (128-pixel) wide column band keeping the last three row minima in registers, left / right
-// pixels come from the neighbouring lanes.  The outer four threads on each side are halo (the stencil of a stencil
-// needs two pixels), so a warp emits 24 x 4 pixels = three bitmap words per row.  Lane <-> column mapping: lanes
-// 0..23 = output columns, 24..27 = right halo, 28..31 = left halo (neighbours by lane rotation).
+// dist.py:277-279 and 116: d = int32(clip(dist, 0, 255)) (truncation), I = 255 - uint8(d).  The comparison is false
+// for NaN, like numpy's, so NaN passes the upper clip; the unsigned truncating conversion then gives 0 for NaN and for
+// every negative value (the lower clip), so NaN is level 255 (outside the mask b = d > 0.5 = I < 255).  Three
+// instructions per pixel in this issue-bound pass, against five for an explicit lower clip and a signed conversion.
+__device__ __forceinline__ unsigned dist_level(float v) {
+    if (v > 255.f) v = 255.f;
+    return 255u - __float2uint_rz(v);
+}
+
+// The walk.  One warp = a 128-column strip x FR_BAND rows walking down, four pixels per thread and row.  Both bitmaps are
+// 3x3 minima: with J = I where a pixel is NOT a candidate and 255 where it is, a candidate p touches an equal-valued
+// non-candidate iff min3x3(J)(p) == I(p) (every neighbour of a candidate is >= it).  A thread holds its four pixels as
+// two u16x2 words (pixels 0,1 / 2,3) so that a three-way minimum of two pixels is ONE instruction (VIMNMX3.U16x2,
+// __vimin3_u16x2); the warp keeps the last row minima in registers and takes left / right pixels from the neighbouring
+// lanes.  The stencil of a stencil needs two pixels beyond the strip on each side: lanes 0 and 31 load them (one pair per
+// row), compute the candidate flag of the column next to the strip with a scalar copy of the stencil, and hand its level
+// (I) and its J to their own horizontal minima.  The band is walked from two rows above it to two rows below it, so the
+// vertical halo costs 4 / FR_BAND of the loads.  Pixels outside the image are level 255: never lower than a neighbour,
+// never a candidate, never in the mask, so every bit beyond W stays zero.
+#define FR_BAND 64
+#define FR_AHEAD 2               // rows of loads in flight per thread
 struct Px4 { unsigned lo, hi; };                      // (px0 | px1 << 16), (px2 | px3 << 16)
-__device__ __forceinline__ Px4 pb_hmin(Px4 v, int lane) {
-    const unsigned hl = __shfl_sync(0xffffffffu, v.hi, (lane + 31) & 31);      // pixels 2,3 of the thread to the left
-    const unsigned lr = __shfl_sync(0xffffffffu, v.lo, (lane + 1) & 31);       // pixels 0,1 of the thread to the right
+// horizontal 3-minimum; `edge` = the value of the column beyond the strip (used by lanes 0 and 31)
+__device__ __forceinline__ Px4 fr_hmin(Px4 v, int lane, unsigned edge) {
+    unsigned hl = __shfl_up_sync(0xffffffffu, v.hi, 1);                        // pixels 2,3 of the thread to the left
+    unsigned lr = __shfl_down_sync(0xffffffffu, v.lo, 1);                      // pixels 0,1 of the thread to the right
+    if (lane == 0) hl = edge << 16;
+    if (lane == 31) lr = edge;
     const unsigned a = __byte_perm(hl, v.lo, 0x5432);                          // (px-1, px0)
     const unsigned m = __byte_perm(v.lo, v.hi, 0x5432);                        // (px1, px2)
     const unsigned z = __byte_perm(v.hi, lr, 0x5432);                          // (px3, px4)
@@ -155,89 +85,221 @@ __device__ __forceinline__ unsigned pb_nibble(unsigned lo, unsigned hi) {
     const unsigned t = lo | (hi << 2);
     return (t | (t >> 15)) & 15u;
 }
-__global__ void __launch_bounds__(TISEG_THREADS)
-k_plateau_bits(Geom g, const uint8_t* __restrict__ I, unsigned* __restrict__ cbits, unsigned* __restrict__ badbits,
-               int* __restrict__ par, uint8_t* __restrict__ low, bool vec, int PB_ROWS) {
-    const int lane = threadIdx.x & 31;
-    const int W4 = (g.W + 3) >> 2, S = (W4 + 23) / 24, bands = (g.H + PB_ROWS - 1) / PB_ROWS;
-    const long long wi = (long long)blockIdx.x * TISEG_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    if (wi >= (long long)S * bands) return;
-    const int band = (int)(wi / S), st = (int)(wi - (long long)band * S), n = blockIdx.y;
-    const int col = lane < 28 ? lane : lane - 32;
-    const int x = (st * 24 + col) * 4, y0 = band * PB_ROWS;
-    const bool inx = x >= 0 && x < g.W;
-    // (tile bases as opaque register pairs + 32-bit offsets: one IMAD.WIDE per access in this issue-bound loop)
-    const uint8_t* It = I + (long long)n * g.P;
-    unsigned* cb = cbits + (long long)n * g.H * g.SEG;
-    unsigned* bb = badbits + (long long)n * g.H * g.SEG;
-    int* parn = par + (long long)n * g.P;
-    uint8_t* lown = low + (long long)n * g.P;
-    asm volatile("" : "+l"(It)); asm volatile("" : "+l"(cb)); asm volatile("" : "+l"(bb)); asm volatile("" : "+l"(parn)); asm volatile("" : "+l"(lown));
-    __builtin_assume(__isGlobal(It)); __builtin_assume(__isGlobal(cb)); __builtin_assume(__isGlobal(bb));
-    __builtin_assume(__isGlobal(parn)); __builtin_assume(__isGlobal(lown));
-    const int seg = st * 3 + (lane >> 3);
-    const bool writer = lane < 24 && (lane & 7) == 0 && seg < g.SEG;
+
+// The sources of the walk.  issue() starts the loads of row y (nothing outside the image); levels() turns them into the
+// thread's four levels (byte k = pixel k) and the pair beyond the strip edge (byte 0 = column xe, byte 1 = xe + 1).
+// VEC: W % 4 == 0 and the rows are aligned to four elements, so a thread's four pixels are in the row or out of it as a
+// whole, and the edge pair (at an even column) is aligned to two.
+// The distance map, fp32 / fp16 / bf16, converted to fp32 at the load.
+template <class TI, bool VEC>
+struct DistSrc {
+    static constexpr bool vec = VEC;
+    struct Raw { float d[4], e[2]; };
+    const TI* t;
+    __device__ __forceinline__ void issue(const Geom& g, int y, int x, int xe, bool oke, Raw& r) const {
+        r.d[0] = r.d[1] = r.d[2] = r.d[3] = 0.f;                      // (0 is level 255)
+        r.e[0] = r.e[1] = 0.f;
+        if (y < 0 || y >= g.H) return;                                // (uniform)
+        const int ro = y * g.W;
+        if (VEC) {
+            if (x < g.W) ld4f_aligned(t + ro + x, r.d);
+            if (oke) {
+                const float2 f = to_f32(*reinterpret_cast<const typename Pair<TI>::type*>(t + ro + xe));
+                r.e[0] = f.x; r.e[1] = f.y;
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) if (x + k < g.W) r.d[k] = to_f32(t[ro + x + k]);
+            if (oke) r.e[0] = to_f32(t[ro + xe]);
+            if (oke && xe + 1 < g.W) r.e[1] = to_f32(t[ro + xe + 1]);
+        }
+    }
+    __device__ __forceinline__ void levels(const Raw& r, unsigned& p, unsigned& e) const {
+        p = dist_level(r.d[0]) | (dist_level(r.d[1]) << 8) | (dist_level(r.d[2]) << 16) | (dist_level(r.d[3]) << 24);
+        e = dist_level(r.e[0]) | (dist_level(r.e[1]) << 8);
+    }
+};
+// A level image (u8), read as it is.
+template <bool VEC>
+struct LevelSrc {
+    static constexpr bool vec = VEC;
+    struct Raw { unsigned p, e; };
+    const uint8_t* t;
+    __device__ __forceinline__ void issue(const Geom& g, int y, int x, int xe, bool oke, Raw& r) const {
+        r.p = 0xffffffffu; r.e = 0xffffu;
+        if (y < 0 || y >= g.H) return;                                // (uniform)
+        const uint8_t* row = t + y * g.W;
+        if (VEC) {
+            if (x < g.W) r.p = *reinterpret_cast<const unsigned*>(row + x);
+        } else {
+            unsigned p = 0u;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) p |= (x + k < g.W ? (unsigned)row[x + k] : 255u) << (8 * k);
+            r.p = p;
+        }
+        if (oke) r.e = row[xe] | ((xe + 1 < g.W ? (unsigned)row[xe + 1] : 255u) << 8);
+    }
+    __device__ __forceinline__ void levels(const Raw& r, unsigned& p, unsigned& e) const { p = r.p; e = r.e; }
+};
+
+// LEVELS: store I (It) and the mask plane (mt) of rows [y0, y1) and add the band's mask pixels to *marea.
+// STENCIL: the candidate (cb) and bad-candidate (bb) bitmaps of rows [y0, y1).
+template <bool LEVELS, bool STENCIL, class Src>
+__device__ __forceinline__ void fr_walk(const Geom& g, const Src& src, uint8_t* __restrict__ It, unsigned* __restrict__ mt,
+                                        unsigned* __restrict__ cb, unsigned* __restrict__ bb, int* __restrict__ marea,
+                                        int lane, int x0, int y0, int y1) {
+    const int W = g.W, x = x0 + lane * 4;
+    const int xe = lane == 0 ? x0 - 2 : x0 + 128;                       // the pair beyond the strip edge
+    const bool oke = STENCIL && ((lane == 0 && x0 > 0) || (lane == 31 && xe < W));
+    const int seg = (x0 >> 5) + (lane >> 3);
+    const bool cwriter = (lane & 7) == 0 && seg < g.SEG, mwriter = (lane & 7) == 4 && seg < g.SEG;
+    const int q = (lane & 3) * 4;
+    const int ylo = STENCIL ? y0 - 2 : y0, yhi = STENCIL ? y1 + 2 : y1;
     const Px4 FF = {0x00ff00ffu, 0x00ff00ffu};
     Px4 hI1 = FF, hI2 = FF;          // row minima of I, rows r-1 and r-2
     Px4 hJ1 = FF, hJ2 = FF;          // row minima of J, rows r-2 and r-3
     Px4 I1 = FF, I2 = FF;            // I of rows r-1, r-2
     Px4 C2 = {0u, 0u};               // candidate flags (bits 0 / 16) of row r-2
-    const int yend = min(y0 + PB_ROWS, g.H);
-    for (int r0 = y0 - 2; r0 < yend + 2; r0 += 4) {
-        unsigned cw[4];
+    unsigned eh1 = 255u, eh2 = 255u, en1 = 255u;   // lanes 0 / 31, the column beyond the edge: row minima (r-1, r-2), I (r-1)
+    int area = 0;
+    typename Src::Raw raw[FR_AHEAD];
+    int yn = ylo;
+    auto issue = [&](typename Src::Raw& r) { src.issue(g, yn < yhi ? yn : -1, x, xe, oke, r); ++yn; };
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {                    // four independent loads in flight
-            const int r = r0 + k;
-            cw[k] = (inx && r >= 0 && r < g.H) ? ld_u8x4(It + r * g.W, x, g.W, 255u, vec) : 0xffffffffu;
+    for (int u = 0; u < FR_AHEAD; ++u) issue(raw[u]);
+    for (int r0 = ylo; r0 < yhi; r0 += FR_AHEAD) {
+        unsigned pv[FR_AHEAD], ev[FR_AHEAD];
+#pragma unroll
+        for (int u = 0; u < FR_AHEAD; ++u) src.levels(raw[u], pv[u], ev[u]);
+        if (r0 + FR_AHEAD < yhi) {                                      // (uniform) always FR_AHEAD rows ahead
+#pragma unroll
+            for (int u = 0; u < FR_AHEAD; ++u) issue(raw[u]);
         }
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int r = r0 + k;
+        for (int u = 0; u < FR_AHEAD; ++u) {
+            const int r = r0 + u;                                       // (rows past yhi: 255, nothing emitted)
+            const unsigned p = pv[u];
             Px4 c;
-            c.lo = __byte_perm(cw[k], 0u, 0x4140);
-            c.hi = __byte_perm(cw[k], 0u, 0x4342);
-            const Px4 hI0 = pb_hmin(c, lane);
-            // candidates of row r-1: the 3x3 minimum (centre included) equals the pixel, and the pixel is below 255
-            Px4 C1, J;
-            {
-                const unsigned mlo = __vimin3_u16x2(hI0.lo, hI1.lo, hI2.lo), mhi = __vimin3_u16x2(hI0.hi, hI1.hi, hI2.hi);
-                const unsigned nlo = pb_nonzero(I1.lo - mlo) | (((I1.lo + 0x00010001u) >> 8) & 0x00010001u);
-                const unsigned nhi = pb_nonzero(I1.hi - mhi) | (((I1.hi + 0x00010001u) >> 8) & 0x00010001u);
-                C1.lo = nlo ^ 0x00010001u;
-                C1.hi = nhi ^ 0x00010001u;
-                J.lo = I1.lo | (C1.lo * 255u);
-                J.hi = I1.hi | (C1.hi * 255u);
-            }
-            const Px4 hJ0 = pb_hmin(J, lane);
-            // bad candidates of row r-2
-            const unsigned jlo = __vimin3_u16x2(hJ0.lo, hJ1.lo, hJ2.lo), jhi = __vimin3_u16x2(hJ0.hi, hJ1.hi, hJ2.hi);
-            const unsigned Blo = C2.lo & ~pb_nonzero(jlo ^ I2.lo), Bhi = C2.hi & ~pb_nonzero(jhi ^ I2.hi);
-            const int y = r - 2;
-            if (y >= y0 && y < yend) {                   // (uniform)
-                unsigned w = (pb_nibble(C2.lo, C2.hi) | (pb_nibble(Blo, Bhi) << 16)) << (lane & 3) * 4;
-                // eight lanes x four pixels -> one 32-bit word of each map: lanes 0..3 of a group fill the low
-                // half-words, lanes 4..7 the high ones
-                w |= __shfl_xor_sync(0xffffffffu, w, 1);
-                w |= __shfl_xor_sync(0xffffffffu, w, 2);
-                const unsigned o = __shfl_xor_sync(0xffffffffu, w, 4);
-                if (writer) {
-                    const unsigned cwd = (w & 0xffffu) | (o << 16), bwd = (w >> 16) | (o & 0xffff0000u);
-                    const int wo = y * g.SEG + seg;
-                    cb[wo] = cwd;
-                    bb[wo] = bwd;
-                    unsigned starts = cwd & ~(cwd << 1);
-                    const int idx0 = y * g.W + seg * 32;
-                    while (starts) {
-                        const int a = __ffs(starts) - 1;
-                        starts &= starts - 1;
-                        parn[idx0 + a] = idx0 + a;
-                        lown[idx0 + a] = 0;
+            c.lo = __byte_perm(p, 0u, 0x4140);
+            c.hi = __byte_perm(p, 0u, 0x4342);
+            const bool lrow = LEVELS && r >= y0 && r < y1;              // (uniform)
+            unsigned mn = 0u;
+            if (LEVELS) {
+                if (lrow) {
+                    uint8_t* dst = It + r * W + x;
+                    if (Src::vec) { if (x < W) *reinterpret_cast<unsigned*>(dst) = p; }
+                    else {
+#pragma unroll
+                        for (int k = 0; k < 4; ++k) if (x + k < W) dst[k] = (uint8_t)(p >> (8 * k));
                     }
                 }
+                mn = pb_nibble(pb_nonzero(c.lo ^ 0x00ff00ffu), pb_nonzero(c.hi ^ 0x00ff00ffu));
             }
-            hI2 = hI1; hI1 = hI0; hJ2 = hJ1; hJ1 = hJ0; I2 = I1; I1 = c; C2 = C1;
+            unsigned cn = 0u, bn = 0u;
+            if (STENCIL) {
+                const unsigned e = ev[u];
+                const unsigned en = lane == 0 ? e >> 8 : e & 255u;     // the column next to the strip
+                const unsigned eh0 = min(min(e & 255u, e >> 8), lane == 0 ? c.lo & 0xffffu : c.hi >> 16);
+                const Px4 hI0 = fr_hmin(c, lane, en);
+                // candidates of row r-1: the 3x3 minimum (centre included) equals the pixel, and the pixel is below 255
+                Px4 C1, J;
+                {
+                    const unsigned mlo = __vimin3_u16x2(hI0.lo, hI1.lo, hI2.lo), mhi = __vimin3_u16x2(hI0.hi, hI1.hi, hI2.hi);
+                    const unsigned nlo = pb_nonzero(I1.lo - mlo) | (((I1.lo + 0x00010001u) >> 8) & 0x00010001u);
+                    const unsigned nhi = pb_nonzero(I1.hi - mhi) | (((I1.hi + 0x00010001u) >> 8) & 0x00010001u);
+                    C1.lo = nlo ^ 0x00010001u;
+                    C1.hi = nhi ^ 0x00010001u;
+                    J.lo = I1.lo | (C1.lo * 255u);
+                    J.hi = I1.hi | (C1.hi * 255u);
+                }
+                const unsigned eJ = (min(min(eh0, eh1), eh2) == en1 && en1 < 255u) ? 255u : en1;
+                const Px4 hJ0 = fr_hmin(J, lane, eJ);
+                // bad candidates of row r-2
+                const unsigned jlo = __vimin3_u16x2(hJ0.lo, hJ1.lo, hJ2.lo), jhi = __vimin3_u16x2(hJ0.hi, hJ1.hi, hJ2.hi);
+                const unsigned Blo = C2.lo & ~pb_nonzero(jlo ^ I2.lo), Bhi = C2.hi & ~pb_nonzero(jhi ^ I2.hi);
+                cn = pb_nibble(C2.lo, C2.hi);
+                bn = pb_nibble(Blo, Bhi);
+                hI2 = hI1; hI1 = hI0; hJ2 = hJ1; hJ1 = hJ0; I2 = I1; I1 = c; C2 = C1;
+                eh2 = eh1; eh1 = eh0; en1 = en;
+            }
+            // eight lanes x four pixels -> one 32-bit word of each map: lanes 0..3 of a group fill the low half-words, lanes
+            // 4..7 the high ones; lane 0 of the group stores the candidate words (row r-2), lane 4 the mask word (row r)
+            unsigned w = (cn | (bn << 16)) << q, m = mn << q;
+            if (STENCIL) { w |= __shfl_xor_sync(0xffffffffu, w, 1); w |= __shfl_xor_sync(0xffffffffu, w, 2); }
+            if (LEVELS) { m |= __shfl_xor_sync(0xffffffffu, m, 1); m |= __shfl_xor_sync(0xffffffffu, m, 2); }
+            const unsigned o = __shfl_xor_sync(0xffffffffu, (lane & 4) ? w : m, 4);
+            const int y = r - 2;
+            if (STENCIL && y >= y0 && y < y1 && cwriter) {
+                cb[y * g.SEG + seg] = (w & 0xffffu) | (o << 16);
+                bb[y * g.SEG + seg] = (w >> 16) | (o & 0xffff0000u);
+            }
+            if (lrow && mwriter) {
+                const unsigned mw = o | (m << 16);
+                mt[r * g.SEG + seg] = mw;
+                area += __popc(mw);
+            }
         }
     }
+    if (LEVELS) {
+        area = __reduce_add_sync(0xffffffffu, area);
+        if (lane == 0 && area) atomicAdd(marea, area);
+    }
+}
+
+// warp -> (strip, band) of tile blockIdx.y; false for the warps past the last band
+__device__ __forceinline__ bool fr_warp(const Geom& g, int& x0, int& y0, int& y1) {
+    const int strips = (g.W + 127) >> 7, bands = (g.H + FR_BAND - 1) / FR_BAND;
+    const long long wi = (long long)blockIdx.x * TISEG_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    if (wi >= (long long)strips * bands) return false;
+    const int band = (int)(wi / strips), strip = (int)(wi - (long long)band * strips);
+    x0 = strip * 128; y0 = band * FR_BAND; y1 = min(y0 + FR_BAND, g.H);
+    return true;
+}
+inline dim3 fr_grid(const Geom& g) {
+    const long long warps = (long long)((g.W + 127) >> 7) * ((g.H + FR_BAND - 1) / FR_BAND);
+    return dim3((unsigned)((warps + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK), (unsigned)g.N);
+}
+
+// the distance map -> I, the mask plane, marea (zeroed beforehand) and, with STENCIL, the candidate / bad-candidate planes.
+// (three blocks per SM at 80 registers, two rows ahead: 0.140 ms per 64 x 1000^2 step on a B200 at 1000 W.  Measured slower
+//  there: four rows ahead at 106 registers, two blocks per SM (+24 %); four blocks per SM with spills (+30 %); bands of 32,
+//  128 or 168 rows instead of 64 (+5 to +12 %).  The pass is bound by instruction issue.)
+template <class TI, bool STENCIL>
+__global__ void __launch_bounds__(TISEG_THREADS, 3)
+k_dist_prep(Geom g, const TI* __restrict__ dist, uint8_t* __restrict__ I, unsigned* __restrict__ mbits, unsigned* __restrict__ cbits,
+            unsigned* __restrict__ bbits, int* __restrict__ marea, bool vec) {
+    int x0, y0, y1;
+    if (!fr_warp(g, x0, y0, y1)) return;
+    const int lane = threadIdx.x & 31, n = blockIdx.y;
+    // (tile bases as opaque register pairs + 32-bit offsets: one IMAD.WIDE per access in this issue-bound loop)
+    const TI* dt = dist + (long long)n * g.P;
+    uint8_t* It = I + (long long)n * g.P;
+    unsigned* mt = mbits + (long long)n * g.H * g.SEG;
+    unsigned* ct = STENCIL ? cbits + (long long)n * g.H * g.SEG : nullptr;
+    unsigned* bt = STENCIL ? bbits + (long long)n * g.H * g.SEG : nullptr;
+    asm volatile("" : "+l"(dt)); asm volatile("" : "+l"(It)); asm volatile("" : "+l"(mt));
+    __builtin_assume(__isGlobal(dt)); __builtin_assume(__isGlobal(It)); __builtin_assume(__isGlobal(mt));
+    if (STENCIL) {
+        asm volatile("" : "+l"(ct)); asm volatile("" : "+l"(bt));
+        __builtin_assume(__isGlobal(ct)); __builtin_assume(__isGlobal(bt));
+    }
+    if (vec) fr_walk<true, STENCIL>(g, DistSrc<TI, true>{dt}, It, mt, ct, bt, marea + n, lane, x0, y0, y1);
+    else fr_walk<true, STENCIL>(g, DistSrc<TI, false>{dt}, It, mt, ct, bt, marea + n, lane, x0, y0, y1);
+}
+
+// the candidate / bad-candidate planes of a level image (the H-reconstruction of I when lambda > 0)
+__global__ void __launch_bounds__(TISEG_THREADS)
+k_plateau_bits(Geom g, const uint8_t* __restrict__ I, unsigned* __restrict__ cbits, unsigned* __restrict__ bbits, bool vec) {
+    int x0, y0, y1;
+    if (!fr_warp(g, x0, y0, y1)) return;
+    const int lane = threadIdx.x & 31, n = blockIdx.y;
+    const uint8_t* It = I + (long long)n * g.P;
+    unsigned* ct = cbits + (long long)n * g.H * g.SEG;
+    unsigned* bt = bbits + (long long)n * g.H * g.SEG;
+    asm volatile("" : "+l"(It)); asm volatile("" : "+l"(ct)); asm volatile("" : "+l"(bt));
+    __builtin_assume(__isGlobal(It)); __builtin_assume(__isGlobal(ct)); __builtin_assume(__isGlobal(bt));
+    if (vec) fr_walk<false, true>(g, LevelSrc<true>{It}, nullptr, nullptr, ct, bt, nullptr, lane, x0, y0, y1);
+    else fr_walk<false, true>(g, LevelSrc<false>{It}, nullptr, nullptr, ct, bt, nullptr, lane, x0, y0, y1);
 }
 
 // seeds: rank of the plateau's root on the pixels of every run of a minimum plateau (the map is zeroed beforehand).  Every
@@ -618,12 +680,16 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
     int* ndense = dense + N;
     TISEG_TRY(zero(c, marea, (2 * (size_t)N + 2) * sizeof(int)));
 
+    // the level image, the mask plane, marea and (lambda = 0) the marker candidates in one pass over the distance map
     TISEG_TRY(with_dtype(dtype, [&](auto z) {
         using TI = decltype(z);
-        const long long warps = (long long)((g.W + 127) / 128) * ((g.H + DP_ROWS - 1) / DP_ROWS);
-        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dist_prep"), k_dist_prep<TI>,
-                        dim3((unsigned)((warps + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK), (unsigned)N), TISEG_THREADS, 0,
-                        g, (const TI*)dist, I0, mbits, (g.W % 4 == 0) && aligned_x4<TI>(dist) && (((uintptr_t)I0) & 3) == 0);
+        const bool vec = (g.W % 4 == 0) && aligned_x4<TI>(dist) && (((uintptr_t)I0) & 3) == 0;
+        if (lamb == 0)
+            TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dist_prep"), (k_dist_prep<TI, true>), fr_grid(g), TISEG_THREADS, 0,
+                            g, (const TI*)dist, I0, mbits, cbits, bbits, marea, vec);
+        else
+            TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dist_prep"), (k_dist_prep<TI, false>), fr_grid(g), TISEG_THREADS, 0,
+                            g, (const TI*)dist, I0, mbits, (unsigned*)nullptr, (unsigned*)nullptr, marea, vec);
         return TISEG_OK;
     }));
     // Hrecons (dist.py:120): the identity for the lambda = 0.0 the reference hard-codes (dist.py:281); a real
@@ -632,6 +698,7 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
         I = ws<uint8_t>(c, total);
         if (!I) return TISEG_ERR_CUDA;
         TISEG_TRY(h_reconstruction_erosion_dev(c, g, I0, lamb, I));
+        TISEG_LAUNCH(c, k_plateau_bits, fr_grid(g), TISEG_THREADS, 0, g, I, cbits, bbits, (g.W % 4 == 0) && (((uintptr_t)I) & 3) == 0);
     }
     // blobs of the mask b from its bit plane (4-connected); their tables are filled by the seed scatter below
     const BitPlanes mask = {mbits, nullptr, nullptr, nullptr, nullptr};
@@ -642,12 +709,6 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
     TISEG_TRY(blobs_ccl(c, g, mask, bpar, brank, first, b));
     // markers: regional-minimum plateaus (8-connected, equal value) of I below 255, via the candidate pixels
     const dim3 word_grid((unsigned)(((long long)g.H * g.SEG + TISEG_THREADS - 1) / TISEG_THREADS), (unsigned)N);
-    {
-        const long long warps = (long long)(((g.W + 3) / 4 + 23) / 24) * ((g.H + PB_ROWS_PER_WARP - 1) / PB_ROWS_PER_WARP);
-        TISEG_LAUNCH(c, k_plateau_bits, dim3((unsigned)((warps + TISEG_WARPS_PER_BLOCK - 1) / TISEG_WARPS_PER_BLOCK), (unsigned)N),
-                     TISEG_THREADS, 0, g, I, cbits, bbits, par, low, (g.W % 4 == 0) && (((uintptr_t)I) & 3) == 0,
-                     PB_ROWS_PER_WARP);
-    }
     const BitPlanes cand = {cbits, nullptr, nullptr, nullptr, nullptr};
     // (a plateau with a pixel that touches an equal-valued non-candidate is not a regional minimum: low[root] = 1, set
     //  inside the labelling from the tile-local roots in shared memory)
@@ -671,7 +732,6 @@ int postproc_dist_dev(tiseg_ctx* c, const Geom& g, int dtype, const void* dist, 
     // background is 0 unless the mask covers more than half of a tile (then the histogram decides, on those tiles only)
     TISEG_TRY(zero(c, nflagged, sizeof(int)));
     TISEG_TRY(zero(c, fbits, (size_t)N * g.H * g.SEG * sizeof(unsigned)));
-    TISEG_LAUNCH(c, k_mask_area, dim3(8, N), TISEG_THREADS, 0, g, mbits, marea);
     TISEG_LAUNCH(c, k_dense_tiles, (N + 255) / 256, 256, 0, marea, N, g.P, bg, dense, ndense);
     Geom gd = listed_geom(g, dense, ndense);
     TISEG_TRY(label_clean_listed(c, g, dense, ndense, mbits, wsl));    // (the histogram reads whole tiles)
