@@ -36,8 +36,8 @@ extern "C" {
 
 /* Element type of the network outputs (logits, distance / HV / foreground maps, direction and point heads) handed to
  * the entries whose second argument is `dtype`: tiseg_softmax_argmax_typed, tiseg_softmax_argmax_tta_typed,
- * tiseg_tta_mean_typed, tiseg_postproc_dist_lambda_typed, tiseg_postproc_hover_ex, tiseg_cdnet_refine_typed and
- * tiseg_mtcdnet_refine_typed.  All network inputs of one call share it.  Half-precision inputs are converted to fp32 as
+ * tiseg_tta_mean_typed, tiseg_postproc_dist_lambda_typed, tiseg_postproc_hover_ex, tiseg_cdnet_refine_typed,
+ * tiseg_mtcdnet_refine_typed, tiseg_cdnet_refine_tta_typed and tiseg_mtcdnet_refine_tta_typed.  All network inputs of one call share it.  Half-precision inputs are converted to fp32 as
  * they are loaded and the arithmetic after the load is the fp32 path's, so a call fed fp16 / bf16 returns the bits the
  * same call returns for the fp32 upcast of its inputs, at half the input bytes (a host buffer crosses PCIe at 2 B per
  * element).  Outputs keep their types: probabilities and means stay fp32.  Another code returns TISEG_ERR_ARG. */
@@ -207,6 +207,25 @@ int tiseg_mtcdnet_refine_typed(tiseg_ctx* ctx, int dtype, const void* tc_logits,
                                const void* dir_logits, const void* point_logits, int N, int T, int Ctc, int Csem, int D,
                                int H, int W, int if_ddm, float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out,
                                uint8_t* sem_cls_out, uint8_t* dir_map_out, float* dd_out);
+
+/* The same two tails fed the RAW outputs of the TTA variants, with the window stitch (base.py:255-295) and
+ * reverse_tta_transform (base.py:365-381) fused into the loads, like tiseg_softmax_argmax_tta_typed: every head is laid
+ * out like its logits (per tile, the T <= 16 variants back to back, whole transformed images when window == 0, else
+ * their windows in the order split_inference visits them), tiseg_tta_input_elems(T, that head's channels, H, W, ...)
+ * elements per tile.  H, W: the original image.  The semantic / three-class heads are averaged by the softmax TTA kernel;
+ * the direction, angle (D == 1) and point heads are staged through shared memory one 32 x 32 tile at a time, so every
+ * head element is read once, coalesced for all eight transforms.  Outputs and arguments otherwise as the entries above,
+ * and equal to them (bit for bit) on the reverse-transformed, stitched heads; dir_map_out is variant 0's map in the
+ * original orientation. */
+int tiseg_cdnet_refine_tta_typed(tiseg_ctx* ctx, int dtype, const void* sem, const void* dir, const void* point, int N,
+                                 int T, int C, int D, int H, int W, const int* rotate_degrees, const int* flips,
+                                 int window, int overlap, int if_ddm, float* sem_prob_out, uint8_t* cls_out,
+                                 uint8_t* dir_map_out, float* dd_out);
+int tiseg_mtcdnet_refine_tta_typed(tiseg_ctx* ctx, int dtype, const void* tc, const void* sem, const void* dir,
+                                   const void* point, int N, int T, int Ctc, int Csem, int D, int H, int W,
+                                   const int* rotate_degrees, const int* flips, int window, int overlap, int if_ddm,
+                                   float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out, uint8_t* sem_cls_out,
+                                   uint8_t* dir_map_out, float* dd_out);
 
 /* ---- A13: align_foreground (tiseg/models/utils/postprocess.py:123-155) -----------------------------------
  * Ordered multi-source BFS growing the labels of `pred` into `foreground` (8-neighbourhood, first claimant

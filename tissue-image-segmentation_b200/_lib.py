@@ -50,6 +50,9 @@ SIGNATURES = {
     "tiseg_postproc_hover_ex": [_vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
     "tiseg_ddm": [_vp, _vp, _i, _i, _i, _vp],
     "tiseg_cdnet_refine_typed": [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp],
+    "tiseg_cdnet_refine_tta_typed": [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp],
+    "tiseg_mtcdnet_refine_tta_typed": [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i,
+                                       _vp, _vp, _vp, _vp, _vp, _vp],
     "tiseg_align_foreground": [_vp, _vp, _vp, _i, _i, _i, _i],
     "tiseg_postproc_multitask": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp],
     "tiseg_pair_metrics_multiclass": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp],

@@ -4,13 +4,17 @@
 //                       the tail of CDNet.inference after the CNN (tiseg/models/segmentors/cdnet.py:183-217):
 //                       softmax + TTA mean of the semantic head, TTA mean of the point head, per variant
 //                       dir[:,0] *= sem[:,0] -> argmax -> DDM, mean DDM, _ddm_enhencement (cdnet.py:354-367), argmax.
+//   tiseg_mtcdnet_refine_typed  the same for MultiTaskCDNet (multi_task_cdnet.py:262-330)
+//   tiseg_cdnet_refine_tta_typed / tiseg_mtcdnet_refine_tta_typed
+//                       both tails on the RAW window / whole-image outputs of the TTA variants: only the fronts that read
+//                       the heads differ (the TTA fronts at the end of this file), the rest is shared (refine_tail).
 // The reference does this with ~60 ATen launches per TTA variant (8 torch.roll temporaries); here the DDM is one
 // wrap-around 3x3 stencil on the uint8 direction map plus a per-tile max/min reduction.
 // The head outputs may be fp32, fp16 or bf16 (TI): the kernels that read them convert at the load; the probabilities,
 // DDM and point mean the library makes from them are fp32.
 #include <cfloat>
 
-#include "common.cuh"
+#include "tta.cuh"
 
 namespace tiseg {
 
@@ -242,7 +246,20 @@ int tiseg_ddm(tiseg_ctx* c, const uint8_t* dir_map, int N, int H, int W, float* 
 
 }  // extern "C"
 
-// the refinement after the front kernels: per-variant direction maps from dir_all on, TI = element type of the heads
+// What every front shares: the DDM of the per-variant direction maps in dir_all, the point-head mean (launched by
+// `point_mean`: the fronts differ in how they read the point head), the enhancement (mode 0 CDNet, 1 MultiTaskCDNet) and
+// the class map.
+template <class PointMean>
+static int refine_tail(tiseg_ctx* c, const Geom& g, int T, int C, int if_ddm, int mode, float* d_prob, uint8_t* d_cls, float* d_dd,
+                       const uint8_t* dir_all, float* pmean, int* pmax, PointMean&& point_mean) {
+    TISEG_TRY(ddm_dev(c, g, dir_all, T, d_dd));
+    TISEG_LAUNCH(c, k_key_init, (g.N + 255) / 256, 256, 0, pmax, g.N);
+    TISEG_TRY(point_mean());
+    TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_prob, C, d_dd, pmean, pmax, if_ddm, mode, d_cls);
+    return TISEG_OK;
+}
+
+// the refinement of reverse-transformed heads [N, T, C, H, W], TI = their element type
 template <class TI>
 static int cdnet_refine_run(tiseg_ctx* c, const Geom& g, const TI* d_sem, const TI* d_dir, const TI* d_pt, int T, int C, int D,
                             int if_ddm, float* d_prob, uint8_t* d_cls, float* d_dd, uint8_t* dir_all, float* pmean, int* pmax) {
@@ -255,11 +272,10 @@ static int cdnet_refine_run(tiseg_ctx* c, const Geom& g, const TI* d_sem, const 
         TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dir_map<9>"), (k_dir_map<TI, 9>), fg, TISEG_THREADS, 0, (long long)g.P, d_dir, d_prob, T, D, C,
                         dir_all, v4);     // D == 9 is checked by the caller
     }
-    TISEG_TRY(ddm_dev(c, g, dir_all, T, d_dd));
-    TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
-    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_point_mean"), k_point_mean<TI>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
-    TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_prob, C, d_dd, pmean, pmax, if_ddm, 0, d_cls);
-    return TISEG_OK;
+    return refine_tail(c, g, T, C, if_ddm, 0, d_prob, d_cls, d_dd, dir_all, pmean, pmax, [&] {
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_point_mean"), k_point_mean<TI>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
+        return TISEG_OK;
+    });
 }
 
 extern "C" {
@@ -355,7 +371,7 @@ k_reg_dir_map(Geom g, const TI* __restrict__ reg, const float* __restrict__ tc_p
 }
 }  // namespace tiseg
 
-// the refinement after the staging, TI = element type of the heads
+// the refinement of reverse-transformed heads [N, T, C, H, W], TI = their element type
 template <class TI>
 static int mtcdnet_refine_run(tiseg_ctx* c, const Geom& g, const TI* d_tc, const TI* d_sem, const TI* d_dir, const TI* d_pt, int T,
                               int Ctc, int Csem, int D, int if_ddm, float* d_tcp, uint8_t* d_tcc, float* d_semp, uint8_t* d_semc,
@@ -376,11 +392,10 @@ static int mtcdnet_refine_run(tiseg_ctx* c, const Geom& g, const TI* d_tc, const
         TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dir_map<9>"), (k_dir_map<TI, 9>), dim3(flat4_grid(g.P), (unsigned)N), TISEG_THREADS, 0,
                         (long long)g.P, d_dir, d_tcp, T, D, Ctc, dir_all, v4);
     }
-    TISEG_TRY(ddm_dev(c, g, dir_all, T, d_dd));
-    TISEG_LAUNCH(c, k_key_init, (N + 255) / 256, 256, 0, pmax, N);
-    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_point_mean"), k_point_mean<TI>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
-    TISEG_LAUNCH(c, k_ddm_enhance, warp_grid(g), TISEG_THREADS, 0, g, d_tcp, Ctc, d_dd, pmean, pmax, if_ddm, 1, d_tcc);
-    return TISEG_OK;
+    return refine_tail(c, g, T, Ctc, if_ddm, 1, d_tcp, d_tcc, d_dd, dir_all, pmean, pmax, [&] {
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_point_mean"), k_point_mean<TI>, warp_grid(g), TISEG_THREADS, 0, g, d_pt, T, pmean, pmax);
+        return TISEG_OK;
+    });
 }
 
 extern "C" {
@@ -418,6 +433,292 @@ int tiseg_mtcdnet_refine_typed(tiseg_ctx* c, int dtype, const void* tc_logits, c
         using TI = decltype(z);
         return mtcdnet_refine_run(c, g, (const TI*)d_tc, (const TI*)d_sem, (const TI*)d_dir, (const TI*)d_pt, T, Ctc, Csem, D, if_ddm,
                                   d_tcp, d_tcc, d_semp, d_semc, d_dd, dir_all, pmean, pmax);
+    }));
+    if (dir_map_out) {
+        uint8_t* d_dm = call.out(dir_map_out, total);
+        TISEG_TRY(call.status());
+        TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
+    }
+    return call.finish();
+}
+
+}  // extern "C"
+
+// ---- TTA fronts: the raw window / whole-image outputs of the T variants in, without a reverse-transformed copy --------
+// The semantic and three-class heads go through tta_launch (k_softmax_argmax_tta: the same arithmetic as
+// k_softmax_argmax).  The direction, angle and point heads go through the kernels below, which do the arithmetic of
+// k_dir_map / k_reg_dir_map / k_point_mean on the same values, so every output equals reverse_tta_transform + stitch +
+// tiseg_*_refine_typed bit for bit.  A block owns a 32 x 32 tile of the ORIGINAL image; the tile's pixels come from a
+// 32 x 32 region of variant t (transposed for 90 / 270 degrees, mirrored by the flips, cut at window edges), staged
+// through shared memory in the original orientation.  Lane l of the staging walks one source row — the tile's columns
+// when the variant is not transposed, its rows when it is — so the reads are coalesced for all eight transforms and
+// every head element is read from HBM once.
+namespace tiseg {
+
+#define TTA_TILE 32
+#define TTA_ROWS (TTA_TILE / TISEG_WARPS_PER_BLOCK)    // tile rows per thread
+
+// the CH channels of variant t of one head, tile (y0, x0) of tile n, into s[ch][ly][lx] (original orientation)
+template <class TI, int CH>
+__device__ __forceinline__ void tta_stage(const Geom& g, const TtaPlan& p, const TI* __restrict__ in, int n, int t, int y0, int x0,
+                                          float (&s)[CH][TTA_TILE][TTA_TILE + 1]) {
+    const bool tr = (p.rot[t] & 1) != 0;            // 90 / 270: a source row runs down the tile's column
+    const int l = threadIdx.x & 31;
+    const TI* base = in + (long long)n * p.tile_stride + p.off[t];
+#pragma unroll
+    for (int i = 0; i < TTA_ROWS; ++i) {
+        const int r = (threadIdx.x >> 5) + i * TISEG_WARPS_PER_BLOCK;
+        const int ly = tr ? l : r, lx = tr ? r : l;       // (row pitch 33: the transposed stores hit 32 banks)
+        if (y0 + ly < g.H && x0 + lx < g.W) {
+            int sy, sx, Ht, Wt;
+            tta_source(p, t, g.H, g.W, y0 + ly, x0 + lx, sy, sx, Ht, Wt);
+            long long cs;
+            const TI* src = base + window_source(p, CH, Ht, Wt, sy, sx, cs);
+#pragma unroll
+            for (int ch = 0; ch < CH; ++ch) s[ch][ly][lx] = to_f32(src[ch * cs]);
+        }
+    }
+}
+
+// k_dir_map per variant from the raw direction head: grid (T * tiles across, tiles down, N), blockIdx.x = tile * T + t so
+// the T blocks of one tile run together and share the background probabilities in L2
+template <class TI>
+__global__ void __launch_bounds__(TISEG_THREADS)
+k_dir_map_tta(Geom g, const TI* __restrict__ dir_logits, TtaPlan plan, const float* __restrict__ sem_prob, int C,
+              uint8_t* __restrict__ dir_map) {
+    __shared__ float s[9][TTA_TILE][TTA_TILE + 1];
+    const int T = plan.T, t = blockIdx.x % T, n = blockIdx.z, x0 = (blockIdx.x / T) * TTA_TILE;
+    const int ty_n = (g.H + TTA_TILE - 1) / TTA_TILE, l = threadIdx.x & 31;
+    for (int ty = blockIdx.y; ty < ty_n; ty += gridDim.y) {
+        const int y0 = ty * TTA_TILE;
+        tta_stage<TI, 9>(g, plan, dir_logits, n, t, y0, x0, s);
+        __syncthreads();
+#pragma unroll
+        for (int i = 0; i < TTA_ROWS; ++i) {
+            const int r = (threadIdx.x >> 5) + i * TISEG_WARPS_PER_BLOCK, y = y0 + r, x = x0 + l;
+            if (y >= g.H || x >= g.W) continue;
+            const int idx = y * g.W + x;
+            const float s0 = sem_prob[(long long)n * C * g.P + idx];
+            float xv[9], m = -INFINITY;                          // the arithmetic of k_dir_map, in its order
+#pragma unroll
+            for (int d = 0; d < 9; ++d) { xv[d] = s[d][r][l]; m = fmaxf(m, xv[d]); }
+            float sum = 0.f;
+#pragma unroll
+            for (int d = 0; d < 9; ++d) { xv[d] = expf(xv[d] - m); sum = sum + xv[d]; }
+            int best = 0;
+            float bv = -INFINITY;
+#pragma unroll
+            for (int d = 0; d < 9; ++d) {
+                float p = xv[d] / sum;
+                if (d == 0) p = p * s0;
+                if (p > bv) { bv = p; best = d; }
+            }
+            dir_map[((long long)n * T + t) * g.P + idx] = (uint8_t)best;
+        }
+        __syncthreads();
+    }
+}
+
+// k_reg_dir_map per variant from the raw angle head (use_regression), grid as k_dir_map_tta
+template <class TI>
+__global__ void __launch_bounds__(TISEG_THREADS)
+k_reg_dir_map_tta(Geom g, const TI* __restrict__ reg, TtaPlan plan, const float* __restrict__ tc_prob, int C,
+                  uint8_t* __restrict__ dir_map) {
+    __shared__ float s[1][TTA_TILE][TTA_TILE + 1];
+    const int T = plan.T, t = blockIdx.x % T, n = blockIdx.z, x0 = (blockIdx.x / T) * TTA_TILE;
+    const int ty_n = (g.H + TTA_TILE - 1) / TTA_TILE, l = threadIdx.x & 31;
+    for (int ty = blockIdx.y; ty < ty_n; ty += gridDim.y) {
+        const int y0 = ty * TTA_TILE;
+        tta_stage<TI, 1>(g, plan, reg, n, t, y0, x0, s);
+        __syncthreads();
+#pragma unroll
+        for (int i = 0; i < TTA_ROWS; ++i) {
+            const int r = (threadIdx.x >> 5) + i * TISEG_WARPS_PER_BLOCK, y = y0 + r, x = x0 + l;
+            if (y >= g.H || x >= g.W) continue;
+            const int idx = y * g.W + x;
+            const float* tp = tc_prob + (long long)n * C * g.P + idx;     // the arithmetic of k_reg_dir_map, in its order
+            float best = tp[0];
+            bool bg = true;
+            for (int k = 1; k < C; ++k) if (tp[(long long)k * g.P] > best) { best = tp[(long long)k * g.P]; bg = false; }
+            float a = s[0][r][l];
+            if (a < 0.f) a = 0.f;
+            if (a > 6.28318548202514648f) a = 6.28318548202514648f;
+            float deg = (a * 180.f) / 3.14159274101257324f;
+            if (deg > 180.f) deg -= 360.f;
+            int bin = 0;
+            for (int j = 1; j < 8; ++j) {
+                const float middle = -180.f + 45.f * (float)j;
+                if (deg > middle - 22.5f && deg <= middle + 22.5f) bin = j;
+            }
+            dir_map[((long long)n * T + t) * g.P + idx] = bg ? (uint8_t)0 : (uint8_t)(bin + 1);
+        }
+        __syncthreads();
+    }
+}
+
+// k_point_mean from the raw point head: the variants summed in order t = 0 .. T-1 in one thread, the per-tile maximum by
+// atomicMax.  grid (tiles across, tiles down, N); variant t is staged into buffer t & 1, one barrier per variant.
+template <class TI>
+__global__ void __launch_bounds__(TISEG_THREADS)
+k_point_mean_tta(Geom g, const TI* __restrict__ point_logits, TtaPlan plan, float* __restrict__ pmean, int* pmax_key) {
+    __shared__ float s[2][1][TTA_TILE][TTA_TILE + 1];
+    const int T = plan.T, n = blockIdx.z, x0 = blockIdx.x * TTA_TILE;
+    const int ty_n = (g.H + TTA_TILE - 1) / TTA_TILE, l = threadIdx.x & 31;
+    for (int ty = blockIdx.y; ty < ty_n; ty += gridDim.y) {
+        const int y0 = ty * TTA_TILE;
+        float acc[TTA_ROWS];
+        for (int t = 0; t < T; ++t) {
+            tta_stage<TI, 1>(g, plan, point_logits, n, t, y0, x0, s[t & 1]);
+            __syncthreads();
+#pragma unroll
+            for (int i = 0; i < TTA_ROWS; ++i) {
+                const float v = s[t & 1][0][(threadIdx.x >> 5) + i * TISEG_WARPS_PER_BLOCK][l];
+                acc[i] = t == 0 ? v : acc[i] + v;
+            }
+        }
+        int k = float_order_key(-INFINITY);
+#pragma unroll
+        for (int i = 0; i < TTA_ROWS; ++i) {
+            const int y = y0 + (threadIdx.x >> 5) + i * TISEG_WARPS_PER_BLOCK, x = x0 + l;
+            if (y >= g.H || x >= g.W) continue;
+            const float a = acc[i] / (float)T;
+            pmean[(long long)n * g.P + y * g.W + x] = a;
+            k = max(k, float_order_key(a));
+        }
+        for (int sh = 16; sh; sh >>= 1) k = max(k, __shfl_xor_sync(0xffffffffu, k, sh));
+        if (l == 0 && k > pmax_key[n]) atomicMax(&pmax_key[n], k);
+        __syncthreads();                                 // the next tile row stages into buffer 0 again
+    }
+}
+
+// grids of the fronts: tiles down are walked by a loop above 65535
+inline dim3 tta_front_grid(const Geom& g, int per_tile) {
+    const unsigned tx = (unsigned)((g.W + TTA_TILE - 1) / TTA_TILE), ty = (unsigned)((g.H + TTA_TILE - 1) / TTA_TILE);
+    return dim3(tx * (unsigned)per_tile, ty < 65535u ? ty : 65535u, (unsigned)g.N);
+}
+
+template <class TI>
+static int point_mean_tta(tiseg_ctx* c, const Geom& g, const TI* d_pt, const TtaPlan& pp, float* pmean, int* pmax) {
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_point_mean_tta"), k_point_mean_tta<TI>, tta_front_grid(g, 1), TISEG_THREADS, 0, g, d_pt, pp,
+                    pmean, pmax);
+    return TISEG_OK;
+}
+
+}  // namespace tiseg
+
+// the refinement of the raw variant outputs, each head through its plan; the tail is cdnet_refine_run's
+template <class TI>
+static int cdnet_refine_tta_run(tiseg_ctx* c, const Geom& g, const TI* d_sem, const TI* d_dir, const TI* d_pt, const TtaPlan& ps,
+                                const TtaPlan& pd, const TtaPlan& pp, int C, int if_ddm, float* d_prob, uint8_t* d_cls, float* d_dd,
+                                uint8_t* dir_all, float* pmean, int* pmax) {
+    TISEG_TRY(tta_launch(c, g, d_sem, ps, C, d_prob, (uint8_t*)nullptr, true));
+    TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dir_map_tta"), k_dir_map_tta<TI>, tta_front_grid(g, ps.T), TISEG_THREADS, 0, g, d_dir, pd,
+                    d_prob, C, dir_all);
+    return refine_tail(c, g, ps.T, C, if_ddm, 0, d_prob, d_cls, d_dd, dir_all, pmean, pmax,
+                       [&] { return point_mean_tta(c, g, d_pt, pp, pmean, pmax); });
+}
+
+// the same for MultiTaskCDNet; the tail is mtcdnet_refine_run's
+template <class TI>
+static int mtcdnet_refine_tta_run(tiseg_ctx* c, const Geom& g, const TI* d_tc, const TI* d_sem, const TI* d_dir, const TI* d_pt,
+                                  const TtaPlan& ptc, const TtaPlan& psem, const TtaPlan& pd, const TtaPlan& pp, int Ctc, int Csem, int D,
+                                  int if_ddm, float* d_tcp, uint8_t* d_tcc, float* d_semp, uint8_t* d_semc, float* d_dd, uint8_t* dir_all,
+                                  float* pmean, int* pmax) {
+    TISEG_TRY(tta_launch(c, g, d_tc, ptc, Ctc, d_tcp, (uint8_t*)nullptr, true));
+    if (d_semp || d_semc) TISEG_TRY(tta_launch(c, g, d_sem, psem, Csem, d_semp, d_semc, true));
+    if (D == 1)
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_reg_dir_map_tta"), k_reg_dir_map_tta<TI>, tta_front_grid(g, ptc.T), TISEG_THREADS, 0, g,
+                        d_dir, pd, d_tcp, Ctc, dir_all);
+    else
+        TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "k_dir_map_tta"), k_dir_map_tta<TI>, tta_front_grid(g, ptc.T), TISEG_THREADS, 0, g, d_dir,
+                        pd, d_tcp, Ctc, dir_all);
+    return refine_tail(c, g, ptc.T, Ctc, if_ddm, 1, d_tcp, d_tcc, d_dd, dir_all, pmean, pmax,
+                       [&] { return point_mean_tta(c, g, d_pt, pp, pmean, pmax); });
+}
+
+extern "C" {
+
+int tiseg_cdnet_refine_tta_typed(tiseg_ctx* c, int dtype, const void* sem, const void* dir, const void* point, int N, int T, int C,
+                                 int D, int H, int W, const int* rotate_degrees, const int* flips, int window, int overlap, int if_ddm,
+                                 float* sem_prob_out, uint8_t* cls_out, uint8_t* dir_map_out, float* dd_out) {
+    static const char* name = "tiseg_cdnet_refine_tta_typed";
+    TISEG_TRY(check_dtype(dtype, name));
+    if (!c || !sem || !dir || !point || T <= 0 || C < 2 || C > 16 || D != 9) {
+        set_error("tiseg_cdnet_refine_tta_typed: bad argument (2 <= C <= 16, D == 9)");
+        return TISEG_ERR_ARG;
+    }
+    TtaPlan ps, pd, pp;
+    TISEG_TRY(tta_plan(ps, T, C, H, W, rotate_degrees, flips, window, overlap, name));
+    TISEG_TRY(tta_plan(pd, T, D, H, W, rotate_degrees, flips, window, overlap, name));
+    TISEG_TRY(tta_plan(pp, T, 1, H, W, rotate_degrees, flips, window, overlap, name));
+    Call call(c, name, N, H, W, T);
+    const Geom& g = call.g;
+    const size_t total = call.total, eb = dtype_bytes(dtype);
+    const void* d_sem = call.in_bytes(sem, (size_t)N * ps.tile_stride * eb);
+    const void* d_dir = call.in_bytes(dir, (size_t)N * pd.tile_stride * eb);
+    const void* d_pt = call.in_bytes(point, (size_t)N * pp.tile_stride * eb);
+    float* d_prob = call.out(sem_prob_out, total * C);
+    uint8_t* d_cls = call.out(cls_out, total);
+    float* d_dd = call.out(dd_out, total);
+    TISEG_TRY(call.status());
+    if (!d_prob) d_prob = ws<float>(c, total * C);         // outputs the caller does not take: scratch
+    if (!d_dd) d_dd = ws<float>(c, total);
+    uint8_t* dir_all = ws<uint8_t>(c, total * T);
+    float* pmean = ws<float>(c, total);
+    int* pmax = ws<int>(c, (size_t)N);
+    if (!d_prob || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
+    TISEG_TRY(with_dtype(dtype, [&](auto z) {
+        using TI = decltype(z);
+        return cdnet_refine_tta_run(c, g, (const TI*)d_sem, (const TI*)d_dir, (const TI*)d_pt, ps, pd, pp, C, if_ddm, d_prob, d_cls, d_dd,
+                                    dir_all, pmean, pmax);
+    }));
+    if (dir_map_out) {
+        // variant 0's map, in the original orientation like every map in dir_all
+        uint8_t* d_dm = call.out(dir_map_out, total);
+        TISEG_TRY(call.status());
+        TISEG_CHECK(cudaMemcpy2DAsync(d_dm, g.P, dir_all, (size_t)T * g.P, g.P, N, cudaMemcpyDeviceToDevice, c->stream));
+    }
+    return call.finish();
+}
+
+int tiseg_mtcdnet_refine_tta_typed(tiseg_ctx* c, int dtype, const void* tc, const void* sem, const void* dir, const void* point, int N,
+                                   int T, int Ctc, int Csem, int D, int H, int W, const int* rotate_degrees, const int* flips, int window,
+                                   int overlap, int if_ddm, float* tc_prob_out, uint8_t* tc_cls_out, float* sem_prob_out,
+                                   uint8_t* sem_cls_out, uint8_t* dir_map_out, float* dd_out) {
+    static const char* name = "tiseg_mtcdnet_refine_tta_typed";
+    TISEG_TRY(check_dtype(dtype, name));
+    if (!c || !tc || !sem || !dir || !point || T <= 0 || Ctc < 2 || Ctc > 16 || Csem < 1 || Csem > 16 || (D != 9 && D != 1)) {
+        set_error("tiseg_mtcdnet_refine_tta_typed: bad argument (2 <= Ctc <= 16, 1 <= Csem <= 16, D == 9, or D == 1: the regression head)");
+        return TISEG_ERR_ARG;
+    }
+    TtaPlan ptc, psem, pd, pp;
+    TISEG_TRY(tta_plan(ptc, T, Ctc, H, W, rotate_degrees, flips, window, overlap, name));
+    TISEG_TRY(tta_plan(psem, T, Csem, H, W, rotate_degrees, flips, window, overlap, name));
+    TISEG_TRY(tta_plan(pd, T, D, H, W, rotate_degrees, flips, window, overlap, name));
+    TISEG_TRY(tta_plan(pp, T, 1, H, W, rotate_degrees, flips, window, overlap, name));
+    Call call(c, name, N, H, W, T);
+    const Geom& g = call.g;
+    const size_t total = call.total, eb = dtype_bytes(dtype);
+    const void* d_tc = call.in_bytes(tc, (size_t)N * ptc.tile_stride * eb);
+    const void* d_sem = call.in_bytes(sem, (size_t)N * psem.tile_stride * eb);
+    const void* d_dir = call.in_bytes(dir, (size_t)N * pd.tile_stride * eb);
+    const void* d_pt = call.in_bytes(point, (size_t)N * pp.tile_stride * eb);
+    float* d_tcp = call.out(tc_prob_out, total * Ctc);
+    uint8_t* d_tcc = call.out(tc_cls_out, total);
+    float* d_semp = call.out(sem_prob_out, total * Csem);
+    uint8_t* d_semc = call.out(sem_cls_out, total);
+    float* d_dd = call.out(dd_out, total);
+    TISEG_TRY(call.status());
+    if (!d_tcp) d_tcp = ws<float>(c, total * Ctc);         // outputs the caller does not take: scratch
+    if (!d_dd) d_dd = ws<float>(c, total);
+    uint8_t* dir_all = ws<uint8_t>(c, total * T);
+    float* pmean = ws<float>(c, total);
+    int* pmax = ws<int>(c, (size_t)N);
+    if (!d_tcp || !d_dd || !dir_all || !pmean || !pmax) return TISEG_ERR_CUDA;
+    TISEG_TRY(with_dtype(dtype, [&](auto z) {
+        using TI = decltype(z);
+        return mtcdnet_refine_tta_run(c, g, (const TI*)d_tc, (const TI*)d_sem, (const TI*)d_dir, (const TI*)d_pt, ptc, psem, pd, pp, Ctc,
+                                      Csem, D, if_ddm, d_tcp, d_tcc, d_semp, d_semc, d_dd, dir_all, pmean, pmax);
     }));
     if (dir_map_out) {
         uint8_t* d_dm = call.out(dir_map_out, total);

@@ -5,7 +5,7 @@
 // fp32 arithmetic in the same order as the reference expression: e = exp(x - max), s = e_0 + e_1 + ...,
 // p = e / s, acc += p per variant, acc / T.  One thread per pixel, channel planes read coalesced.
 // The logits may be fp32, fp16 or bf16 (TI = the element type); they are converted to fp32 as they are loaded.
-#include "common.cuh"
+#include "tta.cuh"
 
 namespace tiseg {
 
@@ -196,54 +196,7 @@ template int softmax_argmax_dev<float>(tiseg_ctx*, const Geom&, const float*, in
 template int softmax_argmax_dev<__half>(tiseg_ctx*, const Geom&, const __half*, int, int, float*, uint8_t*);
 template int softmax_argmax_dev<__nv_bfloat16>(tiseg_ctx*, const Geom&, const __nv_bfloat16*, int, int, float*, uint8_t*);
 
-// ---- the step before K1, fused into its load indexing (SURVEY §8f rank 2) ------------------------------------------
-// The reference stitches the half-overlap window outputs of every TTA variant into a canvas (base.py:255-295), undoes
-// the variant's rotation / flip (base.py:365-381), applies softmax and averages (base.py:321-336).  Those are pure
-// re-indexings, so this kernel reads every logit ONCE, straight from the window tensors:
-//   original pixel (y, x)  ->  pixel of the variant's (transformed) image, by the inverse of reverse_tta_transform
-//                          ->  window (my, mx) whose kept centre region holds it, and the position inside the window.
-// window == 0 means "whole" inference: the variant tensor is the full transformed image.
-struct TtaPlan {
-    int T;
-    int rot[16];                // rotate_degree // 90 of the forward transform (0..3)
-    int flip[16];               // 0 none, 1 horizontal, 2 vertical, 3 diagonal
-    long long off[16];          // element offset of variant t inside one tile's block of the input
-    long long tile_stride;      // elements per tile
-    int window, overlap;
-};
-
-__device__ __forceinline__ void tta_source(const TtaPlan& p, int t, int H, int W, int y, int x, int& sy, int& sx, int& Ht,
-                                           int& Wt) {
-    // Y = rot90(flip(X), k), k = (4 - rot) % 4, with torch.rot90 counter-clockwise: rot90(Z, 1)[i, j] = Z[j, Wz - 1 - i]
-    const int k = (4 - p.rot[t]) & 3;
-    Ht = (k & 1) ? W : H; Wt = (k & 1) ? H : W;       // shape of Z (and of X)
-    int a, b;
-    if (k == 0) { a = y; b = x; }
-    else if (k == 1) { a = x; b = Wt - 1 - y; }
-    else if (k == 2) { a = Ht - 1 - y; b = Wt - 1 - x; }
-    else { a = Ht - 1 - x; b = y; }
-    const int f = p.flip[t];
-    sy = (f & 2) ? Ht - 1 - a : a;
-    sx = (f & 1) ? Wt - 1 - b : b;
-}
-
-// element index (without the channel term) of pixel (sy, sx) of a variant image of shape (Ht, Wt): whole tensor or windows
-__device__ __forceinline__ long long window_source(const TtaPlan& p, int C, int Ht, int Wt, int sy, int sx, long long& cstride) {
-    if (p.window == 0) { cstride = (long long)Ht * Wt; return (long long)sy * Wt + sx; }
-    const int win = p.window, ov = p.overlap, st = win - ov;
-    const int pad_h = Ht - win > 0 ? st - (Ht - win) % st : win - Ht;          // base.py:264-273
-    const int pad_w = Wt - win > 0 ? st - (Wt - win) % st : win - Wt;
-    const int H1 = Ht + pad_h, W1 = Wt + pad_w;
-    const int My = (H1 - win) / st + 1, Mx = (W1 - win) / st + 1;
-    const int Y = sy + (H1 - Ht) / 2, X = sx + (W1 - Wt) / 2;                    // crop of base.py:294
-    int my = (Y - ov / 2) / st; my = my < 0 ? 0 : (my > My - 1 ? My - 1 : my);
-    int mx = (X - ov / 2) / st; mx = mx < 0 ? 0 : (mx > Mx - 1 ? Mx - 1 : mx);
-    if (Y < ov / 2) my = 0;
-    if (X < ov / 2) mx = 0;
-    cstride = (long long)win * win;
-    return ((long long)(my * Mx + mx) * C) * win * win + (long long)(Y - my * st) * win + (X - mx * st);
-}
-
+// ---- the step before K1, fused into its load indexing (SURVEY §8f rank 2): TtaPlan, tta_source, window_source (tta.cuh)
 // SOFTMAX = false: the plain mean of the reverse-transformed variants, what the reference does with its regression heads
 // (`sum(dist_logit_list) / len(dist_logit_list)`, dist.py:398-410; hovernet.py:406 keeps variant 0 only, i.e. T = 1)
 template <class TI, int CMAX, bool SOFTMAX>
@@ -308,9 +261,29 @@ extern "C" long long tiseg_tta_input_elems(int T, int C, int H, int W, const int
     return n;
 }
 
+int tiseg::tta_plan(TtaPlan& plan, int T, int C, int H, int W, const int* rotate_degrees, const int* flips, int window,
+                    int overlap, const char* where) {
+    if (!rotate_degrees || !flips || T <= 0 || T > 16 || window < 0 || (window > 0 && (overlap < 0 || overlap >= window))) {
+        set_error(std::string(where) + ": bad argument (1 <= T <= 16, 0 <= overlap < window)");
+        return TISEG_ERR_ARG;
+    }
+    plan.T = T; plan.window = window; plan.overlap = overlap;
+    long long off = 0;
+    for (int t = 0; t < T; ++t) {
+        if (rotate_degrees[t] % 90 != 0 || flips[t] < 0 || flips[t] > 3) { set_error(std::string(where) + ": bad transform"); return TISEG_ERR_ARG; }
+        plan.rot[t] = ((rotate_degrees[t] / 90) % 4 + 4) % 4;
+        plan.flip[t] = flips[t];
+        plan.off[t] = off;
+        const bool odd = (plan.rot[t] & 1) != 0;
+        off += tta_variant_elems(C, odd ? W : H, odd ? H : W, window, overlap);
+    }
+    plan.tile_stride = off;
+    return TISEG_OK;
+}
+
 template <class TI>
-static int tta_launch(tiseg_ctx* c, const Geom& g, const TI* d_in, const TtaPlan& plan, int C, float* d_prob, uint8_t* d_cls,
-                      bool softmax) {
+int tiseg::tta_launch(tiseg_ctx* c, const Geom& g, const TI* d_in, const TtaPlan& plan, int C, float* d_prob, uint8_t* d_cls,
+                     bool softmax) {
     if (softmax) {
         if (C <= 4) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<4, true>)"), (k_softmax_argmax_tta<TI, 4, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
         else if (C <= 8) TISEG_LAUNCH_AS(c, TISEG_IN_NAME(TI, "(k_softmax_argmax_tta<8, true>)"), (k_softmax_argmax_tta<TI, 8, true>), warp_grid(g), TISEG_THREADS, 0, g, d_in, plan, C, d_prob, d_cls);
@@ -323,6 +296,11 @@ static int tta_launch(tiseg_ctx* c, const Geom& g, const TI* d_in, const TtaPlan
     return TISEG_OK;
 }
 
+template int tiseg::tta_launch<float>(tiseg_ctx*, const Geom&, const float*, const TtaPlan&, int, float*, uint8_t*, bool);
+template int tiseg::tta_launch<__half>(tiseg_ctx*, const Geom&, const __half*, const TtaPlan&, int, float*, uint8_t*, bool);
+template int tiseg::tta_launch<__nv_bfloat16>(tiseg_ctx*, const Geom&, const __nv_bfloat16*, const TtaPlan&, int, float*, uint8_t*,
+                                              bool);
+
 static int tta_entry(tiseg_ctx* c, int dtype, const void* logits, int N, int T, int C, int H, int W, const int* rotate_degrees,
                      const int* flips, int window, int overlap, float* prob, uint8_t* cls, bool softmax) {
     if (!c || !logits || !rotate_degrees || !flips || T <= 0 || T > 16 || C <= 0 || C > 16 || (!prob && !cls) ||
@@ -332,19 +310,9 @@ static int tta_entry(tiseg_ctx* c, int dtype, const void* logits, int N, int T, 
     }
     TISEG_TRY(check_geom(N, H, W));
     TtaPlan plan;
-    plan.T = T; plan.window = window; plan.overlap = overlap;
-    long long off = 0;
-    for (int t = 0; t < T; ++t) {
-        if (rotate_degrees[t] % 90 != 0 || flips[t] < 0 || flips[t] > 3) { set_error("tiseg_softmax_argmax_tta_typed: bad transform"); return TISEG_ERR_ARG; }
-        plan.rot[t] = ((rotate_degrees[t] / 90) % 4 + 4) % 4;
-        plan.flip[t] = flips[t];
-        plan.off[t] = off;
-        const bool odd = (plan.rot[t] & 1) != 0;
-        off += tta_variant_elems(C, odd ? W : H, odd ? H : W, window, overlap);
-    }
-    plan.tile_stride = off;
+    TISEG_TRY(tta_plan(plan, T, C, H, W, rotate_degrees, flips, window, overlap, "tiseg_softmax_argmax_tta_typed"));
     Call call(c, "tiseg_softmax_argmax_tta_typed", N, H, W);
-    const void* d_in = call.in_bytes(logits, (size_t)N * (size_t)off * dtype_bytes(dtype));
+    const void* d_in = call.in_bytes(logits, (size_t)N * (size_t)plan.tile_stride * dtype_bytes(dtype));
     float* d_prob = call.out(prob, call.total * C);
     uint8_t* d_cls = call.out(cls, call.total);
     TISEG_TRY(call.status());

@@ -386,6 +386,27 @@ def reconstruction(seed, mask, method="erosion"):
 _FLIPS = {"none": 0, None: 0, "horizontal": 1, "vertical": 2, "diagonal": 3}
 
 
+def _tta_transforms(T, rotate_degrees, flip_directions):
+    import ctypes
+    if not (T == len(rotate_degrees) == len(flip_directions)):
+        raise ValueError("one rotate_degree and one flip_direction per variant")
+    return (ctypes.c_int * T)(*[int(r) for r in rotate_degrees]), (ctypes.c_int * T)(*[_FLIPS[f] for f in flip_directions])
+
+
+def _tta_pack(vs, rots, H, W, window, overlap, what="variant"):
+    """One head's variants (already through ``net_inputs``) -> ([N, elements per tile] packed in the library's layout, C):
+    per tile, the T variants back to back."""
+    T, N = len(vs), int(vs[0].shape[0])
+    C = int(vs[0].shape[1] if window == 0 else vs[0].shape[2])
+    per_tile = int(_lib.load().tiseg_tta_input_elems(T, C, H, W, rots, int(window), int(overlap)))
+    if sum(int(np.prod(v.shape[1:])) for v in vs) != per_tile or any(int(v.shape[0]) != N for v in vs):
+        raise ValueError("%s shapes do not match the transforms / window geometry" % what)
+    if _lib_is_torch(vs[0]):
+        import torch
+        return torch.cat([v.reshape(N, -1) for v in vs], dim=1).contiguous(), C
+    return np.ascontiguousarray(np.concatenate([v.reshape(N, -1) for v in vs], axis=1)), C
+
+
 def softmax_argmax_tta(variants, rotate_degrees, flip_directions, ori_hw, window=0, overlap=0, want_prob=False):
     """Window stitch + TTA reverse + softmax + mean + argmax in one pass (base.py:255-295, 321-339, 365-381).
 
@@ -395,25 +416,12 @@ def softmax_argmax_tta(variants, rotate_degrees, flip_directions, ori_hw, window
     The variants may be fp32, or all fp16 / bf16: they are packed and read in their dtype, and the outputs are those of
     their fp32 upcast.  Returns the class map [N, H, W] uint8 (and the fp32 mean probabilities [N, C, H, W] with
     ``want_prob``)."""
-    import ctypes
-    from . import _lib
     T = len(variants)
-    if not (T == len(rotate_degrees) == len(flip_directions)):
-        raise ValueError("one rotate_degree and one flip_direction per variant")
+    rots, flips = _tta_transforms(T, rotate_degrees, flip_directions)
     H, W = int(ori_hw[0]), int(ori_hw[1])
     vs, dt = net_inputs(*variants)
     N = int(vs[0].shape[0])
-    C = int(vs[0].shape[1] if window == 0 else vs[0].shape[2])
-    rots = (ctypes.c_int * T)(*[int(r) for r in rotate_degrees])
-    flips = (ctypes.c_int * T)(*[_FLIPS[f] for f in flip_directions])
-    per_tile = int(_lib.load().tiseg_tta_input_elems(T, C, H, W, rots, int(window), int(overlap)))
-    if sum(int(np.prod(v.shape[1:])) for v in vs) != per_tile:
-        raise ValueError("variant shapes do not match the transforms / window geometry")
-    if _lib_is_torch(vs[0]):
-        import torch
-        packed = torch.cat([v.reshape(N, -1) for v in vs], dim=1).contiguous()
-    else:
-        packed = np.ascontiguousarray(np.concatenate([v.reshape(N, -1) for v in vs], axis=1))
+    packed, C = _tta_pack(vs, rots, H, W, window, overlap)
     cls = empty_like_kind(packed, (N, H, W), np.uint8)
     prob = empty_like_kind(packed, (N, C, H, W), np.float32) if want_prob else None
     get_ctx(_dev(packed)).call("tiseg_softmax_argmax_tta_typed", dt, ptr(packed), N, T, C, H, W, rots, flips, int(window),
@@ -425,26 +433,70 @@ def tta_mean(variants, rotate_degrees, flip_directions, ori_hw, window=0, overla
     """Window stitch + TTA reverse + PLAIN mean of a regression head (dist.py:398-410: ``sum(dist_logit_list) /
     len(dist_logit_list)``; hovernet.py:406 keeps ``hv_logit_list[0]``: pass that one variant).  Arguments as
     ``softmax_argmax_tta`` (fp32, or all fp16 / bf16).  -> [N, C, H, W] fp32."""
-    import ctypes
     T = len(variants)
-    if not (T == len(rotate_degrees) == len(flip_directions)):
-        raise ValueError("one rotate_degree and one flip_direction per variant")
+    rots, flips = _tta_transforms(T, rotate_degrees, flip_directions)
     H, W = int(ori_hw[0]), int(ori_hw[1])
     vs, dt = net_inputs(*variants)
     N = int(vs[0].shape[0])
-    C = int(vs[0].shape[1] if window == 0 else vs[0].shape[2])
-    rots = (ctypes.c_int * T)(*[int(r) for r in rotate_degrees])
-    flips = (ctypes.c_int * T)(*[_FLIPS[f] for f in flip_directions])
-    per_tile = int(_lib.load().tiseg_tta_input_elems(T, C, H, W, rots, int(window), int(overlap)))
-    if sum(int(np.prod(v.shape[1:])) for v in vs) != per_tile:
-        raise ValueError("variant shapes do not match the transforms / window geometry")
-    if _lib_is_torch(vs[0]):
-        import torch
-        packed = torch.cat([v.reshape(N, -1) for v in vs], dim=1).contiguous()
-    else:
-        packed = np.ascontiguousarray(np.concatenate([v.reshape(N, -1) for v in vs], axis=1))
+    packed, C = _tta_pack(vs, rots, H, W, window, overlap)
     out = empty_like_kind(packed, (N, C, H, W), np.float32)
     get_ctx(_dev(packed)).call("tiseg_tta_mean_typed", dt, ptr(packed), N, T, C, H, W, rots, flips, int(window), int(overlap), ptr(out))
+    return out
+
+
+def _tta_heads(heads, rotate_degrees, flip_directions, ori_hw, window, overlap, names):
+    """Variant lists of several heads -> (transforms, (H, W), N, dtype code, [(packed head, channels)]).  All heads of the
+    call share one dtype (fp32, or all fp16 / all bf16), like the variants of one head."""
+    T = len(heads[0])
+    if any(len(h) != T for h in heads):
+        raise ValueError("every head needs one output per TTA variant")
+    rots, flips = _tta_transforms(T, rotate_degrees, flip_directions)
+    H, W = int(ori_hw[0]), int(ori_hw[1])
+    flat, dt = net_inputs(*[v for h in heads for v in h])
+    packed = [_tta_pack(flat[k * T:(k + 1) * T], rots, H, W, window, overlap, name) for k, name in enumerate(names)]
+    return rots, flips, H, W, int(flat[0].shape[0]), dt, packed
+
+
+def cdnet_refine_tta(sem_variants, dir_variants, point_variants, rotate_degrees, flip_directions, ori_hw, window=0, overlap=0,
+                     if_ddm=True):
+    """``cdnet_refine`` fed the raw outputs of the TTA variants (cdnet.py:183-217 with base.py:255-295, 365-381 fused into
+    the loads): per head one array per variant, in the reference's loop order, each the head's output on the TRANSFORMED
+    image, [N, C, Ht, Wt] (``window = 0``) or its windows [N, M, C, window, window]; sem C classes, dir 9, point 1.
+    ``ori_hw`` = (H, W) of the image.  fp32, or all fp16 / bf16.  -> dict(sem_prob, cls, dir_map, dd), equal to
+    ``cdnet_refine`` on the stitched, reverse-transformed heads."""
+    rots, flips, H, W, N, dt, ((s, C), (d, D), (p, _)) = _tta_heads(
+        [sem_variants, dir_variants, point_variants], rotate_degrees, flip_directions, ori_hw, window, overlap,
+        ("sem_variants", "dir_variants", "point_variants"))
+    prob = empty_like_kind(s, (N, C, H, W), np.float32)
+    cls = empty_like_kind(s, (N, H, W), np.uint8)
+    dm = empty_like_kind(s, (N, H, W), np.uint8)
+    dd = empty_like_kind(s, (N, H, W), np.float32)
+    get_ctx(_dev(s)).call("tiseg_cdnet_refine_tta_typed", dt, ptr(s), ptr(d), ptr(p), N, len(sem_variants), C, D, H, W, rots, flips,
+                          int(window), int(overlap), 1 if if_ddm else 0, ptr(prob), ptr(cls), ptr(dm), ptr(dd))
+    return dict(sem_prob=prob, cls=cls, dir_map=dm, dd=dd)
+
+
+def mtcdnet_refine_tta(tc_variants, sem_variants, dir_variants, point_variants, rotate_degrees, flip_directions, ori_hw, window=0,
+                       overlap=0, if_ddm=True, want_sem_prob=False):
+    """``mtcdnet_refine`` fed the raw outputs of the TTA variants (multi_task_cdnet.py:262-330 with base.py:255-295,
+    365-381 fused into the loads); variant lists as ``cdnet_refine_tta`` (dir: 9 channels, or 1 for the angle head of
+    use_regression = True).  -> dict(tc_prob, tc_cls, sem_cls, dir_map, dd[, sem_prob]), equal to ``mtcdnet_refine`` on
+    the stitched, reverse-transformed heads."""
+    rots, flips, H, W, N, dt, ((t, Ctc), (s, Csem), (d, D), (p, _)) = _tta_heads(
+        [tc_variants, sem_variants, dir_variants, point_variants], rotate_degrees, flip_directions, ori_hw, window, overlap,
+        ("tc_variants", "sem_variants", "dir_variants", "point_variants"))
+    tcp = empty_like_kind(t, (N, Ctc, H, W), np.float32)
+    tcc = empty_like_kind(t, (N, H, W), np.uint8)
+    semc = empty_like_kind(t, (N, H, W), np.uint8)
+    semp = empty_like_kind(t, (N, Csem, H, W), np.float32) if want_sem_prob else None
+    dm = empty_like_kind(t, (N, H, W), np.uint8)
+    dd = empty_like_kind(t, (N, H, W), np.float32)
+    get_ctx(_dev(t)).call("tiseg_mtcdnet_refine_tta_typed", dt, ptr(t), ptr(s), ptr(d), ptr(p), N, len(tc_variants), Ctc, Csem, D, H, W,
+                          rots, flips, int(window), int(overlap), 1 if if_ddm else 0, ptr(tcp), ptr(tcc), ptr(semp), ptr(semc), ptr(dm),
+                          ptr(dd))
+    out = dict(tc_prob=tcp, tc_cls=tcc, sem_cls=semc, dir_map=dm, dd=dd)
+    if want_sem_prob:
+        out["sem_prob"] = semp
     return out
 
 

@@ -119,9 +119,17 @@ class CDNet(CUNet):
         super().__init__(num_classes, test_cfg)
         self.num_angles = num_angles
 
-    def inference_tail(self, sem_logit, dir_logit, point_logit):
-        """raw head outputs of the T TTA variants -> (refined sem probabilities, dir_map of variant 0)."""
-        r = ops.cdnet_refine(sem_logit, dir_logit, point_logit, if_ddm=self.test_cfg.get('if_ddm', False))
+    def inference_tail(self, sem_logit, dir_logit, point_logit, ori_hw=None, window=0, overlap=0):
+        """head outputs of the T TTA variants -> (refined sem probabilities, dir_map of variant 0, class map).  Without
+        ``ori_hw``: the heads already reverse-transformed, ``[T, C, H, W]`` or ``[N, T, C, H, W]``.  With ``ori_hw`` = (H, W):
+        per head the list of raw variant outputs on the TRANSFORMED image ([N, C, Ht, Wt], or its windows
+        [N, M, C, w, w] for split inference), the transforms from test_cfg, as ``Dist.inference_tail``."""
+        if_ddm = self.test_cfg.get('if_ddm', False)
+        if ori_hw is None:
+            r = ops.cdnet_refine(sem_logit, dir_logit, point_logit, if_ddm=if_ddm)
+        else:
+            rots, flips = _tta_lists(self.test_cfg)
+            r = ops.cdnet_refine_tta(sem_logit, dir_logit, point_logit, rots, flips, ori_hw, window, overlap, if_ddm=if_ddm)
         return r['sem_prob'], r['dir_map'], r['cls']
 
     _enh_mode = 0
@@ -240,13 +248,21 @@ class MultiTaskCDNet(MultiTaskCUNet):
         # use_regression (multi_task_cdnet.py:304-315): dir_logit is then the ONE-channel angle head, in radians
         self.num_angles, self.if_ddm, self.use_regression = num_angles, if_ddm, use_regression
 
-    def inference_tail(self, tc_logit, sem_logit, dir_logit, point_logit):
-        """raw head outputs of the T TTA variants (already reverse-transformed; [T, C, H, W] or [N, T, C, H, W]) ->
-        (refined tc probabilities, sem class map, dir_map of variant 0, tc class map)."""
-        if np.shape(dir_logit)[-3] != (1 if self.use_regression else self.num_angles + 1):
+    def inference_tail(self, tc_logit, sem_logit, dir_logit, point_logit, ori_hw=None, window=0, overlap=0):
+        """head outputs of the T TTA variants -> (refined tc probabilities, sem class map, dir_map of variant 0, tc class
+        map).  Without ``ori_hw``: already reverse-transformed, [T, C, H, W] or [N, T, C, H, W].  With ``ori_hw``: per head
+        the list of raw variant outputs, as ``CDNet.inference_tail``."""
+        # (the channel axis is -3 of a reverse-transformed stack, of a whole variant and of a window stack alike)
+        dch = np.shape(dir_logit if ori_hw is None else dir_logit[0])[-3]
+        if dch != (1 if self.use_regression else self.num_angles + 1):
             raise ValueError("dir_logit has %d channels; use_regression=%s expects %d" % (
-                np.shape(dir_logit)[-3], self.use_regression, 1 if self.use_regression else self.num_angles + 1))
-        r = ops.mtcdnet_refine(tc_logit, sem_logit, dir_logit, point_logit, if_ddm=self.if_ddm)
+                dch, self.use_regression, 1 if self.use_regression else self.num_angles + 1))
+        if ori_hw is None:
+            r = ops.mtcdnet_refine(tc_logit, sem_logit, dir_logit, point_logit, if_ddm=self.if_ddm)
+        else:
+            rots, flips = _tta_lists(self.test_cfg)
+            r = ops.mtcdnet_refine_tta(tc_logit, sem_logit, dir_logit, point_logit, rots, flips, ori_hw, window, overlap,
+                                       if_ddm=self.if_ddm)
         return r['tc_prob'], r['sem_cls'], r['dir_map'], r['tc_cls']
 
     _ddm_enhencement = classmethod(CDNet._ddm_enhencement.__func__)
